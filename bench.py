@@ -11,6 +11,13 @@ A "step" = one generated token for every stream.  `value` = generated tokens/s o
   python bench.py --impl reference [--steps K] [--warmup W]      the reference's algorithm on the host CPU cores
                                                                   (the oracle restatement: the reference itself needs
                                                                   fastai==1.0.61/music21, not installable offline)
+
+`--dump-outputs DIR` (CUDA path) also writes, after the timed steps, what the last timed step of each leg returned to its
+caller, as DIR/<name>.npy: `tokens` (C1: the generated stream; C2 / C5: every stream's token of the last step), `train_losses`
+(C3: loss, ce, ar, tar, grad_norm after the last step), `bert_logits` (C4: the last-position logits of the last forward).  Inputs
+are seeded, so two builds run with the same arguments can be compared output for output.  `tokens` and `bert_logits` repeat bit
+for bit from run to run; `train_losses` do not, because the training kernels accumulate some gradients with atomic adds in no
+fixed order (two runs on a B200 at its 1000 W power limit differed by up to 4e-5 relative in the losses and 9e-4 in grad_norm).
 """
 import argparse
 import ctypes as C
@@ -44,6 +51,19 @@ def measured_peaks():
         return float(p['hbm_gbs']), 'measured (MEASURED_PEAKS.json)'
     except Exception:
         return 6650.0, 'fallback (B200_PROFILING.md)'
+
+
+def dump_outputs(path, outputs):
+    """Writes `outputs` (name -> array) as path/<name>.npy, float64 arrays as float64 and everything else as float32.  The files stay
+    under 64 MB in all: an array above 16 MB (there are at most three) keeps a fixed, seeded sample of its rows."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > 16 << 20:
+            keep = (16 << 20) // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def attention_bytes_per_launch(B, H=8, Dh=64, M=512, e=2):
@@ -167,7 +187,7 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------------------------- C1: the reference's own CPU-runnable case
-def c1_line(args, cpu_only=False):
+def c1_line(args, cpu_only=False, outputs=None):
     """BASELINE.json configs[0]: random-init Transformer-XL (C2's model), seed = the whole encoded fur_elise.mid, 512 greedy tokens,
     fp32.  CPU: the oracle's reference loop (deep_music_genre.py:1853-1972), wall time split into prefill and decode.  GPU: the same
     call through MusicLearner.predict in fp32 mode; the two token streams must be identical."""
@@ -222,6 +242,8 @@ def c1_line(args, cpu_only=False):
     pred, _ = learn.predict(item, n_words=n_words, temperatures=(1., 1., 1.), min_bars=10 ** 6, top_k=1, top_p=0.0)
     torch.cuda.synchronize()
     t_gpu = time.time() - t0
+    if outputs is not None:
+        outputs['tokens'] = np.asarray(pred.data)
     same = list(pred.data) == list(ref)
     return dict(base, value=len(pred.data) / t_gpu, ms_per_step=1e3 * t_gpu / max(len(pred.data), 1),
                 config=dict(base['config'], token_stream_identical_to_oracle=same, gpu_wall_s=t_gpu,
@@ -235,24 +257,27 @@ def c1_line(args, cpu_only=False):
 # --------------------------------------------------------------------------------------------- CUDA arm
 def run_b200(args):
     "C2 headline + (default run) the C3 training step and the C4 encoder forward as sub-records of the one JSON line."
-    line = measure_c2(args)
+    outputs = {} if args.dump_outputs else None
+    line = measure_c2(args, outputs)
     if args.workload == 'c2' and not args.no_extra_legs:
         import argparse
         import bench_bert
         import bench_train
         sub = argparse.Namespace(**vars(args))
         sub.steps, sub.warmup = args.train_steps, 4
-        train = bench_train.measure(sub, sample_clocks=False)
+        train = bench_train.measure(sub, sample_clocks=False, outputs=outputs)
         sub.steps, sub.warmup = args.bert_steps, 3
-        bert = bench_bert.measure(sub, sample_clocks=False)
+        bert = bench_bert.measure(sub, sample_clocks=False, outputs=outputs)
         if line is not None:
             line['train'], line['bert'] = train, bert
             line['gpu_launches_all_legs'] = line['gpu_launches'] + train['gpu_launches'] + bert['gpu_launches']
     if line is not None:
         print(json.dumps(line), flush=True)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
 
 
-def measure_c2(args):
+def measure_c2(args, outputs=None):
     from deepmusicgeneration_b200 import _lib, sharding
     from deepmusicgeneration_b200.app_utils import baseline_config
     from deepmusicgeneration_b200.codec import MusicDataBunch
@@ -322,6 +347,8 @@ def measure_c2(args):
     ms_max = sharding.max_over_ranks(ms, device=dev)
     value = B * world * K / (ms_max / 1e3)
     good = int((toks[:K] >= 0).all().item())
+    if outputs is not None:
+        outputs['tokens'] = toks[K - 1].cpu().numpy()
 
     # ---- end to end through the C ABI with HOST buffers: H2D of the step's input ids, D2H of the sampled tokens
     Ke = min(K, 512)
@@ -441,12 +468,19 @@ def main():
     ap.add_argument('--bert-batch', type=int, default=512, help='c4: sequences per GPU and forward')
     ap.add_argument('--bert-chunk', type=int, default=32, help='c4: sequences per activation chunk of the encoder forward (max_rows / 1024)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the CUDA path (--impl b200)')
     if args.workload == 'c1':
         if args.impl == 'reference':
             return run_reference(args)
         if int(os.environ.get('RANK', '0')) == 0:
-            print(json.dumps(c1_line(args)), flush=True)
+            outputs = {} if args.dump_outputs else None
+            print(json.dumps(c1_line(args, outputs=outputs)), flush=True)
+            if outputs is not None:
+                dump_outputs(args.dump_outputs, outputs)
         return
     if args.workload == 'c3':
         import bench_train

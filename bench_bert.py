@@ -36,12 +36,16 @@ def synthetic(B, gen):
 
 
 def run_b200(args):
-    line = measure(args)
+    outputs = {} if args.dump_outputs else None
+    line = measure(args, outputs=outputs)
     if line is not None:
         print(json.dumps(line), flush=True)
+        if outputs is not None:
+            from bench import dump_outputs
+            dump_outputs(args.dump_outputs, outputs)
 
 
-def measure(args, sample_clocks=True, cpu_leg=True):
+def measure(args, sample_clocks=True, cpu_leg=True, outputs=None):
     "Runs the C4 leg on every rank; returns the JSON record on rank 0 (None elsewhere)."
     from bench import ClockSampler
     from deepmusicgeneration_b200 import _lib, sharding
@@ -103,6 +107,8 @@ def measure(args, sample_clocks=True, cpu_leg=True):
     torch.cuda.synchronize()
     e2e_ms = sharding.max_over_ranks(ev0.elapsed_time(ev1), device=dev)
     e2e_value = B * T * world * Ke / (e2e_ms / 1e3)
+    if outputs is not None:
+        outputs['bert_logits'] = out_host.numpy().copy()
 
     del e, pm
     torch.cuda.empty_cache()

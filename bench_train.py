@@ -47,12 +47,16 @@ def lakh_shaped_tokens(bs, n, gen):
 
 
 def run_b200(args):
-    line = measure(args)
+    outputs = {} if args.dump_outputs else None
+    line = measure(args, outputs=outputs)
     if line is not None:
         print(json.dumps(line), flush=True)
+        if outputs is not None:
+            from bench import dump_outputs
+            dump_outputs(args.dump_outputs, outputs)
 
 
-def measure(args, sample_clocks=True, cpu_leg=True):
+def measure(args, sample_clocks=True, cpu_leg=True, outputs=None):
     "Runs the C3 leg on every rank; returns the JSON record on rank 0 (None elsewhere)."
     from bench import ClockSampler
     from deepmusicgeneration_b200 import _lib, sharding
@@ -113,6 +117,8 @@ def measure(args, sample_clocks=True, cpu_leg=True):
     ms_max = sharding.max_over_ranks(ms, device=dev)
     value = B * T * world * K / (ms_max / 1e3)
     l1 = tr.losses()
+    if outputs is not None:
+        outputs['train_losses'] = np.array([l1[k] for k in ('loss', 'ce', 'ar', 'tar', 'grad_norm')])
     grad_exchange = tr.describe_exchange()
 
     # ---- end to end: every step copies its tokens/targets from pinned host memory and reads the loss back

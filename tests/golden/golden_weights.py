@@ -5,11 +5,18 @@ numpy's compatibility policy, NEP 19), one stream per tensor keyed by (seed, crc
 reference's tensors (the oracle builds encoder + head only) gets the same values; distributions are the ones fastai's
 ``init_transformer`` leaves behind (SURVEY.md App. A.6).
 ``weights_checksum`` of the result is stored in the fixture so a drifted stream would be noticed.
+
+To keep the fixture file under 1 MB, the large outputs keep two positions (axis 1) in five: always the first and the last, the rest
+a fixed, seeded draw.  ``sample_positions`` does that when the fixture is written; ``kept_positions`` picks the same positions out of
+a full output in the tests.
 """
+import re
 import zlib
 
 import numpy as np
 import torch
+
+SAMPLED = re.compile(r'((txl_logits|txl_core|txl_mem_last|bert_logits)\d+|txl_win_logits)$')
 
 
 def golden_state_dict(reference_state, seed):
@@ -43,3 +50,20 @@ def weights_checksum(state):
     "Sum of |w| over the tensors of the hot path (the remix decoder, mha2 and ff blocks are not on it and not in every model)."
     skip = lambda k: k.endswith('pos_enc.freq') or k.startswith('decoder.') or '.mha2.' in k or (k.startswith('encoder.') and '.ff.' in k)
     return float(sum(float(v.double().abs().sum()) for k, v in sorted(state.items()) if not skip(k)))
+
+
+def sample_positions(out, seed=0):
+    "In place: every output named by SAMPLED keeps 2 of 5 positions; `<key>_rows` records which, `<key>_shape` the full shape."
+    rng = np.random.default_rng(seed)
+    for key in sorted(k for k in out if SAMPLED.match(k)):
+        a = out[key]
+        T = a.shape[1]
+        k = -(-2 * T // 5)
+        rows = np.arange(T) if k >= T - 1 else np.sort(np.r_[0, T - 1, 1 + rng.choice(T - 2, k - 2, replace=False)])
+        out[key], out[key + '_rows'], out[key + '_shape'] = a[:, rows], rows, np.array(a.shape)
+
+
+def kept_positions(G, key, full):
+    "The positions of `full` (an output computed in full) that fixture `G` kept for `key`, after checking the full shape."
+    assert tuple(full.shape) == tuple(G[key + '_shape']), (key, full.shape, G[key + '_shape'])
+    return full[:, G[key + '_rows']]

@@ -38,7 +38,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
-from golden_weights import golden_state_dict, weights_checksum      # noqa: E402
+from golden_weights import golden_state_dict, sample_positions, weights_checksum      # noqa: E402
 from oracle import txl                                               # noqa: E402
 
 REF = '/root/reference'
@@ -274,5 +274,6 @@ mitem.position = item.position.copy()               # the app masks after encodi
 res = ref_predict_mask(LearnerStub(bmodel), mitem, temperatures=(1.1, 0.9), top_k=1, top_p=0.0)
 out['predict_mask_in'], out['predict_mask_pos'], out['predict_mask_out'] = masked, mitem.position, res.data
 
+sample_positions(out)
 np.savez_compressed(os.path.join(HERE, 'model_golden.npz'), **out)
 print('wrote', len(out), 'arrays,', os.path.getsize(os.path.join(HERE, 'model_golden.npz')) // 1024, 'KiB')

@@ -16,7 +16,7 @@ import torch
 from oracle import bert as obert, txl
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
-from golden_weights import golden_state_dict      # noqa: E402
+from golden_weights import golden_state_dict, kept_positions      # noqa: E402
 
 pytestmark = pytest.mark.gpu
 V = 324
@@ -61,8 +61,9 @@ def test_txl_forward_override_against_reference_source(G, dtype):
     for s, T in enumerate(G['txl_segments']):
         x, pos = torch.from_numpy(G[f'txl_x{s}']).cuda(), torch.from_numpy(G[f'txl_pos{s}']).cuda()
         logits, raw, outs = pm({'x': x, 'pos': pos})
-        logits, core, mem = logits.cpu().numpy(), outs[0].cpu().numpy(), raw[-1].cpu().numpy()
-        assert mem.shape == G[f'txl_mem_last{s}'].shape, s
+        logits = kept_positions(G, f'txl_logits{s}', logits.cpu().numpy())
+        core = kept_positions(G, f'txl_core{s}', outs[0].cpu().numpy())
+        mem = kept_positions(G, f'txl_mem_last{s}', raw[-1].cpu().numpy())
         if dtype == 'f32':
             assert np.abs(logits - G[f'txl_logits{s}']).max() < 5e-4, s
             assert np.abs(core - G[f'txl_core{s}']).max() < 5e-4, s
@@ -71,6 +72,7 @@ def test_txl_forward_override_against_reference_source(G, dtype):
             worst = max(worst, _bf16_ok(logits, G[f'txl_logits{s}']))
     x, pos = torch.from_numpy(G['txl_win_x']).cuda(), torch.from_numpy(G['txl_win_pos']).cuda()
     lw = pm({'x': x, 'pos': pos}, mask_size=(3, 0))[0].cpu().numpy()           # the training-time window mask over the memory
+    lw = kept_positions(G, 'txl_win_logits', lw)
     if dtype == 'f32':
         assert np.abs(lw - G['txl_win_logits']).max() < 5e-4
     else:
@@ -106,7 +108,7 @@ def test_bert_encoder_against_reference_source(G, dtype):
     worst = 0.
     for T in G['bert_lengths']:
         x, pos = torch.from_numpy(G[f'bert_x{T}']).cuda(), torch.from_numpy(G[f'bert_pos{T}']).cuda()
-        out = pm({'msk': {'x': x, 'pos': pos}})['msk'].cpu().numpy()
+        out = kept_positions(G, f'bert_logits{T}', pm({'msk': {'x': x, 'pos': pos}})['msk'].cpu().numpy())
         if dtype == 'f32':
             assert np.abs(out - G[f'bert_logits{T}']).max() < 5e-4, T
         else:
