@@ -40,7 +40,8 @@ class SamplerParams(C.Structure):
 
 class TrainConfig(C.Structure):
     _fields_ = [('batch', c_i32), ('bptt', c_i32), ('resid_p', c_f32), ('attn_p', c_f32), ('ff_p', c_f32), ('embed_p', c_f32),
-                ('output_p', c_f32), ('alpha', c_f32), ('beta', c_f32), ('seed', c_u64), ('reserved', c_i32 * 4)]
+                ('output_p', c_f32), ('alpha', c_f32), ('beta', c_f32), ('seed', c_u64), ('pad_idx', c_i32),
+                ('reserved', c_i32 * 3)]
 
 
 # name -> (restype, argtypes): every symbol include/dmg_b200.h declares

@@ -13,9 +13,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 OBJDIR = os.path.join(HERE, 'build')
 LIB = os.path.join(HERE, 'libdmg_b200.so')
-SOURCES = ['gemm.cu', 'gemm_train.cu', 'elementwise.cu', 'attention.cu', 'attention_decode2.cu', 'decode_layer.cu', 'attention_flash.cu', 'attention_train.cu', 'attention_train_tc.cu', 'attention_bert_tc.cu',
+SOURCES = ['gemm.cu', 'gemm_train.cu', 'elementwise.cu', 'attention.cu', 'attention_decode2.cu', 'decode_layer.cu', 'attention_flash.cu', 'attention_train.cu', 'attention_train_tc.cu', 'attention_bert_tc.cu', 'attention_bert_train.cu',
            'sampling.cu', 'train_kernels.cu', 'preload.cu', 'model.cu', 'train.cu']
-HEADERS = ['common.cuh', 'kernels.cuh', 'attention_decode2.cuh', 'attention_decode3.cuh', 'sampling.cuh', 'launch.cuh', 'attention_bert_tc_common.cuh', 'model.cuh', 'train_kernels.cuh', 'mma_sync.cuh',
+HEADERS = ['common.cuh', 'kernels.cuh', 'attention_decode2.cuh', 'attention_decode3.cuh', 'sampling.cuh', 'launch.cuh', 'attention_bert_tc_common.cuh', 'model.cuh', 'train_kernels.cuh', 'mma_sync.cuh', 'attention_train_common.cuh',
            os.path.join('..', '..', 'include', 'dmg_b200.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC']

@@ -17,28 +17,17 @@
 //   attn_bwd_dq_kernel: query-tile owner; recomputes P, forms dS, accumulates dQ (content + position parts -> du, dv),
 //                       writes dS in (row, distance) coordinates for the dRk GEMM (ds_dist)
 //   attn_bwd_dkv_kernel: key-tile owner; recomputes P and dS, accumulates dK, dV
-#include <cuda_fp16.h>
 #include "kernels.cuh"
 #include "launch.cuh"
-#include "mma_sync.cuh"
-#include "train_kernels.cuh"
+#include "attention_train_common.cuh"
 
 namespace dmg {
 
 namespace {
 
-constexpr int SKEW_LD = 84;    // elements per row of the warp-private skew strip (80 used)
-typedef __half skew_t;         // fp16 strip (11-bit mantissa: rounding 5e-4 of the position term) - 2.7 KB per warp
 constexpr int DSK_LD = 88;     // bf16 per row of the warp-private dS strip (80 used); 176-byte rows keep ldmatrix aligned
-constexpr float LOG2E = 1.4426950408889634f;
-constexpr float LN2 = 0.6931471805599453f;
-
-// two floats -> packed fp16 pair, saturating to +-65504 instead of overflowing to infinity (lo = first argument)
-__device__ __forceinline__ uint32_t pack_half2_sat(float lo, float hi) {
-  uint32_t r;
-  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-  return r;
-}
+constexpr float LOG2E = ATT_LOG2E;
+constexpr float LN2 = ATT_LN2;
 
 struct MaskP {
   int M, mem_count, win, k;
@@ -51,76 +40,6 @@ __device__ __forceinline__ bool visible(const MaskP& mp, int i, int j) {
   return mp.k == 1 ? jx <= i : jx < (i / mp.win) * mp.win;   // (1,1) causal; (w,0): strictly earlier windows
 }
 
-// (q + bias) A-fragments: a[ks] covers k = 16*ks..16*ks+15; registers hold (g,2t..),(g+8,2t..),(g,2t+8..),(g+8,2t+8..)
-__device__ __forceinline__ uint32_t add_bias2(uint32_t w, float b0, float b1) { return pack_bf16x2(bf16lo(w) + b0, bf16hi(w) + b1); }
-__device__ __forceinline__ void q_frags(uint32_t sQ, int w, int lane, const LaneOff& L, const float* __restrict__ u, const float* __restrict__ v,
-                                        uint32_t (&qu)[4][4], uint32_t (&qv)[4][4]) {
-  const int t = lane & 3;
-#pragma unroll
-  for (int ks = 0; ks < 4; ks++) {
-    uint32_t a[4];
-    frag_a(sQ, 16 * w, ks, L, a);
-    const int c0 = 16 * ks + 2 * t;
-    const float u0 = u[c0], u1 = u[c0 + 1], u8 = u[c0 + 8], u9 = u[c0 + 9];
-    const float v0 = v[c0], v1 = v[c0 + 1], v8 = v[c0 + 8], v9 = v[c0 + 9];
-    qu[ks][0] = add_bias2(a[0], u0, u1); qu[ks][1] = add_bias2(a[1], u0, u1);
-    qu[ks][2] = add_bias2(a[2], u8, u9); qu[ks][3] = add_bias2(a[3], u8, u9);
-    qv[ks][0] = add_bias2(a[0], v0, v1); qv[ks][1] = add_bias2(a[1], v0, v1);
-    qv[ks][2] = add_bias2(a[2], v8, v9); qv[ks][3] = add_bias2(a[3], v8, v9);
-  }
-}
-
-// s[nt][e] = AC + BD (unscaled) for the warp's 16 query rows x the tile's 64 keys.
-// sR0 / sR1: the two Rk tiles of the window (distances D0-64..D0-1 and D0..D0+63).
-__device__ __forceinline__ void scores_tile(const uint32_t (&qu)[4][4], const uint32_t (&qv)[4][4], uint32_t sK, uint32_t sR0,
-                                            uint32_t sR1, skew_t* skew, int w, int lane, const LaneOff& L, float (&s)[8][4]) {
-  const int g = lane >> 2, t = lane & 3;
-  // position term: 16 rows x 80 distances (window columns 16w .. 16w+79)
-#pragma unroll
-  for (int p = 0; p < 5; p++) {
-    const int wc = 16 * w + 16 * p;                 // first window column of this pair of n-tiles
-    const uint32_t sR = (wc < 64 ? sR0 : sR1) + (wc & 63) * 128;
-    float acc[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
-#pragma unroll
-    for (int ks = 0; ks < 4; ks++) {
-      uint32_t r[4];
-      frag_b(sR, 0, ks, L, r);
-      mma_bf16(acc[0], qv[ks], r[0], r[1]);
-      mma_bf16(acc[1], qv[ks], r[2], r[3]);
-    }
-#pragma unroll
-    for (int h = 0; h < 2; h++) {
-      const int col = 16 * p + 8 * h + 2 * t;
-      *(uint32_t*)(skew + g * SKEW_LD + col) = pack_half2_sat(acc[h][0], acc[h][1]);
-      *(uint32_t*)(skew + (g + 8) * SKEW_LD + col) = pack_half2_sat(acc[h][2], acc[h][3]);
-    }
-  }
-  __syncwarp();
-  // content term
-#pragma unroll
-  for (int nt = 0; nt < 8; nt++) { s[nt][0] = 0.f; s[nt][1] = 0.f; s[nt][2] = 0.f; s[nt][3] = 0.f; }
-#pragma unroll
-  for (int ks = 0; ks < 4; ks++) {
-#pragma unroll
-    for (int np = 0; np < 4; np++) {
-      uint32_t r[4];
-      frag_b(sK, 16 * np, ks, L, r);
-      mma_bf16(s[2 * np], qu[ks], r[0], r[1]);
-      mma_bf16(s[2 * np + 1], qu[ks], r[2], r[3]);
-    }
-  }
-  // skewed read: BD[row, jl] = strip[row][64 + row - jl]
-#pragma unroll
-  for (int nt = 0; nt < 8; nt++) {
-    const int jl = 8 * nt + 2 * t;
-    s[nt][0] += __half2float(skew[g * SKEW_LD + 64 + g - jl]);
-    s[nt][1] += __half2float(skew[g * SKEW_LD + 63 + g - jl]);
-    s[nt][2] += __half2float(skew[(g + 8) * SKEW_LD + 72 + g - jl]);
-    s[nt][3] += __half2float(skew[(g + 8) * SKEW_LD + 71 + g - jl]);
-  }
-  __syncwarp();
-}
-
 // pointer to the 64-key tile jt of K (kv=0) or V (kv=1) for stream b, head h
 __device__ __forceinline__ const bf16* kv_tile_ptr(const AttnTrainArgs& a, int b, int h, int jt, int kv, long long* ld) {
   const int HD = a.H * 64;
@@ -131,15 +50,6 @@ __device__ __forceinline__ const bf16* kv_tile_ptr(const AttnTrainArgs& a, int b
   }
   *ld = a.ldx;
   return a.qkv_x + ((long long)b * a.T + (j0 - a.M)) * a.ldx + (1 + kv) * HD + h * 64;
-}
-
-__device__ __forceinline__ float quad_max(float v) {
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1));
-  return fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
-}
-__device__ __forceinline__ float quad_sum(float v) {
-  v += __shfl_xor_sync(0xffffffffu, v, 1);
-  return v + __shfl_xor_sync(0xffffffffu, v, 2);
 }
 
 // =============================================================================================
@@ -326,14 +236,7 @@ __device__ __forceinline__ void bwd_tile_math(const AttnTrainArgs& a, const Mask
 #pragma unroll
   for (int nt = 0; nt < 8; nt++) {
     float keep[4] = {1.f, 1.f, 1.f, 1.f};
-    if (a.drop_thresh) {
-#pragma unroll
-      for (int r = 0; r < 2; r++) {
-        const uint32_t hb = drop_pair_bits(a.drop_seed, drop_base[r] + (uint32_t)(j0 >> 1) + 4 * nt);
-        keep[2 * r] = ((hb & 0xFFFFu) >= a.drop_thresh) ? a.drop_scale : 0.f;
-        keep[2 * r + 1] = ((hb >> 16) >= a.drop_thresh) ? a.drop_scale : 0.f;
-      }
-    }
+    if (a.drop_thresh) attn_keep(a.drop_thresh, a.drop_seed, a.drop_scale, drop_base, j0, nt, keep);
 #pragma unroll
     for (int e = 0; e < 4; e++) {
       const int r = e >> 1;
@@ -363,14 +266,7 @@ __device__ __forceinline__ void bwd_tile_math_saved(const AttnTrainArgs& a, cons
 #pragma unroll
   for (int nt = 0; nt < 8; nt++) {
     float keep[4] = {1.f, 1.f, 1.f, 1.f};
-    if (a.drop_thresh) {
-#pragma unroll
-      for (int r = 0; r < 2; r++) {
-        const uint32_t hb = drop_pair_bits(a.drop_seed, drop_base[r] + (uint32_t)(j0 >> 1) + 4 * nt);
-        keep[2 * r] = ((hb & 0xFFFFu) >= a.drop_thresh) ? a.drop_scale : 0.f;
-        keep[2 * r + 1] = ((hb >> 16) >= a.drop_thresh) ? a.drop_scale : 0.f;
-      }
-    }
+    if (a.drop_thresh) attn_keep(a.drop_thresh, a.drop_seed, a.drop_scale, drop_base, j0, nt, keep);
 #pragma unroll
     for (int e = 0; e < 4; e++) {
       const int r = e >> 1;
@@ -821,8 +717,10 @@ __global__ void __launch_bounds__(128) attn_bwd_dkv_kernel(const AttnTrainBwdArg
 
 // dK / dV from the spilled P and dS tiles (no recomputation of the scores): key-tile owner, loops over the query tiles that
 // see it; per iteration four 64x64 tiles (P, dS, dO, Q) arrive through a double-buffered cp.async ring.
+// ALL_QUERIES: every query tile sees every key (the remix encoder's unmasked attention) instead of the causal range.
 constexpr int LITE_SMEM = 2 * 4 * TILE_BYTES;
 
+template <bool ALL_QUERIES>
 __global__ void __launch_bounds__(128) attn_bwd_dkv_lite_kernel(const AttnTrainBwdArgs ba) {
   const AttnTrainArgs& a = ba.f;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -854,7 +752,7 @@ __global__ void __launch_bounds__(128) attn_bwd_dkv_lite_kernel(const AttnTrainB
     return;
   }
   const int nT = a.T / 64;
-  const int it_lo = j0 < a.M ? 0 : (j0 - a.M) / 64;
+  const int it_lo = (ALL_QUERIES || j0 < a.M) ? 0 : (j0 - a.M) / 64;
   auto load_stage = [&](int it) {
     if (it < nT) {
       uint8_t* st = smem + ((it - it_lo) & 1) * 4 * TILE_BYTES;
@@ -934,6 +832,24 @@ int check_args(const AttnTrainArgs& a) {
 
 }  // namespace
 
+int attn_train_delta(const AttnTrainBwdArgs& ba, cudaStream_t st) {
+  const AttnTrainArgs& a = ba.f;
+  const int rows = a.B * a.T;
+  return launch_np(attn_delta_kernel, dim3((rows * 32 + 255) / 256), dim3(256), 0, st, (const bf16*)a.out, ba.dout, ba.delta, rows, a.T,
+                   a.H);
+}
+
+int attn_bwd_dkv_all_queries(const AttnTrainBwdArgs& ba, cudaStream_t st) {
+  const AttnTrainArgs& a = ba.f;
+  DMG_CHECK(a.M == 0 && ba.p_buf && ba.ds_buf, "attn_bwd_dkv_all_queries: needs M = 0 and the spilled P / dS tiles");
+  static bool configured = false;
+  if (!configured) {
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dkv_lite_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LITE_SMEM));
+    configured = true;
+  }
+  return launch_np(attn_bwd_dkv_lite_kernel<true>, dim3(a.B * a.H * (a.T / 64)), dim3(128), (size_t)LITE_SMEM, st, ba);
+}
+
 int attn_train_fwd(const AttnTrainArgs& a, cudaStream_t st) {
   if (check_args(a)) return -2;
   if (attn_train_fwd_tc_supported(a)) return attn_train_fwd_tc(a, st);
@@ -954,12 +870,10 @@ int attn_train_bwd(const AttnTrainBwdArgs& ba, int num_sms, cudaStream_t st) {
     DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dq_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DQ_SMEM));
     DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dq_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DQ_PS_SMEM));
     DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dkv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DKV_SMEM));
-    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dkv_lite_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LITE_SMEM));
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dkv_lite_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LITE_SMEM));
     configured = true;
   }
-  const int rows = a.B * a.T;
-  if (launch_np(attn_delta_kernel, dim3((rows * 32 + 255) / 256), dim3(256), 0, st, (const bf16*)a.out, ba.dout, ba.delta, rows, a.T, a.H))
-    return -1;
+  if (attn_train_delta(ba, st)) return -1;
   if (attn_bwd_dq_tc_supported(ba)) {   // saved probabilities, 128-aligned shapes: dQ on tcgen05
     if (attn_bwd_dq_tc(ba, st)) return -1;
   } else if (a.p_save && a.m_save) {   // the tcgen05 forward saved the probabilities: no score recomputation
@@ -969,7 +883,7 @@ int attn_train_bwd(const AttnTrainBwdArgs& ba, int num_sms, cudaStream_t st) {
   }
   if (attn_bwd_dkv_tc_supported(ba)) return attn_bwd_dkv_tc(ba, st);   // spilled tiles + (q+u): tcgen05 contraction
   if (ba.p_buf && ba.ds_buf)   // P and dS were spilled by the dQ kernel: no second recomputation of the scores
-    return launch_np(attn_bwd_dkv_lite_kernel, dim3(a.B * a.H * ((a.M + a.T) / 64)), dim3(128), (size_t)LITE_SMEM, st, ba);
+    return launch_np(attn_bwd_dkv_lite_kernel<false>, dim3(a.B * a.H * ((a.M + a.T) / 64)), dim3(128), (size_t)LITE_SMEM, st, ba);
   return launch_np(attn_bwd_dkv_kernel, dim3(a.B * a.H * ((a.M + a.T) / 64)), dim3(128), (size_t)DKV_SMEM, st, ba);
 }
 

@@ -1,8 +1,10 @@
-// Training step of the Transformer-XL path: forward with saved activations, loss, backward, Adam; C ABI (dmg_train_*).
-// What fastai's Learner does for one batch around the reference model (SURVEY.md 3.3, App. A.3, A.7):
-//   model(x) train-mode (deep_music_genre.py:1617-1647), CrossEntropyFlat + RNNTrainer AR/TAR, backward, Adam(true_wd).
-// Memory in training is the reference's own: hidden states of the previous segment per level (detached), re-projected
-// to K/V with the current weights every step (_update_mems, App. A.2).
+// Training step: forward with saved activations, loss, backward, Adam; C ABI (dmg_train_*).
+// What fastai's Learner does for one batch around the reference models (SURVEY.md 3.3, App. A.3, A.7):
+//   Transformer-XL: model(x) train-mode (deep_music_genre.py:1617-1647), CrossEntropyFlat + RNNTrainer AR/TAR, backward, Adam(true_wd).
+//   Memory in training is the reference's own: hidden states of the previous segment per level (detached), re-projected
+//   to K/V with the current weights every step (_update_mems, App. A.2).
+//   Remix encoder (msk task): head(encoder(x_masked, pos)) train-mode (deep_music_remix.py:1874-1881, 1910-2104),
+//   CrossEntropyFlat(ignore_index=pad_idx), backward, the same Adam(true_wd); no memory, no AR/TAR.
 #include <cstring>
 #include <string>
 #include <vector>
@@ -62,6 +64,8 @@ struct dmg_train {
   bf16 *proj = nullptr, *dadd = nullptr, *dh = nullptr, *dattn = nullptr, *dqkv_x = nullptr, *dkv_m = nullptr, *ds_dist = nullptr,
        *qv = nullptr, *drk16 = nullptr, *dlogits = nullptr, *xdrop = nullptr, *dbr = nullptr, *p_buf = nullptr, *ds_buf = nullptr;
   bool dbr_valid = false;                    // dbr holds a branch gradient still to be added to dx32
+  bool bert = false;                         // remix encoder (DMG_ARCH_BERT): the *_bert step functions
+  long long emb_pad = -1;                    // token row of the embedding that lookups do not train (BERT: pad_idx)
   const long long *ids = nullptr, *pos = nullptr;     // of the latest forward (caller-owned, must stay alive until backward ends)
   int win = 1, k = 1, training = 1;
   long long step = 0;
@@ -146,6 +150,47 @@ int build_params(dmg_model* m, dmg_train* t) {
     t->g_beat = add_param(t, reg_name(m, m->beat), m->beat, nullptr, 32ll * d);
     t->g_bar = add_param(t, reg_name(m, m->bar), m->bar, nullptr, 1024ll * d);
   }
+  return 0;
+}
+
+// remix encoder: same order, per layer q | k | v (one contiguous span: the model stores them as one [3*HD, d] matrix),
+// r_attn, their biases, the LayerNorm; tail u, v, embedding (tied head weight), beat, bar
+int build_params_bert(dmg_model* m, dmg_train* t) {
+  const dmg_config& c = m->cfg;
+  const int d = c.d_model, HD = m->HD, L = c.n_layers;
+  const long long w = (long long)HD * d;
+  t->params.clear();
+  t->total = 0;
+  t->g_head_b = add_param(t, "head.decoder.bias", m->head_b, nullptr, c.vocab);
+  t->lg.assign(L, LayerGrad());
+  t->layer_lo_off.assign(L, 0);
+  t->layer_hi_off.assign(L, 0);
+  for (int l = L - 1; l >= 0; l--) {
+    LayerW& W = m->layers[l];
+    LayerGrad& g = t->lg[l];
+    const std::string p = "encoder.layers." + std::to_string(l) + ".mha1.";
+    t->layer_lo_off[l] = t->total;
+    g.wo = g.w1 = g.w2 = g.bo = g.b1 = g.b2 = g.ln2w = g.ln2b = g.bqkv = g.br = -1;
+    g.wqkv = add_param(t, p + "q_wgt.weight", W.wqkv.f32, W.wqkv.b16, w);
+    add_param(t, p + "k_wgt.weight", W.wqkv.f32 + w, W.wqkv.b16 + w, w);
+    add_param(t, p + "v_wgt.weight", W.wqkv.f32 + 2 * w, W.wqkv.b16 + 2 * w, w);
+    g.wr = add_param(t, p + "r_attn.weight", W.wr.f32, W.wr.b16, w);
+    if (c.attn_bias) {
+      g.bqkv = add_param(t, p + "q_wgt.bias", W.bqkv, nullptr, HD);
+      add_param(t, p + "k_wgt.bias", W.bqkv + HD, nullptr, HD);
+      add_param(t, p + "v_wgt.bias", W.bqkv + 2 * HD, nullptr, HD);
+      g.br = add_param(t, p + "r_attn.bias", W.br, nullptr, HD);
+    }
+    g.ln1w = add_param(t, p + "ln.weight", W.ln1w, nullptr, d);
+    g.ln1b = add_param(t, p + "ln.bias", W.ln1b, nullptr, d);
+    t->layer_hi_off[l] = t->total;
+  }
+  t->tail_off = t->total;
+  t->g_u = add_param(t, "encoder.u", m->u, nullptr, HD);
+  t->g_v = add_param(t, "encoder.v", m->v, nullptr, HD);
+  t->g_emb = add_param(t, "encoder.embed.embed.weight", m->emb.f32, m->emb.b16, (long long)c.vocab * d);
+  t->g_beat = add_param(t, "encoder.embed.beat_enc.weight", m->beat, nullptr, 32ll * d);
+  t->g_bar = add_param(t, "encoder.embed.bar_enc.weight", m->bar, nullptr, 1024ll * d);
   return 0;
 }
 
@@ -310,6 +355,25 @@ int train_forward(dmg_model* m, dmg_train* t, const long long* ids, const long l
   return 0;
 }
 
+// dRk[h] = dS_dist[:, h]^T (q + v)[:, h]  ->  dWr = dRk^T PE, r_attn bias = column sums of dRk
+int grad_rel_pos(dmg_model* m, dmg_train* t, const bf16* qv_op, const LayerGrad& g, cudaStream_t st) {
+  const dmg_config& c = m->cfg;
+  const int d = c.d_model, HD = m->HD, rows = t->rows, S = t->S, ns = m->num_sms;
+  DMG_CUDA_OK(cudaMemsetAsync(t->drk32, 0, (size_t)S * HD * sizeof(float), st));
+  {   // one grouped launch: group h reads dS_dist columns [h*S, (h+1)*S) and (q+v) columns [h*64, (h+1)*64)
+    GemmEpi er; er.out = t->drk32; er.ldc = HD; er.out_mode = GEMM_OUT_ATOMIC;
+    er.groups = c.n_heads; er.a_gs = S; er.b_gs = 64; er.c_gs = 64;
+    int sk = (2 * ns) / (c.n_heads * ((S + 127) / 128));
+    if (sk < 1) sk = 1;
+    if (sk > rows / 512) sk = rows / 512 > 0 ? rows / 512 : 1;
+    if (gemm_bf16_tc(t->ds_dist, 1, (long long)c.n_heads * S, qv_op, 1, HD, S, 64, rows, sk, er, ns, st)) return -1;
+  }
+  if (train_cast_bf16(t->drk32, t->drk16, (long long)S * HD, st)) return -1;
+  if (grad_w(m, t, t->drk16, HD, t->pe, d, HD, d, S, g.wr, st)) return -1;
+  if (g.br >= 0 && train_colsum_bf16(t->drk16, HD, S, HD, t->G + g.br, st)) return -1;
+  return 0;
+}
+
 int backward_head(dmg_model* m, dmg_train* t, cudaStream_t st) {
   const dmg_config& c = m->cfg;
   const int d = c.d_model, rows = t->rows, ns = m->num_sms;
@@ -371,21 +435,9 @@ int backward_layer(dmg_model* m, dmg_train* t, int l, cudaStream_t st) {
     const bool q_saved = ba.f.qu_save != nullptr;    // the tcgen05 forward stored q + u and q + v
     if (q_saved) ba.qu = ba.f.qu_save;
     if (attn_train_bwd(ba, ns, st)) return -1;
-    // dRk[h] = dS_dist[:, h]^T (q + v)[:, h]  ->  dWr = dRk^T PE
     const bf16* qv_op = q_saved ? ba.f.qv_save : t->qv;
     if (!q_saved && train_q_plus_bias(A.qkv_x, 3 * HD, m->v, t->qv, rows, HD, st)) return -1;
-    DMG_CUDA_OK(cudaMemsetAsync(t->drk32, 0, (size_t)S * HD * sizeof(float), st));
-    {   // one grouped launch: group h reads dS_dist columns [h*S, (h+1)*S) and (q+v) columns [h*64, (h+1)*64)
-      GemmEpi er; er.out = t->drk32; er.ldc = HD; er.out_mode = GEMM_OUT_ATOMIC;
-      er.groups = c.n_heads; er.a_gs = S; er.b_gs = 64; er.c_gs = 64;
-      int sk = (2 * ns) / (c.n_heads * ((S + 127) / 128));
-      if (sk < 1) sk = 1;
-      if (sk > rows / 512) sk = rows / 512 > 0 ? rows / 512 : 1;
-      if (gemm_bf16_tc(t->ds_dist, 1, (long long)c.n_heads * S, qv_op, 1, HD, S, 64, rows, sk, er, ns, st)) return -1;
-    }
-    if (train_cast_bf16(t->drk32, t->drk16, (long long)S * HD, st)) return -1;
-    if (grad_w(m, t, t->drk16, HD, t->pe, d, HD, d, S, g.wr, st)) return -1;
-    if (g.br >= 0 && train_colsum_bf16(t->drk16, HD, S, HD, t->G + g.br, st)) return -1;
+    if (grad_rel_pos(m, t, qv_op, g, st)) return -1;
     // dWqkv: segment rows, then the memory rows' k|v part
     if (grad_w(m, t, t->dqkv_x, 3 * HD, A.xa_in, d, 3 * HD, d, rows, g.wqkv, st)) return -1;
     if (g.bqkv >= 0 && train_colsum_bf16(t->dqkv_x, 3 * HD, rows, 3 * HD, t->G + g.bqkv, st)) return -1;
@@ -401,12 +453,81 @@ int backward_layer(dmg_model* m, dmg_train* t, int l, cudaStream_t st) {
   return 0;
 }
 
+// remix encoder: per layer ln(x + drop_res(attn(x))) (no out-projection, no FFN), then the head and the masked cross entropy
+int train_forward_bert(dmg_model* m, dmg_train* t, const long long* ids, const long long* pos, const long long* targets, cudaStream_t st) {
+  const dmg_config& c = m->cfg;
+  const int d = c.d_model, HD = m->HD, L = c.n_layers, rows = t->rows, T = t->T, ns = m->num_sms;
+  DMG_CUDA_OK(cudaMemsetAsync(t->acc, 0, 8 * sizeof(float), st));
+  {
+    const Drop dr = make_drop(t, t->cfg.embed_p, SITE_EMBED, 0);
+    if (train_embed(ids, pos, m->emb.f32, m->beat, m->bar, t->x32, t->act[0].xa_in, rows, d, c.vocab, dr.thresh, dr.seed, dr.scale, st))
+      return -1;
+  }
+  for (int l = 0; l < L; l++) {
+    LayerW& W = m->layers[l];
+    LayerAct& A = t->act[l];
+    bf16* xa_out = l + 1 < L ? t->act[l + 1].xa_in : t->xa_last;
+    {   // relative-position keys Rk = PE[0..T) Wr^T (+br)
+      GemmEpi e; e.bias = W.br; e.out = A.rk; e.ldc = HD; e.out_mode = GEMM_OUT_BF16;
+      if (gemm_bf16_tc(t->pe, 0, d, W.wr.b16, 0, d, T, HD, d, 1, e, ns, st)) return -1;
+    }
+    {   // q | k | v
+      GemmEpi e; e.bias = W.bqkv; e.out = A.qkv_x; e.ldc = 3 * HD; e.out_mode = GEMM_OUT_BF16;
+      if (gemm_bf16_tc(A.xa_in, 0, d, W.wqkv.b16, 0, d, rows, 3 * HD, d, 1, e, ns, st)) return -1;
+    }
+    if (attn_bert_train_fwd(attn_args(m, t, l), st)) return -1;
+    const Drop dr = make_drop(t, t->cfg.resid_p, SITE_RES1, l);   // attention output (HD == d) enters the residual directly
+    if (train_residual_ln_fwd(t->x32, A.attn, W.ln1w, W.ln1b, xa_out, A.z1, A.st1, rows, d, dr.thresh, dr.seed, dr.scale, st)) return -1;
+  }
+  const Drop dr = make_drop(t, t->cfg.output_p, SITE_OUT, 0);
+  if (train_rnn_dropout(t->xa_last, t->xdrop, t->B, T, d, dr.thresh, dr.seed, dr.scale, st)) return -1;
+  GemmEpi e; e.bias = m->head_b; e.out = t->logits; e.ldc = t->Vp; e.out_mode = GEMM_OUT_F32;
+  if (gemm_bf16_tc(t->xdrop, 0, d, m->emb.b16, 0, d, rows, c.vocab, d, 1, e, ns, st)) return -1;
+  if (targets && train_ce_loss_masked(t->logits, t->Vp, targets, t->cfg.pad_idx, t->dlogits, t->acc + 0, t->acc + 4, rows, c.vocab, st))
+    return -1;
+  return 0;
+}
+
+int backward_layer_bert(dmg_model* m, dmg_train* t, int l, cudaStream_t st) {
+  const dmg_config& c = m->cfg;
+  const int d = c.d_model, HD = m->HD, H = c.n_heads, rows = t->rows, T = t->T, ns = m->num_sms;
+  LayerW& W = m->layers[l];
+  LayerAct& A = t->act[l];
+  const LayerGrad& g = t->lg[l];
+  const Drop d2 = make_drop(t, t->cfg.resid_p, SITE_RES1, l);
+  // dadd = gradient wrt the attention output
+  if (train_ln_bwd(t->dx32, t->dbr_valid ? t->dbr : nullptr, A.z1, A.st1, W.ln1w, t->dadd, t->G + g.ln1w, t->G + g.ln1b, nullptr, rows, d,
+                   d2.thresh, d2.seed, d2.scale, st)) return -1;
+  AttnTrainBwdArgs ba;
+  ba.f = attn_args(m, t, l);
+  ba.dout = t->dadd; ba.delta = t->delta; ba.dqkv_x = t->dqkv_x; ba.dkv_m = nullptr; ba.ds_dist = t->ds_dist; ba.qv = t->qv;
+  ba.du = t->G + t->g_u; ba.dv = t->G + t->g_v;
+  ba.p_buf = t->p_buf; ba.ds_buf = t->ds_buf;
+  if (attn_bert_train_bwd(ba, st)) return -1;
+  // position part of dq: dq_pos[:, h] = dS_dist[:, h] Rk[:, h] (per head, into dattn); dv = its column sums; dq += dq_pos
+  for (int h = 0; h < H; h++) {
+    GemmEpi e; e.out = t->dattn + h * 64; e.ldc = HD; e.out_mode = GEMM_OUT_BF16;
+    if (gemm_bf16_tc(t->ds_dist + (size_t)h * T, 0, (long long)H * T, A.rk + h * 64, 1, HD, rows, 64, T, 1, e, ns, st)) return -1;
+  }
+  if (train_colsum_bf16(t->dattn, HD, rows, HD, t->G + t->g_v, st)) return -1;
+  if (train_add_bf16(t->dqkv_x, 3 * HD, t->dattn, HD, rows, HD, st)) return -1;
+  if (train_q_plus_bias(A.qkv_x, 3 * HD, m->v, t->qv, rows, HD, st)) return -1;
+  if (grad_rel_pos(m, t, t->qv, g, st)) return -1;
+  if (grad_w(m, t, t->dqkv_x, 3 * HD, A.xa_in, d, 3 * HD, d, rows, g.wqkv, st)) return -1;
+  if (g.bqkv >= 0 && train_colsum_bf16(t->dqkv_x, 3 * HD, rows, 3 * HD, t->G + g.bqkv, st)) return -1;
+  // input gradient of the attention branch, consumed by the next LayerNorm backward (or the embedding backward)
+  GemmEpi e2; e2.out = t->dbr; e2.ldc = d; e2.out_mode = GEMM_OUT_BF16;
+  if (gemm_bf16_tc(t->dqkv_x, 0, 3 * HD, W.wqkv.b16, 1, d, rows, d, 3 * HD, 1, e2, ns, st)) return -1;
+  t->dbr_valid = true;
+  return 0;
+}
+
 int backward_embed(dmg_model* m, dmg_train* t, cudaStream_t st) {
   const dmg_config& c = m->cfg;
   const Drop dr = make_drop(t, t->cfg.embed_p, SITE_EMBED, 0);
   return train_embed_bwd(t->ids, c.encode_position ? t->pos : nullptr, t->dx32, t->dbr_valid ? t->dbr : nullptr, t->G + t->g_emb,
                          t->g_beat >= 0 ? t->G + t->g_beat : nullptr, t->g_bar >= 0 ? t->G + t->g_bar : nullptr, t->rows, c.d_model,
-                         c.vocab, dr.thresh, dr.seed, dr.scale, st);
+                         c.vocab, t->emb_pad, dr.thresh, dr.seed, dr.scale, st);
 }
 
 int check_train(dmg_model* m, const char* who) {
@@ -435,7 +556,8 @@ extern "C" {
 int64_t dmg_train_param_count(dmg_model* m) {
   if (!m) return -1;
   dmg_train tmp;
-  build_params(m, &tmp);
+  if (m->cfg.arch == DMG_ARCH_BERT) build_params_bert(m, &tmp);
+  else build_params(m, &tmp);
   return tmp.total;
 }
 
@@ -451,13 +573,14 @@ void dmg_train_destroy(dmg_model* m) {
 int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat_dev) {
   DMG_CHECK(m && cfg, "dmg_train_create: null argument");
   const dmg_config& c = m->cfg;
-  DMG_CHECK(c.arch == DMG_ARCH_TXL, "dmg_train_create: only the Transformer-XL model trains (remix training is out of scope)");
+  const bool bert = c.arch == DMG_ARCH_BERT;
   DMG_CHECK(m->is_bf16 && m->use_tc, "dmg_train_create: training needs the bf16 tcgen05 model (DMG_BF16, DMG_GEMM_AUTO)");
   DMG_CHECK(m->committed, "dmg_train_create: weights not committed");
   DMG_CHECK(cfg->batch >= 1 && cfg->bptt >= 64 && cfg->bptt % 64 == 0, "dmg_train_create: batch %d / bptt %d (bptt must be a multiple of 64)",
             cfg->batch, cfg->bptt);
   DMG_CHECK(c.mem_len % 64 == 0, "dmg_train_create: mem_len %d must be a multiple of 64", c.mem_len);
-  DMG_CHECK(c.d_inner % 64 == 0 && c.d_model % 128 == 0, "dmg_train_create: d_inner %% 64 and d_model %% 128 required");
+  DMG_CHECK((bert || c.d_inner % 64 == 0) && c.d_model % 128 == 0, "dmg_train_create: d_inner %% 64 and d_model %% 128 required");
+  DMG_CHECK(!bert || (cfg->pad_idx >= 0 && cfg->pad_idx < c.vocab), "dmg_train_create: pad_idx %d outside the vocabulary", cfg->pad_idx);
   const float ps[5] = {cfg->resid_p, cfg->attn_p, cfg->ff_p, cfg->embed_p, cfg->output_p};
   for (float p : ps) DMG_CHECK(p >= 0.f && p < 0.95f, "dmg_train_create: dropout probability %f outside [0, 0.95)", p);
   DMG_CUDA_OK(cudaSetDevice(m->device));
@@ -469,7 +592,14 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
   const int d = c.d_model, HD = m->HD, L = c.n_layers, M = c.mem_len, rows = t->rows, S = M + t->T, di = c.d_inner;
   t->S = S;
   t->Vp = (c.vocab + 63) / 64 * 64;
-  build_params(m, t);
+  t->bert = bert;
+  if (bert) {   // the encoder has no AR / TAR terms
+    t->cfg.alpha = t->cfg.beta = 0.f;
+    t->emb_pad = cfg->pad_idx;
+    build_params_bert(m, t);
+  } else {
+    build_params(m, t);
+  }
   int rc = 0;
 #define TRY(x) do { if (!rc && (x)) rc = -1; } while (0)
   if (grad_flat_dev) { t->G = grad_flat_dev; t->own_G = false; }
@@ -478,7 +608,19 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
   TRY(talloc(t, &t->m2, (size_t)t->total));
   t->act.resize(L);
   const size_t BM = (size_t)t->B * (M > 0 ? M : 1);
-  for (int l = 0; l < L && !rc; l++) {
+  for (int l = 0; l < L && !rc && bert; l++) {
+    LayerAct& A = t->act[l];
+    TRY(talloc(t, &A.xa_in, (size_t)rows * d));
+    TRY(talloc(t, &A.qkv_x, (size_t)(rows + 1) * 3 * HD));   // + the zero row the last query tile reads as "next row"
+    TRY(talloc(t, &A.attn, (size_t)rows * HD));
+    TRY(talloc(t, &A.z1, (size_t)rows * d));
+    bf16* rk = nullptr;   // Rk rows -64 .. T+127: the zero rows the attention's rel-pos windows read past both ends
+    TRY(talloc(t, &rk, (size_t)(S + 192) * HD));
+    A.rk = rk + (size_t)64 * HD;
+    TRY(talloc(t, &A.lse, (size_t)t->B * c.n_heads * t->T));
+    TRY(talloc(t, &A.st1, (size_t)rows));
+  }
+  for (int l = 0; l < L && !rc && !bert; l++) {
     LayerAct& A = t->act[l];
     TRY(talloc(t, &A.xa_in, (size_t)rows * d));
     TRY(talloc(t, &A.qkv_x, (size_t)rows * 3 * HD));
@@ -524,14 +666,14 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
   TRY(talloc(t, &t->proj, (size_t)rows * d));
   TRY(talloc(t, &t->dadd, (size_t)rows * d));
   TRY(talloc(t, &t->dbr, (size_t)rows * d));
-  TRY(talloc(t, &t->dh, (size_t)rows * di));
+  if (!bert) TRY(talloc(t, &t->dh, (size_t)rows * di));
   TRY(talloc(t, &t->dattn, (size_t)rows * HD));
   TRY(talloc(t, &t->dqkv_x, (size_t)rows * 3 * HD));
   TRY(talloc(t, &t->dkv_m, BM * 2 * HD));
   TRY(talloc(t, &t->ds_dist, (size_t)rows * c.n_heads * S));
   TRY(talloc(t, &t->qv, (size_t)rows * HD));
   static const bool bwd_recompute = getenv("DMG_ATTN_BWD_RECOMPUTE") != nullptr;   // measurement switch, read once
-  if (!bwd_recompute) {   // spill P / dS from the dQ kernel instead of recomputing them for dK / dV
+  if (!bwd_recompute || bert) {   // spill P / dS from the dQ kernel instead of recomputing them for dK / dV
     TRY(talloc(t, &t->p_buf, (size_t)rows * c.n_heads * S));
     TRY(talloc(t, &t->ds_buf, (size_t)rows * c.n_heads * S));
   }
@@ -576,11 +718,14 @@ int dmg_train_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_d
   DMG_CHECK(ids_dev, "dmg_train_forward: null ids");
   DMG_CHECK(!m->cfg.encode_position || pos_dev, "dmg_train_forward: model encodes position but pos is NULL");
   DMG_CHECK((mask_win == 1 && mask_k == 1) || (mask_win >= 1 && mask_k == 0), "dmg_train_forward: window mask (%d,%d) unsupported", mask_win, mask_k);
+  DMG_CHECK(!m->train->bert || (mask_win == 1 && mask_k == 1), "dmg_train_forward: the remix encoder has no attention mask, (mask_win, mask_k) must be (1, 1), got (%d,%d)",
+            mask_win, mask_k);
   DMG_CUDA_OK(cudaSetDevice(m->device));
   dmg_train* t = m->train;
   t->ids = (const long long*)ids_dev; t->pos = (const long long*)pos_dev;
   t->win = mask_win; t->k = mask_k; t->training = training ? 1 : 0; t->step = step;
-  if (train_forward(m, t, t->ids, t->pos, (const long long*)targets_dev, (cudaStream_t)stream)) return -1;
+  if (t->bert ? train_forward_bert(m, t, t->ids, t->pos, (const long long*)targets_dev, (cudaStream_t)stream)
+              : train_forward(m, t, t->ids, t->pos, (const long long*)targets_dev, (cudaStream_t)stream)) return -1;
   t->next_layer = targets_dev ? m->cfg.n_layers : -1;
   return 0;
 }
@@ -596,7 +741,7 @@ int dmg_train_backward(dmg_model* m, int layer_hi, int layer_lo, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   if (layer_hi == L && backward_head(m, t, st)) return -1;
   for (int l = layer_hi - 1; l >= layer_lo; l--)
-    if (backward_layer(m, t, l, st)) return -1;
+    if (t->bert ? backward_layer_bert(m, t, l, st) : backward_layer(m, t, l, st)) return -1;
   t->next_layer = layer_lo;
   if (layer_lo == 0) {
     if (backward_embed(m, t, st)) return -1;
@@ -663,10 +808,16 @@ int dmg_train_losses(dmg_model* m, float* out4_host, void* stream) {
   DMG_CHECK(out4_host, "dmg_train_losses: null output");
   dmg_train* t = m->train;
   DMG_CUDA_OK(cudaSetDevice(m->device));
-  float a[4];
+  float a[5];
   DMG_CUDA_OK(cudaMemcpyAsync(a, t->acc, sizeof(a), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
   DMG_CUDA_OK(cudaStreamSynchronize((cudaStream_t)stream));
   const int d = m->cfg.d_model, M = m->cfg.mem_len;
+  if (t->bert) {   // mean over the targets that are not pad_idx (NaN when there are none, as torch gives); no AR / TAR
+    out4_host[0] = a[0] / a[4];
+    out4_host[1] = out4_host[2] = 0.f;
+    out4_host[3] = sqrtf(a[3]);
+    return 0;
+  }
   out4_host[0] = a[0] / t->rows;
   out4_host[1] = t->cfg.alpha * a[1] / ((float)t->rows * d);
   int cnt = t->mem_count + (t->mem_pending ? t->T : 0);

@@ -62,7 +62,7 @@ __global__ void __launch_bounds__(256) train_embed_kernel(const long long* __res
 __global__ void __launch_bounds__(256) train_embed_bwd_kernel(const long long* __restrict__ ids, const long long* __restrict__ pos,
                                                               const float* __restrict__ dx, const bf16* __restrict__ dbr, float* __restrict__ demb,
                                                               float* __restrict__ dbeat, float* __restrict__ dbar, int rows, int d,
-                                                              int vocab, uint32_t thresh, uint32_t seed, float scale) {
+                                                              int vocab, long long pad_idx, uint32_t thresh, uint32_t seed, float scale) {
   const int d4 = d >> 2;
   const long long n = (long long)rows * d4;
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
@@ -79,8 +79,10 @@ __global__ void __launch_bounds__(256) train_embed_bwd_kernel(const long long* _
       keep4(seed, (uint32_t)(row * d + c), thresh, scale, k);
       g.x *= k[0]; g.y *= k[1]; g.z *= k[2]; g.w *= k[3];
     }
-    float* e = demb + id * d + c;
-    atomicAdd(e, g.x); atomicAdd(e + 1, g.y); atomicAdd(e + 2, g.z); atomicAdd(e + 3, g.w);
+    if (id != pad_idx) {   // nn.Embedding(padding_idx): lookups of the pad token contribute no gradient
+      float* e = demb + id * d + c;
+      atomicAdd(e, g.x); atomicAdd(e + 1, g.y); atomicAdd(e + 2, g.z); atomicAdd(e + 3, g.w);
+    }
     if (pos) {
       const long long p = pos[row];
       const long long bt = ((p % 32) + 32) % 32;
@@ -269,11 +271,22 @@ __global__ void __launch_bounds__(256) train_colsum_kernel(const bf16* __restric
 }
 
 // ------------------------------------------------------------------ loss
+// MASKED: rows whose target is `ignore` get zero gradient and no loss; the others are scaled by 1 / count[0] (read on the device)
+template <bool MASKED>
 __global__ void __launch_bounds__(256) train_ce_kernel(const float* __restrict__ logits, long long ldl,
                                                        const long long* __restrict__ targets, bf16* __restrict__ dlogits,
-                                                       float* __restrict__ loss_acc, int rows, int V, float gscale) {
+                                                       float* __restrict__ loss_acc, int rows, int V, float gscale, long long ignore,
+                                                       const float* __restrict__ count) {
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (row >= rows) return;
+  if (MASKED) {
+    if (targets[row] == ignore) {
+      bf16* dr = dlogits + (long long)row * ldl;
+      for (int c = lane; c < (int)ldl; c += 32) dr[c] = __float2bfloat16_rn(0.f);
+      return;
+    }
+    gscale = 1.f / count[0];                        // >= 1: this row counts
+  }
   const float* lr = logits + (long long)row * ldl;
   float mx = -INFINITY;
   for (int c = lane; c < V; c += 32) mx = fmaxf(mx, lr[c]);
@@ -291,6 +304,37 @@ __global__ void __launch_bounds__(256) train_ce_kernel(const float* __restrict__
     dr[c] = __float2bfloat16_rn(gq);
   }
   if (lane == 0) atomicAdd(loss_acc, mx + logf(se) - lr[tg]);
+}
+
+// number of targets != ignore, written to *count (one block)
+__global__ void __launch_bounds__(256) train_count_kernel(const long long* __restrict__ targets, int rows, long long ignore,
+                                                          float* __restrict__ count) {
+  __shared__ int red[8];
+  int n = 0;
+  for (int r = threadIdx.x; r < rows; r += 256) n += targets[r] != ignore;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = n;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int t = 0;
+    for (int q = 0; q < 8; q++) t += red[q];
+    *count = (float)t;
+  }
+}
+
+// dst[r, c] += src[r, c] (bf16, fp32 sum), n even
+__global__ void __launch_bounds__(256) train_add_bf16_kernel(bf16* __restrict__ dst, long long ldd, const bf16* __restrict__ src,
+                                                             long long lds, int rows, int n) {
+  const int n2 = n >> 1;
+  const long long tot = (long long)rows * n2;
+  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < tot; i += (long long)gridDim.x * 256) {
+    const long long r = i / n2;
+    const int c = (int)(i % n2) * 2;
+    uint32_t* dp = (uint32_t*)(dst + r * ldd + c);
+    const uint32_t a = *dp, b = *(const uint32_t*)(src + r * lds + c);
+    *dp = pack_bf16x2(bf16lo(a) + bf16lo(b), bf16hi(a) + bf16hi(b));
+  }
 }
 
 __global__ void __launch_bounds__(256) train_rnn_dropout_kernel(const bf16* __restrict__ x, bf16* __restrict__ y, int B, int T, int d,
@@ -544,9 +588,9 @@ int train_embed(const long long* ids, const long long* pos, const float* emb, co
 }
 
 int train_embed_bwd(const long long* ids, const long long* pos, const float* dx, const bf16* dbr, float* demb, float* dbeat, float* dbar,
-                    int rows, int d, int vocab, uint32_t thresh, uint32_t seed, float scale, cudaStream_t st) {
+                    int rows, int d, int vocab, long long pad_idx, uint32_t thresh, uint32_t seed, float scale, cudaStream_t st) {
   return launch_np(train_embed_bwd_kernel, dim3(grid_for((long long)rows * d / 4)), dim3(256), 0, st, ids, pos, dx, dbr, demb, dbeat, dbar,
-                   rows, d, vocab, thresh, seed, scale);
+                   rows, d, vocab, pad_idx, thresh, seed, scale);
 }
 
 int train_residual_ln_fwd(float* x32, const bf16* add, const float* w, const float* b, bf16* xa, bf16* zsave, float2* stats,
@@ -596,7 +640,19 @@ int train_colsum_bf16(const bf16* x, long long ld, int rows, int n, float* dst, 
 
 int train_ce_loss(const float* logits, long long ldl, const long long* targets, bf16* dlogits, float* loss_acc, int rows, int V,
                   float gscale, cudaStream_t st) {
-  return launch_np(train_ce_kernel, dim3((rows + 7) / 8), dim3(256), 0, st, logits, ldl, targets, dlogits, loss_acc, rows, V, gscale);
+  return launch_np(train_ce_kernel<false>, dim3((rows + 7) / 8), dim3(256), 0, st, logits, ldl, targets, dlogits, loss_acc, rows, V, gscale,
+                   -1ll, (const float*)nullptr);
+}
+
+int train_ce_loss_masked(const float* logits, long long ldl, const long long* targets, long long ignore, bf16* dlogits, float* loss_acc,
+                         float* count, int rows, int V, cudaStream_t st) {
+  if (launch_np(train_count_kernel, dim3(1), dim3(256), 0, st, targets, rows, ignore, count)) return -1;
+  return launch_np(train_ce_kernel<true>, dim3((rows + 7) / 8), dim3(256), 0, st, logits, ldl, targets, dlogits, loss_acc, rows, V, 0.f,
+                   ignore, (const float*)count);
+}
+
+int train_add_bf16(bf16* dst, long long ldd, const bf16* src, long long lds, int rows, int n, cudaStream_t st) {
+  return launch_np(train_add_bf16_kernel, dim3(grid_for((long long)rows * n / 2)), dim3(256), 0, st, dst, ldd, src, lds, rows, n);
 }
 
 int train_rnn_dropout(const bf16* x, bf16* y, int B, int T, int d, uint32_t thresh, uint32_t seed, float scale, cudaStream_t st) {

@@ -149,6 +149,16 @@ struct AttnTrainBwdArgs {
   bf16* ds_buf = nullptr;  // probabilities and dS there and dK/dV come from a kernel that does not recompute the scores
 };
 int attn_train_bwd(const AttnTrainBwdArgs& a, int num_sms, cudaStream_t st);
+// pieces of attn_train_bwd that the remix encoder's backward reuses: delta = rowsum(dO * O); dK / dV from the spilled P / dS
+// tiles with every query tile seeing every key (M = 0, p_buf and ds_buf set)
+int attn_train_delta(const AttnTrainBwdArgs& ba, cudaStream_t st);
+int attn_bwd_dkv_all_queries(const AttnTrainBwdArgs& ba, cudaStream_t st);
+// remix (masked-BERT) encoder attention for training (attention_bert_train.cu): no memory, no mask, _line_shift wrap-around
+// live (lines 1 and 3), T a multiple of 64.  Rk ([T, HD], row = distance) must read as zero for rows -64 .. T+127 and qkv_x
+// needs one readable row past the last stream.  The backward writes the content part of dq (+ du), dk, dv, ds_dist and the
+// P / dS spill (p_buf / ds_buf, required); the position part of dq is ds_dist . Rk (the trainer's per-head GEMMs).
+int attn_bert_train_fwd(const AttnTrainArgs& a, cudaStream_t st);
+int attn_bert_train_bwd(const AttnTrainBwdArgs& ba, cudaStream_t st);
 
 // ------------------------------------------------------------------ elementwise / reductions (train_kernels.cu)
 // x32 = emb[id] (+beat+bar) with embedding dropout; xa = bf16(x32)
@@ -172,6 +182,10 @@ int train_colsum_bf16(const bf16* x, long long ld, int rows, int n, float* dst, 
 // head: logits fp32 [rows, ldl] -> per-row CE loss (sum into loss_acc[0]) and dlogits bf16 [rows, ldl] = (softmax - onehot) * gscale
 int train_ce_loss(const float* logits, long long ldl, const long long* targets, bf16* dlogits, float* loss_acc,
                   int rows, int V, float gscale, cudaStream_t st);
+// CrossEntropyFlat(ignore_index=ignore): *count (device) = number of targets != ignore, counted on the device; rows with the
+// ignore target get no loss and zero dlogits, the others (softmax - onehot) / count.  loss_acc / count is the mean (NaN at count 0).
+int train_ce_loss_masked(const float* logits, long long ldl, const long long* targets, long long ignore, bf16* dlogits, float* loss_acc,
+                         float* count, int rows, int V, cudaStream_t st);
 // output (RNN) dropout of the head input: xd[b,t,:] = xa[b,t,:] * mask[b,:]   (one mask per stream and feature)
 int train_rnn_dropout(const bf16* x, bf16* y, int B, int T, int d, uint32_t thresh, uint32_t seed, float scale,
                       cudaStream_t st);
@@ -184,9 +198,12 @@ int train_sumsq(const float* x, long long n, float* acc, cudaStream_t st);
 int train_sumsq_det(const float* x, long long n, float* part, int part_cap, float* out, cudaStream_t st);
 // TAR value: sum over b, t>=1 of (h[b,t]-h[b,t-1])^2 for h = bf16 [B, n, d] with stream stride bstride elements
 int train_tar(const bf16* h, long long bstride, int B, int n, int d, float* acc, cudaStream_t st);
-// embedding backward: demb[id] += mask * scale * (dx + dbr) (atomics); beat/bar likewise when pos != NULL
+// embedding backward: demb[id] += mask * scale * (dx + dbr) (atomics) except for id == pad_idx (-1: none); beat/bar likewise
+// when pos != NULL (their row 0 is a padding row)
 int train_embed_bwd(const long long* ids, const long long* pos, const float* dx, const bf16* dbr, float* demb, float* dbeat, float* dbar,
-                    int rows, int d, int vocab, uint32_t thresh, uint32_t seed, float scale, cudaStream_t st);
+                    int rows, int d, int vocab, long long pad_idx, uint32_t thresh, uint32_t seed, float scale, cudaStream_t st);
+// dst[rows, n] += src (bf16, row strides ldd / lds)
+int train_add_bf16(bf16* dst, long long ldd, const bf16* src, long long lds, int rows, int n, cudaStream_t st);
 // fp32 [rows, d] -> bf16
 int train_cast_bf16(const float* src, bf16* dst, long long n, cudaStream_t st);
 // gradient bucket <-> its bf16 wire format (any alignment)

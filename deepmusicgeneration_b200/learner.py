@@ -252,10 +252,68 @@ class MultitaskLearner:
         self.data, self.model, self.config = data, model, config
 
     def save(self, file=None, with_opt=True, config=None):
-        state = {'model': self.model.state_dict(), 'opt': None}
+        """{'model': state_dict, 'opt': Adam state of the live trainer (None before any training or with with_opt=False)[, 'config']}:
+        the file multitask_model_learner(pretrained_path=...) reads back."""
+        tr = getattr(self, '_trainer', None)
+        state = {'model': self.model.state_dict(), 'opt': tr.opt_state_dict() if (with_opt and tr is not None) else None}
         if config: state['config'] = config
         torch.save(state, file)
         return file
+
+    # -- training of the mask task: what fastai's Learner.fit_one_cycle does for this learner (MTTrainer, SURVEY.md App. D.8)
+    def trainer(self, bs, bptt, drop_mult=1., seed=0, **kw):
+        "The training-step engine for this model (masked cross entropy, ignore index = the vocabulary's pad); created once per (bs, bptt)."
+        from .training import RemixTrainer
+        key = (bs, bptt, float(drop_mult), int(seed), tuple(sorted(kw.items())))
+        if getattr(self, '_trainer_key', None) != key:
+            if getattr(self, '_trainer', None) is not None:
+                self._trainer.close()
+            self._trainer = RemixTrainer(self.model, bs, bptt, self.config, pad_idx=self.data.vocab.pad_idx, drop_mult=drop_mult,
+                                         seed=seed, **kw)
+            self._trainer_key = key
+        return self._trainer
+
+    def load_opt_state(self, opt_state, bs, bptt, **kw):
+        "learn.opt.load_state_dict(state['opt']) onto the trainer of this (bs, bptt)."
+        if opt_state:
+            self.trainer(bs, bptt, **kw).load_opt_state_dict(opt_state)
+
+    def fit_one_cycle(self, cyc_len, max_lr, batches, bs=None, bptt=None, wd=0.01, clip=0.5, moms=(0.95, 0.85), drop_mult=1.,
+                      mask_p=0.3, mask_range=None, callback=None):
+        """learner.fit_one_cycle(epochs, lr) of the mask task over `batches`: either a list of already-masked ({'x', 'pos'}, y)
+        batches (LongTensors [bs, bptt], y = pad_idx where nothing is predicted), or a deepmusicgeneration_b200.preloader.MusicPreloader
+        built with y_offset=0 and encode_position=True, whose every batch goes through mask_tfm(p=mask_p, mask_range) on the device
+        (deep_music_remix.py:1208-1223).  The default mask_range is (vocab.note_range[0], vocab.dur_range[1]), the range the
+        preloader golden (tests/golden/make_preloader_golden.py) was generated with.  One-cycle LR / momentum schedule over all
+        cyc_len passes, Adam(true_wd), gradient clipping; returns the last step's losses."""
+        from .training import one_cycle_lr
+        from .preloader import MusicPreloader, mask_tfm
+        vocab = self.data.vocab
+        if mask_range is None:
+            mask_range = (vocab.note_range[0], vocab.dur_range[1])
+        is_pl = isinstance(batches, MusicPreloader)
+        n_b = batches.n_batches if is_pl else len(batches)
+        tr = self.trainer(bs or (batches.local_bs if is_pl else batches[0][0]['x'].shape[0]),
+                          bptt or (batches.bptt if is_pl else batches[0][0]['x'].shape[1]), drop_mult=drop_mult)
+        if getattr(self, 'pretrained_opt_state', None):
+            try:    tr.load_opt_state_dict(self.pretrained_opt_state)     # try / except: pass, like the reference
+            except Exception: pass
+            self.pretrained_opt_state = None
+        total, i = cyc_len * n_b, 0
+        for _ in range(cyc_len):
+            for xb, y in batches:
+                if not isinstance(xb, dict):
+                    raise ValueError('the remix encoder needs ({"x", "pos"}, y) batches (MusicPreloader(encode_position=True))')
+                x, pos = xb['x'], xb['pos']
+                if is_pl:
+                    x, y = mask_tfm((x, y), mask_range, vocab.mask_idx, vocab.pad_idx, p=mask_p)
+                lr, mom = one_cycle_lr(i, total, max_lr, moms=moms)
+                tr.step(x, y, pos, lr=lr, betas=(mom, 0.99), wd=wd, clip=clip)
+                if callback is not None:
+                    callback(i, tr)
+                i += 1
+        tr.sync_for_inference()
+        return tr.losses()
 
     def pred_batch(self, batch):
         "fastai Learner.pred_batch: eval-mode forward of one batch."
@@ -303,4 +361,5 @@ def multitask_model_learner(data, config=None, drop_mult=1., pretrained_path=Non
     learn = MultitaskLearner(data, model, config=config)
     if state is not None:
         model.load_state_dict(state['model'], strict=False)
+        learn.pretrained_opt_state = state.get('opt')      # applied by fit_one_cycle to the trainer it creates
     return learn

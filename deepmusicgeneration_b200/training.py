@@ -49,7 +49,7 @@ class TXLTrainer:
     trainer.losses()                                                    # {'ce':.., 'ar':.., 'tar':.., 'loss':.., 'grad_norm':..}
     """
     def __init__(self, model, bs, bptt, config, drop_mult=1., alpha=2., beta=1., seed=0, process_group=None, bucket_layers=4,
-                 distributed=None, wire='bf16', rank_seed=True):
+                 distributed=None, wire='bf16', rank_seed=True, pad_idx=0):
         self.model, self.e = model, model._e
         self.lib = self.e.lib
         self.bs, self.bptt = bs, bptt
@@ -73,7 +73,7 @@ class TXLTrainer:
         tc.batch, tc.bptt = bs, bptt
         for k in ('resid_p', 'attn_p', 'ff_p', 'embed_p', 'output_p'):
             setattr(tc, k, float(config.get(k, 0.)) * drop_mult)
-        tc.alpha, tc.beta, tc.seed = alpha, beta, seed
+        tc.alpha, tc.beta, tc.seed, tc.pad_idx = alpha, beta, seed, pad_idx
         self.tc = tc
         n = self.lib.dmg_train_param_count(self.e.h)
         if n <= 0:
@@ -297,3 +297,27 @@ class TXLTrainer:
         "Re-derive what inference caches from the trained weights (rel-pos key cache)."
         check(self.lib.dmg_commit_weights(self.e.h), 'dmg_commit_weights')
         self.e.committed = True
+
+
+class RemixTrainer(TXLTrainer):
+    """Masked-LM training of the remix encoder: what fastai's ``Learner.fit`` does per batch around ``MultiTransformer`` for the
+    ``msk`` task (deep_music_remix.py:1874-1881, 2734-2741)::
+
+        model.train(); logits = head(encoder(x_masked, pos))
+        loss = CrossEntropyFlat(ignore_index=pad_idx)(logits, y_masked)      # mean over the positions mask_tfm selected
+        loss.backward(); clip; Adam(betas=(0.9, 0.99)) with true_wd
+
+    ``model`` is the ``MultiTransformer`` mirror of ``model.get_multitask_model`` (bf16).  The encoder has no memory (``reset`` is a
+    no-op), no AR/TAR terms (``alpha = beta = 0``) and no attention mask.  ``bptt`` must be a multiple of 64.  Every step needs ``pos``;
+    ``y`` holds ``pad_idx`` at every position that is not predicted.  Data-parallel training is ``TXLTrainer``'s.
+    """
+    def __init__(self, model, bs, bptt, config, pad_idx, drop_mult=1., seed=0, **kw):
+        super().__init__(model, bs, bptt, config, drop_mult=drop_mult, alpha=0., beta=0., seed=seed, pad_idx=int(pad_idx), **kw)
+        self.pad_idx = int(pad_idx)
+
+    def forward(self, x, y=None, pos=None, mask_size=None):
+        if pos is None:
+            raise ValueError('RemixTrainer: the remix encoder adds beat/bar embeddings, pos is required')
+        if mask_size is not None and tuple(mask_size) != (1, 1):
+            raise ValueError(f'RemixTrainer: the remix encoder has no attention mask, mask_size must be (1, 1), got {tuple(mask_size)}')
+        return super().forward(x, y, pos, (1, 1))

@@ -197,9 +197,11 @@ int dmg_gemm_bf16(const void* a_dev, const void* w_dev, const float* bias_dev, v
  * Training step (SURVEY.md 3.3, App. A.7): what fastai's Learner.fit does around the reference model for one batch -
  * model(x) in train mode (deep_music_genre.py:1617-1647 with dropout and rand_window_mask :1586-1590), CrossEntropyFlat
  * + RNNTrainer's AR/TAR terms, loss.backward(), Adam with decoupled weight decay.  bf16 compute (tcgen05 GEMMs, mma.sync
- * flash attention with the rel-pos term), fp32 master weights / residual stream / gradients.  Needs a DMG_BF16
- * DMG_ARCH_TXL model.  Data-parallel training: every rank runs forward/backward on its own sequences and all-reduces the
- * flat gradient buffer (dmg_train_grad_span tells which slice is final after which backward call) before the step.
+ * flash attention with the rel-pos term), fp32 master weights / residual stream / gradients.  Needs a DMG_BF16 model:
+ * DMG_ARCH_TXL, or DMG_ARCH_BERT for masked-LM training of the remix encoder (the msk task of MultiTransformer,
+ * deep_music_remix.py:1874-1881: CrossEntropyFlat(ignore_index=pad_idx), no memory, no AR/TAR, no attention mask).
+ * Data-parallel training: every rank runs forward/backward on its own sequences and all-reduces the flat gradient buffer
+ * (dmg_train_grad_span tells which slice is final after which backward call) before the step.
  * ------------------------------------------------------------------------------------------------------------------ */
 typedef struct dmg_train_config {
   int32_t batch;            /* sequences per step on this GPU (each keeps its own memory, like bs rows of the reference batch) */
@@ -207,7 +209,8 @@ typedef struct dmg_train_config {
   float resid_p, attn_p, ff_p, embed_p, output_p;   /* dropout probabilities, already multiplied by drop_mult (App. A.1/A.2)    */
   float alpha, beta;        /* RNNTrainer activation regularisation (AR) and temporal AR (TAR, value only), App. A.7           */
   uint64_t seed;            /* base seed of the counter-based dropout masks                                                    */
-  int32_t reserved[4];
+  int32_t pad_idx;          /* DMG_ARCH_BERT: the loss's ignore index and the embedding's padding_idx (ignored for DMG_ARCH_TXL) */
+  int32_t reserved[3];
 } dmg_train_config;
 
 /* Allocates activations / gradient / Adam state.  grad_flat_dev: caller-owned fp32 device buffer of
@@ -216,10 +219,12 @@ typedef struct dmg_train_config {
 int64_t dmg_train_param_count(dmg_model* m);
 int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat_dev);
 void dmg_train_destroy(dmg_model* m);
-/* RNNTrainer.on_epoch_begin -> model.reset(): forget the training memory (hidden states of the previous segments). */
+/* RNNTrainer.on_epoch_begin -> model.reset(): forget the training memory (hidden states of the previous segments); a no-op
+ * for DMG_ARCH_BERT, which has no memory. */
 int dmg_train_reset(dmg_model* m);
 /* model(x) in train mode + loss.  ids/targets (and pos when encode_position): int64 [batch, bptt] on the device.
- * (mask_win, mask_k): what rand_window_mask drew on the host, (1,1) or (w,0).  training = 0 disables every dropout
+ * (mask_win, mask_k): what rand_window_mask drew on the host, (1,1) or (w,0); always (1,1) for DMG_ARCH_BERT, whose
+ * targets are the masked copy of x (mask_tfm) with pad_idx at every position not to be predicted.  training = 0 disables every dropout
  * (model.eval() semantics with the training memory).  `step` keys the dropout masks. */
 int dmg_train_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, const int64_t* targets_dev, int mask_win,
                       int mask_k, int training, int64_t step, void* stream);
@@ -245,11 +250,13 @@ int dmg_train_optimizer_step(dmg_model* m, float lr, float beta1, float beta2, f
 int dmg_train_opt_state(dmg_model* m, const char* name, int which, int set, float* buf_host, int64_t numel);
 int64_t dmg_train_opt_steps(dmg_model* m, int64_t value);
 /* Synchronises the stream and returns {cross-entropy (mean), alpha*AR, beta*TAR, gradient norm (after grad_scale; 0 before
- * the first optimizer step)} of the latest step. */
+ * the first optimizer step)} of the latest step.  DMG_ARCH_BERT: {mean CE over the targets != pad_idx (NaN if there are
+ * none; the gradients are then zero), 0, 0, gradient norm}. */
 int dmg_train_losses(dmg_model* m, float* out4_host, void* stream);
 /* Tests: gradient of one parameter by its state-dict name; the dropout mask (keep ? 1/(1-p) : 0) of a site as the kernels
  * generate it (site 0 embedding [rows,d], 1 attention [B,H,T,S], 2 attention-residual [rows,d], 3 FFN inner [rows,d_inner],
- * 4 FFN residual [rows,d], 5 output RNN dropout [B,d]); the device pointer of the owned gradient buffer. */
+ * 4 FFN residual [rows,d], 5 output RNN dropout [B,d]; DMG_ARCH_BERT uses 0, 1 [B,H,T,T], 2 and 5); the device pointer of the
+ * owned gradient buffer. */
 int dmg_train_get_grad(dmg_model* m, const char* name, float* out_host, int64_t numel);
 int dmg_train_dropout_mask(dmg_model* m, int site, int layer, int64_t step, float* out_dev, int64_t numel, void* stream);
 float* dmg_train_grad_buffer(dmg_model* m);
