@@ -961,4 +961,26 @@ int dmg_attn_train_bwd(const void* qkv_x, int64_t ldx, const void* kv_m, int64_t
   return attn_train_bwd(ba, 148, (cudaStream_t)stream);
 }
 
+int dmg_attn_bert_train_fwd(const void* qkv_x, int64_t ldx, const void* rk, const float* u, const float* v, void* out, float* lse,
+                            int B, int T, int H, float drop_p, uint32_t drop_seed_v, void* stream) {
+  DMG_CHECK(qkv_x && rk && u && v && out && lse, "dmg_attn_bert_train_fwd: null argument");
+  return attn_bert_train_fwd(make_attn_args(qkv_x, ldx, nullptr, 0, rk, u, v, out, lse, B, T, H, 0, 0, 1, 1, drop_p, drop_seed_v),
+                             (cudaStream_t)stream);
+}
+
+int dmg_attn_bert_train_bwd(const void* qkv_x, int64_t ldx, const void* rk, const float* u, const float* v, const void* out,
+                            const float* lse, const void* dout, int B, int T, int H, float drop_p, uint32_t drop_seed_v, float* delta,
+                            void* dqkv_x, void* ds_dist, float* du, void* p_buf, void* ds_buf, void* stream) {
+  DMG_CHECK(qkv_x && rk && u && v && out && lse && dout && delta && dqkv_x && du, "dmg_attn_bert_train_bwd: null argument");
+  DMG_CHECK(ds_dist, "dmg_attn_bert_train_bwd: ds_dist [B*T, H*T] is required");
+  DMG_CHECK(p_buf && ds_buf, "dmg_attn_bert_train_bwd: p_buf and ds_buf [B*H, T, T] are required");
+  AttnTrainBwdArgs ba;
+  ba.f = make_attn_args(qkv_x, ldx, nullptr, 0, rk, u, v, const_cast<void*>(out), const_cast<float*>(lse), B, T, H, 0, 0, 1, 1, drop_p,
+                        drop_seed_v);
+  ba.dout = (const bf16*)dout; ba.delta = delta; ba.dqkv_x = (bf16*)dqkv_x; ba.dkv_m = nullptr; ba.ds_dist = (bf16*)ds_dist;
+  ba.qv = nullptr; ba.du = du; ba.dv = nullptr;
+  ba.p_buf = (bf16*)p_buf; ba.ds_buf = (bf16*)ds_buf;
+  return attn_bert_train_bwd(ba, (cudaStream_t)stream);
+}
+
 }  // extern "C"

@@ -277,6 +277,21 @@ int dmg_attn_train_bwd(const void* qkv_x, int64_t ldx, const void* kv_m, int64_t
                        const float* v, const void* out, const float* lse, const void* dout, int B, int T, int H, int M,
                        int mem_count, int win, int k, float drop_p, uint32_t drop_seed, float* delta, void* dqkv_x, void* dkv_m,
                        void* ds_dist, float* du, float* dv, const void* p_save, const float* m_save, void* stream);
+/* Unit-test entries of the remix (masked-BERT) encoder's training attention (attention_bert_train.cu): no memory, no mask,
+ * T a multiple of 64, head size 64, HD = H*64.  Layouts:
+ *   qkv_x   [B*T + 1 rows, ldx] bf16, q | k | v at columns 0 | HD | 2*HD; the row past the last sequence must be readable
+ *   rk      points at row 0 (distance 0) of [T, HD] bf16 with 64 readable rows before it and 128 after it
+ *   out, dout [B*T, HD] dense (the kernels hard-code the row stride HD); lse, delta [B, H, T] fp32
+ *   dqkv_x  [B*T, ldx]: the q columns get the CONTENT part of dq only (the position part is ds_dist . Rk), k | v all of dk | dv
+ *   ds_dist [B*T, H*T] bf16: dS in (query row, distance) coordinates, head h at column h*T
+ *   du      [HD] fp32, accumulated into (not overwritten): u is shared by all layers
+ *   p_buf, ds_buf [B*H, T, T] bf16 workspaces, owned by the caller. */
+int dmg_attn_bert_train_fwd(const void* qkv_x, int64_t ldx, const void* rk, const float* u, const float* v, void* out,
+                            float* lse, int B, int T, int H, float drop_p, uint32_t drop_seed, void* stream);
+int dmg_attn_bert_train_bwd(const void* qkv_x, int64_t ldx, const void* rk, const float* u, const float* v,
+                            const void* out, const float* lse, const void* dout, int B, int T, int H, float drop_p,
+                            uint32_t drop_seed, float* delta, void* dqkv_x, void* ds_dist, float* du,
+                            void* p_buf, void* ds_buf, void* stream);
 
 /* ---- training data feed (SURVEY.md section 8 f4) ------------------------------------------------------------------------
  * dmg_preload_fill = MusicPreloader.__getitem__ / fill_row (deep_music_genre.py:1088-1125) for all `bs` rows of one batch.

@@ -6,6 +6,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+import remix_attention_ref
 from deepmusicgeneration_b200 import _lib
 from oracle import bert
 from oracle import bert_train
@@ -37,6 +38,57 @@ def test_line_shift_lines_and_ds_dist_identity(T):
             elif r >= 1: dist[r, x] = dS[r - 1, T + r - x]
     assert torch.allclose(qv.grad, dist @ R)
     assert torch.allclose(Rk.grad, dist.t() @ q)
+
+
+@pytest.mark.parametrize('T', [1, 2, 5, 8, 13])
+@pytest.mark.parametrize('dropout', [False, True])
+def test_float64_attention_reference_matches_the_oracle(T, dropout):
+    """remix_attention_ref (the reference of tests/test_gpu_remix_attention.py) against the oracle's _apply_attention fed q, k, v
+    and Rk directly (identity projections): same output, same gradients, and the gradients rebuilt from dS the way the kernels
+    and the trainer's GEMMs split them (content part of dq from dS K, position part and dRk from ds_dist)."""
+    B, H, D = 2, 2, 64
+    g = torch.Generator().manual_seed(100 + T)
+    q, k, v = (torch.randn(B, H, T, D, dtype=torch.float64, generator=g) for _ in range(3))
+    rk = torch.randn(T, H, D, dtype=torch.float64, generator=g)
+    u, vb = (0.3 * torch.randn(H, D, dtype=torch.float64, generator=g) for _ in range(2))
+    mask = (torch.rand(B, H, T, T, generator=g) > 0.3).double() / 0.7 if dropout else None
+    dout = torch.randn(B, H, T, D, dtype=torch.float64, generator=g)
+
+    att = bert.MemMultiHeadRelativeAttentionKV(H, H * D, D, mem_len=0, r_mask=False).double()
+    with torch.no_grad():
+        for lin in (att.q_wgt, att.k_wgt, att.v_wgt, att.r_attn):
+            lin.weight.copy_(torch.eye(H * D, dtype=torch.float64))
+            lin.bias.zero_()
+    att.drop_att = bert_train.FixedMask()
+    att.drop_att.mask = mask
+    leaves = [t.clone().requires_grad_(True) for t in (q, k, v, rk, u, vb)]
+    lq, lk, lv, lrk, lu, lvb = leaves
+    flat = lambda t: t.permute(0, 2, 1, 3).reshape(B, T, H * D)
+    want = att._apply_attention(flat(lq), flat(lk), flat(lv), r=lrk.flip(0).reshape(T, H * D), g_u=lu[:, None], g_v=lvb[:, None])
+    want.backward(flat(dout))
+    want_grads = [t.grad for t in leaves]
+
+    leaves = [t.clone().requires_grad_(True) for t in (q, k, v, rk, u, vb)]
+    out, lse, raw = remix_attention_ref.remix_attention(*leaves, drop_mask=mask)
+    raw.retain_grad()
+    assert torch.allclose(flat(out), want, rtol=1e-12, atol=1e-12)
+    assert torch.allclose(lse, torch.logsumexp(raw / 8, -1))
+    out.backward(dout)
+    for got, ref in zip([t.grad for t in leaves], want_grads):
+        assert torch.allclose(got, ref, rtol=1e-10, atol=1e-12)
+
+    dS = raw.grad
+    dist = remix_attention_ref.ds_to_dist(dS)
+    assert (dist[:, 0, :, 1:] == 0).all()
+    qv = (q + vb[:, None]).permute(0, 2, 1, 3)
+    dq_pos, dvb, drk = remix_attention_ref.position_grads(dist, rk, qv)
+    dq_content = dS @ k
+    gq, gk, gv, grk, gu, gvb = want_grads
+    assert torch.allclose(dq_content + dq_pos.permute(0, 2, 1, 3), gq, rtol=1e-10, atol=1e-12)
+    assert torch.allclose(dq_content.sum((0, 2)), gu, rtol=1e-10, atol=1e-12)
+    assert torch.allclose(dvb, gvb, rtol=1e-10, atol=1e-12)
+    assert torch.allclose(drk, grk, rtol=1e-10, atol=1e-12)
+    assert torch.allclose(dS.transpose(-1, -2) @ (q + u[:, None]), gk, rtol=1e-10, atol=1e-12)
 
 
 def small_model(pad_idx, V=40):
