@@ -57,6 +57,9 @@ SYMBOLS = {
     'dmg_select_hidden': (c_i32, [c_vp, c_vp, c_i32]),
     'dmg_mem_count': (c_i32, [c_vp]),
     'dmg_forward': (c_i32, [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp]),
+    'dmg_forward_varlen': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp]),
+    'dmg_predict_mask_batch': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, C.POINTER(VocabLayout),
+                                       C.POINTER(SamplerParams), c_vp]),
     'dmg_get_hidden': (c_i32, [c_vp, c_i32, c_vp, c_vp]),
     'dmg_sampler_init': (c_i32, [c_vp, C.POINTER(VocabLayout), C.POINTER(SamplerParams), c_vp, c_vp, c_i32]),
     'dmg_generate': (c_i32, [c_vp, c_i32, c_vp, c_vp]),
@@ -99,6 +102,7 @@ SYMBOLS = {
                                    c_i32, c_i32, c_f32, c_u32, c_vp, c_vp, c_vp]),
     'dmg_attn_train_bwd': (c_i32, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32,
                                    c_i32, c_i32, c_i32, c_f32, c_u32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'dmg_attn_bert_varlen': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp]),
     'dmg_attn_bert_train_fwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32, c_vp]),
     'dmg_attn_bert_train_bwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32,
                                         c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),

@@ -30,7 +30,9 @@ __host__ __device__ constexpr int gen_smem_floats() {
          (BERT ? 63 * GLD : 0) /*R upper*/ + GQ * (GK + 1) /*P*/;
 }
 
-template <class T, bool BERT>
+// VARLEN (BERT only): sequence b has a.lens[b] tokens in rows [b*a.T, b*a.T + a.lens[b]) of the padded layout; query tiles past
+// its end do nothing (the caller zeroes those output rows)
+template <class T, bool BERT, bool VARLEN>
 __global__ void __launch_bounds__(128) attn_general_kernel(AttnGeneralArgs a) {
   extern __shared__ float sm[];
   float* Qu = sm;
@@ -45,7 +47,8 @@ __global__ void __launch_bounds__(128) attn_general_kernel(AttnGeneralArgs a) {
   pdl_launch_dependents();
   pdl_wait();
   const int i0 = blockIdx.x * GQ, h = blockIdx.y, b = blockIdx.z;
-  const int T_len = a.T, H = a.H, HD = H * 64, M = a.M;
+  const int T_len = VARLEN ? a.lens[b] : a.T, H = a.H, HD = H * 64, M = a.M;
+  if (VARLEN && i0 >= T_len) return;
   const int m = a.mem_count, S = m + T_len;
   const T* kring = (const T*)a.kring;
   const T* vring = (const T*)a.vring;
@@ -56,7 +59,7 @@ __global__ void __launch_bounds__(128) attn_general_kernel(AttnGeneralArgs a) {
     const int r = idx >> 4, c4 = (idx & 15) * 4;
     const int i = i0 + r;
     float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (i < T_len) q = *(const float4*)(a.qkv + ((size_t)b * T_len + i) * 3 * HD + h * 64 + c4);
+    if (i < T_len) q = *(const float4*)(a.qkv + ((size_t)b * a.T + i) * 3 * HD + h * 64 + c4);
     const float4 uu = *(const float4*)(a.u + h * 64 + c4), vv = *(const float4*)(a.v + h * 64 + c4);
     if (r < GQ) *(float4*)(Qu + r * GLD + c4) = make_float4(q.x + uu.x, q.y + uu.y, q.z + uu.z, q.w + uu.w);
     *(float4*)(Qv + r * GLD + c4) = make_float4(q.x + vv.x, q.y + vv.y, q.z + vv.z, q.w + vv.w);
@@ -89,7 +92,7 @@ __global__ void __launch_bounds__(128) attn_general_kernel(AttnGeneralArgs a) {
             vv[e] = to_f32(vring[off + e]);
           }
         } else {
-          const float* row = a.qkv + ((size_t)b * T_len + (j - m)) * 3 * HD + h * 64 + c16;
+          const float* row = a.qkv + ((size_t)b * a.T + (j - m)) * 3 * HD + h * 64 + c16;
 #pragma unroll
           for (int e = 0; e < 16; e++) {
             kv[e] = row[HD + e];
@@ -201,28 +204,32 @@ __global__ void __launch_bounds__(128) attn_general_kernel(AttnGeneralArgs a) {
   }
   if (i < T_len) {
     const float inv = l_run > 0.f ? 1.f / l_run : 0.f;
-    T* out = (T*)a.out + ((size_t)b * T_len + i) * HD + h * 64 + kg * 16;
+    T* out = (T*)a.out + ((size_t)b * a.T + i) * HD + h * 64 + kg * 16;
 #pragma unroll
     for (int e = 0; e < 16; e++) out[e] = from_f32<T>(o[e] * inv);
   }
 }
 
-template <class T, bool BERT>
+template <class T, bool BERT, bool VARLEN = false>
 static int launch_general(const AttnGeneralArgs& a, cudaStream_t st) {
   const int smem = gen_smem_floats<BERT>() * 4;
   static bool configured = false;
   if (!configured) {
-    DMG_CUDA_OK(cudaFuncSetAttribute(attn_general_kernel<T, BERT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_general_kernel<T, BERT, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     configured = true;
   }
   dim3 grid((a.T + GQ - 1) / GQ, a.H, a.B);
-  return launch_k(attn_general_kernel<T, BERT>, grid, dim3(128), smem, st, 1, a);
+  return launch_k(attn_general_kernel<T, BERT, VARLEN>, grid, dim3(128), smem, st, 1, a);
 }
 
 template <class T>
 int attn_general(const AttnGeneralArgs& a, cudaStream_t st) {
   DMG_CHECK(a.win >= 1, "attn_general: window size must be >= 1");
   if (a.B <= 0 || a.T <= 0) return 0;
+  if (a.lens) {
+    DMG_CHECK(a.bert && a.M == 0, "attn_general: per-sequence lengths need the memory-less BERT encoder");
+    return launch_general<T, true, true>(a, st);
+  }
   return a.bert ? launch_general<T, true>(a, st) : launch_general<T, false>(a, st);
 }
 template int attn_general<float>(const AttnGeneralArgs&, cudaStream_t);

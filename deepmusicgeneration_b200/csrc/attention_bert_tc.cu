@@ -50,7 +50,11 @@ static_assert(BT_SOFT_WARPS * 32 * BT_LINE16 <= BT_SOFT_WARPS * 32 * BT_STRIP_LD
 // operands): the thread's two 64-column windows overlap in 32 columns, so it reads 96 distinct columns once (three tcgen05.ld.x32
 // instead of four), stores 12 instead of 32 16-byte chunks and reads its 64 scores back as 33 aligned words + funnel shifts - 40 % of
 // the shared-memory wavefronts of the fp32 line (the kernel sits on the shared-memory pipe, profiles/r1g_attn_bert_tc_ncu.txt).
-template <bool H16>
+//
+// VARLEN: a padded batch of sequences of their own lengths (a.lens, each >= 128) walked through the host-built item list a.items; every
+// item is computed as it would be with T = its sequence's length, at row stride a.T.  Keys past the end are masked by a select and
+// the V rows there are zeroed in shared memory, so the padding rows may hold anything (NaN included).
+template <bool H16, bool VARLEN>
 __global__ void __launch_bounds__(BT_THREADS, 1)
 attn_bert_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmR, const BertTcArgs a) {
   extern __shared__ __align__(1024) uint8_t bt_smem_raw[];
@@ -59,8 +63,8 @@ attn_bert_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
   uint32_t* tmem_holder = (uint32_t*)(bar + Q_COUNT);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int NT = (a.T + 127) / 128;                  // a ragged last tile: keys >= T are masked, rows >= T are not stored
-  const int n_items = a.B * a.H * NT;               // every query tile sees all NT key tiles: uniform work
+  const int NT_all = (a.T + 127) / 128;              // a ragged last tile: keys >= T are masked, rows >= T are not stored
+  const int n_items = VARLEN ? a.n_items : a.B * a.H * NT_all;   // every query tile sees all NT key tiles: uniform work
   const int HD = a.H * 64;
 
   if (warp == BT_SOFT_WARPS && lane == 0) {
@@ -81,13 +85,13 @@ attn_bert_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     asm volatile("setmaxnreg.dec.sync.aligned.u32 64;");
     if (warp == BT_SOFT_WARPS) {
       // =========================================== TMA producer ===========================================
-      if (lane == 0) bt_producer<H16 ? 2 : 1>(smem, bar, tmX, tmR, a, NT, n_items);
+      if (lane == 0) bt_producer<H16 ? 2 : 1, VARLEN>(smem, bar, tmX, tmR, a, NT_all, n_items);
     } else if (warp == BT_SOFT_WARPS + 1) {
       // =========================================== MMA issuer ===========================================
-      bt_mma_issuer<H16 ? 2 : 1>(smem, bar, tmem_base, NT, n_items, a.H, a.dbg);   // the whole warp: uniform control flow
+      bt_mma_issuer<H16 ? 2 : 1, VARLEN>(smem, bar, tmem_base, NT_all, n_items, a, a.dbg);   // the whole warp: uniform control flow
     } else {
       // =========================================== transform warps ===========================================
-      bt_transform(smem, bar, a, NT, n_items, threadIdx.x - 32 * (BT_SOFT_WARPS + 2));
+      bt_transform<VARLEN>(smem, bar, a, NT_all, n_items, threadIdx.x - 32 * (BT_SOFT_WARPS + 2));
     }
   } else {
     // =========================================== softmax warps ===========================================
@@ -99,11 +103,19 @@ attn_bert_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     const float c = a.scale * BT_LOG2E;
     uint8_t* prow = smem + BO_P + hf * BT16K + (r >> 3) * 1024 + (r & 7) * 128;
 
-    int kit = 0;                                    // items this CTA has finished: the barriers count on across items
+    int kit = 0, gsum = 0;                          // items this CTA has finished: the barriers count on across items
     for (int item = blockIdx.x; item < n_items; item += gridDim.x, kit++) {
-    const BtItem wi = bt_item(item, NT, a.H);
-    const int b = wi.b, h = wi.h, it = wi.it, i0 = it * 128, row = i0 + r;
-    const int g0 = kit * NT;
+    int b, h, it, T, NT;
+    if constexpr (VARLEN) {
+      const BtVarItem wi = bt_var_item(a, item);
+      b = wi.b; h = wi.h; it = wi.it; T = wi.T; NT = wi.NT;
+    } else {
+      const BtItem wi = bt_item(item, NT_all, a.H);
+      b = wi.b; h = wi.h; it = wi.it; T = a.T; NT = NT_all;
+    }
+    const int i0 = it * 128, row = i0 + r;
+    const int g0 = VARLEN ? gsum : kit * NT;
+    if constexpr (VARLEN) gsum += NT;
 
     float o[64];
 #pragma unroll
@@ -214,8 +226,8 @@ attn_bert_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
 
       }
 
-      if (n == NT - 1 && (a.T & 127)) {              // ragged last tile: keys past the sequence end
-        const int jlim = a.T - n * 128 - 64 * hf;
+      if (n == NT - 1 && (T & 127)) {                // ragged last tile: keys past the sequence end
+        const int jlim = T - n * 128 - 64 * hf;
 #pragma unroll
         for (int jj = 0; jj < 64; jj++) s[jj] = jj < jlim ? s[jj] : -INFINITY;
       }
@@ -302,7 +314,7 @@ attn_bert_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     wr_s[0] = m_run;
     wr_s[1] = l_run;
     asm volatile("bar.sync 1, 256;" ::: "memory");
-    if (row < a.T) {
+    if (row < T) {
       const float m1 = rd_s[0], l1 = rd_s[1];
       const float m = fmaxf(m_run, m1);
       const float w0 = ex2_fast((m_run - m) * c), w1 = ex2_fast((m1 - m) * c);
@@ -340,8 +352,8 @@ int attn_bert_tc(const bf16* qkv, const bf16* rd, int Dcap, const float* u, cons
                  int fp32_strip, cudaStream_t st) {
   static bool configured = false;
   if (!configured) {
-    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bert_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BT_SMEM));
-    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bert_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BT_SMEM));
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bert_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BT_SMEM));
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bert_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BT_SMEM));
     configured = true;
   }
   const int HD = H * 64;
@@ -351,6 +363,7 @@ int attn_bert_tc(const bf16* qkv, const bf16* rd, int Dcap, const float* u, cons
   BertTcArgs a;
   a.u = u; a.v = v; a.out = out; a.B = B; a.T = T; a.H = H; a.Dcap = Dcap; a.scale = scale;
   a.dbg = nullptr;
+  a.lens = nullptr; a.items = nullptr; a.n_items = 0;
   // persistent: one CTA per SM (shared memory and all 512 TMEM columns allow one), items dealt round-robin.  DMG_BERT_TC_ONE_ITEM=1
   // (measurement only) launches one CTA per item, the schedule of rounds 1 and 2.
   static int num_sms = 0, one_item = -1;
@@ -370,9 +383,9 @@ int attn_bert_tc(const bf16* qkv, const bf16* rd, int Dcap, const float* u, cons
     if (!tl_dev) DMG_CUDA_OK(cudaMalloc(&tl_dev, 2048 * sizeof(unsigned long long)));
     DMG_CUDA_OK(cudaMemsetAsync(tl_dev, 0, 2048 * sizeof(unsigned long long), st));
     a.dbg = tl_dev;
-    const int rc = fp32_strip ? launch_k(attn_bert_tc_kernel<false>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
+    const int rc = fp32_strip ? launch_k(attn_bert_tc_kernel<false, false>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
                                          *(const CUtensorMap*)tr->bytes, a)
-                              : launch_k(attn_bert_tc_kernel<true>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
+                              : launch_k(attn_bert_tc_kernel<true, false>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
                                          *(const CUtensorMap*)tr->bytes, a);
     if (rc) return rc;
     static unsigned long long host[2048];
@@ -383,9 +396,40 @@ int attn_bert_tc(const bf16* qkv, const bf16* rd, int Dcap, const float* u, cons
     return 0;
   }
   if (fp32_strip)
-    return launch_k(attn_bert_tc_kernel<false>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
+    return launch_k(attn_bert_tc_kernel<false, false>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
                     *(const CUtensorMap*)tr->bytes, a);
-  return launch_k(attn_bert_tc_kernel<true>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
+  return launch_k(attn_bert_tc_kernel<true, false>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
+                  *(const CUtensorMap*)tr->bytes, a);
+}
+
+// Padded batch of B sequences (qkv rows b*T_max + i): the n_items work items items_dev[] (see BertTcArgs) of the sequences with
+// lens_dev[b] >= 128.  Writes only rows < lens[b].
+int attn_bert_tc_varlen(const bf16* qkv, const bf16* rd, int Dcap, const float* u, const float* v, bf16* out, const int* lens_dev,
+                        const int* items_dev, int n_items, int B, int T_max, int H, float scale, int fp32_strip, cudaStream_t st) {
+  DMG_CHECK(T_max >= 128 && Dcap >= T_max && H <= 256 && B <= 32768, "attn_bert_tc_varlen: T_max %d / H %d / B %d outside the kernel's range", T_max, H, B);
+  if (n_items <= 0) return 0;
+  static bool configured = false;
+  if (!configured) {
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bert_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BT_SMEM));
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bert_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BT_SMEM));
+    configured = true;
+  }
+  const int HD = H * 64;
+  const TensorMap2D *tx = nullptr, *tr = nullptr;
+  if (train_get_tmap(qkv, 3 * HD, (long long)B * T_max, 3 * HD, 128, &tx)) return -1;
+  if (train_get_tmap(rd, 64, (long long)H * Dcap, 64, 128, &tr)) return -1;
+  BertTcArgs a;
+  a.u = u; a.v = v; a.out = out; a.B = B; a.T = T_max; a.H = H; a.Dcap = Dcap; a.scale = scale;
+  a.dbg = nullptr;
+  a.lens = lens_dev; a.items = items_dev; a.n_items = n_items;
+  int dev = 0, num_sms = 0;
+  DMG_CUDA_OK(cudaGetDevice(&dev));
+  DMG_CUDA_OK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
+  const dim3 grid(n_items < num_sms ? n_items : num_sms);
+  if (fp32_strip)
+    return launch_k(attn_bert_tc_kernel<false, true>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
+                    *(const CUtensorMap*)tr->bytes, a);
+  return launch_k(attn_bert_tc_kernel<true, true>, grid, dim3(BT_THREADS), (size_t)BT_SMEM, st, 1, *(const CUtensorMap*)tx->bytes,
                   *(const CUtensorMap*)tr->bytes, a);
 }
 

@@ -48,6 +48,11 @@ struct BertTcArgs {
   int B, T, H, Dcap;
   float scale;
   unsigned long long* dbg;          // measurement only (DMG_BERT_TC_TIMELINE): %globaltimer marks of CTA 0, nullptr in the product path
+  // per-sequence lengths (the VARLEN kernels): T is the padded length (row stride of a sequence), sequence b has lens[b] >= 128 tokens,
+  // items[0, n_items) lists the work items as (b << 16) | (h << 8) | query tile
+  const int* lens;
+  const int* items;
+  int n_items;
 };
 // timeline slots: softmax warp 0 / 4 at [256 hf + 48 item + 5 tile + mark], issuer at [512 + 48 item + 6 tile + mark], transform warps at
 // [768 + 4 item + mark], producer at [832 + 4 item + mark]; the first four items of CTA 0
@@ -95,18 +100,35 @@ __device__ __forceinline__ BtItem bt_item(int item, int nT, int H) {
   const int bh = item / nT;
   return {bh / H, bh % H, item % nT};
 }
+// VARLEN: the item list and the sequence's own length T / tile count NT.  Every role keeps the running sums of NT and NT + 3 over the
+// items it has walked (the barrier use counts g0 / r0 of the fixed-length kernel, k * NT and k * (NT + 3)).
+struct BtVarItem {
+  int b, h, it, T, NT;
+};
+__device__ __forceinline__ BtVarItem bt_var_item(const BertTcArgs& a, int item) {
+  const int e = __ldg(a.items + item), b = e >> 16, T = __ldg(a.lens + b);
+  return {b, (e >> 8) & 255, e & 255, T, (T + 127) / 128};
+}
 
 // TMA producer (one thread): per item q / q_next, then per key tile K, the position-key blocks and V
-template <int VS>
+template <int VS, bool VARLEN>
 __device__ __forceinline__ void bt_producer(uint8_t* smem, uint64_t* bar, const CUtensorMap& tmX, const CUtensorMap& tmR, const BertTcArgs& a,
-                                            int NT, int n_items) {
+                                            int NT_all, int n_items) {
   const int HD = a.H * 64;
   pdl_wait();                                  // q | k | v come from the predecessor kernel (the QKV GEMM)
-  int k = 0;
+  int k = 0, gsum = 0, rsum = 0;
   for (int item = blockIdx.x; item < n_items; item += gridDim.x, k++) {
-    const BtItem w = bt_item(item, NT, a.H);
-    const int b = w.b, h = w.h, it = w.it, i0 = it * 128;
-    const int g0 = k * NT, r0 = k * (NT + 3);  // tiles / slot loads of the earlier items
+    int b, h, it, T, NT;
+    if constexpr (VARLEN) {
+      const BtVarItem w = bt_var_item(a, item);
+      b = w.b; h = w.h; it = w.it; T = w.T; NT = w.NT;
+    } else {
+      const BtItem w = bt_item(item, NT_all, a.H);
+      b = w.b; h = w.h; it = w.it; T = a.T; NT = NT_all;
+    }
+    const int i0 = it * 128;
+    const int g0 = VARLEN ? gsum : k * NT, r0 = VARLEN ? rsum : k * (NT + 3);  // tiles / slot loads of the earlier items
+    if constexpr (VARLEN) { gsum += NT; rsum += NT + 3; }
     auto slot_wait = [&](int j) {               // the slot of load j of this item, once its previous tenant has been released
       const int gl = r0 + j, s = gl & 1;
       bt_wait(&bar[Q_REMPTY0 + s], ((gl >> 1) & 1) ^ 1);
@@ -121,7 +143,7 @@ __device__ __forceinline__ void bt_producer(uint8_t* smem, uint64_t* bar, const 
     auto load_r = [&](int j) {                  // load 0 = upper block of tile 0; load j >= 1 = lower block of tile j-1
       // line 1: Rk rows (it-j)*128 ...; line 3: Rk rows T + 1 + (it-j)*128 ... (distance T + 1 + i - j; rows below 0 or past T - 1
       // only meet masked keys or the zero pad)
-      const int row = j <= it ? (it - j) * 128 : a.T + 1 + (it - j) * 128;
+      const int row = j <= it ? (it - j) * 128 : T + 1 + (it - j) * 128;
       const int s = slot_wait(2 + j);
       mbar_expect_tx(&bar[Q_RFULL0 + s], BT16K);
       tma_load_2d(smem + BO_R + s * BT16K, &tmR, 0, h * a.Dcap + row, &bar[Q_RFULL0 + s]);
@@ -165,16 +187,24 @@ __device__ __forceinline__ void bt_producer(uint8_t* smem, uint64_t* bar, const 
 // swizzled layout.  Eight consecutive threads take the eight 16-byte chunks of one row (128 contiguous bytes: no bank conflicts); a
 // thread's rows are 8 apart, so its physical chunk maps to the same logical columns in all of them and it needs one 8-wide slice of
 // u and v only (requested before the wait for q).
-__device__ __forceinline__ void bt_transform(uint8_t* smem, uint64_t* bar, const BertTcArgs& a, int NT, int n_items, int tid) {
+template <bool VARLEN>
+__device__ __forceinline__ void bt_transform(uint8_t* smem, uint64_t* bar, const BertTcArgs& a, int NT_all, int n_items, int tid) {
   const int pc = tid & 7, rb = tid >> 3;
   const int col = 8 * (pc ^ rb);
-  int k = 0;
+  int k = 0, rsum = 0;
   for (int item = blockIdx.x; item < n_items; item += gridDim.x, k++) {
-    const int h = (item / NT) % a.H;
+    int h, NT;
+    if constexpr (VARLEN) {
+      const BtVarItem w = bt_var_item(a, item);
+      h = w.h; NT = w.NT;
+    } else {
+      h = (item / NT_all) % a.H; NT = NT_all;
+    }
     const float4 ua = __ldg((const float4*)(a.u + h * 64 + col)), ub = __ldg((const float4*)(a.u + h * 64 + col + 4));
     const float4 va = __ldg((const float4*)(a.v + h * 64 + col)), vb = __ldg((const float4*)(a.v + h * 64 + col + 4));
     const float uu[8] = {ua.x, ua.y, ua.z, ua.w, ub.x, ub.y, ub.z, ub.w}, vv8[8] = {va.x, va.y, va.z, va.w, vb.x, vb.y, vb.z, vb.w};
-    const int g0 = k * (NT + 3), g1 = g0 + 1;
+    const int g0 = VARLEN ? rsum : k * (NT + 3), g1 = g0 + 1;
+    if constexpr (VARLEN) rsum += NT + 3;
     // the slots were released by the last S MMA of the previous item: nothing reads the three operand tiles any more
     bt_wait(&bar[Q_QFULL], k & 1);
     if (tid == 0) bt_mark(a.dbg, 768 + 4 * k, k);
@@ -226,8 +256,8 @@ __device__ __forceinline__ void bt_transform(uint8_t* smem, uint64_t* bar, const
 // `if (lane == 0)` branch the same loop cost ~400 instructions per tile (per MMA a vector-to-uniform move loop, elect, predicate
 // shuffles, descriptor rebuild) = 2 us of one thread's time - and THAT was the tile period of the kernel, with the tensor pipe
 // 24 % busy and the softmax warps waiting for scores (profiles/r2h_attn_bert_tc_timeline_single_v.txt).
-template <int VS>
-__device__ __forceinline__ void bt_mma_issuer(uint8_t* smem, uint64_t* bar, uint32_t tmem_base, int NT, int n_items, int H,
+template <int VS, bool VARLEN>
+__device__ __forceinline__ void bt_mma_issuer(uint8_t* smem, uint64_t* bar, uint32_t tmem_base, int NT_all, int n_items, const BertTcArgs& a,
                                               unsigned long long* dbg) {
   constexpr uint32_t idesc_s = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
   constexpr uint32_t idesc_pv = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((64u >> 3) << 17) | ((128u >> 4) << 24);
@@ -236,9 +266,17 @@ __device__ __forceinline__ void bt_mma_issuer(uint8_t* smem, uint64_t* bar, uint
                  d_k = bt_desc_k(smem_u32(smem + BO_K)), d_r0 = bt_desc_k(smem_u32(smem + BO_R)), d_r1 = bt_desc_k(smem_u32(smem + BO_R + BT16K)),
                  d_p0 = bt_desc_k(smem_u32(smem + BO_P)), d_p1 = bt_desc_k(smem_u32(smem + BO_P + BT16K)),
                  d_v0 = bt_desc_mn(smem_u32(smem + BO_V)), d_v1 = bt_desc_mn(smem_u32(smem + (VS == 2 ? BO_V2 : BO_V)));
-  auto issue_pv = [&](int g, int ms, int k) {  // g: tile count over all items of this CTA; ms, k: timeline slot / item
+  // g: tile count over all items of this CTA; ms, k: timeline slot / item; vzero (VARLEN): V rows from vzero on lie past the sequence end
+  // and are zeroed before the MMA reads them (the probabilities there are 0, but 0 * NaN is not)
+  auto issue_pv = [&](int g, int ms, int k, int vzero) {
     const int vs = g % VS, vu = g / VS;
     bt_wait(&bar[vs ? Q_VFULL1 : Q_VFULL], vu & 1);
+    if (VARLEN && vzero < 128) {
+      uint8_t* vt = smem + (vs ? BO_V2 : BO_V);
+      for (int c = vzero * 8 + (int)(threadIdx.x & 31); c < 128 * 8; c += 32) *(uint4*)(vt + 16 * c) = make_uint4(0u, 0u, 0u, 0u);
+      bt_fence_async();
+      __syncwarp();
+    }
 #pragma unroll
     for (int hf = 0; hf < 2; hf++) {
       bt_wait(&bar[Q_PFULL0 + hf], g & 1);
@@ -258,10 +296,17 @@ __device__ __forceinline__ void bt_mma_issuer(uint8_t* smem, uint64_t* bar, uint
       __syncwarp();
     }
   };
-  int k = 0;
+  int k = 0, gsum = 0, rsum = 0;
   for (int item = blockIdx.x; item < n_items; item += gridDim.x, k++) {
-    const int it = item % NT;
-    const int g0 = k * NT, r0 = k * (NT + 3) + 2;
+    int it, NT, vzero = 128;
+    if constexpr (VARLEN) {
+      const BtVarItem w = bt_var_item(a, item);
+      it = w.it; NT = w.NT; vzero = w.T - (NT - 1) * 128;
+    } else {
+      it = item % NT_all; NT = NT_all;
+    }
+    const int g0 = VARLEN ? gsum : k * NT, r0 = (VARLEN ? rsum : k * (NT + 3)) + 2;
+    if constexpr (VARLEN) { gsum += NT; rsum += NT + 3; }
     bt_wait(&bar[Q_QREADY], k & 1);
     for (int n = 0; n < NT; n++) {
       const int g = g0 + n, gu = r0 + n, gl = gu + 1;                   // load gu = this tile's upper block, gl = its lower block
@@ -290,9 +335,9 @@ __device__ __forceinline__ void bt_mma_issuer(uint8_t* smem, uint64_t* bar, uint
         bt_mark(dbg, 512 + 48 * k + 6 * n, k);
       }
       __syncwarp();
-      if (n > 0) issue_pv(g - 1, 512 + 48 * k + 6 * (n - 1), k);
+      if (n > 0) issue_pv(g - 1, 512 + 48 * k + 6 * (n - 1), k, 128);
     }
-    issue_pv(g0 + NT - 1, 512 + 48 * k + 6 * (NT - 1), k);
+    issue_pv(g0 + NT - 1, 512 + 48 * k + 6 * (NT - 1), k, vzero);
   }
 }
 

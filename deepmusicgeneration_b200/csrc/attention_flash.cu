@@ -107,11 +107,16 @@ struct FlashArgs {
   bf16* out;           // [B*T, HD]
   int B, T, H;
   float scale;
+  // per-sequence lengths (BERT): block row bh / H walks sequence seqs[bh / H], whose lens[.] tokens are rows [b*T, b*T + len) of the
+  // padded layout (T = the padded length); nTg 64-row query tiles per (sequence, head), tiles past the sequence end do nothing
+  const int* lens;
+  const int* seqs;
+  int nTg;
 };
 
 constexpr int FL_SMEM = 4 * TILE_BYTES /*Q, Qnext, K, V*/ + 4 * TILE_BYTES /*two Rk windows*/ + 4 * 16 * FL_SKEW_LD * 4;
 
-template <bool BERT>
+template <bool BERT, bool VARLEN>
 __global__ void __launch_bounds__(128) attn_flash_kernel(const FlashArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
   uint8_t* sQ = smem;
@@ -127,17 +132,20 @@ __global__ void __launch_bounds__(128) attn_flash_kernel(const FlashArgs a) {
   pdl_launch_dependents();
   pdl_wait();
 
-  const int nT = (a.T + 63) / 64, T64 = nT * 64;
-  const int it = nT - 1 - (blockIdx.x % nT);
-  const int bh = blockIdx.x / nT, b = bh / a.H, h = bh % a.H;
+  const int nTb = VARLEN ? a.nTg : (a.T + 63) / 64;   // query tiles per block row
+  const int it = nTb - 1 - (blockIdx.x % nTb);
+  const int bh = blockIdx.x / nTb, b = VARLEN ? a.seqs[bh / a.H] : bh / a.H, h = bh % a.H;
+  const int T = VARLEN ? a.lens[b] : a.T;           // this sequence's length
+  const int nT = (T + 63) / 64, T64 = nT * 64;
+  if (VARLEN && it >= nT) return;
   const int i0 = it * 64, HD = a.H * 64;
   const long long ldx = 3 * HD;
   const bf16* qkv_b = a.qkv + (long long)b * a.T * ldx + h * 64;     // q of (b, h); k at +HD, v at +2*HD
   const bf16* rk_h = a.rk + (long long)h * a.rk_hs;
-  const int shift3 = a.T + 1 - T64;                 // line-3 table: Rk3[x] = Rk[x + shift3], x = T64 + i - j
+  const int shift3 = T + 1 - T64;                   // line-3 table: Rk3[x] = Rk[x + shift3], x = T64 + i - j
 
-  tile_load_guard(sQ, qkv_b, ldx, i0, a.T, tid);
-  if (BERT) tile_load_guard(sQn, qkv_b, ldx, i0 + 1, a.T, tid);
+  tile_load_guard(sQ, qkv_b, ldx, i0, T, tid);
+  if (BERT) tile_load_guard(sQn, qkv_b, ldx, i0 + 1, T, tid);
   cp_async_commit();
   cp_async_wait<0>();
   __syncthreads();
@@ -158,8 +166,8 @@ __global__ void __launch_bounds__(128) attn_flash_kernel(const FlashArgs a) {
     const int j0 = jt * 64;
     const bool use1 = jt <= it, use3 = BERT && jt >= it;
     __syncthreads();
-    tile_load_guard(sK, qkv_b + HD, ldx, j0, a.T, tid);
-    tile_load_guard(sV, qkv_b + 2 * HD, ldx, j0, a.T, tid);
+    tile_load_guard(sK, qkv_b + HD, ldx, j0, T, tid);
+    tile_load_guard(sV, qkv_b + 2 * HD, ldx, j0, T, tid);
     if (use1) {                                      // distances D0-64 .. D0+63, D0 = i0 - j0 >= 0
       const int D0 = i0 - j0;
       tile_load_guard(sR, rk_h, a.rk_ld, D0 - 64, a.rk_rows, tid);
@@ -191,7 +199,7 @@ __global__ void __launch_bounds__(128) attn_flash_kernel(const FlashArgs a) {
         if (j <= i) { if (use1) bdv = bd1[nt][e]; }
         else if (BERT && j > i + 1) { if (use3) bdv = bd3[nt][e]; }
         float x = s[nt][e] + bdv;
-        const bool vis = BERT ? (j < a.T) : (j <= i);
+        const bool vis = BERT ? (j < T) : (j <= i);
         if (!vis) x = -INFINITY;
         s[nt][e] = x;
         mx[e >> 1] = fmaxf(mx[e >> 1], x);
@@ -239,14 +247,18 @@ __global__ void __launch_bounds__(128) attn_flash_kernel(const FlashArgs a) {
       }
     }
   }
+  // VARLEN: the sequence index is read again rather than kept in a register across the key loop (52 instead of 12 bytes of spill
+  // stores with it kept)
+  int bo = b;
+  if constexpr (VARLEN) bo = *(volatile const int*)(a.seqs + blockIdx.x / nTb / a.H);
 #pragma unroll
   for (int r = 0; r < 2; r++) {
     float l = l_run[r];
     l += __shfl_xor_sync(0xffffffffu, l, 1);
     l += __shfl_xor_sync(0xffffffffu, l, 2);
-    if (row_g[r] >= a.T) continue;
+    if (row_g[r] >= T) continue;
     const float inv = l > 0.f ? 1.f / l : 0.f;
-    bf16* orow = a.out + ((long long)b * a.T + row_g[r]) * HD + h * 64;
+    bf16* orow = a.out + ((long long)bo * a.T + row_g[r]) * HD + h * 64;
 #pragma unroll
     for (int nt = 0; nt < 8; nt++)
       *(uint32_t*)(orow + 8 * nt + 2 * t) = pack_bf16x2(o[nt][2 * r] * inv, o[nt][2 * r + 1] * inv);
@@ -262,15 +274,35 @@ int attn_flash(const bf16* qkv, const bf16* rd, int Dcap, const float* u, const 
   FlashArgs a;
   a.qkv = qkv; a.rk = rd; a.rk_hs = (long long)Dcap * 64; a.rk_ld = 64; a.rk_rows = Dcap; a.u = u; a.v = v; a.out = out;
   a.B = B; a.T = T; a.H = H; a.scale = scale;
+  a.lens = nullptr; a.seqs = nullptr; a.nTg = 0;
   static bool configured = false;
   if (!configured) {
-    DMG_CUDA_OK(cudaFuncSetAttribute(attn_flash_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FL_SMEM));
-    DMG_CUDA_OK(cudaFuncSetAttribute(attn_flash_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FL_SMEM));
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_flash_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FL_SMEM));
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_flash_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FL_SMEM));
     configured = true;
   }
   const dim3 grid(B * H * ((T + 63) / 64));
-  if (bert) return launch_k(attn_flash_kernel<true>, grid, dim3(128), (size_t)FL_SMEM, st, 1, a);
-  return launch_k(attn_flash_kernel<false>, grid, dim3(128), (size_t)FL_SMEM, st, 1, a);
+  if (bert) return launch_k(attn_flash_kernel<true, false>, grid, dim3(128), (size_t)FL_SMEM, st, 1, a);
+  return launch_k(attn_flash_kernel<false, false>, grid, dim3(128), (size_t)FL_SMEM, st, 1, a);
+}
+
+// BERT encoder over the n_seqs sequences seqs_dev[] of a padded batch (qkv rows b*T_max + i, lengths lens_dev[b]); max_len = the longest
+// of them (sizes the grid).  Writes only rows < lens[b].
+int attn_flash_varlen(const bf16* qkv, const bf16* rd, int Dcap, const float* u, const float* v, bf16* out, const int* lens_dev,
+                      const int* seqs_dev, int n_seqs, int max_len, int T_max, int H, float scale, cudaStream_t st) {
+  DMG_CHECK(max_len >= 1 && max_len <= T_max && Dcap >= max_len, "attn_flash_varlen: length %d outside [1, T_max=%d] or past the rel-pos cache (%d)",
+            max_len, T_max, Dcap);
+  if (n_seqs <= 0) return 0;
+  FlashArgs a;
+  a.qkv = qkv; a.rk = rd; a.rk_hs = (long long)Dcap * 64; a.rk_ld = 64; a.rk_rows = Dcap; a.u = u; a.v = v; a.out = out;
+  a.B = n_seqs; a.T = T_max; a.H = H; a.scale = scale;
+  a.lens = lens_dev; a.seqs = seqs_dev; a.nTg = (max_len + 63) / 64;
+  static bool configured = false;
+  if (!configured) {
+    DMG_CUDA_OK(cudaFuncSetAttribute(attn_flash_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FL_SMEM));
+    configured = true;
+  }
+  return launch_k(attn_flash_kernel<true, true>, dim3(n_seqs * H * a.nTg), dim3(128), (size_t)FL_SMEM, st, 1, a);
 }
 
 }  // namespace dmg

@@ -1,5 +1,7 @@
 // Internal launcher declarations shared by the .cu files of libdmg_b200.so.
 #pragma once
+#include <vector>
+
 #include "common.cuh"
 
 namespace dmg {
@@ -119,6 +121,7 @@ struct AttnGeneralArgs {
   int bert;             // 1: no mask, _line_shift wrap-around live (deep_music_remix.py:2096, r_mask=False)
   int win, k;           // window_mask (win_size, k); eval = (1, 1)
   float scale;          // 1/sqrt(Dh)
+  const int* lens = nullptr;   // BERT only, device [B]: sequence b is rows [b*T, b*T + lens[b]) (T = the padded length); NULL = all T
 };
 template <class T>
 int attn_general(const AttnGeneralArgs& a, cudaStream_t st);
@@ -148,6 +151,32 @@ bool attn_bert_tc_supported(int T, int H, int Dcap);
 // fp32_strip = 1: the first version of the strip skew (fp32 lines, 2.5 x the shared-memory wavefronts); kept for the parity tests
 int attn_bert_tc(const bf16* qkv, const bf16* rd, int Dcap, const float* u, const float* v, bf16* out, int B, int T, int H, float scale,
                  int fp32_strip, cudaStream_t st);
+// Per-sequence lengths (the batched remix): qkv / out are a padded batch, rows b*T_max + i, sequence b has lens_dev[b] tokens.  Both
+// write only the rows < lens[b] of the sequences they cover.  attn_bert_tc_varlen walks the host-built item list items_dev[n_items]
+// ((b << 16) | (h << 8) | 128-row query tile) of the sequences with lens >= 128; attn_flash_varlen the n_seqs sequences seqs_dev[]
+// (max_len = the longest of them).
+int attn_bert_tc_varlen(const bf16* qkv, const bf16* rd, int Dcap, const float* u, const float* v, bf16* out, const int* lens_dev,
+                        const int* items_dev, int n_items, int B, int T_max, int H, float scale, int fp32_strip, cudaStream_t st);
+int attn_flash_varlen(const bf16* qkv, const bf16* rd, int Dcap, const float* u, const float* v, bf16* out, const int* lens_dev,
+                      const int* seqs_dev, int n_seqs, int max_len, int T_max, int H, float scale, cudaStream_t st);
+
+// remix_batch.cu.  A padded batch of BERT sequences of their own lengths: lens (device [B]) and the host-built routing of
+// bert_varlen_plan - the tcgen05 kernel's item list for the sequences of at least 128 tokens (use_tc), the mma.sync flash kernel for
+// the others - so that every sequence runs on the kernel it would get alone.
+struct VarlenPlan {
+  const int* lens = nullptr;
+  const int* tc_items = nullptr;
+  int n_tc_items = 0;
+  const int* fl_seqs = nullptr;
+  int n_fl_seqs = 0, fl_max_len = 0;
+};
+void bert_varlen_plan(const int* lens_host, int B, int H, bool use_tc, std::vector<int>& tc_items, std::vector<int>& fl_seqs,
+                      int* fl_max_len);
+// both attention launches of the plan, then zeroes the output rows >= lens[b]
+int attn_bert_varlen_bf16(const bf16* qkv, const bf16* rd, int Dcap, const float* u, const float* v, bf16* out, const VarlenPlan& p,
+                          int B, int T_max, int H, float scale, int fp32_strip, cudaStream_t st);
+template <class T>
+int varlen_zero_rows(T* out, const int* lens_dev, int B, int T_max, int HD, cudaStream_t st);
 // x_len == 1 over the bf16 ring: persistent, TMA-2D swizzled K/V tiles, resident rel-pos keys, mma.sync dot products
 // (attention_decode2.cu).  tmK/tmV: ring viewed as [max_batch*H*M rows, 64 cols]; tmR: Rd viewed as [H*Dcap rows, 64 cols];
 // 64-row boxes.

@@ -138,9 +138,10 @@ struct DecodeStep {
   }
 };
 
+// vp (BERT only): the nb sequences have their own lengths (a padded batch, T_len = the padded length; see remix_batch.cu)
 template <class T>
 static int forward_chunk(dmg_model* m, const long long* ids, const long long* pos, int b0, int nb, int T_len, int win,
-                         int k, int logits_mode, float* logits, float* core_out, cudaStream_t st) {
+                         int k, int logits_mode, float* logits, float* core_out, cudaStream_t st, const VarlenPlan* vp = nullptr) {
   const dmg_config& c = m->cfg;
   const int d = c.d_model, HD = m->HD, rows = nb * T_len, M = c.mem_len;
   const bool bert = c.arch == DMG_ARCH_BERT;
@@ -189,7 +190,10 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
     if (flash) {
       // memory-less segment: bf16 q|k|v straight from the GEMM epilogue, tensor-core flash attention (attention_flash.cu)
       if (linear(m, A_XA, xa, L.wqkv, L.bqkv, m->qkv16, 3 * HD, rows, 0, 1, st)) return -1;
-      if (bert && !(m->kflags & DMG_KF_BERT_MMA_SYNC) && attn_bert_tc_supported(T_len, c.n_heads, m->Dcap)) {
+      if (vp) {
+        if (attn_bert_varlen_bf16(m->qkv16, (const bf16*)L.rd, m->Dcap, m->u, m->v, (bf16*)m->attn, *vp, nb, T_len, c.n_heads,
+                                  1.f / sqrtf((float)c.d_head), (m->kflags & DMG_KF_BERT_FP32_STRIP) ? 1 : 0, st)) return -1;
+      } else if (bert && !(m->kflags & DMG_KF_BERT_MMA_SYNC) && attn_bert_tc_supported(T_len, c.n_heads, m->Dcap)) {
         // tcgen05 / TMEM / TMA kernel (sequences of at least 128 tokens)
         if (attn_bert_tc(m->qkv16, (const bf16*)L.rd, m->Dcap, m->u, m->v, (bf16*)m->attn, nb, T_len, c.n_heads,
                          1.f / sqrtf((float)c.d_head), (m->kflags & DMG_KF_BERT_FP32_STRIP) ? 1 : 0, st)) return -1;
@@ -228,7 +232,9 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
       a.B = nb; a.T = T_len; a.H = c.n_heads; a.M = M; a.Dcap = m->Dcap;
       a.mem_count = m->mem_count; a.pos_total = m->pos_total; a.b0 = b0; a.bert = bert ? 1 : 0; a.win = win; a.k = k;
       a.scale = 1.f / sqrtf((float)c.d_head);
+      a.lens = vp ? vp->lens : nullptr;
       if (attn_general<T>(a, st)) return -1;
+      if (vp && varlen_zero_rows<T>((T*)m->attn, vp->lens, nb, T_len, HD, st)) return -1;
       if (M > 0 && ring_append_kv<T, float>(m->qkv, (T*)L.kring, (T*)L.vring, nb, T_len, c.n_heads, c.d_head, M, m->pos_total, b0,
                                             c.max_batch, st)) return -1;
     }
@@ -284,6 +290,38 @@ static int forward_impl(dmg_model* m, const long long* ids, const long long* pos
     m->mem_count = m->mem_count + T_len > c.mem_len ? c.mem_len : m->mem_count + T_len;
   }
   return 0;
+}
+
+// A padded batch of bs BERT sequences of their own lengths (lens_host [bs], each in [1, T_max]): validates, uploads the lengths and
+// the attention routing (bert_varlen_plan) into the model's buffers.  The plan stays valid until the next call.
+static int varlen_setup(dmg_model* m, const int32_t* lens_host, int bs, int T_max, VarlenPlan* p, cudaStream_t st) {
+  const dmg_config& c = m->cfg;
+  DMG_CHECK(m->committed, "varlen: weights not committed (call dmg_commit_weights)");
+  DMG_CHECK(c.arch == DMG_ARCH_BERT, "varlen: per-sequence lengths are for the BERT encoder only");
+  DMG_CHECK(bs >= 1 && bs <= c.max_batch, "varlen: batch %d outside [1, max_batch=%d]", bs, c.max_batch);
+  DMG_CHECK(T_max >= 1 && T_max <= c.max_seq, "varlen: T_max %d outside [1, max_seq=%d]", T_max, c.max_seq);
+  DMG_CHECK((long long)bs * T_max <= m->max_rows, "varlen: %d x %d rows exceed the activation workspace (%d rows)", bs, T_max, m->max_rows);
+  for (int b = 0; b < bs; b++)
+    DMG_CHECK(lens_host[b] >= 1 && lens_host[b] <= T_max, "varlen: length %d of sequence %d outside [1, T_max=%d]", lens_host[b], b, T_max);
+  const bool use_tc = m->is_bf16 && m->use_tc && T_max > 1 && !(m->kflags & (DMG_KF_BERT_MMA_SYNC | DMG_KF_NO_FLASH)) &&
+                      attn_bert_tc_supported(T_max, c.n_heads, m->Dcap);
+  std::vector<int> items, seqs;
+  int fl_max = 0;
+  bert_varlen_plan(lens_host, bs, c.n_heads, use_tc, items, seqs, &fl_max);
+  DMG_CUDA_OK(cudaMemcpyAsync(m->vl_lens, lens_host, (size_t)bs * 4, cudaMemcpyHostToDevice, st));
+  if (!items.empty()) DMG_CUDA_OK(cudaMemcpyAsync(m->vl_items, items.data(), items.size() * 4, cudaMemcpyHostToDevice, st));
+  if (!seqs.empty()) DMG_CUDA_OK(cudaMemcpyAsync(m->vl_seqs, seqs.data(), seqs.size() * 4, cudaMemcpyHostToDevice, st));
+  p->lens = m->vl_lens;
+  p->tc_items = m->vl_items; p->n_tc_items = (int)items.size();
+  p->fl_seqs = m->vl_seqs; p->n_fl_seqs = (int)seqs.size(); p->fl_max_len = fl_max;
+  m->mem_count = 0; m->pos_total = 0; m->batch = bs;
+  return 0;
+}
+
+static int forward_varlen(dmg_model* m, const long long* ids, const long long* pos, const VarlenPlan& p, int bs, int T_max,
+                          int logits_mode, float* logits, float* core_out, cudaStream_t st) {
+  return m->is_bf16 ? forward_chunk<bf16>(m, ids, pos, 0, bs, T_max, 1, 1, logits_mode, logits, core_out, st, &p)
+                    : forward_chunk<float>(m, ids, pos, 0, bs, T_max, 1, 1, logits_mode, logits, core_out, st, &p);
 }
 
 static int build_rd(dmg_model* m) {
@@ -555,6 +593,15 @@ int dmg_create(const dmg_config* cfg, int device, dmg_model** out) {
       if (!rc && getenv("DMG_DECODE_TIMELINE")) TRY(dalloc(m, &m->dl_dbg, 64));
     }
   }
+  if (bert) {
+    const size_t items = (size_t)c.max_batch * c.n_heads * ((c.max_seq + 127) / 128);
+    TRY(dalloc(m, &m->vl_lens, (size_t)c.max_batch));
+    TRY(dalloc(m, &m->vl_items, items));
+    TRY(dalloc(m, &m->vl_seqs, (size_t)c.max_batch));
+    TRY(dalloc(m, &m->mk_pos, (size_t)c.max_batch * c.max_seq));
+    for (int** p : {&m->mk_n, &m->mk_streams, &m->mk_prev, &m->mk_rc, &m->mk_tok, &m->mk_nc}) TRY(dalloc(m, p, (size_t)c.max_batch));
+    TRY(dalloc(m, &m->mk_step, 1));
+  }
   if (!rc && cudaStreamCreateWithFlags(&m->cap_stream, cudaStreamNonBlocking) != cudaSuccess) {
     set_error("dmg_create: cudaStreamCreate failed");
     rc = -1;
@@ -660,6 +707,120 @@ int dmg_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, in
   DMG_CUDA_OK(cudaSetDevice(m->device));
   return forward_impl(m, (const long long*)ids_dev, (const long long*)pos_dev, bs, x_len, mask_win, mask_k, logits_mode,
                       logits_dev, core_out_dev, (cudaStream_t)stream);
+}
+
+int dmg_forward_varlen(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, const int32_t* lens_host, int bs, int T_max,
+                       int logits_mode, float* logits_dev, float* core_out_dev, void* stream) {
+  DMG_CHECK(m && ids_dev && pos_dev && lens_host, "dmg_forward_varlen: null argument");
+  DMG_CHECK(logits_mode == DMG_LOGITS_NONE || logits_mode == DMG_LOGITS_ALL, "dmg_forward_varlen: logits_mode must be NONE or ALL");
+  DMG_CUDA_OK(cudaSetDevice(m->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  VarlenPlan p;
+  if (varlen_setup(m, lens_host, bs, T_max, &p, st)) return -1;
+  return forward_varlen(m, (const long long*)ids_dev, (const long long*)pos_dev, p, bs, T_max, logits_mode, logits_dev, core_out_dev, st);
+}
+
+int dmg_predict_mask_batch(dmg_model* m, int64_t* ids_dev, const int64_t* pos_dev, const int32_t* lens_host, const int32_t* mask_pos_host,
+                           const int32_t* n_masks_host, const int32_t* stream_idx_host, int B, int T_max, int n_max,
+                           const dmg_vocab_layout* vocab, const dmg_sampler_params* params, void* stream) {
+  DMG_CHECK(m && ids_dev && pos_dev && lens_host && n_masks_host && stream_idx_host && vocab && params,
+            "dmg_predict_mask_batch: null argument");
+  DMG_CHECK(n_max >= 0 && n_max <= T_max && (n_max == 0 || mask_pos_host), "dmg_predict_mask_batch: n_max %d outside [0, T_max=%d]", n_max, T_max);
+  DMG_CHECK(B >= 1 && B <= m->cfg.max_batch, "dmg_predict_mask_batch: %d items outside [1, max_batch=%d]", B, m->cfg.max_batch);
+  for (int b = 0; b < B; b++) {
+    const int L = lens_host[b], n = n_masks_host[b];
+    DMG_CHECK(L >= 1 && L <= T_max, "dmg_predict_mask_batch: length %d of item %d outside [1, T_max=%d]", L, b, T_max);
+    DMG_CHECK(n >= 0 && n <= n_max && n <= L, "dmg_predict_mask_batch: item %d has %d masks (n_max %d, length %d)", b, n, n_max, L);
+    DMG_CHECK(stream_idx_host[b] >= 0, "dmg_predict_mask_batch: negative stream index of item %d", b);
+    for (int s = 0; s < n; s++) {
+      const int p = mask_pos_host[(size_t)b * n_max + s];
+      DMG_CHECK(p >= 0 && p < L && (s == 0 || p > mask_pos_host[(size_t)b * n_max + s - 1]),
+                "dmg_predict_mask_batch: mask position %d of item %d is outside [0, %d) or not ascending", p, b, L);
+    }
+  }
+  DMG_CUDA_OK(cudaSetDevice(m->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  VarlenPlan p;
+  if (varlen_setup(m, lens_host, B, T_max, &p, st)) return -1;
+  int steps = 0;
+  for (int b = 0; b < B; b++) steps = n_masks_host[b] > steps ? n_masks_host[b] : steps;
+  if (steps == 0) return 0;
+  DMG_CUDA_OK(cudaMemcpyAsync(m->mk_pos, mask_pos_host, (size_t)B * n_max * 4, cudaMemcpyHostToDevice, st));
+  DMG_CUDA_OK(cudaMemcpyAsync(m->mk_n, n_masks_host, (size_t)B * 4, cudaMemcpyHostToDevice, st));
+  DMG_CUDA_OK(cudaMemcpyAsync(m->mk_streams, stream_idx_host, (size_t)B * 4, cudaMemcpyHostToDevice, st));
+  DMG_CUDA_OK(cudaMemsetAsync(m->mk_rc, 0, (size_t)B * 4, st));
+  DMG_CUDA_OK(cudaMemsetAsync(m->mk_step, 0, 4, st));
+  const dmg_config& c = m->cfg;
+  MaskStepArgs a;
+  a.ids = (long long*)ids_dev; a.lens = m->vl_lens; a.mask_pos = m->mk_pos; a.n_masks = m->mk_n; a.step = m->mk_step;
+  a.prev = m->mk_prev; a.repeat_count = m->mk_rc; a.logits = m->logits_buf; a.bias = m->head_b; a.tok = m->mk_tok;
+  a.num_choices = m->mk_nc; a.B = B; a.T_max = T_max; a.n_max = n_max; a.d = c.d_model; a.V = c.vocab;
+  SampleArgs sa;
+  memset(&sa, 0, sizeof(sa));
+  sa.logits = m->logits_buf; sa.V = c.vocab; sa.vocab = *vocab; sa.params = *params; sa.loop_mode = 0;
+  sa.prev_idx = m->mk_prev; sa.repeat_count = m->mk_rc; sa.out_tokens = m->mk_tok; sa.num_choices = m->mk_nc;
+  sa.stream_ids = m->mk_streams; sa.dev_offset = m->mk_step;
+  const void* emb = m->is_bf16 ? (const void*)m->emb.b16 : (const void*)m->emb.f32;
+  // one step: the encoder forward (no logits) over the current ids, then the mask step; its launches read the step counter on the
+  // device, so from the second step on they are replayed as one CUDA graph (the first, eager step performs the one-time set-up)
+  auto step = [&](cudaStream_t s) -> int {
+    if (forward_varlen(m, (const long long*)ids_dev, (const long long*)pos_dev, p, B, T_max, DMG_LOGITS_NONE, nullptr, nullptr, s)) return -1;
+    return mask_step_launch(a, m->xa, emb, m->is_bf16, sa, s);
+  };
+  const bool graphed = !(m->kflags & DMG_KF_NO_GRAPH) && steps > 1;
+  cudaGraphExec_t exec = nullptr;
+  int rc = step(st);
+  for (int s = 1; s < steps && !rc; s++) {
+    if (!graphed) { rc = step(st); continue; }
+    if (exec == nullptr) {
+      const long long before = g_launch_count;
+      cudaGraph_t g = nullptr;
+      DMG_CUDA_OK(cudaStreamBeginCapture(m->cap_stream, cudaStreamCaptureModeThreadLocal));
+      rc = step(m->cap_stream);
+      const cudaError_t e = cudaStreamEndCapture(m->cap_stream, &g);
+      m->graph_launches = g_launch_count - before;
+      g_launch_count = before;
+      if (!rc && e != cudaSuccess) { set_error("dmg_predict_mask_batch: graph capture failed: %s", cudaGetErrorString(e)); rc = -1; }
+      if (!rc && cudaGraphInstantiate(&exec, g, 0) != cudaSuccess) { set_error("dmg_predict_mask_batch: cudaGraphInstantiate failed"); rc = -1; }
+      if (g) cudaGraphDestroy(g);
+      if (rc) break;
+    }
+    if (cudaGraphLaunch(exec, st) != cudaSuccess) { set_error("dmg_predict_mask_batch: cudaGraphLaunch failed"); rc = -1; break; }
+    g_launch_count += m->graph_launches;
+  }
+  if (exec) cudaGraphExecDestroy(exec);
+  return rc;
+}
+
+int dmg_attn_bert_varlen(const void* qkv_dev, const void* rk_dev, int Dcap, const float* u, const float* v, void* out_dev,
+                         const int32_t* lens_host, int B, int T_max, int H, int mma_sync_only, void* stream) {
+  DMG_CHECK(qkv_dev && rk_dev && u && v && out_dev && lens_host, "dmg_attn_bert_varlen: null argument");
+  DMG_CHECK(B >= 1 && T_max >= 1 && H >= 1 && H <= 256 && Dcap >= T_max, "dmg_attn_bert_varlen: B %d, T_max %d, H %d, Dcap %d", B, T_max, H, Dcap);
+  for (int b = 0; b < B; b++)
+    DMG_CHECK(lens_host[b] >= 1 && lens_host[b] <= T_max, "dmg_attn_bert_varlen: length %d of sequence %d outside [1, T_max=%d]", lens_host[b], b, T_max);
+  cudaStream_t st = (cudaStream_t)stream;
+  std::vector<int> items, seqs;
+  int fl_max = 0;
+  bert_varlen_plan(lens_host, B, H, !mma_sync_only && attn_bert_tc_supported(T_max, H, Dcap), items, seqs, &fl_max);
+  int* buf = nullptr;
+  DMG_CUDA_OK(cudaMalloc(&buf, (size_t)(B + items.size() + seqs.size() + 1) * 4));
+  VarlenPlan p;
+  p.lens = buf; p.tc_items = buf + B; p.n_tc_items = (int)items.size(); p.fl_seqs = buf + B + items.size();
+  p.n_fl_seqs = (int)seqs.size(); p.fl_max_len = fl_max;
+  int rc = 0;
+  if (cudaMemcpyAsync(buf, lens_host, (size_t)B * 4, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+      (!items.empty() && cudaMemcpyAsync(buf + B, items.data(), items.size() * 4, cudaMemcpyHostToDevice, st) != cudaSuccess) ||
+      (!seqs.empty() && cudaMemcpyAsync(buf + B + items.size(), seqs.data(), seqs.size() * 4, cudaMemcpyHostToDevice, st) != cudaSuccess)) {
+    set_error("dmg_attn_bert_varlen: upload failed");
+    rc = -1;
+  }
+  if (!rc) rc = attn_bert_varlen_bf16((const bf16*)qkv_dev, (const bf16*)rk_dev, Dcap, u, v, (bf16*)out_dev, p, B, T_max, H,
+                                      0.125f, 0, st);
+  const cudaError_t e = cudaStreamSynchronize(st);
+  cudaFree(buf);
+  if (rc) return rc;
+  DMG_CUDA_OK(e);
+  return 0;
 }
 
 int dmg_get_hidden(dmg_model* m, int level, float* out_dev, void* stream) {

@@ -86,6 +86,10 @@ struct dmg_model {
   int graph_bs = -1;
   long long graph_launches = 0;
   dmg_train* train = nullptr;   // training state (train.cu), created by dmg_train_create
+  // batched remix (remix_batch.cu), BERT models: per-sequence lengths with their attention routing, and the mask loop's device state
+  int *vl_lens = nullptr, *vl_items = nullptr, *vl_seqs = nullptr;
+  int *mk_pos = nullptr, *mk_n = nullptr, *mk_streams = nullptr, *mk_prev = nullptr, *mk_rc = nullptr, *mk_tok = nullptr, *mk_nc = nullptr,
+      *mk_step = nullptr;
 };
 
 namespace dmg {

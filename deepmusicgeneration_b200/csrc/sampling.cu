@@ -272,7 +272,8 @@ __global__ void __launch_bounds__(SAMP_THREADS) sample_kernel(SampleArgs a) {
   __syncthreads();
   if (tid == 0) sh_int[0] = V;
   __syncthreads();
-  const float u = philox_uniform(sp.seed, a.offset + (a.loop_mode ? (uint64_t)step : 0ull), (uint32_t)sidx);
+  const uint64_t draw = a.offset + (a.loop_mode ? (uint64_t)step : 0ull) + (a.dev_offset ? (uint64_t)*a.dev_offset : 0ull);
+  const float u = philox_uniform(sp.seed, draw, a.stream_ids ? (uint32_t)a.stream_ids[sidx] : (uint32_t)sidx);
   const float target = u * pr[V - 1];
   for (int i = tid; i < V; i += SAMP_THREADS) {
     const float prevc = i > 0 ? pr[i - 1] : 0.f;

@@ -26,9 +26,30 @@ struct SampleArgs {
   long long* next_pos;        // [n] beat position of the next token (loop mode, may be NULL)
   int* num_choices;           // [n] optional
   float* probs;               // [n, V] optional: the final probabilities (after filter / top-k / top-p / softmax)
+  // optional (the batched remix): Philox stream of row i = stream_ids[i] instead of i; *dev_offset is added to the counter
+  const int* stream_ids;
+  const int* dev_offset;
 };
 
 int sample_launch(const SampleArgs& a, int n, cudaStream_t st);
+
+// The mask step of the batched remix (remix_batch.cu): device state of B items of a padded batch (row b*T_max + t)
+struct MaskStepArgs {
+  long long* ids;             // [B*T_max] in / out: the sampled tokens replace the masks
+  const int* lens;            // [B]
+  const int* mask_pos;        // [B, n_max] ascending mask positions of each item
+  const int* n_masks;         // [B]
+  int* step;                  // [1] the loop step s (advanced by the step itself: the launches can be replayed as a graph)
+  int* prev;                  // [B] the token before the masked position (the sampler's prev_idx)
+  int* repeat_count;          // [B]
+  float* logits;              // [B, V] the masked positions' logits
+  const float* bias;          // [V] head bias
+  int* tok;                   // [B] sampled ids
+  int* num_choices;           // [B]
+  int B, T_max, n_max, d, V;
+};
+// head row -> sampler (samp: the remix sampler over a.logits, prev, repeat_count, tok, num_choices) -> write-back
+int mask_step_launch(const MaskStepArgs& a, const void* h, const void* emb, bool bf16_operands, const SampleArgs& samp, cudaStream_t st);
 
 struct BeamArgs {
   const float* logits;      // [nb, V] fp32: last-position logits of the live beams

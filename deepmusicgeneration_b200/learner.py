@@ -346,6 +346,62 @@ class MultitaskLearner:
             x[midx] = idx
         return vocab.to_music_item(x.cpu().numpy())
 
+    def predict_mask_batch(self, items, temperatures=(1.0, 1.0), top_k=20, top_p=0.8, seed=None):
+        """predict_mask over many items at once: returns one MusicItem per item.  The items (of any lengths up to max_seq) run as
+        padded batches of up to max_batch items through dmg_predict_mask_batch: every step is one encoder forward over the batch and
+        one sampled token per item that still has masks, with no host round trip.  Item i draws from Philox stream i of `seed` (its
+        n-th mask uses counter n), so item 0 makes the draws of predict_mask(items[0], ..., seed=seed).  Its logit row is summed in another
+        order than the head GEMM's, so a near-tie can still go the other way.  In fp32 no result depends on how the items are grouped;
+        in bf16 the GEMM kernel follows the row count of a group (max_batch / max_rows), which can likewise flip a near-tie.  Items
+        are sorted by length before they are grouped, which keeps the padding small."""
+        e = self.model._e
+        vocab = self.data.vocab
+        cfg = e.cfg
+        max_rows = cfg.max_rows if cfg.max_rows > 0 else cfg.max_batch * cfg.max_seq
+        datas = [np.asarray(it.data, dtype=np.int64) for it in items]
+        poss = [np.asarray(it.position, dtype=np.int64) for it in items]
+        for i, x in enumerate(datas):
+            if len(x) > cfg.max_seq:
+                raise ValueError(f'item {i} has {len(x)} tokens and exceeds max_seq={cfg.max_seq}: build the learner with '
+                                 f'multitask_model_learner(..., max_seq=<longest item>) or cut the item with item.trim_to_beat(...)')
+            if len(x) == 0:
+                raise ValueError(f'item {i} is empty')
+        vl = vocab_layout(vocab)
+        params = sampler_params(vocab, 1, temperatures, 0, top_k, top_p, None, flags=_lib.SAMPLE_REMIX_FILTER, seed=seed)
+        out = [None] * len(items)
+        order = sorted(range(len(items)), key=lambda i: len(datas[i]))
+        k = 0
+        while k < len(order):
+            chunk = [order[k]]                         # ascending lengths: the last item of a chunk sets its padded length
+            while (k + len(chunk) < len(order) and len(chunk) < cfg.max_batch and
+                   (len(chunk) + 1) * len(datas[order[k + len(chunk)]]) <= max_rows):
+                chunk.append(order[k + len(chunk)])
+            k += len(chunk)
+            B, T = len(chunk), max(len(datas[i]) for i in chunk)
+            lens = np.array([len(datas[i]) for i in chunk], dtype=np.int32)
+            x = np.full((B, T), vocab.pad_idx, dtype=np.int64)
+            pos = np.zeros((B, T), dtype=np.int64)
+            masks = [np.flatnonzero(datas[i] == vocab.mask_idx).astype(np.int32) for i in chunk]
+            n_max = max(1, max(len(mp) for mp in masks))
+            mask_pos = np.zeros((B, n_max), dtype=np.int32)
+            for j, i in enumerate(chunk):
+                x[j, :lens[j]] = datas[i]
+                pos[j, :lens[j]] = poss[i]
+                mask_pos[j, :len(masks[j])] = masks[j]
+            n_masks = np.array([len(mp) for mp in masks], dtype=np.int32)
+            streams = np.array(chunk, dtype=np.int32)
+            xd = torch.from_numpy(x).to(e.device)
+            pd = torch.from_numpy(pos).to(e.device)
+            with torch.cuda.device(e.device):
+                check(e.lib.dmg_predict_mask_batch(e.h, _ptr(xd), _ptr(pd), lens.ctypes.data_as(C.c_void_p),
+                                                   mask_pos.ctypes.data_as(C.c_void_p), n_masks.ctypes.data_as(C.c_void_p),
+                                                   streams.ctypes.data_as(C.c_void_p), B, T, n_max, C.byref(vl), C.byref(params),
+                                                   _stream_ptr()), 'dmg_predict_mask_batch')
+            res = xd.cpu().numpy()
+            for j, i in enumerate(chunk):
+                out[i] = vocab.to_music_item(res[j, :lens[j]].copy())
+        return out
+
 
 def multitask_model_learner(data, config=None, drop_mult=1., pretrained_path=None, dtype='bf16', device=0, max_batch=1,
                             max_seq=1024, seed=None, **learn_kwargs):

@@ -123,7 +123,9 @@ class _Engine:
         return out
 
     # ---- forward
-    def forward(self, ids, pos, logits_mode, want_core=False, mask=(1, 1)):
+    def forward(self, ids, pos, logits_mode, want_core=False, mask=(1, 1), lens=None):
+        """One forward over ids [bs, T].  lens (BERT encoder only): the length of every row, a padded batch of sequences that are each
+        computed as if alone at their length (dmg_forward_varlen); logits_mode LOGITS_NONE or LOGITS_ALL."""
         assert ids.dim() == 2
         ids = ids.to(self.device, torch.int64).contiguous()
         if pos is not None:
@@ -137,8 +139,15 @@ class _Engine:
             logits = torch.empty(bs, V, device=self.device, dtype=torch.float32)
         core = torch.empty(bs, T, d, device=self.device, dtype=torch.float32) if want_core else None
         with torch.cuda.device(self.device):
-            check(self.lib.dmg_forward(self.h, _ptr(ids), _ptr(pos), bs, T, int(mask[0]), int(mask[1]), logits_mode,
-                                       _ptr(logits), _ptr(core), _stream_ptr()), 'dmg_forward')
+            if lens is not None:
+                ln = np.ascontiguousarray(np.asarray(lens, dtype=np.int32))
+                if ln.shape != (bs,):
+                    raise ValueError(f'lens must hold one length per row ({bs}), got shape {ln.shape}')
+                check(self.lib.dmg_forward_varlen(self.h, _ptr(ids), _ptr(pos), ln.ctypes.data_as(C.c_void_p), bs, T, logits_mode,
+                                                  _ptr(logits), _ptr(core), _stream_ptr()), 'dmg_forward_varlen')
+            else:
+                check(self.lib.dmg_forward(self.h, _ptr(ids), _ptr(pos), bs, T, int(mask[0]), int(mask[1]), logits_mode,
+                                           _ptr(logits), _ptr(core), _stream_ptr()), 'dmg_forward')
         return logits, core
 
     def reset(self, batch=0):

@@ -122,6 +122,30 @@ int dmg_mem_count(dmg_model* m);
 int dmg_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, int bs, int x_len, int mask_win,
                 int mask_k, int logits_mode, float* logits_dev, float* core_out_dev, void* stream);
 
+/* The BERT encoder (DMG_ARCH_BERT) over a padded batch of bs sequences of their own lengths: ids_dev / pos_dev int64 [bs, T_max],
+ * sequence b is row b of length lens_host[b] in [1, T_max] (host memory); what its padding positions hold does not matter.  Every
+ * sequence is computed as if it were alone at its length (dmg_forward with x_len = lens[b]): the same attention kernel - except a
+ * one-token sequence in a batch with T_max > 1, which runs on the flash kernel in bf16 where alone it runs on the FFMA kernel - and
+ * rows < lens[b] equal to that forward's up to the GEMMs' row-count-dependent summation order (bf16: the GEMM kernel is chosen by
+ * the number of rows, bs * T_max here).  logits_mode DMG_LOGITS_NONE or DMG_LOGITS_ALL
+ * (logits_dev fp32 [bs, T_max, V]); core_out_dev fp32 [bs, T_max, d_model] or NULL.  Rows past a sequence's end hold finite values
+ * of no meaning.  bs * T_max must fit the activation workspace (max_rows). */
+int dmg_forward_varlen(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, const int32_t* lens_host, int bs, int T_max,
+                       int logits_mode, float* logits_dev, float* core_out_dev, void* stream);
+
+/* MultitaskLearner.predict_mask (deep_music_remix.py:2563-2613) for B items at once, on the device.  ids_dev / pos_dev int64 [B, T_max]
+ * (padded as in dmg_forward_varlen; ids_dev is updated in place: every mask position receives its sampled token); host arrays:
+ * lens_host [B], mask_pos_host [B, n_max] (the ascending positions of the masks of item b in its first n_masks_host[b] entries),
+ * stream_idx_host [B] (Philox stream of the item).  Step s runs the varlen forward and, for every item with more than s masks, the
+ * logits of its s-th mask position, the remix sampler of dmg_sample_logits with counter offset s and its stream, and the
+ * write-back; repeat_count per item as the reference keeps it.  With stream_idx = 0 an item makes the draws of the one-item loop of
+ * predict_mask (offset n = mask number, stream 0); its logit row is summed in another order than the head GEMM's.  In fp32 results do not depend on which other items share the batch; in bf16
+ * the GEMM kernel is chosen by the row count B * T_max, so another grouping may round differently and change a near-tied pick.  The steps are
+ * replayed as a CUDA graph (DMG_KF_NO_GRAPH: launched one by one).  Everything is validated before anything launches. */
+int dmg_predict_mask_batch(dmg_model* m, int64_t* ids_dev, const int64_t* pos_dev, const int32_t* lens_host, const int32_t* mask_pos_host,
+                           const int32_t* n_masks_host, const int32_t* stream_idx_host, int B, int T_max, int n_max,
+                           const dmg_vocab_layout* vocab, const dmg_sampler_params* params, void* stream);
+
 /* raw_outputs[level] of the reference forward (= model[0].hidden[level]): fp32 [bs, mem_count, d_model].
  * Needs cfg.keep_hidden. */
 int dmg_get_hidden(dmg_model* m, int level, float* out_dev, void* stream);
@@ -292,6 +316,14 @@ int dmg_attn_bert_train_bwd(const void* qkv_x, int64_t ldx, const void* rk, cons
                             const void* out, const float* lse, const void* dout, int B, int T, int H, float drop_p,
                             uint32_t drop_seed, float* delta, void* dqkv_x, void* ds_dist, float* du,
                             void* p_buf, void* ds_buf, void* stream);
+
+/* Unit-test entry of the per-sequence-length inference attention of the BERT encoder (the launches of dmg_forward_varlen): qkv_dev
+ * bf16 [B*T_max, 3*H*64] (q | k | v, sequence b = rows b*T_max + [0, lens_host[b])), rk_dev bf16 [H][Dcap][64] (rel-pos keys by distance,
+ * Dcap >= T_max + 1), u / v fp32 [H*64], out_dev bf16 [B*T_max, H*64]; head size 64 (scale 1/8).  mma_sync_only = 0: sequences of at
+ * least 128 tokens on the tcgen05 kernel, shorter ones on the mma.sync flash kernel; 1: every sequence on the flash kernel.  Output
+ * rows past a sequence's end are written as zeros; the padding rows of qkv may hold anything.  Synchronises the stream. */
+int dmg_attn_bert_varlen(const void* qkv_dev, const void* rk_dev, int Dcap, const float* u, const float* v, void* out_dev,
+                         const int32_t* lens_host, int B, int T_max, int H, int mma_sync_only, void* stream);
 
 /* ---- training data feed (SURVEY.md section 8 f4) ------------------------------------------------------------------------
  * dmg_preload_fill = MusicPreloader.__getitem__ / fill_row (deep_music_genre.py:1088-1125) for all `bs` rows of one batch.
