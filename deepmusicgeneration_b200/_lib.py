@@ -90,6 +90,10 @@ SYMBOLS = {
     'dmg_train_opt_state': (c_i32, [c_vp, C.c_char_p, c_i32, c_i32, c_vp, c_i64]),
     'dmg_train_opt_steps': (c_i64, [c_vp, c_i64]),
     'dmg_train_losses': (c_i32, [c_vp, c_vp, c_vp]),
+    'dmg_train_eval_begin': (c_i32, [c_vp, c_i32]),
+    'dmg_train_eval_batch': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp]),
+    'dmg_train_eval_end': (c_i32, [c_vp, c_vp, c_i32, c_vp]),
+    'dmg_eval_metrics': (c_i32, [c_vp, c_i64, c_vp, c_i64, c_i32, c_i32, c_vp, c_vp]),
     'dmg_train_get_grad': (c_i32, [c_vp, C.c_char_p, c_vp, c_i64]),
     'dmg_train_dropout_mask': (c_i32, [c_vp, c_i32, c_i32, c_i64, c_vp, c_i64, c_vp]),
     'dmg_train_grad_buffer': (c_vp, [c_vp]),

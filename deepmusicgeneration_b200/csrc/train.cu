@@ -72,6 +72,13 @@ struct dmg_train {
   int opt_steps = 0;
   int next_layer = -1;                       // backward progress: next layer_hi expected (-1: no forward pending)
   bool mem_pending = false;
+  // validation (dmg_train_eval_*): forward-only batches write (ce_sum, kept, correct) to row eval_n of eval_tab, never to acc
+  bool eval_fwd = false;                     // the running forward is a validation batch: save nothing for a backward
+  bool eval_last = false;                    // the latest forward was a validation batch: its activations are incomplete
+  bool eval_open = false;                    // between dmg_train_eval_begin and dmg_train_eval_end
+  int eval_cap = 0, eval_max = 0, eval_n = 0;   // allocated rows, rows of this validation, rows written
+  double *eval_tab = nullptr, *eval_part = nullptr;   // [eval_cap][3], [EVAL_PART_SLOTS][3]
+  const long long* eval_targets = nullptr;
   AdamTensor* adam_tensors = nullptr;
   AdamChunk* adam_chunks = nullptr;
   int n_adam_chunks = 0;
@@ -279,10 +286,19 @@ AttnTrainArgs attn_args(dmg_model* m, dmg_train* t, int l) {
   a.scale = 1.f / sqrtf((float)c.d_head);
   const Drop dr = make_drop(t, t->cfg.attn_p, SITE_ATTN, l);
   a.drop_thresh = dr.thresh; a.drop_seed = dr.seed; a.drop_scale = dr.scale;
-  if (A.p_save && attn_train_fwd_tc_supported(a)) {   // same predicate as the forward dispatch
+  if (A.p_save && !t->eval_fwd && attn_train_fwd_tc_supported(a)) {   // same predicate as the forward dispatch
     a.p_save = A.p_save; a.m_save = A.m_save; a.qu_save = A.qu_save; a.qv_save = A.qv_save;
   }
   return a;
+}
+
+// validation head: tied decoder on the last layer's output (the output dropout is the identity in eval mode) and the metrics of
+// the batch into row eval_n of the validation table
+int eval_head(dmg_model* m, dmg_train* t, long long ignore, cudaStream_t st) {
+  const dmg_config& c = m->cfg;
+  GemmEpi e; e.bias = m->head_b; e.out = t->logits; e.ldc = t->Vp; e.out_mode = GEMM_OUT_F32;
+  if (gemm_bf16_tc(t->xa_last, 0, c.d_model, m->emb.b16, 0, c.d_model, t->rows, c.vocab, c.d_model, 1, e, m->num_sms, st)) return -1;
+  return train_eval_metrics(t->logits, t->Vp, t->eval_targets, ignore, t->rows, c.vocab, t->eval_part, t->eval_tab + 3ll * t->eval_n, st);
 }
 
 int train_forward(dmg_model* m, dmg_train* t, const long long* ids, const long long* pos, const long long* targets,
@@ -290,7 +306,7 @@ int train_forward(dmg_model* m, dmg_train* t, const long long* ids, const long l
   const dmg_config& c = m->cfg;
   const int d = c.d_model, HD = m->HD, L = c.n_layers, M = c.mem_len, rows = t->rows, S = M + t->T, ns = m->num_sms;
   if (finish_pending_mem(m, t, st)) return -1;
-  DMG_CUDA_OK(cudaMemsetAsync(t->acc, 0, 4 * sizeof(float), st));
+  if (!t->eval_fwd) DMG_CUDA_OK(cudaMemsetAsync(t->acc, 0, 4 * sizeof(float), st));
   {
     const Drop dr = make_drop(t, t->cfg.embed_p, SITE_EMBED, 0);
     if (train_embed(ids, c.encode_position ? pos : nullptr, m->emb.f32, m->beat, m->bar, t->x32, t->act[0].xa_in, rows, d, c.vocab,
@@ -328,6 +344,7 @@ int train_forward(dmg_model* m, dmg_train* t, const long long* ids, const long l
       static const bool old_epi = getenv("DMG_FFN_SAVE_PRE") != nullptr;
       GemmEpi e; e.bias = W.b1; e.act = old_epi ? GEMM_ACT_GELU : GEMM_ACT_GELU_GRADSAVE; e.out = A.hact; e.ldc = c.d_inner; e.out_mode = GEMM_OUT_BF16;
       e.out2 = A.hpre; e.ld2 = c.d_inner; e.drop_thresh = d3.thresh; e.drop_seed = d3.seed; e.drop_scale = d3.scale;
+      if (t->eval_fwd) { e.act = GEMM_ACT_GELU; e.out2 = nullptr; }   // validation: the activation only
       if (gemm_bf16_tc(A.xa1, 0, d, W.w1.b16, 0, d, rows, c.d_inner, d, 1, e, ns, st)) return -1;
       GemmEpi e2; e2.bias = W.b2; e2.out = t->proj; e2.ldc = d; e2.out_mode = GEMM_OUT_BF16;
       if (gemm_bf16_tc(A.hact, 0, c.d_inner, W.w2.b16, 0, c.d_inner, rows, d, c.d_inner, 1, e2, ns, st)) return -1;
@@ -336,7 +353,10 @@ int train_forward(dmg_model* m, dmg_train* t, const long long* ids, const long l
     }
   }
   // head: RNN dropout, tied decoder, cross entropy (+ gradient of the logits), AR, TAR
-  {
+  if (t->eval_fwd) {   // validation: no dropout, the metrics instead of the loss and dlogits; no AR / TAR (CrossEntropyFlat only)
+    if (eval_head(m, t, -1, st)) return -1;
+    if (M > 0 && apply_mem_update(m, t, st, L, L)) return -1;   // level L keeps what a training forward leaves there
+  } else {
     const Drop dr = make_drop(t, t->cfg.output_p, SITE_OUT, 0);
     if (train_rnn_dropout(t->xa_last, t->xdrop, t->B, t->T, d, dr.thresh, dr.seed, dr.scale, st)) return -1;
     GemmEpi e; e.bias = m->head_b; e.out = t->logits; e.ldc = t->Vp; e.out_mode = GEMM_OUT_F32;
@@ -457,7 +477,7 @@ int backward_layer(dmg_model* m, dmg_train* t, int l, cudaStream_t st) {
 int train_forward_bert(dmg_model* m, dmg_train* t, const long long* ids, const long long* pos, const long long* targets, cudaStream_t st) {
   const dmg_config& c = m->cfg;
   const int d = c.d_model, HD = m->HD, L = c.n_layers, rows = t->rows, T = t->T, ns = m->num_sms;
-  DMG_CUDA_OK(cudaMemsetAsync(t->acc, 0, 8 * sizeof(float), st));
+  if (!t->eval_fwd) DMG_CUDA_OK(cudaMemsetAsync(t->acc, 0, 8 * sizeof(float), st));
   {
     const Drop dr = make_drop(t, t->cfg.embed_p, SITE_EMBED, 0);
     if (train_embed(ids, pos, m->emb.f32, m->beat, m->bar, t->x32, t->act[0].xa_in, rows, d, c.vocab, dr.thresh, dr.seed, dr.scale, st))
@@ -479,6 +499,7 @@ int train_forward_bert(dmg_model* m, dmg_train* t, const long long* ids, const l
     const Drop dr = make_drop(t, t->cfg.resid_p, SITE_RES1, l);   // attention output (HD == d) enters the residual directly
     if (train_residual_ln_fwd(t->x32, A.attn, W.ln1w, W.ln1b, xa_out, A.z1, A.st1, rows, d, dr.thresh, dr.seed, dr.scale, st)) return -1;
   }
+  if (t->eval_fwd) return eval_head(m, t, t->cfg.pad_idx, st);
   const Drop dr = make_drop(t, t->cfg.output_p, SITE_OUT, 0);
   if (train_rnn_dropout(t->xa_last, t->xdrop, t->B, T, d, dr.thresh, dr.seed, dr.scale, st)) return -1;
   GemmEpi e; e.bias = m->head_b; e.out = t->logits; e.ldc = t->Vp; e.out_mode = GEMM_OUT_F32;
@@ -566,6 +587,8 @@ void dmg_train_destroy(dmg_model* m) {
   cudaSetDevice(m->device);
   cudaDeviceSynchronize();
   for (void* p : m->train->allocs) cudaFree(p);
+  cudaFree(m->train->eval_tab);
+  cudaFree(m->train->eval_part);
   delete m->train;
   m->train = nullptr;
 }
@@ -724,6 +747,7 @@ int dmg_train_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_d
   dmg_train* t = m->train;
   t->ids = (const long long*)ids_dev; t->pos = (const long long*)pos_dev;
   t->win = mask_win; t->k = mask_k; t->training = training ? 1 : 0; t->step = step;
+  t->eval_last = false;
   if (t->bert ? train_forward_bert(m, t, t->ids, t->pos, (const long long*)targets_dev, (cudaStream_t)stream)
               : train_forward(m, t, t->ids, t->pos, (const long long*)targets_dev, (cudaStream_t)stream)) return -1;
   t->next_layer = targets_dev ? m->cfg.n_layers : -1;
@@ -735,6 +759,8 @@ int dmg_train_backward(dmg_model* m, int layer_hi, int layer_lo, void* stream) {
   dmg_train* t = m->train;
   const int L = m->cfg.n_layers;
   DMG_CHECK(layer_hi >= layer_lo && layer_lo >= 0 && layer_hi <= L, "dmg_train_backward: bad slice [%d, %d)", layer_lo, layer_hi);
+  DMG_CHECK(!t->eval_last, "dmg_train_backward: the latest forward was a validation batch (dmg_train_eval_batch), which saves nothing "
+            "for a backward; run dmg_train_forward with targets first");
   DMG_CHECK(t->next_layer == layer_hi, "dmg_train_backward: slice starts at layer %d but %d is next (forward with targets first, slices in descending order)",
             layer_hi, t->next_layer);
   DMG_CUDA_OK(cudaSetDevice(m->device));
@@ -749,6 +775,75 @@ int dmg_train_backward(dmg_model* m, int layer_hi, int layer_lo, void* stream) {
     t->next_layer = -1;
   }
   return 0;
+}
+
+int dmg_train_eval_begin(dmg_model* m, int max_batches) {
+  if (check_train(m, "dmg_train_eval_begin")) return -2;
+  DMG_CHECK(max_batches >= 1, "dmg_train_eval_begin: max_batches %d must be at least 1", max_batches);
+  dmg_train* t = m->train;
+  DMG_CUDA_OK(cudaSetDevice(m->device));
+  DMG_CUDA_OK(cudaDeviceSynchronize());   // a previous table may still be read by queued work
+  if (t->eval_part == nullptr) DMG_CUDA_OK(cudaMalloc(&t->eval_part, (size_t)EVAL_PART_SLOTS * 3 * sizeof(double)));
+  if (t->eval_cap < max_batches) {
+    cudaFree(t->eval_tab);
+    t->eval_tab = nullptr;
+    t->eval_cap = 0;
+    DMG_CUDA_OK(cudaMalloc(&t->eval_tab, (size_t)max_batches * 3 * sizeof(double)));
+    t->eval_cap = max_batches;
+  }
+  DMG_CUDA_OK(cudaMemset(t->eval_tab, 0, (size_t)t->eval_cap * 3 * sizeof(double)));
+  DMG_CUDA_OK(cudaDeviceSynchronize());
+  t->eval_max = max_batches;
+  t->eval_n = 0;
+  t->eval_open = true;
+  return 0;
+}
+
+int dmg_train_eval_batch(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, const int64_t* targets_dev, void* stream) {
+  if (check_train(m, "dmg_train_eval_batch")) return -2;
+  dmg_train* t = m->train;
+  DMG_CHECK(t->eval_open, "dmg_train_eval_batch: no validation table (call dmg_train_eval_begin first)");
+  DMG_CHECK(t->eval_n < t->eval_max, "dmg_train_eval_batch: batch %d is past max_batches = %d of dmg_train_eval_begin", t->eval_n + 1,
+            t->eval_max);
+  DMG_CHECK(ids_dev && targets_dev, "dmg_train_eval_batch: null ids or targets");
+  DMG_CHECK(!t->bert || pos_dev, "dmg_train_eval_batch: the remix encoder adds beat/bar embeddings, pos is required");
+  DMG_CHECK(!m->cfg.encode_position || pos_dev, "dmg_train_eval_batch: model encodes position but pos is NULL");
+  DMG_CUDA_OK(cudaSetDevice(m->device));
+  // model.eval(): no dropout, the (1,1) mask; ids / pos / step of the latest training forward stay as they are
+  t->win = 1; t->k = 1; t->training = 0;
+  t->eval_fwd = true;
+  t->eval_targets = (const long long*)targets_dev;
+  const int rc = t->bert ? train_forward_bert(m, t, (const long long*)ids_dev, (const long long*)pos_dev, nullptr, (cudaStream_t)stream)
+                         : train_forward(m, t, (const long long*)ids_dev, (const long long*)pos_dev, nullptr, (cudaStream_t)stream);
+  t->eval_fwd = false;
+  t->eval_targets = nullptr;
+  t->eval_last = true;
+  t->next_layer = -1;
+  if (rc) return -1;
+  t->eval_n++;
+  return 0;
+}
+
+int dmg_train_eval_end(dmg_model* m, double* out_host, int n_batches, void* stream) {
+  if (check_train(m, "dmg_train_eval_end")) return -2;
+  dmg_train* t = m->train;
+  DMG_CHECK(t->eval_open, "dmg_train_eval_end: no validation table (call dmg_train_eval_begin first)");
+  DMG_CHECK(out_host, "dmg_train_eval_end: null output");
+  DMG_CHECK(n_batches == t->eval_n, "dmg_train_eval_end: n_batches = %d but %d batches were validated", n_batches, t->eval_n);
+  DMG_CUDA_OK(cudaSetDevice(m->device));
+  t->eval_open = false;
+  if (n_batches == 0) return 0;
+  DMG_CUDA_OK(cudaMemcpyAsync(out_host, t->eval_tab, (size_t)n_batches * 3 * sizeof(double), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  DMG_CUDA_OK(cudaStreamSynchronize((cudaStream_t)stream));
+  return 0;
+}
+
+int dmg_eval_metrics(const float* logits_dev, int64_t ldl, const int64_t* targets_dev, int64_t ignore, int rows, int V, double* out3_dev,
+                     void* stream) {
+  DMG_CHECK(logits_dev && targets_dev && out3_dev, "dmg_eval_metrics: null argument");
+  DMG_CHECK(rows >= 0 && V >= 1 && ldl >= V, "dmg_eval_metrics: rows %d, V %d, ldl %lld (need rows >= 0, V >= 1, ldl >= V)", rows, V,
+            (long long)ldl);
+  return train_eval_metrics(logits_dev, ldl, (const long long*)targets_dev, ignore, rows, V, nullptr, out3_dev, (cudaStream_t)stream);
 }
 
 int dmg_train_grad_span(dmg_model* m, int layer_hi, int layer_lo, int64_t* offset, int64_t* count) {

@@ -323,6 +323,78 @@ __global__ void __launch_bounds__(256) train_count_kernel(const long long* __res
   }
 }
 
+// ------------------------------------------------------------------ validation metrics
+// (value, index) order of torch.argmax: NaN above everything, then the larger value, then the lower index
+__device__ __forceinline__ bool argmax_better(float v, int i, float bv, int bi) {
+  const bool vn = isnan(v), bn = isnan(bv);
+  if (vn != bn) return vn;
+  if (vn || v == bv) return i < bi;
+  return v > bv;
+}
+
+// One warp per row (rows strided over the grid in a fixed assignment): the first maximal index, then logsumexp.  Lane 0 of
+// each warp sums its rows in row order; the block adds its 8 warps in order and writes (ce_sum, kept, correct) to part[block].
+// No floating-point atomics: the result depends on the grid size only, which depends on `rows` only.
+__global__ void __launch_bounds__(256) train_eval_metrics_kernel(const float* __restrict__ logits, long long ldl,
+                                                                 const long long* __restrict__ targets, long long ignore, int rows,
+                                                                 int V, double* __restrict__ part) {
+  __shared__ double red[8][3];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double ce = 0.0, kept = 0.0, correct = 0.0;
+  for (int row = blockIdx.x * 8 + warp; row < rows; row += gridDim.x * 8) {
+    long long tg = targets[row];
+    if (ignore >= 0 && tg == ignore) continue;
+    tg = tg < 0 ? 0 : (tg >= V ? V - 1 : tg);      // as train_ce_kernel
+    const float* lr = logits + (long long)row * ldl;
+    float mx = -INFINITY;
+    int am = 0x7fffffff;
+#pragma unroll 4
+    for (int c = lane; c < V; c += 32) {
+      const float x = lr[c];
+      if (argmax_better(x, c, mx, am)) { mx = x; am = c; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float omx = __shfl_xor_sync(0xffffffffu, mx, o);
+      const int oam = __shfl_xor_sync(0xffffffffu, am, o);
+      if (argmax_better(omx, oam, mx, am)) { mx = omx; am = oam; }
+    }
+    float se = 0.f;
+#pragma unroll 4
+    for (int c = lane; c < V; c += 32) se += expf(lr[c] - mx);
+    se = warp_sum(se);
+    if (lane == 0) {
+      ce += (double)(mx - lr[tg]) + (double)logf(se);
+      kept += 1.0;
+      correct += am == (int)tg ? 1.0 : 0.0;
+    }
+  }
+  if (lane == 0) { red[warp][0] = ce; red[warp][1] = kept; red[warp][2] = correct; }
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    double s = 0.0;
+    for (int w = 0; w < 8; w++) s += red[w][threadIdx.x];
+    part[blockIdx.x * 3 + threadIdx.x] = s;
+  }
+}
+
+// out3 = the sums of the n partial triples, in a fixed order (one block)
+__global__ void __launch_bounds__(96) train_eval_metrics_final_kernel(const double* __restrict__ part, int n, double* __restrict__ out3) {
+  __shared__ double red[96];
+  const int k = threadIdx.x % 3, j0 = threadIdx.x / 3;     // 32 strided lanes per quantity
+  double s = 0.0;
+  for (int j = j0; j < n; j += 32) s += part[j * 3 + k];
+  red[threadIdx.x] = s;
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    double t = 0.0;
+    for (int j = 0; j < 32; j++) t += red[j * 3 + threadIdx.x];
+    out3[threadIdx.x] = t;
+  }
+}
+
+__device__ double g_eval_part[EVAL_PART_SLOTS * 3];   // scratch of the test entry dmg_eval_metrics: one per device, not reentrant
+
 // dst[r, c] += src[r, c] (bf16, fp32 sum), n even
 __global__ void __launch_bounds__(256) train_add_bf16_kernel(bf16* __restrict__ dst, long long ldd, const bf16* __restrict__ src,
                                                              long long lds, int rows, int n) {
@@ -649,6 +721,18 @@ int train_ce_loss_masked(const float* logits, long long ldl, const long long* ta
   if (launch_np(train_count_kernel, dim3(1), dim3(256), 0, st, targets, rows, ignore, count)) return -1;
   return launch_np(train_ce_kernel<true>, dim3((rows + 7) / 8), dim3(256), 0, st, logits, ldl, targets, dlogits, loss_acc, rows, V, 0.f,
                    ignore, (const float*)count);
+}
+
+int train_eval_metrics(const float* logits, long long ldl, const long long* targets, long long ignore, int rows, int V, double* part,
+                       double* out3, cudaStream_t st) {
+  DMG_CHECK(logits && targets && out3 && rows >= 0 && V >= 1 && ldl >= V, "eval metrics: bad arguments (rows %d, V %d, ldl %lld)", rows,
+            V, ldl);
+  if (part == nullptr) DMG_CUDA_OK(cudaGetSymbolAddress((void**)&part, g_eval_part));
+  int g = (rows + 7) / 8;
+  if (g > EVAL_PART_SLOTS) g = EVAL_PART_SLOTS;
+  if (g < 1) g = 1;
+  if (launch_np(train_eval_metrics_kernel, dim3(g), dim3(256), 0, st, logits, ldl, targets, ignore, rows, V, part)) return -1;
+  return launch_np(train_eval_metrics_final_kernel, dim3(1), dim3(96), 0, st, (const double*)part, g, out3);
 }
 
 int train_add_bf16(bf16* dst, long long ldd, const bf16* src, long long lds, int rows, int n, cudaStream_t st) {

@@ -186,6 +186,13 @@ int train_ce_loss(const float* logits, long long ldl, const long long* targets, 
 // ignore target get no loss and zero dlogits, the others (softmax - onehot) / count.  loss_acc / count is the mean (NaN at count 0).
 int train_ce_loss_masked(const float* logits, long long ldl, const long long* targets, long long ignore, bf16* dlogits, float* loss_acc,
                          float* count, int rows, int V, cudaStream_t st);
+// Validation metrics of one batch, no gradient: out3[0] = sum over kept rows of logsumexp(row) - row[target], out3[1] = kept rows
+// (target != ignore; ignore < 0: every row), out3[2] = kept rows whose first maximal logit is the target.  Targets outside [0, V)
+// are clamped as in train_ce_loss.  Summed in a fixed order (per-block partials in `part`, EVAL_PART_SLOTS triples; NULL: a
+// module-wide scratch, for the test entry only: not reentrant), so a batch gives the same bits on every run.
+constexpr int EVAL_PART_SLOTS = 148 * 8;
+int train_eval_metrics(const float* logits, long long ldl, const long long* targets, long long ignore, int rows, int V, double* part,
+                       double* out3, cudaStream_t st);
 // output (RNN) dropout of the head input: xd[b,t,:] = xa[b,t,:] * mask[b,:]   (one mask per stream and feature)
 int train_rnn_dropout(const bf16* x, bf16* y, int B, int T, int d, uint32_t thresh, uint32_t seed, float scale,
                       cudaStream_t st);

@@ -7,6 +7,7 @@ multinomial -> bookkeeping) runs on the device without a host round trip per tok
 same loop over many independent streams (the batched-generation workload of BASELINE.json).
 """
 import ctypes as C
+import time
 
 import numpy as np
 import torch
@@ -45,10 +46,62 @@ def sampler_params(vocab, n_words, temperatures, min_bars, top_k, top_p, allowed
     return p
 
 
+def _load_checkpoint(learn, file):
+    """fastai Learner.load(with_opt=True) for a file of learn.save: the weights into the model, the Adam state into the live trainer
+    (if there is one), then the inference caches."""
+    state = torch.load(file, map_location='cpu', weights_only=False)
+    learn.model.load_state_dict(state['model'], strict=False)
+    tr = getattr(learn, '_trainer', None)
+    if tr is not None:
+        if state.get('opt'):
+            tr.load_opt_state_dict(state['opt'])
+        tr.sync_for_inference()
+    return learn
+
+
+def _epoch_end(learn, tr, epoch, t0, validate, metric, callbacks):
+    """fastai's end of an epoch in fit(): validate (if there are validation batches), one recorder row, the callbacks.  train_loss is
+    the last training batch's loss (dropout on; not fastai's smoothed value).  Returns True when a callback stops training."""
+    row = {'epoch': epoch, 'train_loss': tr.losses()['loss'], 'valid_loss': None, metric: None}
+    if validate is not None:
+        row['valid_loss'], row[metric] = validate()
+    row['time'] = time.time() - t0
+    learn.recorder.append(row)
+    stop = False
+    for cb in callbacks:
+        stop = bool(cb.on_epoch_end(epoch, row)) or stop
+    return stop
+
+
+def _trainer_for(learn, batches, x_of):
+    "the live trainer, or one sized by the first batch of `batches` (a list or a MusicPreloader)"
+    from .preloader import MusicPreloader
+    tr = getattr(learn, '_trainer', None)
+    if tr is not None:
+        return tr
+    if isinstance(batches, MusicPreloader):
+        return learn.trainer(batches.local_bs, batches.bptt)
+    x = x_of(batches[0])
+    return learn.trainer(x.shape[0], x.shape[1])
+
+
 class MusicLearner:
     "deep_music_genre.py:1811-1972"
     def __init__(self, data, model, config=None):
         self.data, self.model, self.config = data, model, config
+        self.recorder = []         # one row per epoch of fit_one_cycle(valid_batches=... or callbacks=...)
+
+    def load(self, file):
+        "Weights and Adam state of a learn.save file (fastai Learner.load)."
+        return _load_checkpoint(self, file)
+
+    def validate(self, valid_batches):
+        """fastai Learner.validate: [valid_loss, accuracy] of `valid_batches` (a list of (x, y[, pos]) [bs, bptt] or a MusicPreloader) in
+        eval mode, on the device (TXLTrainer.validate).  The training memory is reset first (fastai runs on_epoch_begin = RNNTrainer's
+        reset there) and carried across the batches.  Uses the live trainer, or creates one sized by the batches."""
+        tr = _trainer_for(self, valid_batches, lambda b: b[0]['x'] if isinstance(b[0], dict) else b[0])
+        r = tr.validate(valid_batches, reset=True)
+        return [r['valid_loss'], r['accuracy']]
 
     # -- checkpoints: {'model': state_dict (fastai key names), 'config': ...}  (:1812-1821, :1789-1805)
     def save(self, file=None, with_opt=True, config=None):
@@ -79,12 +132,19 @@ class MusicLearner:
         return self._trainer
 
     def fit_one_cycle(self, cyc_len, max_lr, batches, bs=None, bptt=None, wd=0.01, clip=0.5, moms=(0.95, 0.85), drop_mult=1.,
-                      callback=None):
+                      callback=None, valid_batches=None, callbacks=None):
         """learner.fit_one_cycle(epochs, lr) over `batches`: a list of (x, y[, pos]) LongTensors [bs, bptt], or a
         deepmusicgeneration_b200.preloader.MusicPreloader (the reference's contiguous streams with per-item random transpose,
         deep_music_genre.py:1001-1125, assembled on the GPU; every pass is a new epoch = new shuffle / transposes, like the
         reference's DataLoader): one-cycle LR / momentum schedule over all cyc_len passes, memory reset at every epoch start
-        (RNNTrainer.on_epoch_begin), Adam(true_wd), gradient clipping."""
+        (RNNTrainer.on_epoch_begin), Adam(true_wd), gradient clipping.
+
+        valid_batches (same forms, same [bs, bptt]): after every epoch the model is validated on them in eval mode, straight after
+        the training batches and without a memory reset, as fastai's fit loop does.  With valid_batches or callbacks
+        (callbacks.EarlyStoppingCallback, callbacks.SaveModelCallback), every epoch appends {'epoch', 'train_loss', 'valid_loss',
+        'accuracy', 'time'} to self.recorder (train_loss: the epoch's last batch loss, dropout on, read once per epoch - not
+        fastai's smoothed loss; time: seconds) and the callbacks may stop training early.  Without either, nothing is added to
+        the loop.  `callback(i, trainer)` still runs after every step."""
         from .training import one_cycle_lr
         from .preloader import MusicPreloader
         is_pl = isinstance(batches, MusicPreloader)
@@ -95,8 +155,16 @@ class MusicLearner:
             try:    tr.load_opt_state_dict(self.pretrained_opt_state)     # try / except: pass, like the reference
             except Exception: pass
             self.pretrained_opt_state = None
+        track = valid_batches is not None or bool(callbacks)
+        cbs = list(callbacks or [])
+        if track:
+            self.recorder = []
+            for cb in cbs:
+                cb.on_train_begin(self)
+        validate = (lambda: list(tr.validate(valid_batches, reset=False).values())) if valid_batches is not None else None
         total, i = cyc_len * n_b, 0
-        for _ in range(cyc_len):
+        for epoch in range(cyc_len):
+            t0 = time.time()
             tr.reset()
             for b in batches:
                 if is_pl:                           # (x, y) or ({'x', 'pos'}, y)
@@ -106,6 +174,10 @@ class MusicLearner:
                 if callback is not None:
                     callback(i, tr)
                 i += 1
+            if track and _epoch_end(self, tr, epoch, t0, validate, 'accuracy', cbs):
+                break
+        for cb in cbs:
+            cb.on_train_end()
         tr.sync_for_inference()
         return tr.losses()
 
@@ -250,6 +322,19 @@ class MultitaskLearner:
     "deep_music_remix.py:2479-2613 (mask task)."
     def __init__(self, data, model, config=None):
         self.data, self.model, self.config = data, model, config
+        self.recorder = []         # one row per epoch of fit_one_cycle(valid_batches=... or callbacks=...)
+
+    def load(self, file):
+        "Weights and Adam state of a learn.save file (fastai Learner.load)."
+        return _load_checkpoint(self, file)
+
+    def validate(self, valid_batches, mask_p=0.3, mask_range=None, seed=None):
+        """fastai Learner.validate of the mask task: [valid_loss, mask_acc] of `valid_batches` (already-masked ({'x', 'pos'}, y)
+        batches, or a MusicPreloader whose batches go through mask_tfm first; see RemixTrainer.validate), in eval mode on the device.
+        Uses the live trainer, or creates one sized by the batches."""
+        tr = _trainer_for(self, valid_batches, lambda b: b[0]['x'])
+        r = tr.validate(valid_batches, mask_p=mask_p, mask_range=mask_range, seed=seed, vocab=self.data.vocab)
+        return [r['valid_loss'], r['mask_acc']]
 
     def save(self, file=None, with_opt=True, config=None):
         """{'model': state_dict, 'opt': Adam state of the live trainer (None before any training or with with_opt=False)[, 'config']}:
@@ -279,13 +364,19 @@ class MultitaskLearner:
             self.trainer(bs, bptt, **kw).load_opt_state_dict(opt_state)
 
     def fit_one_cycle(self, cyc_len, max_lr, batches, bs=None, bptt=None, wd=0.01, clip=0.5, moms=(0.95, 0.85), drop_mult=1.,
-                      mask_p=0.3, mask_range=None, callback=None):
+                      mask_p=0.3, mask_range=None, callback=None, valid_batches=None, callbacks=None, valid_seed=None):
         """learner.fit_one_cycle(epochs, lr) of the mask task over `batches`: either a list of already-masked ({'x', 'pos'}, y)
         batches (LongTensors [bs, bptt], y = pad_idx where nothing is predicted), or a deepmusicgeneration_b200.preloader.MusicPreloader
         built with y_offset=0 and encode_position=True, whose every batch goes through mask_tfm(p=mask_p, mask_range) on the device
         (deep_music_remix.py:1208-1223).  The default mask_range is (vocab.note_range[0], vocab.dur_range[1]), the range the
         preloader golden (tests/golden/make_preloader_golden.py) was generated with.  One-cycle LR / momentum schedule over all
-        cyc_len passes, Adam(true_wd), gradient clipping; returns the last step's losses."""
+        cyc_len passes, Adam(true_wd), gradient clipping; returns the last step's losses.
+
+        valid_batches (same forms, same [bs, bptt]; a preloader's batches are masked with mask_p / mask_range, seeded by valid_seed):
+        validated in eval mode after every epoch.  With valid_batches or callbacks (callbacks.EarlyStoppingCallback,
+        callbacks.SaveModelCallback), every epoch appends {'epoch', 'train_loss', 'valid_loss', 'mask_acc', 'time'} to self.recorder
+        (train_loss: the epoch's last batch loss, dropout on, read once per epoch - not fastai's smoothed loss; time: seconds) and
+        the callbacks may stop training early.  Without either, nothing is added to the loop."""
         from .training import one_cycle_lr
         from .preloader import MusicPreloader, mask_tfm
         vocab = self.data.vocab
@@ -299,8 +390,17 @@ class MultitaskLearner:
             try:    tr.load_opt_state_dict(self.pretrained_opt_state)     # try / except: pass, like the reference
             except Exception: pass
             self.pretrained_opt_state = None
+        track = valid_batches is not None or bool(callbacks)
+        cbs = list(callbacks or [])
+        if track:
+            self.recorder = []
+            for cb in cbs:
+                cb.on_train_begin(self)
+        validate = (lambda: list(tr.validate(valid_batches, mask_p=mask_p, mask_range=mask_range, seed=valid_seed,
+                                             vocab=vocab).values())) if valid_batches is not None else None
         total, i = cyc_len * n_b, 0
-        for _ in range(cyc_len):
+        for epoch in range(cyc_len):
+            t0 = time.time()
             for xb, y in batches:
                 if not isinstance(xb, dict):
                     raise ValueError('the remix encoder needs ({"x", "pos"}, y) batches (MusicPreloader(encode_position=True))')
@@ -312,6 +412,10 @@ class MultitaskLearner:
                 if callback is not None:
                     callback(i, tr)
                 i += 1
+            if track and _epoch_end(self, tr, epoch, t0, validate, 'mask_acc', cbs):
+                break
+        for cb in cbs:
+            cb.on_train_end()
         tr.sync_for_inference()
         return tr.losses()
 

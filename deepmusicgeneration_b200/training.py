@@ -40,6 +40,25 @@ def one_cycle_lr(step, total, lr_max, div_factor=25., pct_start=0.3, final_div=N
     return cos(lr_max, lr_max / final_div, pct), cos(moms[1], moms[0], pct)
 
 
+def _tuples(batches):
+    """(iterator of (x, y, pos or None), upper bound of its length) for a list of (x, y[, pos]) / ({'x', 'pos'}, y) batches or a
+    MusicPreloader (whose len() counts items, not batches)."""
+    from .preloader import MusicPreloader
+    if isinstance(batches, MusicPreloader):
+        n = batches.n_batches
+    else:
+        batches = batches if hasattr(batches, '__len__') else list(batches)
+        n = len(batches)
+
+    def gen():
+        for b in batches:
+            if isinstance(b[0], dict):
+                yield b[0]['x'], b[1], b[0].get('pos')
+            else:
+                yield b[0], b[1], (b[2] if len(b) > 2 else None)
+    return gen(), n
+
+
 class TXLTrainer:
     """One training step at a time.  ``model`` is the ``SequentialRNN`` mirror from ``model.get_language_model`` (bf16).
 
@@ -234,6 +253,82 @@ class TXLTrainer:
             if callback is not None:
                 callback(i, self)
 
+    # ------------------------------------------------------------------ validation
+    def _check_shape(self, what, t):
+        if t is not None and tuple(t.shape) != (self.bs, self.bptt):
+            raise ValueError(f'validation batch: {what} must be [bs, bptt] = [{self.bs}, {self.bptt}] like the training batches, '
+                             f'got {list(t.shape)}')
+
+    def _batches(self, batches):
+        """_tuples(batches); a list of batches has every shape checked here, before anything is launched (a MusicPreloader's batches
+        are checked one by one as they come)."""
+        it, n = _tuples(batches)
+        from .preloader import MusicPreloader
+        if not isinstance(batches, MusicPreloader):
+            tuples = list(it)
+            for x, y, pos in tuples:
+                for what, t in (('x', x), ('y', y), ('pos', pos)):
+                    self._check_shape(what, t)
+            it = iter(tuples)
+        return it, n
+
+    def _eval_table(self, batches, n_max):
+        """Forward-only eval-mode batches (x, y, pos) through dmg_train_eval_*: returns the per-batch table, float64 [n, 3] =
+        (CE sum, kept targets, correct argmax).  One device-to-host copy at the end, no sync per batch."""
+        dev, h = self.e.device, self.e.h
+        keep = []
+        with torch.cuda.device(dev):
+            check(self.lib.dmg_train_eval_begin(h, max(1, n_max)), 'dmg_train_eval_begin')
+            n = 0
+            for x, y, pos in batches:
+                for what, t in (('x', x), ('y', y), ('pos', pos)):
+                    self._check_shape(what, t)
+                x = x.to(dev, torch.int64).contiguous()
+                y = y.to(dev, torch.int64).contiguous()
+                pos = pos.to(dev, torch.int64).contiguous() if pos is not None else None
+                keep.append((x, y, pos))          # the launches read them asynchronously
+                check(self.lib.dmg_train_eval_batch(h, _ptr(x), _ptr(pos), _ptr(y), _stream_ptr()), 'dmg_train_eval_batch')
+                n += 1
+            tab = np.zeros((n, 3), dtype=np.float64)
+            check(self.lib.dmg_train_eval_end(h, tab.ctypes.data_as(C.c_void_p), n, _stream_ptr()), 'dmg_train_eval_end')
+        return tab
+
+    def _average(self, per_batch, weights):
+        """fastai's validate / AverageMetric: the batch-size-weighted mean of per-batch values ([n, k] float64).  Data parallel: the
+        per-batch values are first averaged over the ranks (one all-reduce, as the reference's AverageMultiMetric does for its metric;
+        here for the loss too, so that every rank holds the same bits and takes the same early-stopping decision)."""
+        vals = torch.from_numpy(np.ascontiguousarray(per_batch, dtype=np.float64))
+        if self.distributed:
+            # the table all-reduce needs the same number of batches on every rank: check it first (max of n and of -n)
+            n = torch.tensor([len(vals), -len(vals)], dtype=torch.int64, device=self.e.device)
+            torch.distributed.all_reduce(n, op=torch.distributed.ReduceOp.MAX, group=self.pg)
+            hi, lo = int(n[0]), -int(n[1])
+            if hi != lo:
+                raise ValueError(f'validation: the ranks validated between {lo} and {hi} batches; data-parallel validation needs the '
+                                 f'same number of batches on every rank')
+            if len(vals):
+                d = vals.to(self.e.device)
+                torch.distributed.all_reduce(d, group=self.pg)
+                vals = (d / self.world).cpu()
+        w = torch.as_tensor(np.asarray(weights, dtype=np.float64))
+        if len(vals) == 0:
+            return [float('nan')] * per_batch.shape[1]
+        return [float(v) for v in (vals * w[:, None]).sum(0) / w.sum()]
+
+    def validate(self, batches, reset=True):
+        """fastai Learner.validate for the language model: model.eval() over `batches` - (x, y) or (x, y, pos) LongTensors [bs, bptt],
+        or a MusicPreloader - with the training memory carried from batch to batch (``reset=True`` forgets it first, as fastai's
+        RNNTrainer.on_epoch_begin does).  Returns {'valid_loss': mean CrossEntropyFlat, 'accuracy': fraction of positions whose
+        argmax (first maximal logit) is the target}, each the batch-size-weighted mean over the batches.  Weights, optimizer state,
+        step_count and losses() are left as they were."""
+        it, n_max = self._batches(batches)
+        if reset:
+            self.reset()
+        tab = self._eval_table(it, n_max)
+        rows = float(self.bs * self.bptt)
+        loss, acc = self._average(np.stack([tab[:, 0] / rows, tab[:, 2] / rows], 1), [self.bs] * len(tab))
+        return {'valid_loss': loss, 'accuracy': acc}
+
     # ------------------------------------------------------------------ test / inspection helpers
     def grads(self):
         "name -> gradient (CPU fp32) in state-dict naming."
@@ -321,3 +416,32 @@ class RemixTrainer(TXLTrainer):
         if mask_size is not None and tuple(mask_size) != (1, 1):
             raise ValueError(f'RemixTrainer: the remix encoder has no attention mask, mask_size must be (1, 1), got {tuple(mask_size)}')
         return super().forward(x, y, pos, (1, 1))
+
+    def validate(self, batches, mask_p=0.3, mask_range=None, seed=None, vocab=None):
+        """fastai Learner.validate of the mask task: model.eval() over `batches` - already-masked ({'x', 'pos'}, y) or (x, y, pos)
+        batches [bs, bptt], or a MusicPreloader(y_offset=0, encode_position=True) whose batches go through mask_tfm(p=mask_p,
+        mask_range) first, as fastai applies the batch transforms to the validation loader too.  `seed` makes those masks (and so the
+        result) reproducible: batch i uses a seed derived from (seed, i); None draws them from torch's CPU generator.  `vocab` (default
+        MusicVocab.create()) gives mask_idx and the default mask_range (note_range[0], dur_range[1]).  Returns {'valid_loss': mean
+        CrossEntropyFlat(ignore_index=pad_idx), 'mask_acc': fraction of the predicted positions whose argmax is the target}: per
+        batch over its kept targets (NaN for a batch with none, as torch gives, and the NaN carries into the result), then the
+        batch-size-weighted mean.  Weights, optimizer state, step_count and losses() are left as they were."""
+        from .preloader import MusicPreloader, mask_tfm
+        it, n_max = self._batches(batches)
+        if isinstance(batches, MusicPreloader):
+            if vocab is None:
+                from .codec import MusicVocab
+                vocab = MusicVocab.create()
+            rng = mask_range or (vocab.note_range[0], vocab.dur_range[1])
+
+            def masked(src):
+                for i, (x, y, pos) in enumerate(src):
+                    s = None if seed is None else (int(seed) * 1000003 + 7919 * (i + 1)) & 0x7FFFFFFF
+                    xm, ym = mask_tfm((x, y), rng, vocab.mask_idx, self.pad_idx, p=mask_p, seed=s)
+                    yield xm, ym, pos
+            it = masked(it)
+        with np.errstate(invalid='ignore', divide='ignore'):
+            tab = self._eval_table(it, n_max)
+            per = np.stack([tab[:, 0] / tab[:, 1], tab[:, 2] / tab[:, 1]], 1)
+        loss, acc = self._average(per, [self.bs] * len(tab))
+        return {'valid_loss': loss, 'mask_acc': acc}

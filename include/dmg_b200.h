@@ -277,6 +277,23 @@ int64_t dmg_train_opt_steps(dmg_model* m, int64_t value);
  * the first optimizer step)} of the latest step.  DMG_ARCH_BERT: {mean CE over the targets != pad_idx (NaN if there are
  * none; the gradients are then zero), 0, 0, gradient norm}. */
 int dmg_train_losses(dmg_model* m, float* out4_host, void* stream);
+/* Validation (fastai Learner.validate: model.eval() over held-out batches, CrossEntropyFlat and the accuracy metric) without a host
+ * sync per batch.  dmg_train_eval_begin sizes and zeroes a device table of max_batches rows (the only allocation of a validation).
+ * dmg_train_eval_batch runs a forward-only eval-mode batch: no dropout, mask (1,1), nothing saved for a backward, no AR / TAR, no
+ * logit gradient; row b of the table receives {sum over kept rows of logsumexp - logit[target], kept rows, kept rows whose first
+ * maximal logit is the target}, kept = target != pad_idx for DMG_ARCH_BERT (which needs pos), every row for DMG_ARCH_TXL.  The
+ * Transformer-XL memory advances exactly as in a training forward.  It leaves weights, optimizer state and dmg_train_losses alone;
+ * a dmg_train_backward after it is refused.  dmg_train_eval_end copies the n_batches x 3 table (fp64, row-major; n_batches =
+ * the batches run since begin) to the host and synchronises the stream. */
+int dmg_train_eval_begin(dmg_model* m, int max_batches);
+int dmg_train_eval_batch(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, const int64_t* targets_dev, void* stream);
+int dmg_train_eval_end(dmg_model* m, double* out_host, int n_batches, void* stream);
+/* Unit-test entry of the validation metrics kernel: logits fp32 [rows, ldl] (valid width V), targets int64 [rows] (clamped to
+ * [0, V) as in the training loss), ignore < 0 for no ignore index; out3_dev (fp64, device) = {ce_sum, kept, correct} as above.
+ * Summed in a fixed order: the same input gives the same bits.  Not reentrant: its partial sums live in one module-wide device buffer
+ * per GPU, so two calls must not run concurrently on the same device (the trainer's own validation uses a buffer of its own). */
+int dmg_eval_metrics(const float* logits_dev, int64_t ldl, const int64_t* targets_dev, int64_t ignore, int rows, int V,
+                     double* out3_dev, void* stream);
 /* Tests: gradient of one parameter by its state-dict name; the dropout mask (keep ? 1/(1-p) : 0) of a site as the kernels
  * generate it (site 0 embedding [rows,d], 1 attention [B,H,T,S], 2 attention-residual [rows,d], 3 FFN inner [rows,d_inner],
  * 4 FFN residual [rows,d], 5 output RNN dropout [B,d]; DMG_ARCH_BERT uses 0, 1 [B,H,T,T], 2 and 5); the device pointer of the
