@@ -44,6 +44,17 @@ class TrainConfig(C.Structure):
                 ('reserved', c_i32 * 3)]
 
 
+class DecodeAttnArgs(C.Structure):
+    _fields_ = [(n, c_vp) for n in ('qkv', 'kring', 'vring', 'rd', 'u', 'v', 'out', 'state')] + [('pos_total', c_i64)] + \
+               [(n, c_i32) for n in ('B', 'H', 'Dh', 'M', 'Dcap', 'Bcap', 'b0', 'kernel')]
+
+
+class DecodeLayerArgs(C.Structure):
+    _fields_ = [(n, c_vp) for n in ('x32', 'attn', 'wo', 'w1', 'w2', 'wqkv', 'bo', 'ln1w', 'ln1b', 'b1', 'b2', 'ln2w', 'ln2b', 'bqkv',
+                                    'qkv', 'xa_out', 'pp')] + [('pp_stride', c_i64)] + \
+               [(n, c_i32) for n in ('attn_rows', 'row_base', 'B', 'mode', 'd_model', 'n_heads', 'd_head', 'd_inner')]
+
+
 # name -> (restype, argtypes): every symbol include/dmg_b200.h declares
 SYMBOLS = {
     'dmg_last_error': (C.c_char_p, []),
@@ -107,6 +118,9 @@ SYMBOLS = {
     'dmg_attn_train_bwd': (c_i32, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32,
                                    c_i32, c_i32, c_i32, c_f32, c_u32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'dmg_attn_bert_varlen': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp]),
+    'dmg_attn_decode': (c_i32, [C.POINTER(DecodeAttnArgs), c_vp]),
+    'dmg_decode_layer_step': (c_i32, [C.POINTER(DecodeLayerArgs), c_vp]),
+    'dmg_decode_dual': (c_i32, [C.POINTER(DecodeLayerArgs), C.POINTER(DecodeAttnArgs), c_i32, c_vp]),
     'dmg_attn_bert_train_fwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32, c_vp]),
     'dmg_attn_bert_train_bwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32,
                                         c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),

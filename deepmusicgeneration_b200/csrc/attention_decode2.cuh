@@ -176,14 +176,17 @@ __device__ __forceinline__ void attn_decode2_body(const CUtensorMap& tmK, const 
       pdl_wait();
       for (int it = lo, n = 0; it < hi; ++it, ++n) {
         const int h = it / B, b = it - h * B;
+        const int qs = n & 1;
+        // q slot first: it means the consumers are done with item n - 2, so r_free's phase n - 1 is the only phase of that parity
+        // that can still be open.  (Waiting on r_free first, with the consumers still scoring item n - 2, the finished phase n - 3
+        // has the parity of phase n - 1 and passed: the next head's Rd overwrote the keys of items n - 2 and n - 1.)
+        mbar_wait(&q_empty[qs], (uint32_t)(((n >> 1) & 1) ^ 1));
         if (h != cur_h) {
           if (cur_h >= 0) mbar_wait(r_free, (uint32_t)((n - 1) & 1));   // previous item's score phase is done with Rd
           mbar_expect_tx(r_full, (uint32_t)(L.r_boxes * 8192));
           for (int bx = 0; bx < L.r_boxes; bx++) tma_load_2d(Rres + bx * 8192, &tmR, 0, h * a.Dcap + bx * 64, r_full);
           cur_h = h;
         }
-        const int qs = n & 1;
-        mbar_wait(&q_empty[qs], (uint32_t)(((n >> 1) & 1) ^ 1));
         mbar_expect_tx(&q_full[qs], 768);
         const float* qrow = a.qkv + (size_t)b * 3 * HD + h * 64;
         bulk_g2s(qbuf + qs * 192, qrow, 256, &q_full[qs]);

@@ -389,7 +389,7 @@ __device__ __forceinline__ void decode_layer_body(const CUtensorMap& tmAttn, con
     }
     float acc[16];
     if (body) {
-      // ---- out-projection slice -> scratch P[row][feature]
+      // ---- out-projection slice
       mbar_wait(&tmem_full[0], 0);
       tc_fence_after();
       if (mk) dl_mark(a.dbg, 2, 2);

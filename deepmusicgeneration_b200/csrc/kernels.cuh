@@ -40,7 +40,6 @@ struct DecodeLayerArgs {
   float* x32;            // [rows, d] fp32 residual stream, in / out
   bf16* xa_out;          // [rows, d] bf16 copy of the final rows (input of the head GEMM) or NULL
   float* qkv;            // [rows, n3] fp32: the next layer's q|k|v (mode & 2)
-  float* P;              // scratch [rows padded to DL_ROWS, d] fp32: out-projection slices before LayerNorm 1
   float* PP;             // scratch [DL_CLUSTER][pp_stride] fp32: the FFN-down partial sums of the 8 K slices, [row, d] each
   long long pp_stride;   // elements between two slabs of PP
   const float *bo, *b1, *b2, *bq;            // biases (any may be NULL)

@@ -79,7 +79,7 @@ struct DecodeStep {
     LayerW& Lb = m->layers[body ? l - 1 : 0];        // the layer whose body runs
     LayerW& Ln = m->layers[next ? l : 0];            // the layer whose q|k|v are produced
     DecodeLayerArgs da;
-    da.x32 = m->x32; da.qkv = m->qkv; da.P = m->dl_P; da.PP = m->dl_PP; da.pp_stride = m->dl_pp_stride;
+    da.x32 = m->x32; da.qkv = m->qkv; da.PP = m->dl_PP; da.pp_stride = m->dl_pp_stride;
     da.row_base = r0; da.B = r1; da.d = c.d_model; da.HD = m->HD; da.di = c.d_inner; da.n3 = 3 * m->HD;
     da.mode = (body ? 1 : 0) | (next ? 2 : 0);
     da.dbg = (l == c.n_layers / 2 && r0 == 0) ? m->dl_dbg : nullptr;      // timeline probe: one mid-stack launch
@@ -579,10 +579,9 @@ int dmg_create(const dmg_config* cfg, int device, dmg_model** out) {
       if (bufs[i] == nullptr || m->a_cols[i] % 64 != 0) continue;
       TRY(make_tmap_bf16(&m->tmA[i], bufs[i], m->a_cols[i], m->a_rows[i], m->a_cols[i], 128));
     }
-    // fused one-token layer step: the out-projection scratch is `proj` (unused by that path otherwise), the FFN-down partial sums
-    // get their own [8][rows, d] fp32 scratch; DL_ROWS-row boxes over the attention output
+    // fused one-token layer step: the FFN-down partial sums get their own [8][rows, d] fp32 scratch; DL_ROWS-row boxes over the
+    // attention output
     if (!rc && !bert && c.mem_len > 0 && !(m->kflags & DMG_KF_NO_FUSED_DECODE) && decode_layer_supported(d, HD, c.d_inner, 3 * HD)) {
-      m->dl_P = m->proj;
       m->dl_rows = (int)(R < 512 ? R : 512);                      // one-token steps run max_batch <= 512 rows through this path
       m->dl_pp_stride = (long long)m->dl_rows * d;
       TRY(dalloc(m, &m->dl_PP, (size_t)DL_CLUSTER * m->dl_pp_stride));
@@ -994,6 +993,142 @@ int dmg_decode_dual_launch(dmg_model* m, int layer, void* stream) {
   int hx = 0;
   DMG_CHECK(m->fused_decode && ds.pipelined(m->batch, &hx), "dmg_decode_dual_launch: the two-half pipeline is off for this model / batch");
   return ds.dual(layer + 1, 0, hx, layer, hx, m->batch);      // A_layer(second half) + F_{layer+1}(first half), as in the step
+}
+
+}  // extern "C"
+
+// ---- unit-test entries of the one-token decode kernels: the checks and tensor maps of dmg_attn_decode / dmg_decode_layer_step /
+// dmg_decode_dual, made before anything is launched
+namespace dmg {
+
+static_assert(sizeof(dmg_decode_attn_args) == 104 && sizeof(dmg_decode_layer_args) == 176, "tests/test_abi.py mirrors these layouts");
+
+struct DecodeAttnPlan {
+  AttnDecodeArgs a;
+  TensorMap2D tmK, tmV, tmR;
+  int b0 = 0, num_sms = 0;
+  int state[2] = {0, 0};
+};
+
+static int plan_decode_attn(const dmg_decode_attn_args* p, DecodeAttnPlan& o, const char* who) {
+  DMG_CHECK(p && p->qkv && p->kring && p->vring && p->rd && p->u && p->v && p->out && p->state, "%s: null argument", who);
+  DMG_CHECK(p->Dh == 64, "%s: head size %d (only 64)", who, p->Dh);
+  DMG_CHECK(p->kernel == 0 || p->kernel == 1, "%s: kernel %d (0 = the step's choice, 1 = the second-generation kernel)", who, p->kernel);
+  // kernel 0 falls back to the second kernel where the third does not apply, so both choices need what the second one supports
+  DMG_CHECK(attn_decode2_supported(64, p->M), "%s: mem_len %d not supported by the decode attention", who, p->M);
+  DMG_CHECK(p->Dcap >= p->M + 1, "%s: rel-pos cache too small (Dcap %d < M + 1 = %d)", who, p->Dcap, p->M + 1);
+  DMG_CHECK(p->B >= 1 && p->H >= 1 && p->H <= 64 && p->b0 >= 0 && (long long)p->b0 + p->B <= p->Bcap,
+            "%s: B %d, H %d, streams [%d, %d) outside the ring's %d", who, p->B, p->H, p->b0, p->b0 + p->B, p->Bcap);
+  DMG_CHECK(p->pos_total >= 0 && p->pos_total <= 0x7fffffffLL, "%s: pos_total %lld outside [0, 2^31)", who, (long long)p->pos_total);
+  const long long ring_rows = (long long)p->Bcap * p->H * p->M;
+  if (make_tmap_bf16(&o.tmK, p->kring, 64, ring_rows, 64, 64) || make_tmap_bf16(&o.tmV, p->vring, 64, ring_rows, 64, 64) ||
+      make_tmap_bf16(&o.tmR, p->rd, 64, (long long)p->H * p->Dcap, 64, 64)) return -1;
+  int dev = 0;
+  DMG_CUDA_OK(cudaGetDevice(&dev));
+  DMG_CUDA_OK(cudaDeviceGetAttribute(&o.num_sms, cudaDevAttrMultiProcessorCount, dev));
+  AttnDecodeArgs& a = o.a;
+  const size_t chunk = (size_t)p->b0 * p->H * p->M * 64;      // the kernels take ring pointers offset by b0 streams
+  a.qkv = p->qkv; a.kring = (bf16*)p->kring + chunk; a.vring = (bf16*)p->vring + chunk; a.rd = (const bf16*)p->rd;
+  a.u = p->u; a.v = p->v; a.out = (bf16*)p->out; a.dev_state = p->state;
+  a.B = p->B; a.H = p->H; a.M = p->M; a.Dcap = p->Dcap;
+  a.scale = 0.125f;
+  a.force_v2 = p->kernel;
+  o.b0 = p->b0;
+  o.state[0] = (int)p->pos_total;
+  o.state[1] = (int)(p->pos_total < p->M ? p->pos_total : p->M);   // mem_count, as state_advance keeps it
+  return 0;
+}
+
+struct DecodeLayerPlan {
+  DecodeLayerArgs a;
+  TensorMap2D tmAttn, tmWo, tmW1, tmW2, tmWq;
+};
+
+static int plan_decode_layer(const dmg_decode_layer_args* p, DecodeLayerPlan& o, const char* who) {
+  DMG_CHECK(p, "%s: null argument", who);
+  const bool body = (p->mode & 1) != 0, next = (p->mode & 2) != 0;
+  DMG_CHECK(p->mode >= 1 && p->mode <= 3, "%s: mode %d (bit 0 = layer body, bit 1 = next q|k|v)", who, p->mode);
+  const int HD = p->n_heads * p->d_head;
+  DMG_CHECK(p->d_head == 64 && decode_layer_supported(p->d_model, HD, p->d_inner, 3 * HD),
+            "%s: geometry d_model %d, %d heads of %d, d_inner %d not supported", who, p->d_model, p->n_heads, p->d_head, p->d_inner);
+  DMG_CHECK(p->x32 && p->pp, "%s: null argument", who);
+  DMG_CHECK(!body || (p->attn && p->wo && p->w1 && p->w2 && p->ln1w && p->ln1b && p->ln2w && p->ln2b), "%s: null argument (layer body)", who);
+  DMG_CHECK(!next || (p->wqkv && p->qkv), "%s: null argument (next q|k|v)", who);
+  DMG_CHECK(p->row_base >= 0 && p->B > p->row_base, "%s: rows [%d, %d) empty", who, p->row_base, p->B);
+  DMG_CHECK(!body || p->attn_rows >= p->B, "%s: attn_rows %d < B %d", who, p->attn_rows, p->B);
+  const long long rows_pad = p->row_base + (long long)(p->B - p->row_base + DL_ROWS - 1) / DL_ROWS * DL_ROWS;
+  DMG_CHECK(p->pp_stride >= rows_pad * p->d_model, "%s: pp_stride %lld < %lld rows x %d (whole %d-row clusters are written)", who,
+            (long long)p->pp_stride, rows_pad, p->d_model, DL_ROWS);
+  const int d = p->d_model, di = p->d_inner;
+  // the kernel takes all five maps; a weight the mode does not read gets the map of one it does
+  if (body) {
+    if (make_tmap_bf16(&o.tmAttn, p->attn, HD, p->attn_rows, HD, DL_ROWS) || make_tmap_bf16(&o.tmWo, p->wo, HD, d, HD, 64) ||
+        make_tmap_bf16(&o.tmW1, p->w1, d, di, d, 64) || make_tmap_bf16(&o.tmW2, p->w2, di, d, di, 64)) return -1;
+  }
+  if (next && make_tmap_bf16(&o.tmWq, p->wqkv, d, 3 * HD, d, 64)) return -1;
+  if (!body) o.tmAttn = o.tmWo = o.tmW1 = o.tmW2 = o.tmWq;
+  if (!next) o.tmWq = o.tmWo;
+  DecodeLayerArgs& a = o.a;
+  a.x32 = p->x32; a.xa_out = (bf16*)p->xa_out; a.qkv = p->qkv; a.PP = p->pp; a.pp_stride = p->pp_stride;
+  a.bo = p->bo; a.b1 = p->b1; a.b2 = p->b2; a.bq = p->bqkv;
+  a.ln1w = p->ln1w; a.ln1b = p->ln1b; a.ln2w = p->ln2w; a.ln2b = p->ln2b;
+  a.row_base = p->row_base; a.B = p->B;
+  a.d = d; a.HD = HD; a.di = di; a.n3 = 3 * HD;
+  a.mode = p->mode;
+  return 0;
+}
+
+}  // namespace dmg
+
+extern "C" {
+
+int dmg_attn_decode(const dmg_decode_attn_args* p, void* stream) {
+  DecodeAttnPlan o;
+  if (plan_decode_attn(p, o, "dmg_attn_decode")) return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  DMG_CUDA_OK(cudaMemcpyAsync(p->state, o.state, sizeof(o.state), cudaMemcpyHostToDevice, st));
+  const int rc = attn_decode2(&o.tmK, &o.tmV, &o.tmR, o.a, o.b0, o.num_sms, st);
+  const cudaError_t e = cudaStreamSynchronize(st);
+  if (rc) return rc;
+  DMG_CUDA_OK(e);
+  return 0;
+}
+
+int dmg_decode_layer_step(const dmg_decode_layer_args* f, void* stream) {
+  DecodeLayerPlan o;
+  if (plan_decode_layer(f, o, "dmg_decode_layer_step")) return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int rc = decode_layer(&o.tmAttn, &o.tmWo, &o.tmW1, &o.tmW2, &o.tmWq, o.a, st);
+  const cudaError_t e = cudaStreamSynchronize(st);
+  if (rc) return rc;
+  DMG_CUDA_OK(e);
+  return 0;
+}
+
+int dmg_decode_dual(const dmg_decode_layer_args* f, const dmg_decode_attn_args* a, int attn_clusters, void* stream) {
+  DecodeLayerPlan lo;
+  DecodeAttnPlan ao;
+  if (plan_decode_layer(f, lo, "dmg_decode_dual") || plan_decode_attn(a, ao, "dmg_decode_dual")) return -1;
+  DMG_CHECK(a->kernel == 0 && decode_dual_supported(a->M), "dmg_decode_dual: the attention role runs the third-generation kernel only "
+            "(kernel 0, M a multiple of 128 up to 512; got kernel %d, M %d)", a->kernel, a->M);
+  DMG_CHECK(attn_clusters >= 0, "dmg_decode_dual: attn_clusters %d", attn_clusters);
+  const long long items = (long long)a->B * a->H;
+  if (attn_clusters == 0) {   // as DecodeStep::dual sizes the attention role
+    const int n_fused = (f->B - f->row_base + DL_ROWS - 1) / DL_ROWS;
+    attn_clusters = decode_dual_max_clusters() - n_fused;
+    if ((long long)attn_clusters * DL_CLUSTER > items) attn_clusters = (int)((items + DL_CLUSTER - 1) / DL_CLUSTER);
+    DMG_CHECK(attn_clusters >= 1, "dmg_decode_dual: no cluster left for the attention role");
+  }
+  DMG_CHECK(items <= decode_dual_max_items(attn_clusters), "dmg_decode_dual: %d x %d items do not fit %d attention clusters", a->B,
+            a->H, attn_clusters);
+  cudaStream_t st = (cudaStream_t)stream;
+  DMG_CUDA_OK(cudaMemcpyAsync(a->state, ao.state, sizeof(ao.state), cudaMemcpyHostToDevice, st));
+  const int rc = decode_dual(&lo.tmAttn, &lo.tmWo, &lo.tmW1, &lo.tmW2, &lo.tmWq, lo.a, &ao.tmK, &ao.tmV, &ao.tmR, ao.a, ao.b0,
+                             attn_clusters, st);
+  const cudaError_t e = cudaStreamSynchronize(st);
+  if (rc) return rc;
+  DMG_CUDA_OK(e);
+  return 0;
 }
 
 int dmg_gemm_bf16(const void* a_dev, const void* w_dev, const float* bias_dev, void* c_dev, int M, int N, int K, int gelu,

@@ -69,7 +69,7 @@ struct dmg_model {
   TensorMap2D tmA[A_COUNT];
   // fused one-token layer step (decode_layer.cu)
   bool fused_decode = false;
-  float *dl_P = nullptr, *dl_PP = nullptr;
+  float* dl_PP = nullptr;
   long long dl_pp_stride = 0;
   int dl_rows = 0, dl_max_clusters = 0;
   bool dl_dual = false;                    // the two-half software pipeline with dual-role launches

@@ -342,6 +342,57 @@ int dmg_attn_bert_train_bwd(const void* qkv_x, int64_t ldx, const void* rk, cons
 int dmg_attn_bert_varlen(const void* qkv_dev, const void* rk_dev, int Dcap, const float* u, const float* v, void* out_dev,
                          const int32_t* lens_host, int B, int T_max, int H, int mma_sync_only, void* stream);
 
+/* Unit-test entries of the one-token decode kernels (attention_decode2.cuh, attention_decode3.cuh, decode_layer.cu) on caller-owned
+ * buffers, laid out as the model lays them out.  Arguments are checked before anything is launched; each entry synchronises the stream.
+ *
+ * dmg_decode_attn_args: the decode attention over the bf16 K/V ring for rows [0, B) of qkv / out, ring streams [b0, b0 + B).
+ *   qkv fp32 [B, 3*H*Dh] (q | k | v of the new token); kring / vring bf16 [Bcap][H][M][Dh]; rd bf16 [H][Dcap][Dh] (rel-pos keys by
+ *   distance); u / v fp32 [H*Dh]; out bf16 [B, H*Dh]; state a device int32[2] that receives {pos_total, min(pos_total, M)} (the
+ *   invariant the model's ring state keeps) and that the kernel reads.  The kernel reads the M ring slots, then writes the new
+ *   token's k / v (rounded to bf16) into slot pos_total % M.  kernel: 0 = what the one-token step runs (the third-generation kernel where
+ *   it supports M, else the second), 1 = the second-generation kernel.  Dh must be 64, Dcap >= M + 1.
+ *   Precondition: the kernels request their first K/V tiles before they wait for the previous kernel on the stream, so the ring must
+ *   not have been written by the kernel launched immediately before on the same stream (synchronise after preparing it). */
+typedef struct dmg_decode_attn_args {
+  const float* qkv;
+  void* kring;
+  void* vring;
+  const void* rd;
+  const float* u;
+  const float* v;
+  void* out;
+  int32_t* state;
+  int64_t pos_total;
+  int32_t B, H, Dh, M, Dcap, Bcap, b0, kernel;
+} dmg_decode_attn_args;
+int dmg_attn_decode(const dmg_decode_attn_args* a, void* stream);
+
+/* dmg_decode_layer_args: the fused one-token layer step over rows [row_base, B) (d_model 512, d_inner 2048, 8 heads of 64: the
+ * geometry the kernel supports).  mode bit 0 = layer body: x32 = LN2(x1 + W2 gelu_tanh(W1 x1 + b1) + b2) with
+ * x1 = LN1(x32 + attn Wo^T + bo), also copied to xa_out (bf16, nullable); bit 1 = the next layer's q|k|v = Wqkv x32 + bqkv into
+ * qkv (fp32 [B, 3*H*64]).  x32 fp32 [B, 512] in / out; attn bf16 [attn_rows, H*64], attn_rows >= B (rows past B are read and their
+ * results discarded); weights bf16 in nn.Linear layout; biases fp32 (nullable), LayerNorm weights fp32.  pp: fp32 scratch of 8 slabs
+ * pp_stride elements apart; the kernel writes the partial sums of whole 32-row clusters, so pp_stride >=
+ * (row_base + round_up(B - row_base, 32)) * 512. */
+typedef struct dmg_decode_layer_args {
+  float* x32;
+  const void* attn;
+  const void *wo, *w1, *w2, *wqkv;
+  const float *bo, *ln1w, *ln1b, *b1, *b2, *ln2w, *ln2b, *bqkv;
+  float* qkv;
+  void* xa_out;
+  float* pp;
+  int64_t pp_stride;
+  int32_t attn_rows, row_base, B, mode;
+  int32_t d_model, n_heads, d_head, d_inner;
+} dmg_decode_layer_args;
+int dmg_decode_layer_step(const dmg_decode_layer_args* f, void* stream);
+
+/* The dual-role launch of the pipelined one-token step: the fused layer step `f` and the attention `a` (the third-generation kernel:
+ * a->kernel must be 0 and M supported by it) in ONE launch.  attn_clusters = 0: as many 8-CTA attention clusters as the step gives
+ * it (the co-resident clusters left by the fused role, at most one per 8 items); > 0: that many, if the items fit them. */
+int dmg_decode_dual(const dmg_decode_layer_args* f, const dmg_decode_attn_args* a, int attn_clusters, void* stream);
+
 /* ---- training data feed (SURVEY.md section 8 f4) ------------------------------------------------------------------------
  * dmg_preload_fill = MusicPreloader.__getitem__ / fill_row (deep_music_genre.py:1088-1125) for all `bs` rows of one batch.
  * Everything is device memory: `tokens` / `positions` the flat ragged corpus (int32), `offsets` [n_items+1] (int64), `perm` the

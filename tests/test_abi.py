@@ -41,6 +41,10 @@ def test_struct_layouts_match_header():
     assert C.sizeof(_lib.VocabLayout) == 14 * 4
     assert C.sizeof(_lib.SamplerParams) == 3 * 8 + 4 * 4 + 2 * 4 + 8
     assert _lib.SamplerParams.seed.offset == 48
+    assert C.sizeof(_lib.DecodeAttnArgs) == 8 * 8 + 8 + 8 * 4
+    assert _lib.DecodeAttnArgs.pos_total.offset == 64 and _lib.DecodeAttnArgs.kernel.offset == 100
+    assert C.sizeof(_lib.DecodeLayerArgs) == 17 * 8 + 8 + 8 * 4
+    assert _lib.DecodeLayerArgs.pp_stride.offset == 136 and _lib.DecodeLayerArgs.d_inner.offset == 172
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason='CPU-only check')
