@@ -15,8 +15,8 @@
 // Backward = three kernels, none with floating-point atomics on activations:
 //   attn_delta_kernel : delta_i = dO_i . O_i
 //   attn_bwd_dq_kernel: query-tile owner; recomputes P, forms dS, accumulates dQ (content + position parts -> du, dv),
-//                       writes dS in (row, distance) coordinates for the dRk GEMM (ds_dist)
-//   attn_bwd_dkv_kernel: key-tile owner; recomputes P and dS, accumulates dK, dV
+//                       writes dS in (row, distance) coordinates for the dRk GEMM (ds_dist) and spills P (dropped) and dS
+//   attn_bwd_dkv_lite_kernel: key-tile owner; accumulates dK, dV from the spilled P and dS tiles
 #include "kernels.cuh"
 #include "launch.cuh"
 #include "attention_train_common.cuh"
@@ -223,14 +223,13 @@ __global__ void __launch_bounds__(256) attn_delta_kernel(const bf16* __restrict_
   }
 }
 
-// recompute P (normalised), dP and dS for one tile; returns ds (scaled gradient wrt AC+BD) and pd (dropped P) in s / pd
+// recompute P (normalised), dP and dS for one tile; returns ds (scaled gradient wrt AC+BD) in s
 __device__ __forceinline__ void bwd_tile_math(const AttnTrainArgs& a, const MaskP& mp, float (&s)[8][4], float (&dpd)[8][4],
                                               const int (&row_g)[2], const float (&lse2)[2], const float (&dl)[2], int j0,
-                                              const uint32_t (&drop_base)[2], int t, bool want_pd, float (&pd)[8][4],
-                                              bf16* p_row0 = nullptr, bf16* p_row1 = nullptr, bf16* ds_row0 = nullptr,
-                                              bf16* ds_row1 = nullptr) {
-  // p_row*/ds_row*: when set, the dropped probabilities and dS of this thread's two rows are also written (bf16 pairs) at
-  // column offset 8*nt + 2*t of the given row pointers - the input of the dK/dV kernel (attn_bwd_dkv_lite_kernel)
+                                              const uint32_t (&drop_base)[2], int t, bf16* p_row0, bf16* p_row1, bf16* ds_row0,
+                                              bf16* ds_row1) {
+  // p_row*/ds_row*: the dropped probabilities and dS of this thread's two rows are also written (bf16 pairs) at column
+  // offset 8*nt + 2*t of the given row pointers - the input of the dK/dV kernel (attn_bwd_dkv_lite_kernel)
   const float c = a.scale * LOG2E;
   const bool need_mask = (j0 + 63 >= a.M) || (j0 < a.M - a.mem_count);
 #pragma unroll
@@ -244,15 +243,12 @@ __device__ __forceinline__ void bwd_tile_math(const AttnTrainArgs& a, const Mask
       if (need_mask && !visible(mp, row_g[r], j0 + 8 * nt + 2 * t + (e & 1))) p = 0.f;
       const float dp = dpd[nt][e] * keep[e];
       s[nt][e] = p * (dp - dl[r]) * a.scale;
-      if (want_pd) pd[nt][e] = p * keep[e];
-      if (p_row0) keep[e] *= p;                     // keep[] now holds the dropped probability
+      keep[e] *= p;                                 // keep[] now holds the dropped probability
     }
-    if (p_row0) {
-      *(uint32_t*)(p_row0 + 8 * nt + 2 * t) = pack_bf16x2(keep[0], keep[1]);
-      *(uint32_t*)(p_row1 + 8 * nt + 2 * t) = pack_bf16x2(keep[2], keep[3]);
-      *(uint32_t*)(ds_row0 + 8 * nt + 2 * t) = pack_bf16x2(s[nt][0], s[nt][1]);
-      *(uint32_t*)(ds_row1 + 8 * nt + 2 * t) = pack_bf16x2(s[nt][2], s[nt][3]);
-    }
+    *(uint32_t*)(p_row0 + 8 * nt + 2 * t) = pack_bf16x2(keep[0], keep[1]);
+    *(uint32_t*)(p_row1 + 8 * nt + 2 * t) = pack_bf16x2(keep[2], keep[3]);
+    *(uint32_t*)(ds_row0 + 8 * nt + 2 * t) = pack_bf16x2(s[nt][0], s[nt][1]);
+    *(uint32_t*)(ds_row1 + 8 * nt + 2 * t) = pack_bf16x2(s[nt][2], s[nt][3]);
   }
 }
 
@@ -275,6 +271,8 @@ __device__ __forceinline__ void bwd_tile_math_saved(const AttnTrainArgs& a, cons
       s[nt][e] = p * (dp - dl[r]) * a.scale;
       keep[e] *= p;                                 // keep[] now holds the dropped probability
     }
+    // p_row0 is never null: the branch only keeps ptxas from hoisting the caller's loads of the next tile's words above these
+    // stores, which needs a second set of pw registers (without it the kernel spills at 255 registers)
     if (p_row0) {
       *(uint32_t*)(p_row0 + 8 * nt + 2 * t) = pack_bf16x2(keep[0], keep[1]);
       *(uint32_t*)(p_row1 + 8 * nt + 2 * t) = pack_bf16x2(keep[2], keep[3]);
@@ -408,7 +406,7 @@ __global__ void __launch_bounds__(128, PS ? DQ_PS_MINB : 1) attn_bwd_dq_kernel(c
     uint8_t* sV = sK + TILE_BYTES;
     const uint32_t sR0 = smem_u32(sR + (rt_lo % NR) * TILE_BYTES), sR1 = smem_u32(sR + (rt_hi % NR) * TILE_BYTES);
 
-    float s[8][4], dpd[8][4], unused[8][4];
+    float s[8][4], dpd[8][4];
     if (!PS) scores_tile(qu, qv, smem_u32(sK), sR0, sR1, skew, w, lane, L, s);
     // dPd = dO V^T
 #pragma unroll
@@ -429,8 +427,7 @@ __global__ void __launch_bounds__(128, PS ? DQ_PS_MINB : 1) attn_bwd_dq_kernel(c
 #pragma unroll
       for (int r = 0; r < 2; r++) fac[r] = ex2_fast(mblk[r] * (a.scale * LOG2E) - lse2[r]);
       const long long o0 = (bhT + row_g[0]) * S + j0, o1 = (bhT + row_g[1]) * S + j0;
-      bwd_tile_math_saved(a, pw, fac, s, dpd, dl, j0, drop_base, t, ba.p_buf ? ba.p_buf + o0 : nullptr, ba.p_buf ? ba.p_buf + o1 : nullptr,
-                          ba.p_buf ? ba.ds_buf + o0 : nullptr, ba.p_buf ? ba.ds_buf + o1 : nullptr);
+      bwd_tile_math_saved(a, pw, fac, s, dpd, dl, j0, drop_base, t, ba.p_buf + o0, ba.p_buf + o1, ba.ds_buf + o0, ba.ds_buf + o1);
       if (jt < jt_hi) {                              // next tile's words and maxima
 #pragma unroll
         for (int nt = 0; nt < 8; nt++)
@@ -439,12 +436,9 @@ __global__ void __launch_bounds__(128, PS ? DQ_PS_MINB : 1) attn_bwd_dq_kernel(c
 #pragma unroll
         for (int r = 0; r < 2; r++) mblk[r] = __ldg(msrc[r] + jt + 1);
       }
-    } else if (ba.p_buf) {                            // spill P (dropped) and dS for the dK/dV kernel: [b*H+h][T][S] bf16
+    } else {                                         // spill P (dropped) and dS for the dK/dV kernel: [b*H+h][T][S] bf16
       const long long o0 = (bhT + row_g[0]) * S + j0, o1 = (bhT + row_g[1]) * S + j0;
-      bwd_tile_math(a, mp, s, dpd, row_g, lse2, dl, j0, drop_base, t, false, unused, ba.p_buf + o0, ba.p_buf + o1, ba.ds_buf + o0,
-                    ba.ds_buf + o1);
-    } else {
-      bwd_tile_math(a, mp, s, dpd, row_g, lse2, dl, j0, drop_base, t, false, unused);   // s := dS
+      bwd_tile_math(a, mp, s, dpd, row_g, lse2, dl, j0, drop_base, t, ba.p_buf + o0, ba.p_buf + o1, ba.ds_buf + o0, ba.ds_buf + o1);
     }
 
     // dS into the skewed strip (bf16): strip[row][64 + row - jl]
@@ -540,177 +534,6 @@ __global__ void __launch_bounds__(128, PS ? DQ_PS_MINB : 1) attn_bwd_dq_kernel(c
         atomicAdd(ba.du + h * 64 + 8 * nt + 2 * t + e, su);
         atomicAdd(ba.dv + h * 64 + 8 * nt + 2 * t + e, sv);
       }
-    }
-  }
-}
-
-// Q / dO tiles double-buffered, Rk tiles in a 3-slot ring (the window slides UP with the query tile: iteration `it` needs
-// rt_hi = (M + i0 - j0)/64 and rt_hi - 1 and loads exactly one new tile, rt_hi); (q+u) overwrites Q in place.
-constexpr int DKV_NST = 2;
-constexpr int DKV_NR = 3;
-constexpr int DKV_SMEM = 2 * TILE_BYTES /*K,V*/ + 2 * DKV_NST * TILE_BYTES /*Q,dO ring*/ + 2 * TILE_BYTES /*P,dS*/ + DKV_NR * TILE_BYTES +
-                         4 * 16 * SKEW_LD * (int)sizeof(skew_t);
-
-__global__ void __launch_bounds__(128) attn_bwd_dkv_kernel(const AttnTrainBwdArgs ba) {
-  const AttnTrainArgs& a = ba.f;
-  extern __shared__ __align__(128) uint8_t smem[];
-  uint8_t* sK = smem;
-  uint8_t* sV = sK + TILE_BYTES;
-  uint8_t* sQdO = sV + TILE_BYTES;                  // stage s: Q at sQdO + 2*s*TILE, dO right behind it
-  uint8_t* sP = sQdO + 2 * DKV_NST * TILE_BYTES;
-  uint8_t* sdS = sP + TILE_BYTES;
-  uint8_t* sR = sdS + TILE_BYTES;
-  skew_t* skew_all = (skew_t*)(sR + DKV_NR * TILE_BYTES);
-  const int tid = threadIdx.x, w = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-  skew_t* skew = skew_all + w * 16 * SKEW_LD;
-  LaneOff L;
-  lane_off_init(L, lane, w);
-
-  const int nS = (a.M + a.T) / 64;
-  const int jt = blockIdx.x % nS;                     // memory tiles (longest loops) come first
-  const int bh = blockIdx.x / nS, b = bh / a.H, h = bh % a.H;
-  const int j0 = jt * 64, HD = a.H * 64, S = a.M + a.T;
-  const MaskP mp = {a.M, a.mem_count, a.win, a.k};
-  const long long bhT = (long long)bh * a.T;
-
-  // destination rows of this key tile
-  bf16 *dk_dst, *dv_dst;
-  long long ldd;
-  if (j0 < a.M) {
-    ldd = a.ldm;
-    dk_dst = ba.dkv_m + ((long long)b * a.M + j0) * a.ldm + h * 64;
-    dv_dst = dk_dst + HD;
-  } else {
-    ldd = a.ldx;
-    dk_dst = ba.dqkv_x + ((long long)b * a.T + (j0 - a.M)) * a.ldx + HD + h * 64;
-    dv_dst = dk_dst + HD;
-  }
-  if (j0 < a.M - a.mem_count) {                       // memory slots not filled yet: no gradient
-    for (int i = tid; i < 64 * 32; i += 128) {
-      const int r = i >> 5, cidx = (i & 31) * 2;
-      *(uint32_t*)(dk_dst + (long long)r * ldd + cidx) = 0u;
-      *(uint32_t*)(dv_dst + (long long)r * ldd + cidx) = 0u;
-    }
-    return;
-  }
-
-  const int nT = a.T / 64;
-  const int it_lo = j0 < a.M ? 0 : (j0 - a.M) / 64;
-  const int rt_base = (a.M - j0) / 64;              // rt_hi of iteration `it` is rt_base + it (>= 0 from it_lo on)
-
-  auto load_stage = [&](int it) {                   // one cp.async group: Q, dO of query tile `it` and the new Rk tile(s)
-    if (it < nT) {
-      const int st = (it - it_lo) % DKV_NST;
-      const int i0 = it * 64;
-      tile_load_async(sQdO + 2 * st * TILE_BYTES, a.qkv_x + ((long long)b * a.T + i0) * a.ldx + h * 64, a.ldx, tid, 128);
-      tile_load_async(sQdO + (2 * st + 1) * TILE_BYTES, ba.dout + ((long long)b * a.T + i0) * HD + h * 64, HD, tid, 128);
-      const int rt_hi = rt_base + it;
-      tile_load_async(sR + (rt_hi % DKV_NR) * TILE_BYTES, a.rk + (long long)rt_hi * 64 * HD + h * 64, HD, tid, 128);
-      if (it == it_lo && rt_hi > 0)
-        tile_load_async(sR + ((rt_hi - 1) % DKV_NR) * TILE_BYTES, a.rk + (long long)(rt_hi - 1) * 64 * HD + h * 64, HD, tid, 128);
-    }
-    cp_async_commit();
-  };
-
-  {
-    long long ld;
-    const bf16* kp = kv_tile_ptr(a, b, h, jt, 0, &ld);
-    tile_load_async(sK, kp, ld, tid, 128);
-    const bf16* vp = kv_tile_ptr(a, b, h, jt, 1, &ld);
-    tile_load_async(sV, vp, ld, tid, 128);
-  }
-#pragma unroll
-  for (int s2 = 0; s2 < DKV_NST - 1; s2++) load_stage(it_lo + s2);     // K, V ride in the first group
-
-  float dk[8][4], dv[8][4];
-#pragma unroll
-  for (int nt = 0; nt < 8; nt++)
-#pragma unroll
-    for (int e = 0; e < 4; e++) { dk[nt][e] = 0.f; dv[nt][e] = 0.f; }
-
-  for (int it = it_lo; it < nT; it++) {
-    const int i0 = it * 64;
-    const int rt_hi = rt_base + it, rt_lo = rt_hi > 0 ? rt_hi - 1 : 0;
-    cp_async_wait<DKV_NST - 2>();
-    __syncthreads();                                 // tile `it` visible; everybody finished iteration it-1 (sP, sdS, old stage)
-    load_stage(it + DKV_NST - 1);
-    const int st = (it - it_lo) % DKV_NST;
-    uint8_t* sQ = sQdO + 2 * st * TILE_BYTES;
-    uint8_t* sdO = sQ + TILE_BYTES;
-    uint8_t* sQu = sQ;                               // (q+u) replaces q in place once the fragments are in registers
-    const uint32_t sR0 = smem_u32(sR + (rt_lo % DKV_NR) * TILE_BYTES), sR1 = smem_u32(sR + (rt_hi % DKV_NR) * TILE_BYTES);
-
-    uint32_t qu[4][4], qv[4][4], dof[4][4];
-    q_frags(smem_u32(sQ), w, lane, L, a.u + h * 64, a.v + h * 64, qu, qv);
-#pragma unroll
-    for (int ks = 0; ks < 4; ks++) frag_a(smem_u32(sdO), 16 * w, ks, L, dof[ks]);
-    // (q+u) tile for the dK contraction (B operand, [k = query][n = dh])
-#pragma unroll
-    for (int ks = 0; ks < 4; ks++) {
-      *(uint32_t*)(sQu + tile_off(16 * w + g, 2 * ks) + 4 * t) = qu[ks][0];
-      *(uint32_t*)(sQu + tile_off(16 * w + g + 8, 2 * ks) + 4 * t) = qu[ks][1];
-      *(uint32_t*)(sQu + tile_off(16 * w + g, 2 * ks + 1) + 4 * t) = qu[ks][2];
-      *(uint32_t*)(sQu + tile_off(16 * w + g + 8, 2 * ks + 1) + 4 * t) = qu[ks][3];
-    }
-    const int row_g[2] = {i0 + 16 * w + g, i0 + 16 * w + g + 8};
-    const uint32_t drop_base[2] = {(uint32_t)(((bhT + row_g[0]) * S) >> 1) + t, (uint32_t)(((bhT + row_g[1]) * S) >> 1) + t};
-    float lse2[2], dl[2];
-#pragma unroll
-    for (int r = 0; r < 2; r++) {
-      lse2[r] = a.lse[bhT + row_g[r]] * LOG2E;
-      dl[r] = ba.delta[bhT + row_g[r]];
-    }
-    float s[8][4], dpd[8][4], pd[8][4];
-    scores_tile(qu, qv, smem_u32(sK), sR0, sR1, skew, w, lane, L, s);
-#pragma unroll
-    for (int nt = 0; nt < 8; nt++) { dpd[nt][0] = 0.f; dpd[nt][1] = 0.f; dpd[nt][2] = 0.f; dpd[nt][3] = 0.f; }
-    const uint32_t sVa = smem_u32(sV);
-#pragma unroll
-    for (int ks = 0; ks < 4; ks++) {
-#pragma unroll
-      for (int np = 0; np < 4; np++) {
-        uint32_t r[4];
-        frag_b(sVa, 16 * np, ks, L, r);
-        mma_bf16(dpd[2 * np], dof[ks], r[0], r[1]);
-        mma_bf16(dpd[2 * np + 1], dof[ks], r[2], r[3]);
-      }
-    }
-    bwd_tile_math(a, mp, s, dpd, row_g, lse2, dl, j0, drop_base, t, true, pd);   // s := dS, pd := dropped P
-    // P and dS tiles [query][key] for the transposed contractions
-#pragma unroll
-    for (int nt = 0; nt < 8; nt++) {
-      *(uint32_t*)(sP + tile_off(16 * w + g, nt) + 4 * t) = pack_bf16x2(pd[nt][0], pd[nt][1]);
-      *(uint32_t*)(sP + tile_off(16 * w + g + 8, nt) + 4 * t) = pack_bf16x2(pd[nt][2], pd[nt][3]);
-      *(uint32_t*)(sdS + tile_off(16 * w + g, nt) + 4 * t) = pack_bf16x2(s[nt][0], s[nt][1]);
-      *(uint32_t*)(sdS + tile_off(16 * w + g + 8, nt) + 4 * t) = pack_bf16x2(s[nt][2], s[nt][3]);
-    }
-    __syncthreads();
-    // dV (keys 16w..) += P^T dO ; dK += dS^T (Q+u)
-    const uint32_t sPa = smem_u32(sP), sdSa = smem_u32(sdS), sdOa = smem_u32(sdO), sQua = smem_u32(sQu);
-#pragma unroll
-    for (int ks = 0; ks < 4; ks++) {
-      uint32_t ap[4], as[4];
-      frag_a_t(sPa, 16 * ks, L, ap);
-      frag_a_t(sdSa, 16 * ks, L, as);
-#pragma unroll
-      for (int np = 0; np < 4; np++) {
-        uint32_t r[4];
-        frag_b_t(sdOa, np, 16 * ks, L, r);
-        mma_bf16(dv[2 * np], ap, r[0], r[1]);
-        mma_bf16(dv[2 * np + 1], ap, r[2], r[3]);
-        frag_b_t(sQua, np, 16 * ks, L, r);
-        mma_bf16(dk[2 * np], as, r[0], r[1]);
-        mma_bf16(dk[2 * np + 1], as, r[2], r[3]);
-      }
-    }
-  }
-#pragma unroll
-  for (int r = 0; r < 2; r++) {
-    const long long ro = (long long)(16 * w + g + 8 * r) * ldd;
-#pragma unroll
-    for (int nt = 0; nt < 8; nt++) {
-      *(uint32_t*)(dk_dst + ro + 8 * nt + 2 * t) = pack_bf16x2(dk[nt][2 * r], dk[nt][2 * r + 1]);
-      *(uint32_t*)(dv_dst + ro + 8 * nt + 2 * t) = pack_bf16x2(dv[nt][2 * r], dv[nt][2 * r + 1]);
     }
   }
 }
@@ -861,15 +684,14 @@ int attn_train_fwd(const AttnTrainArgs& a, cudaStream_t st) {
   return launch_np(attn_train_fwd_kernel, dim3(a.B * a.H * (a.T / 64)), dim3(128), (size_t)FWD_SMEM, st, a);
 }
 
-int attn_train_bwd(const AttnTrainBwdArgs& ba, int num_sms, cudaStream_t st) {
-  (void)num_sms;
+int attn_train_bwd(const AttnTrainBwdArgs& ba, cudaStream_t st) {
   const AttnTrainArgs& a = ba.f;
   if (check_args(a)) return -2;
+  DMG_CHECK(ba.p_buf && ba.ds_buf, "training attention backward: the P / dS workspaces p_buf and ds_buf are required");
   static bool configured = false;
   if (!configured) {
     DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dq_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DQ_SMEM));
     DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dq_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DQ_PS_SMEM));
-    DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dkv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DKV_SMEM));
     DMG_CUDA_OK(cudaFuncSetAttribute(attn_bwd_dkv_lite_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LITE_SMEM));
     configured = true;
   }
@@ -882,9 +704,7 @@ int attn_train_bwd(const AttnTrainBwdArgs& ba, int num_sms, cudaStream_t st) {
     return -1;
   }
   if (attn_bwd_dkv_tc_supported(ba)) return attn_bwd_dkv_tc(ba, st);   // spilled tiles + (q+u): tcgen05 contraction
-  if (ba.p_buf && ba.ds_buf)   // P and dS were spilled by the dQ kernel: no second recomputation of the scores
-    return launch_np(attn_bwd_dkv_lite_kernel<false>, dim3(a.B * a.H * ((a.M + a.T) / 64)), dim3(128), (size_t)LITE_SMEM, st, ba);
-  return launch_np(attn_bwd_dkv_kernel, dim3(a.B * a.H * ((a.M + a.T) / 64)), dim3(128), (size_t)DKV_SMEM, st, ba);
+  return launch_np(attn_bwd_dkv_lite_kernel<false>, dim3(a.B * a.H * ((a.M + a.T) / 64)), dim3(128), (size_t)LITE_SMEM, st, ba);
 }
 
 }  // namespace dmg

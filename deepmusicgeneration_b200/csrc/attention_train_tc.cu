@@ -1005,9 +1005,8 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_cons
 }  // namespace
 
 bool attn_bwd_dq_tc_supported(const AttnTrainBwdArgs& ba) {
-  static const bool off = getenv("DMG_ATTN_DQ_MMA_SYNC") != nullptr;
   const AttnTrainArgs& a = ba.f;
-  return !off && a.p_save && a.m_save && ba.p_buf && ba.ds_buf && a.T % 128 == 0 && a.M % 128 == 0 && a.mem_count % 128 == 0 &&
+  return a.p_save && a.m_save && a.T % 128 == 0 && a.M % 128 == 0 && a.mem_count % 128 == 0 &&
          a.ldx % 8 == 0 && (a.M == 0 || a.ldm % 8 == 0);
 }
 
@@ -1037,9 +1036,8 @@ int attn_bwd_dq_tc(const AttnTrainBwdArgs& ba, cudaStream_t st) {
 
 
 bool attn_bwd_dkv_tc_supported(const AttnTrainBwdArgs& ba) {
-  static const bool off = getenv("DMG_ATTN_DKV_MMA_SYNC") != nullptr;
   const AttnTrainArgs& a = ba.f;
-  return !off && ba.p_buf && ba.ds_buf && ba.qu && a.T % 128 == 0 && a.M % 128 == 0 && a.mem_count % 128 == 0 && a.ldx % 8 == 0 &&
+  return ba.qu && a.T % 128 == 0 && a.M % 128 == 0 && a.mem_count % 128 == 0 && a.ldx % 8 == 0 &&
          (a.M == 0 || a.ldm % 8 == 0);
 }
 
@@ -1061,12 +1059,8 @@ int attn_bwd_dkv_tc(const AttnTrainBwdArgs& ba, cudaStream_t st) {
                    *(const CUtensorMap*)ts->bytes, *(const CUtensorMap*)td->bytes, *(const CUtensorMap*)tq->bytes, ba);
 }
 
-namespace {
-}  // namespace
-
 bool attn_train_fwd_tc_supported(const AttnTrainArgs& a) {
-  static const bool off = getenv("DMG_ATTN_FWD_MMA_SYNC") != nullptr;
-  return !off && a.T % 128 == 0 && a.M % 128 == 0 && a.mem_count % 128 == 0 && a.ldx % 8 == 0 && (a.M == 0 || a.ldm % 8 == 0);
+  return a.T % 128 == 0 && a.M % 128 == 0 && a.mem_count % 128 == 0 && a.ldx % 8 == 0 && (a.M == 0 || a.ldm % 8 == 0);
 }
 
 int attn_train_fwd_tc(const AttnTrainArgs& a, cudaStream_t st) {

@@ -329,13 +329,6 @@ gemm_train_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           if (lane == 0) tma_store_wait_read<0>();     // the boxes of the previous chunk have been read out
           __syncwarp();
           float g2[32];                               // act = 2: the saved backward factor gelu'(pre) (dropout applied below)
-          if (p.out2 && p.act != GEMM_ACT_GELU_GRADSAVE) {
-#pragma unroll
-            for (int j = 0; j < 4; j++)
-              *(uint4*)(strip + 2048 + lane * 64 + ((j ^ sw) << 4)) =
-                  make_uint4(pack_bf16x2(v[8 * j], v[8 * j + 1]), pack_bf16x2(v[8 * j + 2], v[8 * j + 3]),
-                             pack_bf16x2(v[8 * j + 4], v[8 * j + 5]), pack_bf16x2(v[8 * j + 6], v[8 * j + 7]));
-          }
           if (p.act == GEMM_ACT_GELU_GRADSAVE) {
 #pragma unroll
             for (int j = 0; j < 32; j++) {
@@ -363,13 +356,12 @@ gemm_train_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
               const float a8[8] = {bf16lo(w.x), bf16hi(w.x), bf16lo(w.y), bf16hi(w.y), bf16lo(w.z), bf16hi(w.z), bf16lo(w.w), bf16hi(w.w)};
 #pragma unroll
               for (int e = 0; e < 8; e++) {
-                if (p.aux_mode == GEMM_AUX_GELU_GRAD) v[8 * j + e] *= gelu_tanh_grad_fast(a8[e]);
-                else if (p.aux_mode == GEMM_AUX_MUL_BF16) v[8 * j + e] *= a8[e];
+                if (p.aux_mode == GEMM_AUX_MUL_BF16) v[8 * j + e] *= a8[e];
                 else v[8 * j + e] += a8[e];
               }
             }
             xcnt++;
-          } else if (p.aux_mode == GEMM_AUX_GELU_GRAD || p.aux_mode == GEMM_AUX_ADD_BF16 || p.aux_mode == GEMM_AUX_MUL_BF16) {
+          } else if (p.aux_mode == GEMM_AUX_ADD_BF16 || p.aux_mode == GEMM_AUX_MUL_BF16) {
             if (row < p.M) {
               const bf16* ax = (const bf16*)p.aux + (size_t)row * p.ld_aux + col0;
 #pragma unroll
@@ -379,8 +371,7 @@ gemm_train_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                   const float a8[8] = {bf16lo(w.x), bf16hi(w.x), bf16lo(w.y), bf16hi(w.y), bf16lo(w.z), bf16hi(w.z), bf16lo(w.w), bf16hi(w.w)};
 #pragma unroll
                   for (int e = 0; e < 8; e++) {
-                    if (p.aux_mode == GEMM_AUX_GELU_GRAD) v[8 * j + e] *= gelu_tanh_grad_fast(a8[e]);
-                    else if (p.aux_mode == GEMM_AUX_MUL_BF16) v[8 * j + e] *= a8[e];
+                    if (p.aux_mode == GEMM_AUX_MUL_BF16) v[8 * j + e] *= a8[e];
                     else v[8 * j + e] += a8[e];
                   }
                 }
@@ -400,7 +391,7 @@ gemm_train_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
               }
             }
           }
-          if (p.out2 && p.act == GEMM_ACT_GELU_GRADSAVE) {
+          if (p.act == GEMM_ACT_GELU_GRADSAVE) {
 #pragma unroll
             for (int j = 0; j < 4; j++)
               *(uint4*)(strip + 2048 + lane * 64 + ((j ^ sw) << 4)) =
@@ -441,21 +432,15 @@ gemm_train_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             if (row >= p.M) continue;
             const float4 sv = stg[rloc * 8 + (cq ^ (rloc & 7))];
             float v[4] = {sv.x + bias4.x, sv.y + bias4.y, sv.z + bias4.z, sv.w + bias4.w};
-            if (p.out2) *(uint2*)(p.out2 + (size_t)row * p.ld2 + col) = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
             if (p.act) {
 #pragma unroll
               for (int e = 0; e < 4; e++) v[e] = gelu_tanh_fast(v[e]);
             }
-            if (p.aux_mode == GEMM_AUX_GELU_GRAD || p.aux_mode == GEMM_AUX_ADD_BF16) {
+            if (p.aux_mode == GEMM_AUX_ADD_BF16) {
               const uint2 w = __ldg((const uint2*)((const bf16*)p.aux + (size_t)row * p.ld_aux + col));
               const float a[4] = {bf16lo(w.x), bf16hi(w.x), bf16lo(w.y), bf16hi(w.y)};
-              if (p.aux_mode == GEMM_AUX_GELU_GRAD) {
 #pragma unroll
-                for (int e = 0; e < 4; e++) v[e] *= gelu_tanh_grad_fast(a[e]);
-              } else {
-#pragma unroll
-                for (int e = 0; e < 4; e++) v[e] += a[e];
-              }
+              for (int e = 0; e < 4; e++) v[e] += a[e];
             } else if (p.aux_mode == GEMM_AUX_ADD_F32) {
               const float4 w = *((const float4*)((const float*)p.aux + (size_t)row * p.ld_aux + col));
               v[0] += w.x; v[1] += w.y; v[2] += w.z; v[3] += w.w;
@@ -553,14 +538,17 @@ int gemm_bf16_tc(const bf16* A, int a_mn, long long lda, const bf16* B, int b_mn
   DMG_CHECK(lda % 8 == 0 && ldb % 8 == 0, "gemm_bf16_tc: operand row strides must be multiples of 8 (lda=%lld ldb=%lld)", lda, ldb);
   DMG_CHECK(splitk >= 1 && (splitk == 1 || e.out_mode == GEMM_OUT_ATOMIC), "gemm_bf16_tc: split-K needs the atomic output mode");
   DMG_CHECK(e.out_mode == GEMM_OUT_BF16 ? e.ldc % 8 == 0 : e.ldc % 4 == 0, "gemm_bf16_tc: output row stride %lld misaligned", e.ldc);
+  DMG_CHECK((e.out2 != nullptr) == (e.act == GEMM_ACT_GELU_GRADSAVE),
+            "gemm_bf16_tc: a second output goes with the gradient-saving GeLU epilogue (act 2) and only with it (act=%d)", e.act);
   DMG_CHECK(!e.out2 || e.ld2 % 8 == 0, "gemm_bf16_tc: second output row stride misaligned");
+  DMG_CHECK(e.aux_mode == GEMM_AUX_NONE || e.aux_mode == GEMM_AUX_ADD_BF16 || e.aux_mode == GEMM_AUX_ADD_F32 || e.aux_mode == GEMM_AUX_MUL_BF16,
+            "gemm_bf16_tc: unknown aux_mode %d", e.aux_mode);
   DMG_CHECK(e.aux_mode == GEMM_AUX_NONE || (e.aux && (e.aux_mode == GEMM_AUX_ADD_F32 ? e.ld_aux % 4 == 0 : e.ld_aux % 8 == 0)),
             "gemm_bf16_tc: aux operand missing or misaligned");
   DMG_CHECK(N % 4 == 0, "gemm_bf16_tc: N=%d must be a multiple of 4 (16-byte epilogue accesses)", N);
   // CTA pairs (256-row tiles) whenever there are at least two 128-row blocks; tile width: the widest that still yields
   // about one wave of tiles
-  static const bool force_1cta = getenv("DMG_GEMM_1CTA") != nullptr;
-  const int CG = (!force_1cta && M > GT_BM && N > 64 && num_sms >= 2) ? 2 : 1;   // a pair stages N/2 >= 64 columns of B per CTA
+  const int CG = (M > GT_BM && N > 64 && num_sms >= 2) ? 2 : 1;   // a pair stages N/2 >= 64 columns of B per CTA
   const int units = num_sms / CG;
   const int num_m = (M + GT_BM * CG - 1) / (GT_BM * CG);
   // tile width: the candidate with the smallest estimated time = waves x (k-blocks x (MMA + fixed cost) + epilogue); a
@@ -597,11 +585,9 @@ int gemm_bf16_tc(const bf16* A, int a_mn, long long lda, const bf16* B, int b_mn
   if (!b_mn) { if (get_tmap(B, K, Next, ldb, BN / CG, &tb)) return -1; }
   else       { if (get_tmap(B, Next, K, ldb, 64, &tb)) return -1; }
   // bf16 outputs leave through TMA stores (dense boxes; the map clips at M and N); needs N-extent columns in a group-free launch
-  static const bool no_tma_store = getenv("DMG_GEMM_NO_TMA_STORE") != nullptr;
-  p.tma_store = (!no_tma_store && e.out_mode == GEMM_OUT_BF16 && groups == 1 && e.aux_mode != GEMM_AUX_ADD_F32) ? 1 : 0;
-  p.aux_tma = (p.tma_store && !e.out2 && (e.aux_mode == GEMM_AUX_GELU_GRAD || e.aux_mode == GEMM_AUX_ADD_BF16 || e.aux_mode == GEMM_AUX_MUL_BF16) &&
-               !getenv("DMG_GEMM_NO_AUX_TMA")) ? 1 : 0;
-  DMG_CHECK(e.act != GEMM_ACT_GELU_GRADSAVE || (p.tma_store && e.out2), "gemm_bf16_tc: the gradient-saving GeLU epilogue needs bf16 TMA-store outputs and a second output");
+  p.tma_store = (e.out_mode == GEMM_OUT_BF16 && groups == 1 && e.aux_mode != GEMM_AUX_ADD_F32) ? 1 : 0;
+  p.aux_tma = (p.tma_store && !e.out2 && (e.aux_mode == GEMM_AUX_ADD_BF16 || e.aux_mode == GEMM_AUX_MUL_BF16)) ? 1 : 0;
+  DMG_CHECK(e.act != GEMM_ACT_GELU_GRADSAVE || p.tma_store, "gemm_bf16_tc: the gradient-saving GeLU epilogue needs bf16 TMA-store outputs");
   const TensorMap2D *tc = ta, *tc2 = ta, *tx = ta;   // placeholders when unused
   if (p.tma_store) {
     if (get_tmap(e.out, N, M, e.ldc, -1, &tc)) return -1;

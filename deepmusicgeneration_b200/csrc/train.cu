@@ -236,8 +236,7 @@ int apply_mem_update(dmg_model* m, dmg_train* t, cudaStream_t st, int level_lo, 
   const int M = c.mem_len;
   if (M <= 0) return 0;
   for (int l = level_lo; l <= level_hi; l++) {
-    static const bool no_swap = getenv("DMG_TRAIN_NO_SWAP") != nullptr;
-    if (t->T == M && !no_swap) {   // the whole memory is replaced: trade buffers instead of copying (the old memory becomes next step's scratch)
+    if (t->T == M) {   // the whole memory is replaced: trade buffers instead of copying (the old memory becomes next step's scratch)
       std::swap(t->mem[l], l < c.n_layers ? t->act[l].xa_in : t->xa_last);
       continue;
     }
@@ -341,8 +340,7 @@ int train_forward(dmg_model* m, dmg_train* t, const long long* ids, const long l
     {   // FFN
       const Drop d3 = make_drop(t, t->cfg.ff_p, SITE_FF, l);
       // hpre receives the backward factor gelu'(pre) * dropout instead of the pre-activation (GEMM_ACT_GELU_GRADSAVE)
-      static const bool old_epi = getenv("DMG_FFN_SAVE_PRE") != nullptr;
-      GemmEpi e; e.bias = W.b1; e.act = old_epi ? GEMM_ACT_GELU : GEMM_ACT_GELU_GRADSAVE; e.out = A.hact; e.ldc = c.d_inner; e.out_mode = GEMM_OUT_BF16;
+      GemmEpi e; e.bias = W.b1; e.act = GEMM_ACT_GELU_GRADSAVE; e.out = A.hact; e.ldc = c.d_inner; e.out_mode = GEMM_OUT_BF16;
       e.out2 = A.hpre; e.ld2 = c.d_inner; e.drop_thresh = d3.thresh; e.drop_seed = d3.seed; e.drop_scale = d3.scale;
       if (t->eval_fwd) { e.act = GEMM_ACT_GELU; e.out2 = nullptr; }   // validation: the activation only
       if (gemm_bf16_tc(A.xa1, 0, d, W.w1.b16, 0, d, rows, c.d_inner, d, 1, e, ns, st)) return -1;
@@ -423,14 +421,8 @@ int backward_layer(dmg_model* m, dmg_train* t, int l, cudaStream_t st) {
     if (train_ln_bwd(t->dx32, t->dbr_valid ? t->dbr : nullptr, A.z2, A.st2, W.ln2w, t->dadd, t->G + g.ln2w, t->G + g.ln2b, t->G + g.b2, rows, d,
                      d4.thresh, d4.seed, d4.scale, st)) return -1;   // also the FFN-down bias gradient
     if (grad_w(m, t, t->dadd, d, A.hact, di, d, di, rows, g.w2, st)) return -1;
-    const Drop d3 = make_drop(t, t->cfg.ff_p, SITE_FF, l);
-    static const bool old_epi = getenv("DMG_FFN_SAVE_PRE") != nullptr;
-    GemmEpi e; e.aux = A.hpre; e.ld_aux = di; e.out = t->dh; e.ldc = di; e.out_mode = GEMM_OUT_BF16;
-    if (old_epi) {   // hpre = pre-activation: recompute gelu' and the dropout mask here
-      e.aux_mode = GEMM_AUX_GELU_GRAD; e.drop_thresh = d3.thresh; e.drop_seed = d3.seed; e.drop_scale = d3.scale;
-    } else {         // hpre = gelu'(pre) * keep * scale, stored by the forward: one multiply
-      e.aux_mode = GEMM_AUX_MUL_BF16;
-    }
+    // hpre = gelu'(pre) * keep * scale, stored by the forward: one multiply
+    GemmEpi e; e.aux = A.hpre; e.ld_aux = di; e.aux_mode = GEMM_AUX_MUL_BF16; e.out = t->dh; e.ldc = di; e.out_mode = GEMM_OUT_BF16;
     if (gemm_bf16_tc(t->dadd, 0, d, W.w2.b16, 1, di, rows, di, d, 1, e, ns, st)) return -1;
     if (grad_w(m, t, t->dh, di, A.xa1, d, di, d, rows, g.w1, st)) return -1;
     if (train_colsum_bf16(t->dh, di, rows, di, t->G + g.b1, st)) return -1;
@@ -454,7 +446,7 @@ int backward_layer(dmg_model* m, dmg_train* t, int l, cudaStream_t st) {
     ba.p_buf = t->p_buf; ba.ds_buf = t->ds_buf;
     const bool q_saved = ba.f.qu_save != nullptr;    // the tcgen05 forward stored q + u and q + v
     if (q_saved) ba.qu = ba.f.qu_save;
-    if (attn_train_bwd(ba, ns, st)) return -1;
+    if (attn_train_bwd(ba, st)) return -1;
     const bf16* qv_op = q_saved ? ba.f.qv_save : t->qv;
     if (!q_saved && train_q_plus_bias(A.qkv_x, 3 * HD, m->v, t->qv, rows, HD, st)) return -1;
     if (grad_rel_pos(m, t, qv_op, g, st)) return -1;
@@ -656,8 +648,7 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
     TRY(talloc(t, &A.z2, (size_t)rows * d));
     TRY(talloc(t, &A.rk, (size_t)S * HD));
     TRY(talloc(t, &A.lse, (size_t)t->B * c.n_heads * t->T));
-    static const bool no_psave = getenv("DMG_ATTN_NO_PSAVE") != nullptr;   // measurement switch, read once
-    if (t->T % 128 == 0 && c.mem_len % 128 == 0 && !no_psave) {   // geometry the tcgen05 forward serves
+    if (t->T % 128 == 0 && c.mem_len % 128 == 0) {   // geometry the tcgen05 forward serves
       TRY(talloc(t, &A.p_save, (size_t)t->B * c.n_heads * t->T * S));
       TRY(talloc(t, &A.m_save, (size_t)t->B * c.n_heads * t->T * (S / 64)));
       TRY(talloc(t, &A.qu_save, (size_t)rows * HD));
@@ -695,11 +686,8 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
   TRY(talloc(t, &t->dkv_m, BM * 2 * HD));
   TRY(talloc(t, &t->ds_dist, (size_t)rows * c.n_heads * S));
   TRY(talloc(t, &t->qv, (size_t)rows * HD));
-  static const bool bwd_recompute = getenv("DMG_ATTN_BWD_RECOMPUTE") != nullptr;   // measurement switch, read once
-  if (!bwd_recompute || bert) {   // spill P / dS from the dQ kernel instead of recomputing them for dK / dV
-    TRY(talloc(t, &t->p_buf, (size_t)rows * c.n_heads * S));
-    TRY(talloc(t, &t->ds_buf, (size_t)rows * c.n_heads * S));
-  }
+  TRY(talloc(t, &t->p_buf, (size_t)rows * c.n_heads * S));    // P / dS spilled by the dQ kernel for dK / dV
+  TRY(talloc(t, &t->ds_buf, (size_t)rows * c.n_heads * S));
   {   // multi-tensor Adam tables
     std::vector<AdamTensor> ht;
     std::vector<AdamChunk> hc;
@@ -1030,30 +1018,27 @@ int dmg_attn_train_bwd(const void* qkv_x, int64_t ldx, const void* kv_m, int64_t
   ba.dout = (const bf16*)dout; ba.delta = delta; ba.dqkv_x = (bf16*)dqkv_x; ba.dkv_m = (bf16*)dkv_m; ba.ds_dist = (bf16*)ds_dist;
   ba.qv = nullptr; ba.du = du; ba.dv = dv;
   if (p_save && m_save) { ba.f.p_save = (bf16*)const_cast<void*>(p_save); ba.f.m_save = const_cast<float*>(m_save); }
-  static const bool recompute = getenv("DMG_ATTN_BWD_RECOMPUTE") != nullptr;
   static bf16* ws = nullptr;          // spill workspace of this test hook: kept between calls, regrown on demand
   static size_t ws_elems = 0;
   const size_t n = (size_t)B * H * T * (M + T);
-  if (!recompute) {
-    if (ws_elems < 2 * n) {
-      if (ws) { DMG_CUDA_OK(cudaDeviceSynchronize()); cudaFree(ws); ws = nullptr; ws_elems = 0; }
-      DMG_CUDA_OK(cudaMalloc(&ws, 2 * n * sizeof(bf16)));
-      ws_elems = 2 * n;
-    }
-    ba.p_buf = ws; ba.ds_buf = ws + n;
-    // (q + u) operand of the tcgen05 dK/dV kernel (in the trainer the tcgen05 forward stores it)
-    static bf16* qu_ws = nullptr;
-    static size_t qu_elems = 0;
-    const size_t nq = (size_t)B * T * H * 64;
-    if (qu_elems < nq) {
-      if (qu_ws) { DMG_CUDA_OK(cudaDeviceSynchronize()); cudaFree(qu_ws); qu_ws = nullptr; qu_elems = 0; }
-      DMG_CUDA_OK(cudaMalloc(&qu_ws, nq * sizeof(bf16)));
-      qu_elems = nq;
-    }
-    if (train_q_plus_bias((const bf16*)qkv_x, ldx, u, qu_ws, B * T, H * 64, (cudaStream_t)stream)) return -1;
-    ba.qu = qu_ws;
+  if (ws_elems < 2 * n) {
+    if (ws) { DMG_CUDA_OK(cudaDeviceSynchronize()); cudaFree(ws); ws = nullptr; ws_elems = 0; }
+    DMG_CUDA_OK(cudaMalloc(&ws, 2 * n * sizeof(bf16)));
+    ws_elems = 2 * n;
   }
-  return attn_train_bwd(ba, 148, (cudaStream_t)stream);
+  ba.p_buf = ws; ba.ds_buf = ws + n;
+  // (q + u) operand of the tcgen05 dK/dV kernel (in the trainer the tcgen05 forward stores it)
+  static bf16* qu_ws = nullptr;
+  static size_t qu_elems = 0;
+  const size_t nq = (size_t)B * T * H * 64;
+  if (qu_elems < nq) {
+    if (qu_ws) { DMG_CUDA_OK(cudaDeviceSynchronize()); cudaFree(qu_ws); qu_ws = nullptr; qu_elems = 0; }
+    DMG_CUDA_OK(cudaMalloc(&qu_ws, nq * sizeof(bf16)));
+    qu_elems = nq;
+  }
+  if (train_q_plus_bias((const bf16*)qkv_x, ldx, u, qu_ws, B * T, H * 64, (cudaStream_t)stream)) return -1;
+  ba.qu = qu_ws;
+  return attn_train_bwd(ba, (cudaStream_t)stream);
 }
 
 int dmg_attn_bert_train_fwd(const void* qkv_x, int64_t ldx, const void* rk, const float* u, const float* v, void* out, float* lse,

@@ -45,11 +45,6 @@ __device__ __forceinline__ float tanh_fast(float x) {
 __device__ __forceinline__ float gelu_tanh_fast(float x) {
   return 0.5f * x * (1.f + tanh_fast(0.7978845608028654f * (x + 0.044715f * x * x * x)));
 }
-__device__ __forceinline__ float gelu_tanh_grad_fast(float x) {
-  const float k = 0.7978845608028654f, c = 0.044715f;
-  const float t = tanh_fast(k * (x + c * x * x * x));
-  return 0.5f * (1.f + t) + 0.5f * x * (1.f - t * t) * k * (1.f + 3.f * c * x * x);
-}
 
 // ------------------------------------------------------------------ persistent tcgen05 GEMM
 // C[M,N] = A * B with the reduction over K; operand storage:
@@ -61,8 +56,7 @@ enum { GEMM_OUT_F32 = 0, GEMM_OUT_BF16 = 1, GEMM_OUT_ATOMIC = 2 };
 // factor gelu'(pre) * keep * drop_scale instead of the pre-activation (it is the only thing the backward needs the
 // pre-activation for), so that the input-gradient GEMM's epilogue is one multiply (GEMM_AUX_MUL_BF16): no tanh, no dropout hash.
 enum { GEMM_ACT_NONE = 0, GEMM_ACT_GELU = 1, GEMM_ACT_GELU_GRADSAVE = 2 };
-enum { GEMM_AUX_NONE = 0,
-       GEMM_AUX_GELU_GRAD = 1,   // value *= gelu'(aux[m,n])                 (aux bf16: the saved pre-activation)
+enum { GEMM_AUX_NONE = 0,       // the values are the aux_mode numbers of dmg_gemm_train
        GEMM_AUX_ADD_BF16 = 2,    // value += aux[m,n]                        (bf16 residual)
        GEMM_AUX_ADD_F32 = 3,     // value += aux[m,n]                        (fp32 residual)
        GEMM_AUX_MUL_BF16 = 4 };  // value *= aux[m,n]                        (bf16: a saved gradient factor)
@@ -75,7 +69,7 @@ struct GemmEpi {
   void* out = nullptr;
   long long ldc = 0;
   int out_mode = GEMM_OUT_F32;
-  bf16* out2 = nullptr;          // optional: value before act / aux / dropout (bf16), e.g. the FFN pre-activation
+  bf16* out2 = nullptr;          // act = 2 only, and required there: the saved backward factor (bf16)
   long long ld2 = 0;
   uint32_t drop_thresh = 0;      // dropout applied last (after act / aux): 0 = none
   uint32_t drop_seed = 0;
@@ -143,12 +137,12 @@ struct AttnTrainBwdArgs {
   bf16* qv;              // [B*T, HD] bf16: q + v (operand of the dRk GEMM)
   float* du;             // [HD] accumulated (atomics)
   float* dv;             // [HD]
-  const bf16* qu = nullptr; // optional [B*T, HD] bf16: q + u; with p_buf / ds_buf and T, M, mem_count multiples of 128 it selects the
-                            // tcgen05 dK/dV kernel (attention_train_tc.cu)
-  bf16* p_buf = nullptr;   // optional workspaces [B*H, T, M+T] bf16: when both are set the dQ kernel spills the dropped
-  bf16* ds_buf = nullptr;  // probabilities and dS there and dK/dV come from a kernel that does not recompute the scores
+  const bf16* qu = nullptr; // optional [B*T, HD] bf16: q + u; with T, M, mem_count multiples of 128 it selects the tcgen05 dK/dV
+                            // kernel (attention_train_tc.cu)
+  bf16* p_buf = nullptr;   // required workspaces [B*H, T, M+T] bf16: the dQ kernel spills the dropped probabilities and dS
+  bf16* ds_buf = nullptr;  // there, and dK / dV are contracted from them without recomputing the scores
 };
-int attn_train_bwd(const AttnTrainBwdArgs& a, int num_sms, cudaStream_t st);
+int attn_train_bwd(const AttnTrainBwdArgs& a, cudaStream_t st);
 // pieces of attn_train_bwd that the remix encoder's backward reuses: delta = rowsum(dO * O); dK / dV from the spilled P / dS
 // tiles with every query tile seeing every key (M = 0, p_buf and ds_buf set)
 int attn_train_delta(const AttnTrainBwdArgs& ba, cudaStream_t st);

@@ -303,7 +303,9 @@ int dmg_train_dropout_mask(dmg_model* m, int site, int layer, int64_t step, floa
 float* dmg_train_grad_buffer(dmg_model* m);
 /* Unit-test entry of the training GEMM (persistent tcgen05 kernel): C[M,N] = op(A) op(B); a_mn / b_mn = 1 when the
  * reduction index is the slow one in memory; out_mode 0 fp32, 1 bf16, 2 fp32 atomic accumulate (split-K allowed);
- * aux_mode 0 none, 1 multiply by gelu'(aux bf16), 2 add aux bf16, 3 add aux fp32. */
+ * gelu 0 none, 1 tanh-GeLU, 2 tanh-GeLU whose second output out2 (bf16, required; out_mode 1) receives gelu'(pre) times the
+ * dropout factor - out2 is an error with any other gelu;
+ * aux_mode 0 none, 2 add aux bf16, 3 add aux fp32, 4 multiply by aux bf16 - any other value is an error. */
 int dmg_gemm_train(const void* a_dev, int a_mn, int64_t lda, const void* b_dev, int b_mn, int64_t ldb, int M, int N, int K,
                    int splitk, const float* bias_dev, int gelu, const void* aux_dev, int64_t ld_aux, int aux_mode, void* out_dev,
                    int64_t ldc, int out_mode, void* out2_dev, int64_t ld2, float drop_p, uint32_t drop_seed, void* stream);

@@ -38,11 +38,10 @@ def timeit(fn, R=20):
     for i in range(R): fn(i)
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / R * 1e3
-tc = 'off' if os.environ.get('DMG_ATTN_FWD_MMA_SYNC') else 'on'
 for pdrop in (0.1, 0.0):
-    for save in ((False, True) if tc == 'on' else (False,)):
+    for save in (False, True):
         us = timeit(lambda i: fwd(i, pdrop, save))
-        print(f'attn_train_fwd p={pdrop} tc={tc} save={save}: {us:.1f} us  {3 * 2 * B * T * HD * S / us / 1e6:.0f} TFLOP/s dense-count')
+        print(f'attn_train_fwd p={pdrop} save={save}: {us:.1f} us  {3 * 2 * B * T * HD * S / us / 1e6:.0f} TFLOP/s dense-count')
         fwd(0, pdrop, save)
         if os.environ.get('BWD', '1') == '1':
             us = timeit(lambda i: bwd(0, pdrop, save), R=10)

@@ -15,7 +15,7 @@ def run(name, M, N, K, a_mn, b_mn, out_mode, splitk=1, bias=False, gelu=0, aux_m
     pres = [torch.zeros(M, N, device=dev, dtype=torch.bfloat16) for _ in range(nb)] if pre else [None] * nb
     b = torch.randn(N, device=dev) if bias else None
     aux = None
-    if aux_mode in (1, 2): aux = torch.randn(M, N, device=dev).bfloat16()
+    if aux_mode in (2, 4): aux = torch.randn(M, N, device=dev).bfloat16()
     if aux_mode == 3: aux = torch.randn(M, N, device=dev)
     def call(i):
         rc = lib.dmg_gemm_train(P(As[i]), a_mn, As[i].stride(0), P(Bs[i]), b_mn, Bs[i].stride(0), M, N, K, splitk, P(b), gelu, P(aux),
@@ -45,14 +45,14 @@ if os.environ.get('GEMM_MAJORS'):
 only = os.environ.get('GEMM_ONLY')
 if only:
     run('QKV fwd', rows, 1536, 512, 0, 0, 1, reps=2)
-    run('FF1 fwd (bias gelu drop pre)', rows, 2048, 512, 0, 0, 1, bias=True, gelu=1, pre=True, drop=0.1, reps=2)
+    run('FF1 fwd (bias gelu drop gfac)', rows, 2048, 512, 0, 0, 1, bias=True, gelu=2, pre=True, drop=0.1, reps=2)
     sys.exit(0)
 run('QKV fwd', rows, 1536, 512, 0, 0, 1)
 run('KVmem fwd', rows, 1024, 512, 0, 0, 1)
 run('out-proj fwd', rows, 512, 512, 0, 0, 1)
-run('FF1 fwd (bias gelu drop pre)', rows, 2048, 512, 0, 0, 1, bias=True, gelu=1, pre=True, drop=0.1)
+run('FF1 fwd (bias gelu drop gfac)', rows, 2048, 512, 0, 0, 1, bias=True, gelu=2, pre=True, drop=0.1)
 run('FF2 fwd (bias)', rows, 512, 2048, 0, 0, 1, bias=True)
-run('dh = dY W2 (gelu grad drop)', rows, 2048, 512, 0, 1, 1, aux_mode=1, drop=0.1)
+run('dh = dY W2 (x gfac)', rows, 2048, 512, 0, 1, 1, aux_mode=4)
 run('dbranch = dh W1 (bf16)', rows, 512, 2048, 0, 1, 1)
 run('dbranch = dqkv Wqkv (bf16)', rows, 512, 1536, 0, 1, 1)
 run('dattn = dY Wo (bf16)', rows, 512, 512, 0, 1, 1)

@@ -8,7 +8,7 @@ import pytest
 import torch
 
 from deepmusicgeneration_b200 import _lib
-from deepmusicgeneration_b200._lib import check
+from deepmusicgeneration_b200._lib import DmgError, check
 from oracle import txl
 
 pytestmark = pytest.mark.gpu
@@ -83,23 +83,16 @@ def test_gemm_train_splitk_atomic_accumulates():
     assert rel_err(out, ref) < 2e-3
 
 
-def test_gemm_train_epilogues():
+def test_gemm_train_residual_and_dropout_epilogues():
+    "residual adds (bf16 / fp32 aux, in place) and the fused dropout on the fp32 output path"
     torch.manual_seed(2)
     M, N, K = 640, 768, 256
     A = torch.randn(M, K, device='cuda').bfloat16()
     W = (torch.randn(N, K, device='cuda') * 0.1).bfloat16()
     bias = torch.randn(N, device='cuda')
     acc = A.float() @ W.float().t() + bias
-    # bias + GeLU + pre-activation copy, bf16 out
-    out, pre = gemm_train(A, 0, W, 0, M, N, K, bias=bias, gelu=1, out_mode=1, want_pre=True)
-    assert rel_err(pre, acc) < 5e-3 and rel_err(out, gelu_tanh(acc)) < 5e-3
-    # multiply by gelu'(aux)
-    aux = torch.randn(M, N, device='cuda').bfloat16()
-    x = aux.float().requires_grad_(True)
-    gelu_tanh(x).sum().backward()
-    out = gemm_train(A, 0, W, 0, M, N, K, aux=aux, aux_mode=1, out_mode=1)
-    assert rel_err(out, (acc - bias) * x.grad) < 5e-3
     # residual adds
+    aux = torch.randn(M, N, device='cuda').bfloat16()
     res32 = torch.randn(M, N, device='cuda')
     out = gemm_train(A, 0, W, 0, M, N, K, aux=res32, aux_mode=3, out_mode=0)
     assert rel_err(out, acc - bias + res32) < 2e-3
@@ -140,7 +133,7 @@ def test_gemm_train_gradient_saving_gelu_epilogue():
     assert rel_err(dh, (dy.float() @ W2.float()) * gfac.float()) < 5e-3
 
 
-def test_gemm_train_persistent_many_tiles_per_cta():
+def test_gemm_train_persistent_loop_wraps_around():
     "more tiles than CTA pairs: the persistent loop, both TMEM stages, the TMA-store strips and the aux-box prefetch wrap around"
     torch.manual_seed(4)
     M, N, K = 8192, 2048, 192
@@ -148,14 +141,14 @@ def test_gemm_train_persistent_many_tiles_per_cta():
     W = (torch.randn(N, K, device='cuda') * 0.1).bfloat16()
     bias = torch.randn(N, device='cuda')
     acc = A.float() @ W.float().t()
-    out, pre = gemm_train(A, 0, W, 0, M, N, K, bias=bias, gelu=1, out_mode=1, want_pre=True)
-    assert rel_err(pre, acc + bias) < 5e-3 and rel_err(out, gelu_tanh(acc + bias)) < 5e-3
-    aux = torch.randn(M, N, device='cuda').bfloat16()
-    x = aux.float().requires_grad_(True)
+    x = (acc + bias).requires_grad_(True)
     gelu_tanh(x).sum().backward()
-    out = gemm_train(A, 0, W, 0, M, N, K, aux=aux, aux_mode=1, out_mode=1)
+    out, gfac = gemm_train(A, 0, W, 0, M, N, K, bias=bias, gelu=2, out_mode=1, want_pre=True)
+    assert rel_err(gfac, x.grad) < 5e-3 and rel_err(out, gelu_tanh(x.detach())) < 5e-3
+    out = gemm_train(A, 0, W, 0, M, N, K, aux=gfac, aux_mode=4, out_mode=1)
     assert torch.isfinite(out.float()).all()
-    assert rel_err(out, acc * x.grad) < 5e-3
+    assert rel_err(out, acc * gfac.float()) < 5e-3
+    aux = torch.randn(M, N, device='cuda').bfloat16()
     out = gemm_train(A, 0, W, 0, M, N, K, aux=aux, aux_mode=2, out_mode=1)
     assert rel_err(out, acc + aux.float()) < 5e-3
     out = gemm_train(A, 0, W, 0, M, N, K, out_mode=0)
@@ -163,6 +156,25 @@ def test_gemm_train_persistent_many_tiles_per_cta():
     Wm = W.t().contiguous()                                   # [K, N]: MN-major B
     out = gemm_train(A, 0, Wm, 1, M, N, K, out_mode=1)
     assert rel_err(out, acc) < 5e-3
+
+
+def test_gemm_train_rejects_unsupported_epilogues():
+    "aux_mode 1, and a second output with any GeLU but the gradient-saving one, are refused before anything is launched"
+    torch.manual_seed(7)
+    lib = _lib.load()
+    M, N, K = 256, 256, 128
+    A = torch.randn(M, K, device='cuda').bfloat16()
+    W = torch.randn(N, K, device='cuda').bfloat16()
+    aux = torch.randn(M, N, device='cuda').bfloat16()
+    out = torch.full((M, N), 5.0, device='cuda', dtype=torch.bfloat16)
+    torch.cuda.synchronize()
+    launches = lib.dmg_launch_count()
+    with pytest.raises(DmgError, match='aux_mode 1'):
+        gemm_train(A, 0, W, 0, M, N, K, aux=aux, aux_mode=1, out_mode=1, out=out)
+    with pytest.raises(DmgError, match='second output'):
+        gemm_train(A, 0, W, 0, M, N, K, gelu=1, out_mode=1, out=out, want_pre=True)
+    assert lib.dmg_launch_count() == launches
+    assert (out == 5.0).all()
 
 
 def test_gemm_train_grouped_heads():
