@@ -110,6 +110,16 @@ SYMBOLS = {
     'dmg_train_grad_buffer': (c_vp, [c_vp]),
     'dmg_gemm_train': (c_i32, [c_vp, c_i32, c_i64, c_vp, c_i32, c_i64, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32, c_vp, c_i64,
                                c_i32, c_vp, c_i64, c_i32, c_vp, c_i64, c_f32, c_u32, c_vp]),
+    'dmg_train_embed': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32, c_vp]),
+    'dmg_train_embed_bwd': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i64, c_f32, c_u32, c_vp]),
+    'dmg_train_ln_fwd': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_f32, c_u32, c_vp]),
+    'dmg_train_ln_bwd': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_f32, c_u32, c_vp]),
+    'dmg_train_ce': (c_i32, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_i32, c_i32, c_vp]),
+    'dmg_train_rnn_dropout': (c_i32, [c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32, c_vp]),
+    'dmg_train_head_bwd': (c_i32, [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32, c_f32, c_vp]),
+    'dmg_train_sumsq': (c_i32, [c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp]),
+    'dmg_train_tar': (c_i32, [c_vp, c_i64, c_i32, c_i32, c_i32, c_vp, c_vp]),
+    'dmg_train_colsum': (c_i32, [c_vp, c_i64, c_i32, c_i32, c_vp, c_vp]),
     'dmg_preload_fill': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_vp, c_i32, c_i32, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp,
                                  c_vp]),
     'dmg_mask_tfm': (c_i32, [c_vp, c_vp, c_i64, c_i32, c_i32, c_i32, c_i32, C.c_double, c_u32, c_vp, c_vp, c_vp]),

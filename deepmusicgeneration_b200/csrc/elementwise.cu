@@ -27,10 +27,8 @@ __global__ void embed_kernel(const long long* __restrict__ ids, const long long*
   const float4* e = (const float4*)(emb + (size_t)id * d);
   const float4 *be = nullptr, *ba = nullptr;
   if (pos != nullptr && beat != nullptr) {
-    long long p = pos[row];
-    long long bp = p % 32;
-    long long br = (p / 32) % 1024;
-    if (br >= 1024) br = 1023;
+    const long long p = pos[row];
+    const long long bp = p & 31, br = (p >> 5) & 1023;   // p mod 32, floor(p / 32) mod 1024 (Python floor semantics, also for p < 0)
     be = (const float4*)(beat + (size_t)bp * d);
     ba = (const float4*)(bar + (size_t)br * d);
   }

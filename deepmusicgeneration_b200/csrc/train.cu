@@ -579,6 +579,7 @@ void dmg_train_destroy(dmg_model* m) {
   cudaSetDevice(m->device);
   cudaDeviceSynchronize();
   for (void* p : m->train->allocs) cudaFree(p);
+  for (auto& W : m->layers) W.wr.b16 = nullptr;   // allocated by ensure_wr_b16 among the trainer's buffers, freed just above
   cudaFree(m->train->eval_tab);
   cudaFree(m->train->eval_part);
   delete m->train;
@@ -595,6 +596,8 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
             cfg->batch, cfg->bptt);
   DMG_CHECK(c.mem_len % 64 == 0, "dmg_train_create: mem_len %d must be a multiple of 64", c.mem_len);
   DMG_CHECK((bert || c.d_inner % 64 == 0) && c.d_model % 128 == 0, "dmg_train_create: d_inner %% 64 and d_model %% 128 required");
+  DMG_CHECK(train_ln_supported(c.d_model), "dmg_train_create: d_model=%d unsupported: the training LayerNorm kernels serve d_model = "
+            "128, 256, 384, 512, 768 or 1024", c.d_model);
   DMG_CHECK(!bert || (cfg->pad_idx >= 0 && cfg->pad_idx < c.vocab), "dmg_train_create: pad_idx %d outside the vocabulary", cfg->pad_idx);
   const float ps[5] = {cfg->resid_p, cfg->attn_p, cfg->ff_p, cfg->embed_p, cfg->output_p};
   for (float p : ps) DMG_CHECK(p >= 0.f && p < 0.95f, "dmg_train_create: dropout probability %f outside [0, 0.95)", p);
@@ -608,6 +611,10 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
   t->S = S;
   t->Vp = (c.vocab + 63) / 64 * 64;
   t->bert = bert;
+  int rc = 0;
+#define TRY(x) do { if (!rc && (x)) rc = -1; } while (0)
+  // the r_attn bf16 copies first: the parameter list records every bf16 copy, which the Adam kernel refreshes after each update
+  TRY(ensure_wr_b16(m, t));
   if (bert) {   // the encoder has no AR / TAR terms
     t->cfg.alpha = t->cfg.beta = 0.f;
     t->emb_pad = cfg->pad_idx;
@@ -615,8 +622,6 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
   } else {
     build_params(m, t);
   }
-  int rc = 0;
-#define TRY(x) do { if (!rc && (x)) rc = -1; } while (0)
   if (grad_flat_dev) { t->G = grad_flat_dev; t->own_G = false; }
   else { TRY(talloc(t, &t->G, (size_t)t->total)); t->own_G = true; }
   TRY(talloc(t, &t->m1, (size_t)t->total));
@@ -707,7 +712,6 @@ int dmg_train_create(dmg_model* m, const dmg_train_config* cfg, float* grad_flat
     if (!rc && cudaMemcpy(t->adam_chunks, hc.data(), hc.size() * sizeof(AdamChunk), cudaMemcpyHostToDevice) != cudaSuccess) rc = -1;
   }
   TRY(train_posenc(t->pe, S, d, 0));
-  TRY(ensure_wr_b16(m, t));
 #undef TRY
   if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("dmg_train_create: device error after setup"); rc = -1; }
   if (rc) { dmg_train_destroy(m); return rc; }
@@ -980,6 +984,124 @@ int dmg_gemm_train(const void* a_dev, int a_mn, int64_t lda, const void* b_dev, 
   e.out_mode = out_mode; e.out2 = (bf16*)out2_dev; e.ld2 = ld2;
   if (drop_p > 0.f) { e.drop_thresh = drop_thresh16(drop_p); e.drop_scale = drop_scale(drop_p); e.drop_seed = drop_seed_v; }
   return gemm_bf16_tc((const bf16*)a_dev, a_mn, lda, (const bf16*)b_dev, b_mn, ldb, M, N, K, splitk, e, sms, (cudaStream_t)stream);
+}
+
+// ---- unit-test entries of the elementwise training kernels: plain device pointers, dropout as (p, seed) like dmg_gemm_train
+static Drop hook_drop(float p, uint32_t seed) {
+  Drop d;
+  d.thresh = p > 0.f ? drop_thresh16(p) : 0u;
+  d.scale = d.thresh ? drop_scale(p) : 1.f;
+  d.seed = seed;
+  return d;
+}
+
+int dmg_train_embed(const int64_t* ids_dev, const int64_t* pos_dev, const float* emb, const float* beat, const float* bar, float* x32,
+                    void* xa, int rows, int d, int vocab, float drop_p, uint32_t drop_seed_v, void* stream) {
+  DMG_CHECK(ids_dev && emb && x32 && xa, "dmg_train_embed: null argument");
+  DMG_CHECK(!pos_dev || (beat && bar), "dmg_train_embed: pos given without the beat / bar tables");
+  DMG_CHECK(rows >= 0 && d > 0 && d % 4 == 0 && vocab >= 1, "dmg_train_embed: rows %d, d %d, vocab %d (need rows >= 0, d a positive "
+            "multiple of 4, vocab >= 1)", rows, d, vocab);
+  DMG_CHECK(drop_p >= 0.f && drop_p < 1.f, "dmg_train_embed: dropout probability %f outside [0, 1)", drop_p);
+  if (rows == 0) return 0;
+  const Drop dr = hook_drop(drop_p, drop_seed_v);
+  return train_embed((const long long*)ids_dev, (const long long*)pos_dev, emb, beat, bar, x32, (bf16*)xa, rows, d, vocab, dr.thresh,
+                     dr.seed, dr.scale, (cudaStream_t)stream);
+}
+
+int dmg_train_embed_bwd(const int64_t* ids_dev, const int64_t* pos_dev, const float* dx, const void* dbr, float* demb, float* dbeat,
+                        float* dbar, int rows, int d, int vocab, int64_t pad_idx, float drop_p, uint32_t drop_seed_v, void* stream) {
+  DMG_CHECK(ids_dev && dx && demb, "dmg_train_embed_bwd: null argument");
+  DMG_CHECK(!pos_dev || (dbeat && dbar), "dmg_train_embed_bwd: pos given without the beat / bar gradients");
+  DMG_CHECK(rows >= 0 && d > 0 && d % 4 == 0 && vocab >= 1, "dmg_train_embed_bwd: rows %d, d %d, vocab %d (need rows >= 0, d a "
+            "positive multiple of 4, vocab >= 1)", rows, d, vocab);
+  DMG_CHECK(drop_p >= 0.f && drop_p < 1.f, "dmg_train_embed_bwd: dropout probability %f outside [0, 1)", drop_p);
+  if (rows == 0) return 0;
+  const Drop dr = hook_drop(drop_p, drop_seed_v);
+  return train_embed_bwd((const long long*)ids_dev, (const long long*)pos_dev, dx, (const bf16*)dbr, demb, dbeat, dbar, rows, d, vocab,
+                         pad_idx, dr.thresh, dr.seed, dr.scale, (cudaStream_t)stream);
+}
+
+int dmg_train_ln_fwd(float* x32, const void* add, const float* w, const float* b, void* xa, void* zsave, float* stats, int rows, int d,
+                     float drop_p, uint32_t drop_seed_v, void* stream) {
+  DMG_CHECK(x32 && add && w && b && xa, "dmg_train_ln_fwd: null argument");
+  DMG_CHECK(rows >= 0, "dmg_train_ln_fwd: rows %d < 0", rows);
+  DMG_CHECK(train_ln_supported(d), "dmg_train_ln_fwd: d=%d unsupported (128, 256, 384, 512, 768, 1024)", d);
+  DMG_CHECK(drop_p >= 0.f && drop_p < 1.f, "dmg_train_ln_fwd: dropout probability %f outside [0, 1)", drop_p);
+  if (rows == 0) return 0;
+  const Drop dr = hook_drop(drop_p, drop_seed_v);
+  return train_residual_ln_fwd(x32, (const bf16*)add, w, b, (bf16*)xa, (bf16*)zsave, (float2*)stats, rows, d, dr.thresh, dr.seed, dr.scale,
+                               (cudaStream_t)stream);
+}
+
+int dmg_train_ln_bwd(float* dy, const void* dbr, const void* zsave, const float* stats, const float* w, void* dadd, float* dw, float* db,
+                     float* dsum, int rows, int d, float drop_p, uint32_t drop_seed_v, void* stream) {
+  DMG_CHECK(dy && zsave && stats && w && dadd && dw && db, "dmg_train_ln_bwd: null argument");
+  DMG_CHECK(rows >= 0, "dmg_train_ln_bwd: rows %d < 0", rows);
+  DMG_CHECK(train_ln_supported(d), "dmg_train_ln_bwd: d=%d unsupported (128, 256, 384, 512, 768, 1024)", d);
+  DMG_CHECK(drop_p >= 0.f && drop_p < 1.f, "dmg_train_ln_bwd: dropout probability %f outside [0, 1)", drop_p);
+  if (rows == 0) return 0;
+  const Drop dr = hook_drop(drop_p, drop_seed_v);
+  return train_ln_bwd(dy, (const bf16*)dbr, (const bf16*)zsave, (const float2*)stats, w, (bf16*)dadd, dw, db, dsum, rows, d, dr.thresh,
+                      dr.seed, dr.scale, (cudaStream_t)stream);
+}
+
+int dmg_train_ce(const float* logits, int64_t ldl, const int64_t* targets_dev, int64_t ignore, void* dlogits, float* loss_acc,
+                 float* count, int rows, int V, void* stream) {
+  DMG_CHECK(logits && targets_dev && dlogits && loss_acc, "dmg_train_ce: null argument");
+  DMG_CHECK(ignore < 0 || count, "dmg_train_ce: ignore = %lld needs the count output", (long long)ignore);
+  DMG_CHECK(rows >= 0 && V >= 1 && ldl >= V, "dmg_train_ce: rows %d, V %d, ldl %lld (need rows >= 0, V >= 1, ldl >= V)", rows, V,
+            (long long)ldl);
+  if (rows == 0) return 0;
+  if (ignore < 0)   // the Transformer-XL loss: mean over all rows
+    return train_ce_loss(logits, ldl, (const long long*)targets_dev, (bf16*)dlogits, loss_acc, rows, V, 1.f / rows, (cudaStream_t)stream);
+  return train_ce_loss_masked(logits, ldl, (const long long*)targets_dev, ignore, (bf16*)dlogits, loss_acc, count, rows, V,
+                              (cudaStream_t)stream);
+}
+
+int dmg_train_rnn_dropout(const void* x, void* y, int B, int T, int d, float drop_p, uint32_t drop_seed_v, void* stream) {
+  DMG_CHECK(x && y, "dmg_train_rnn_dropout: null argument");
+  DMG_CHECK(B >= 0 && T >= 0 && d > 0 && d % 4 == 0, "dmg_train_rnn_dropout: B %d, T %d, d %d (need B, T >= 0, d a positive multiple of 4)",
+            B, T, d);
+  DMG_CHECK(drop_p >= 0.f && drop_p < 1.f, "dmg_train_rnn_dropout: dropout probability %f outside [0, 1)", drop_p);
+  if (B == 0 || T == 0) return 0;
+  const Drop dr = hook_drop(drop_p, drop_seed_v);
+  return train_rnn_dropout((const bf16*)x, (bf16*)y, B, T, d, dr.thresh, dr.seed, dr.scale, (cudaStream_t)stream);
+}
+
+int dmg_train_head_bwd(const void* dxd, const float* core, float* dx32, int B, int T, int d, float drop_p, uint32_t drop_seed_v,
+                       float ar_coef, void* stream) {
+  DMG_CHECK(dxd && core && dx32, "dmg_train_head_bwd: null argument");
+  DMG_CHECK(B >= 0 && T >= 0 && d > 0 && d % 4 == 0, "dmg_train_head_bwd: B %d, T %d, d %d (need B, T >= 0, d a positive multiple of 4)",
+            B, T, d);
+  DMG_CHECK(drop_p >= 0.f && drop_p < 1.f, "dmg_train_head_bwd: dropout probability %f outside [0, 1)", drop_p);
+  if (B == 0 || T == 0) return 0;
+  const Drop dr = hook_drop(drop_p, drop_seed_v);
+  return train_head_bwd((const bf16*)dxd, core, dx32, B, T, d, dr.thresh, dr.seed, dr.scale, ar_coef, (cudaStream_t)stream);
+}
+
+int dmg_train_sumsq(const float* x, int64_t n, int deterministic, float* part, int part_cap, float* out, void* stream) {
+  DMG_CHECK(x && out, "dmg_train_sumsq: null argument");
+  DMG_CHECK(((uintptr_t)x & 15) == 0, "dmg_train_sumsq: x must be 16-byte aligned");
+  DMG_CHECK(n >= 0, "dmg_train_sumsq: n %lld < 0", (long long)n);
+  DMG_CHECK(!deterministic || (part && part_cap >= 1), "dmg_train_sumsq: the deterministic sum needs part (part_cap %d floats)", part_cap);
+  if (deterministic) return train_sumsq_det(x, n, part, part_cap, out, (cudaStream_t)stream);
+  return train_sumsq(x, n, out, (cudaStream_t)stream);
+}
+
+int dmg_train_tar(const void* h, int64_t bstride, int B, int n, int d, float* acc, void* stream) {
+  DMG_CHECK(h && acc, "dmg_train_tar: null argument");
+  DMG_CHECK(B >= 0 && n >= 0 && d > 0 && d % 2 == 0 && bstride >= (int64_t)n * d && bstride % 2 == 0,
+            "dmg_train_tar: B %d, n %d, d %d, bstride %lld (need d even, bstride even and >= n*d)", B, n, d, (long long)bstride);
+  if (B == 0) return 0;
+  return train_tar((const bf16*)h, bstride, B, n, d, acc, (cudaStream_t)stream);
+}
+
+int dmg_train_colsum(const void* x, int64_t ld, int rows, int n, float* dst, void* stream) {
+  DMG_CHECK(x && dst, "dmg_train_colsum: null argument");
+  DMG_CHECK(rows >= 0 && n >= 1 && ld >= n && ld % 2 == 0, "dmg_train_colsum: rows %d, n %d, ld %lld (need rows >= 0, n >= 1, ld even and "
+            ">= n)", rows, n, (long long)ld);
+  if (rows == 0) return 0;
+  return train_colsum_bf16((const bf16*)x, ld, rows, n, dst, (cudaStream_t)stream);
 }
 
 static AttnTrainArgs make_attn_args(const void* qkv_x, int64_t ldx, const void* kv_m, int64_t ldm, const void* rk, const float* u,

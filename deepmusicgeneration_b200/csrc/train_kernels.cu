@@ -43,9 +43,7 @@ __global__ void __launch_bounds__(256) train_embed_kernel(const long long* __res
     float4 v = *(const float4*)(emb + id * d + c);
     if (pos) {
       const long long p = pos[row];
-      const long long bt = ((p % 32) + 32) % 32;
-      long long br = (p / 32) % 1024;
-      br = br < 0 ? 0 : (br > 1023 ? 1023 : br);
+      const long long bt = p & 31, br = (p >> 5) & 1023;   // p mod 32, floor(p / 32) mod 1024 (Python floor semantics, also for p < 0)
       const float4 x = *(const float4*)(beat + bt * d + c), y = *(const float4*)(bar + br * d + c);
       v.x += x.x + y.x; v.y += x.y + y.y; v.z += x.z + y.z; v.w += x.w + y.w;
     }
@@ -85,9 +83,7 @@ __global__ void __launch_bounds__(256) train_embed_bwd_kernel(const long long* _
     }
     if (pos) {
       const long long p = pos[row];
-      const long long bt = ((p % 32) + 32) % 32;
-      long long br = (p / 32) % 1024;
-      br = br < 0 ? 0 : (br > 1023 ? 1023 : br);
+      const long long bt = p & 31, br = (p >> 5) & 1023;   // as train_embed_kernel
       if (bt != 0) {   // padding_idx = 0 rows receive no gradient
         float* q = dbeat + bt * d + c;
         atomicAdd(q, g.x); atomicAdd(q + 1, g.y); atomicAdd(q + 2, g.z); atomicAdd(q + 3, g.w);
@@ -227,30 +223,6 @@ __global__ void __launch_bounds__(256) train_ln_bwd_kernel(float* __restrict__ d
         atomicAdd(dst + k * 128 + threadIdx.x, s);
       }
     }
-  }
-}
-
-// dst0[c] += sum_blk partial[blk][0][c]; dst1[c] += sum_blk partial[blk][1][c]   (dst1 may be NULL: single plane)
-// 32 columns per block, 8 row-groups of threads walk the partial blocks, shared-memory tree at the end (coalesced reads).
-__global__ void __launch_bounds__(256) train_partial_finish_kernel(const float* __restrict__ partial, int nblk, int n,
-                                                                   float* __restrict__ dst0, float* __restrict__ dst1) {
-  __shared__ float red[8][33];
-  const int planes = dst1 ? 2 : 1;
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-  const int c = blockIdx.x * 32 + tx;
-  float s = 0.f;
-  if (c < n * planes) {
-    const int which = c / n, col = c % n;
-    for (int b = ty; b < nblk; b += 8) s += partial[((long long)b * planes + which) * n + col];
-  }
-  red[ty][tx] = s;
-  __syncthreads();
-  if (ty == 0 && c < n * planes) {
-    float t = 0.f;
-#pragma unroll
-    for (int q = 0; q < 8; q++) t += red[q][tx];
-    const int which = c / n, col = c % n;
-    (which ? dst1 : dst0)[col] += t;
   }
 }
 
@@ -695,11 +667,6 @@ int train_ln_bwd(float* dy, const bf16* dbr, const bf16* zsave, const float2* st
   }
   DMG_CHECK(false, "training LayerNorm backward: d_model=%d unsupported", d);
   return -2;
-}
-
-int train_partial_finish(const float* partial, int nblk, int n, float* dst0, float* dst1, cudaStream_t st) {
-  const int tot = n * (dst1 ? 2 : 1);
-  return launch_np(train_partial_finish_kernel, dim3((tot + 31) / 32), dim3(256), 0, st, partial, nblk, n, dst0, dst1);
 }
 
 int train_colsum_bf16(const bf16* x, long long ld, int rows, int n, float* dst, cudaStream_t st) {

@@ -160,6 +160,8 @@ int train_embed(const long long* ids, const long long* pos, const float* emb, co
                 float* x32, bf16* xa, int rows, int d, int vocab, uint32_t thresh, uint32_t seed, float scale,
                 cudaStream_t st);
 // z = x32 + dropout(add); save zsave = bf16(z), stats = (mean, rstd); x32 = LN(z)*w+b; xa = bf16(x32)
+// the widths the two training LayerNorm kernels are instantiated for (d / 128 = 1, 2, 3, 4, 6, 8)
+inline bool train_ln_supported(int d) { return d == 128 || d == 256 || d == 384 || d == 512 || d == 768 || d == 1024; }
 int train_residual_ln_fwd(float* x32, const bf16* add, const float* w, const float* b, bf16* xa, bf16* zsave,
                           float2* stats, int rows, int d, uint32_t thresh, uint32_t seed, float scale, cudaStream_t st);
 // LayerNorm backward: incoming gradient = dy (fp32 [rows,d]) + dbr (bf16 [rows,d] or NULL: the branch gradient a preceding
@@ -169,7 +171,6 @@ int train_residual_ln_fwd(float* x32, const bf16* add, const float* w, const flo
 // dsum (may be NULL) += column sums of dadd: the bias gradient of the Linear whose output entered the residual sum.
 int train_ln_bwd(float* dy, const bf16* dbr, const bf16* zsave, const float2* stats, const float* w, bf16* dadd, float* dw, float* db,
                  float* dsum, int rows, int d, uint32_t thresh, uint32_t seed, float scale, cudaStream_t st);
-int train_partial_finish(const float* partial, int nblk, int n, float* dst0, float* dst1, cudaStream_t st);   // dst += sums
 // column sums of a bf16 matrix [rows, n] (row stride ld) added into dst[n] (bias gradients)
 int train_colsum_bf16(const bf16* x, long long ld, int rows, int n, float* dst, cudaStream_t st);
 // column sums of a fp32 matrix, added into dst (du/dv from dq accumulators are not needed: attention does them)

@@ -309,6 +309,42 @@ float* dmg_train_grad_buffer(dmg_model* m);
 int dmg_gemm_train(const void* a_dev, int a_mn, int64_t lda, const void* b_dev, int b_mn, int64_t ldb, int M, int N, int K,
                    int splitk, const float* bias_dev, int gelu, const void* aux_dev, int64_t ld_aux, int aux_mode, void* out_dev,
                    int64_t ldc, int out_mode, void* out2_dev, int64_t ld2, float drop_p, uint32_t drop_seed, void* stream);
+/* Unit-test entries of the training step's elementwise kernels (train_kernels.cu), device pointers, no model; each calls the
+ * launcher the training step calls.  Dropout is (drop_p, drop_seed): element i of a site is kept iff the 16-bit half (i & 1) of
+ * the hash mix32((i >> 1) ^ seed) is >= round(drop_p * 65536), and kept values are scaled by 1 / (1 - that threshold / 65536).
+ * Arguments are checked before anything is launched; rows = 0 launches nothing.  bf16 buffers are void*.
+ *   dmg_train_embed: x32 [rows, d] = emb[clamp(id)] (+ beat[pos mod 32] + bar[floor(pos / 32) mod 1024] when pos is given), dropped
+ *     at element row*d + c; xa = bf16(x32).  dmg_train_embed_bwd: demb / dbeat / dbar += the dropped (dx + dbr) rows (dbr bf16, may be
+ *     NULL), except lookups of pad_idx (< 0: none) and of beat / bar row 0.
+ *   dmg_train_ln_fwd: z = x32 + dropout(add) (add bf16); stats [rows] (mean, rstd) and zsave = bf16(z) when given (both may be NULL);
+ *     x32 = LayerNorm(z) * w + b (eps 1e-5), xa = bf16(x32); d in {128, 256, 384, 512, 768, 1024}.
+ *   dmg_train_ln_bwd: dy (+ dbr bf16, may be NULL) is the gradient wrt the LayerNorm output, overwritten with dz (wrt z);
+ *     dadd = bf16(dropout(dz)); dw, db += the affine-parameter gradients; dsum (may be NULL) += the column sums of dropout(dz).
+ *   dmg_train_ce: ignore < 0: loss_acc += sum over rows of logsumexp - logit[target], dlogits [rows, ldl] bf16 = (softmax -
+ *     onehot) / rows, zero in columns V..ldl; ignore >= 0: rows with target == ignore get no loss and zero dlogits, *count (device,
+ *     required) = the other rows, which are scaled by 1 / count.  Targets are clamped to [0, V).
+ *   dmg_train_rnn_dropout: y [B, T, d] = x * mask[b, :] (one mask per stream, element b*d + c), bf16 both.
+ *   dmg_train_head_bwd: dx32 [B, T, d] fp32 = dxd (bf16) * mask[b, :] + ar_coef * core (fp32).
+ *   dmg_train_sumsq: deterministic = 0: *out += sum of x^2 (atomics); 1: *out = sum of x^2 in a fixed order through part (part_cap
+ *     floats, the trainer uses 592).  x 16-byte aligned.
+ *   dmg_train_tar: *acc += sum over b < B, 1 <= t < n of ||h[b*bstride + t*d ..] - h[b*bstride + (t-1)*d ..]||^2, h bf16.
+ *   dmg_train_colsum: dst[c] += sum over rows of x[r*ld + c], c < n, x bf16. */
+int dmg_train_embed(const int64_t* ids_dev, const int64_t* pos_dev, const float* emb, const float* beat, const float* bar, float* x32,
+                    void* xa, int rows, int d, int vocab, float drop_p, uint32_t drop_seed, void* stream);
+int dmg_train_embed_bwd(const int64_t* ids_dev, const int64_t* pos_dev, const float* dx, const void* dbr, float* demb, float* dbeat,
+                        float* dbar, int rows, int d, int vocab, int64_t pad_idx, float drop_p, uint32_t drop_seed, void* stream);
+int dmg_train_ln_fwd(float* x32, const void* add, const float* w, const float* b, void* xa, void* zsave, float* stats, int rows, int d,
+                     float drop_p, uint32_t drop_seed, void* stream);
+int dmg_train_ln_bwd(float* dy, const void* dbr, const void* zsave, const float* stats, const float* w, void* dadd, float* dw, float* db,
+                     float* dsum, int rows, int d, float drop_p, uint32_t drop_seed, void* stream);
+int dmg_train_ce(const float* logits, int64_t ldl, const int64_t* targets_dev, int64_t ignore, void* dlogits, float* loss_acc,
+                 float* count, int rows, int V, void* stream);
+int dmg_train_rnn_dropout(const void* x, void* y, int B, int T, int d, float drop_p, uint32_t drop_seed, void* stream);
+int dmg_train_head_bwd(const void* dxd, const float* core, float* dx32, int B, int T, int d, float drop_p, uint32_t drop_seed,
+                       float ar_coef, void* stream);
+int dmg_train_sumsq(const float* x, int64_t n, int deterministic, float* part, int part_cap, float* out, void* stream);
+int dmg_train_tar(const void* h, int64_t bstride, int B, int n, int d, float* acc, void* stream);
+int dmg_train_colsum(const void* x, int64_t ld, int rows, int n, float* dst, void* stream);
 /* Unit-test entries of the training attention kernels (attention_train.cu, attention_train_tc.cu): see AttnTrainArgs for
  * the layouts.  p_save [B*H, T, M+T] bf16 and m_save [B*H, T, (M+T)/64] fp32 are optional (both or neither, tcgen05
  * forward only = T, M, mem_count multiples of 128): the forward saves the undropped probabilities there and the backward,
