@@ -16,6 +16,7 @@ ARCH_TXL, ARCH_BERT = 0, 1
 F32, BF16 = 0, 1
 GEMM_AUTO, GEMM_SIMT, GEMM_TC_TILE = 0, 1, 2
 LOGITS_NONE, LOGITS_ALL, LOGITS_LAST = 0, 1, 2
+SEG_AUTO, SEG_GENERAL, SEG_FLASH, SEG_TC_RING, SEG_BERT_TC = 0, 1, 2, 3, 4     # dmg_segment_attn_args.kernel (DMG_SEG_*)
 SAMPLE_EARLY_STOP, SAMPLE_MASK_UNUSED, SAMPLE_REMIX_FILTER = 1, 2, 4
 # dmg_config.kernel_flags (DMG_KF_*): non-default kernels for parity tests / reproducing measurements; 0 = the product path
 (KF_NO_DECODE_KERNEL, KF_NO_FLASH, KF_NO_GRAPH, KF_BERT_MMA_SYNC, KF_BERT_FP32_STRIP, KF_NO_SPLITK, KF_NO_BIG_GEMM, KF_GEMM_SIMT,
@@ -53,6 +54,12 @@ class DecodeLayerArgs(C.Structure):
     _fields_ = [(n, c_vp) for n in ('x32', 'attn', 'wo', 'w1', 'w2', 'wqkv', 'bo', 'ln1w', 'ln1b', 'b1', 'b2', 'ln2w', 'ln2b', 'bqkv',
                                     'qkv', 'xa_out', 'pp')] + [('pp_stride', c_i64)] + \
                [(n, c_i32) for n in ('attn_rows', 'row_base', 'B', 'mode', 'd_model', 'n_heads', 'd_head', 'd_inner')]
+
+
+class SegmentAttnArgs(C.Structure):
+    _fields_ = [(n, c_vp) for n in ('qkv', 'kring', 'vring', 'rd', 'u', 'v', 'out')] + [('pos_total', c_i64)] + \
+               [(n, c_i32) for n in ('arch', 'dtype', 'B', 'T', 'H', 'M', 'Dcap', 'Bcap', 'b0', 'win', 'k', 'append', 'kernel',
+                                     'kernel_ran')]
 
 
 # name -> (restype, argtypes): every symbol include/dmg_b200.h declares
@@ -131,6 +138,7 @@ SYMBOLS = {
     'dmg_attn_decode': (c_i32, [C.POINTER(DecodeAttnArgs), c_vp]),
     'dmg_decode_layer_step': (c_i32, [C.POINTER(DecodeLayerArgs), c_vp]),
     'dmg_decode_dual': (c_i32, [C.POINTER(DecodeLayerArgs), C.POINTER(DecodeAttnArgs), c_i32, c_vp]),
+    'dmg_attn_segment': (c_i32, [C.POINTER(SegmentAttnArgs), c_vp]),
     'dmg_attn_bert_train_fwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32, c_vp]),
     'dmg_attn_bert_train_bwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32,
                                         c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),

@@ -138,6 +138,97 @@ struct DecodeStep {
   }
 };
 
+// ---- the attention of one segment: which kernel runs it (segment_route) and its launch with the ring append that follows
+// (segment_attention).  forward_chunk and the unit-test entry dmg_attn_segment both go through these two functions.
+constexpr int SEG_DECODE = -1;   // a one-token bf16 step: the decode kernel (attention_decode2.cu), which appends to the ring itself
+
+struct SegShape {
+  bool bf16, use_tc, bert;
+  bool ring_tm;                 // the rings and Rd have the decode kernel's tensor maps
+  int T, H, M, Dcap, mem_count, win, k, kflags;
+  long long pos_total;
+};
+
+// What each kernel supports (head size 64).  Flash: segments without memory (prefill after reset(), every BERT forward).  tcgen05
+// ring: whole 128-token tiles over a warm memory.  BERT tcgen05: sequences of at least 128 tokens.
+static bool seg_flash_ok(const SegShape& s) {
+  return s.bf16 && s.T > 1 && (s.bert || (s.mem_count == 0 && s.win == 1 && s.k == 1)) && s.Dcap >= s.T;
+}
+static bool seg_tc_ring_ok(const SegShape& s) {
+  return s.bf16 && !s.bert && s.T > 1 && attn_fwd_tc_ring_supported(s.T, 64, s.M, s.mem_count, (int)s.pos_total);
+}
+static bool seg_bert_tc_ok(const SegShape& s) { return s.bf16 && s.bert && attn_bert_tc_supported(s.T, s.H, s.Dcap); }
+static bool seg_decode_ok(const SegShape& s) {
+  return s.bf16 && !s.bert && s.T == 1 && s.M > 0 && s.ring_tm && attn_decode2_supported(64, s.M);
+}
+
+// DMG_SEG_* (or SEG_DECODE) for the segment under the kernel flags s.kflags.  Known before the q|k|v GEMM: the flash and tcgen05
+// kernels read q|k|v as bf16, the general and decode kernels as fp32.
+static int segment_route(const SegShape& s) {
+  if (seg_decode_ok(s) && !(s.kflags & DMG_KF_NO_DECODE_KERNEL)) return SEG_DECODE;
+  // memory-less bf16 segments: tensor-core flash attention, or for BERT sequences of >= 128 tokens the tcgen05 kernel
+  if (s.use_tc && seg_flash_ok(s) && !(s.kflags & DMG_KF_NO_FLASH))
+    return seg_bert_tc_ok(s) && !(s.kflags & DMG_KF_BERT_MMA_SYNC) ? DMG_SEG_BERT_TC : DMG_SEG_FLASH;
+  // bf16 segments of whole 128-token tiles over a WARM memory (chunked prefill of long seeds, validation passes): the tcgen05 attention of
+  // the training forward reading the K/V rings and the per-head Rd cache in place (attention_train_tc.cu)
+  if (s.use_tc && seg_tc_ring_ok(s) && !(s.kflags & DMG_KF_NO_FLASH)) return DMG_SEG_TC_RING;
+  return DMG_SEG_GENERAL;
+}
+
+static bool seg_qkv_bf16(int kernel) { return kernel != DMG_SEG_GENERAL && kernel != SEG_DECODE; }
+
+struct SegBufs {
+  const void* qkv;              // [B*T, 3*H*64]: bf16 where seg_qkv_bf16, else fp32
+  void *kring, *vring;          // [Bcap][H][M][64], element type of the model (bf16 / fp32)
+  const void* rd;               // [H][Dcap][64]
+  const float *u, *v;
+  void* out;                    // [B*T, H*64]
+  int Bcap;
+  int fp32_strip;               // BERT tcgen05 kernel: DMG_KF_BERT_FP32_STRIP
+  const VarlenPlan* vp;         // BERT only: per-sequence lengths, or NULL
+};
+
+// The attention of streams [b0, b0 + B) on the kernel `kernel` (not SEG_DECODE), then - over a memory and with `append` - the K/V of
+// the segment's last min(T, M) tokens into the rings.  T: element type of the rings / Rd / output of the general kernel.
+template <class T>
+static int segment_attention(int kernel, const SegShape& s, const SegBufs& p, int B, int b0, bool append, cudaStream_t st) {
+  const float scale = 0.125f;   // 1 / sqrt(64)
+  if (kernel == DMG_SEG_FLASH || kernel == DMG_SEG_BERT_TC) {
+    const bf16* qkv = (const bf16*)p.qkv;
+    if (p.vp) {
+      if (attn_bert_varlen_bf16(qkv, (const bf16*)p.rd, s.Dcap, p.u, p.v, (bf16*)p.out, *p.vp, B, s.T, s.H, scale, p.fp32_strip, st))
+        return -1;
+    } else if (kernel == DMG_SEG_BERT_TC) {
+      if (attn_bert_tc(qkv, (const bf16*)p.rd, s.Dcap, p.u, p.v, (bf16*)p.out, B, s.T, s.H, scale, p.fp32_strip, st)) return -1;
+    } else if (attn_flash(qkv, (const bf16*)p.rd, s.Dcap, p.u, p.v, (bf16*)p.out, B, s.T, s.H, s.bert ? 1 : 0, scale, st)) {
+      return -1;
+    }
+    if (append && s.M > 0 && ring_append_kv<bf16, bf16>(qkv, (bf16*)p.kring, (bf16*)p.vring, B, s.T, s.H, 64, s.M, s.pos_total, b0,
+                                                       p.Bcap, st)) return -1;
+    return 0;
+  }
+  if (kernel == DMG_SEG_TC_RING) {
+    const bf16* qkv = (const bf16*)p.qkv;
+    if (attn_fwd_tc_ring(qkv, (const bf16*)p.kring, (const bf16*)p.vring, (const bf16*)p.rd, s.Dcap, p.u, p.v, (bf16*)p.out, B, s.T, s.H,
+                         s.M, s.mem_count, s.win, s.k, (int)s.pos_total, b0, p.Bcap, scale, st)) return -1;
+    if (append && ring_append_kv<bf16, bf16>(qkv, (bf16*)p.kring, (bf16*)p.vring, B, s.T, s.H, 64, s.M, s.pos_total, b0, p.Bcap, st))
+      return -1;
+    return 0;
+  }
+  DMG_CHECK(kernel == DMG_SEG_GENERAL, "segment attention: kernel %d", kernel);
+  AttnGeneralArgs a;
+  a.qkv = (const float*)p.qkv; a.kring = p.kring; a.vring = p.vring; a.rd = p.rd; a.u = p.u; a.v = p.v; a.out = p.out;
+  a.B = B; a.T = s.T; a.H = s.H; a.M = s.M; a.Dcap = s.Dcap;
+  a.mem_count = s.mem_count; a.pos_total = s.pos_total; a.b0 = b0; a.bert = s.bert ? 1 : 0; a.win = s.win; a.k = s.k;
+  a.scale = scale;
+  a.lens = p.vp ? p.vp->lens : nullptr;
+  if (attn_general<T>(a, st)) return -1;
+  if (p.vp && varlen_zero_rows<T>((T*)p.out, p.vp->lens, B, s.T, s.H * 64, st)) return -1;
+  if (append && s.M > 0 && ring_append_kv<T, float>((const float*)p.qkv, (T*)p.kring, (T*)p.vring, B, s.T, s.H, 64, s.M, s.pos_total,
+                                                    b0, p.Bcap, st)) return -1;
+  return 0;
+}
+
 // vp (BERT only): the nb sequences have their own lengths (a padded batch, T_len = the padded length; see remix_batch.cu)
 template <class T>
 static int forward_chunk(dmg_model* m, const long long* ids, const long long* pos, int b0, int nb, int T_len, int win,
@@ -148,15 +239,12 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
   T* xa = (T*)m->xa;
   if (embed<T>(ids, c.encode_position ? pos : nullptr, m->emb.f32, m->beat, m->bar, m->x32, xa, rows, d, c.vocab, st)) return -1;
   if (c.keep_hidden && M > 0 && ring_append_hidden(m->x32, m->hrings[0], nb, T_len, d, M, m->pos_total, b0, st)) return -1;
-  const bool fast_decode = m->is_bf16 && !bert && T_len == 1 && M > 0 && m->layers[0].has_ring_tm &&
-                           attn_decode2_supported(c.d_head, M) && !(m->kflags & DMG_KF_NO_DECODE_KERNEL);
-  // segments without memory (prefill after reset(), every BERT forward) in bf16: flash attention on the tensor cores
-  const bool flash = m->is_bf16 && m->use_tc && T_len > 1 && (bert || (m->mem_count == 0 && win == 1 && k == 1)) &&
-                     m->Dcap >= T_len && !(m->kflags & DMG_KF_NO_FLASH);
-  // bf16 segments of whole 128-token tiles over a WARM memory (chunked prefill of long seeds, validation passes): the tcgen05 attention of
-  // the training forward reading the K/V rings and the per-head Rd cache in place (attention_train_tc.cu)
-  const bool tc_warm = m->is_bf16 && m->use_tc && !bert && !flash && !fast_decode && T_len > 1 && !(m->kflags & DMG_KF_NO_FLASH) &&
-                       m->qkv16 != nullptr && attn_fwd_tc_ring_supported(T_len, c.d_head, M, m->mem_count, m->pos_total);
+  SegShape sh;
+  sh.bf16 = m->is_bf16; sh.use_tc = m->use_tc; sh.bert = bert; sh.ring_tm = m->layers[0].has_ring_tm;
+  sh.T = T_len; sh.H = c.n_heads; sh.M = M; sh.Dcap = m->Dcap; sh.mem_count = m->mem_count; sh.win = win; sh.k = k; sh.kflags = m->kflags;
+  sh.pos_total = m->pos_total;
+  const int route = segment_route(sh);
+  const bool fast_decode = route == SEG_DECODE, qkv_bf16 = seg_qkv_bf16(route);
   // one-token step, product path: per layer ONE decode-attention launch + ONE fused layer launch (decode_layer.cu)
   const bool fused = fast_decode && m->fused_decode && !c.keep_hidden && m->layers[0].wqkv.has_tm && rows <= m->dl_rows;
   if (fused) {
@@ -187,33 +275,9 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
   }
   for (int l = 0; l < c.n_layers && !fused; l++) {
     LayerW& L = m->layers[l];
-    if (flash) {
-      // memory-less segment: bf16 q|k|v straight from the GEMM epilogue, tensor-core flash attention (attention_flash.cu)
-      if (linear(m, A_XA, xa, L.wqkv, L.bqkv, m->qkv16, 3 * HD, rows, 0, 1, st)) return -1;
-      if (vp) {
-        if (attn_bert_varlen_bf16(m->qkv16, (const bf16*)L.rd, m->Dcap, m->u, m->v, (bf16*)m->attn, *vp, nb, T_len, c.n_heads,
-                                  1.f / sqrtf((float)c.d_head), (m->kflags & DMG_KF_BERT_FP32_STRIP) ? 1 : 0, st)) return -1;
-      } else if (bert && !(m->kflags & DMG_KF_BERT_MMA_SYNC) && attn_bert_tc_supported(T_len, c.n_heads, m->Dcap)) {
-        // tcgen05 / TMEM / TMA kernel (sequences of at least 128 tokens)
-        if (attn_bert_tc(m->qkv16, (const bf16*)L.rd, m->Dcap, m->u, m->v, (bf16*)m->attn, nb, T_len, c.n_heads,
-                         1.f / sqrtf((float)c.d_head), (m->kflags & DMG_KF_BERT_FP32_STRIP) ? 1 : 0, st)) return -1;
-      } else if (attn_flash(m->qkv16, (const bf16*)L.rd, m->Dcap, m->u, m->v, (bf16*)m->attn, nb, T_len, c.n_heads, bert ? 1 : 0,
-                            1.f / sqrtf((float)c.d_head), st)) {
-        return -1;
-      }
-      if (M > 0 && ring_append_kv<bf16, bf16>(m->qkv16, (bf16*)L.kring, (bf16*)L.vring, nb, T_len, c.n_heads, c.d_head, M,
-                                               m->pos_total, b0, c.max_batch, st)) return -1;
-    } else if (tc_warm) {
-      if (linear(m, A_XA, xa, L.wqkv, L.bqkv, m->qkv16, 3 * HD, rows, 0, 1, st)) return -1;
-      if (attn_fwd_tc_ring(m->qkv16, (const bf16*)L.kring, (const bf16*)L.vring, (const bf16*)L.rd, m->Dcap, m->u, m->v, (bf16*)m->attn, nb,
-                           T_len, c.n_heads, M, m->mem_count, win, k, m->pos_total, b0, c.max_batch, 1.f / sqrtf((float)c.d_head), st)) return -1;
-      if (ring_append_kv<bf16, bf16>(m->qkv16, (bf16*)L.kring, (bf16*)L.vring, nb, T_len, c.n_heads, c.d_head, M, m->pos_total, b0,
-                                     c.max_batch, st)) return -1;
-    } else if (linear(m, A_XA, xa, L.wqkv, L.bqkv, m->qkv, 3 * HD, rows, 0, 0, st)) {
-      return -1;
-    }
-    if (flash || tc_warm) {
-    } else if (fast_decode) {
+    // q|k|v as the attention kernel reads it: bf16 straight from the GEMM epilogue for the flash / tcgen05 kernels, else fp32
+    if (linear(m, A_XA, xa, L.wqkv, L.bqkv, qkv_bf16 ? (void*)m->qkv16 : (void*)m->qkv, 3 * HD, rows, 0, qkv_bf16 ? 1 : 0, st)) return -1;
+    if (fast_decode) {
       AttnDecodeArgs a;
       a.qkv = m->qkv;
       a.kring = (bf16*)L.kring + (size_t)b0 * c.n_heads * M * 64;
@@ -227,16 +291,11 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
       a.force_v2 = (m->kflags & DMG_KF_ATTN_DECODE_V2) ? 1 : 0;
       if (attn_decode2(&L.tmK, &L.tmV, &L.tmR, a, b0, m->num_sms, st)) return -1;
     } else {
-      AttnGeneralArgs a;
-      a.qkv = m->qkv; a.kring = L.kring; a.vring = L.vring; a.rd = L.rd; a.u = m->u; a.v = m->v; a.out = m->attn;
-      a.B = nb; a.T = T_len; a.H = c.n_heads; a.M = M; a.Dcap = m->Dcap;
-      a.mem_count = m->mem_count; a.pos_total = m->pos_total; a.b0 = b0; a.bert = bert ? 1 : 0; a.win = win; a.k = k;
-      a.scale = 1.f / sqrtf((float)c.d_head);
-      a.lens = vp ? vp->lens : nullptr;
-      if (attn_general<T>(a, st)) return -1;
-      if (vp && varlen_zero_rows<T>((T*)m->attn, vp->lens, nb, T_len, HD, st)) return -1;
-      if (M > 0 && ring_append_kv<T, float>(m->qkv, (T*)L.kring, (T*)L.vring, nb, T_len, c.n_heads, c.d_head, M, m->pos_total, b0,
-                                            c.max_batch, st)) return -1;
+      SegBufs p;
+      p.qkv = qkv_bf16 ? (const void*)m->qkv16 : (const void*)m->qkv;
+      p.kring = L.kring; p.vring = L.vring; p.rd = L.rd; p.u = m->u; p.v = m->v; p.out = m->attn;
+      p.Bcap = c.max_batch; p.fp32_strip = (m->kflags & DMG_KF_BERT_FP32_STRIP) ? 1 : 0; p.vp = vp;
+      if (segment_attention<T>(route, sh, p, nb, b0, true, st)) return -1;
     }
     if (bert) {
       if (residual_layernorm<T, T>(m->x32, (const T*)m->attn, L.ln1w, L.ln1b, xa, rows, d, st)) return -1;
@@ -703,6 +762,10 @@ int dmg_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, in
                 int logits_mode, float* logits_dev, float* core_out_dev, void* stream) {
   DMG_CHECK(m && ids_dev, "dmg_forward: null argument");
   DMG_CHECK(mask_win >= 1, "dmg_forward: mask_win must be >= 1");
+  // the attention kernels hide every key after the query (they stop their key loops there), which is what window_mask does for
+  // (1, 1) and (w, 0) and only for those
+  DMG_CHECK(m->cfg.arch == DMG_ARCH_BERT || (mask_win == 1 && mask_k == 1) || mask_k == 0, "dmg_forward: window mask (%d,%d) unsupported",
+            mask_win, mask_k);
   DMG_CUDA_OK(cudaSetDevice(m->device));
   return forward_impl(m, (const long long*)ids_dev, (const long long*)pos_dev, bs, x_len, mask_win, mask_k, logits_mode,
                       logits_dev, core_out_dev, (cudaStream_t)stream);
@@ -1125,6 +1188,56 @@ int dmg_decode_dual(const dmg_decode_layer_args* f, const dmg_decode_attn_args* 
   DMG_CUDA_OK(cudaMemcpyAsync(a->state, ao.state, sizeof(ao.state), cudaMemcpyHostToDevice, st));
   const int rc = decode_dual(&lo.tmAttn, &lo.tmWo, &lo.tmW1, &lo.tmW2, &lo.tmWq, lo.a, &ao.tmK, &ao.tmV, &ao.tmR, ao.a, ao.b0,
                              attn_clusters, st);
+  const cudaError_t e = cudaStreamSynchronize(st);
+  if (rc) return rc;
+  DMG_CUDA_OK(e);
+  return 0;
+}
+
+int dmg_attn_segment(dmg_segment_attn_args* p, void* stream) {
+  static_assert(sizeof(dmg_segment_attn_args) == 120, "tests/test_abi.py mirrors this layout");
+  const char* who = "dmg_attn_segment";
+  DMG_CHECK(p, "%s: null argument", who);
+  DMG_CHECK(p->arch == DMG_ARCH_TXL || p->arch == DMG_ARCH_BERT, "%s: arch %d (0 = Transformer-XL, 1 = BERT)", who, p->arch);
+  DMG_CHECK(p->dtype == DMG_F32 || p->dtype == DMG_BF16, "%s: dtype %d (0 = fp32, 1 = bf16)", who, p->dtype);
+  DMG_CHECK(p->kernel >= DMG_SEG_AUTO && p->kernel <= DMG_SEG_BERT_TC,
+            "%s: kernel %d (0 = dmg_forward's choice, 1 general, 2 flash, 3 tcgen05 ring, 4 BERT tcgen05)", who, p->kernel);
+  DMG_CHECK(p->append == 0 || p->append == 1, "%s: append %d (0 or 1)", who, p->append);
+  const bool bert = p->arch == DMG_ARCH_BERT;
+  DMG_CHECK(p->B >= 1 && p->T >= 1 && p->H >= 1 && p->H <= 256 && p->M >= 0, "%s: B %d, T %d, H %d, M %d", who, p->B, p->T, p->H, p->M);
+  DMG_CHECK(p->pos_total >= 0 && p->pos_total + p->T <= 0x7fffffffLL, "%s: pos_total %lld outside [0, 2^31 - T)", who,
+            (long long)p->pos_total);
+  DMG_CHECK(!bert || (p->M == 0 && p->pos_total == 0), "%s: the BERT encoder has no memory (M %d, pos_total %lld)", who, p->M,
+            (long long)p->pos_total);
+  DMG_CHECK(p->qkv && p->rd && p->u && p->v && p->out && (p->M == 0 || (p->kring && p->vring)), "%s: null argument", who);
+  DMG_CHECK(p->b0 >= 0 && (long long)p->b0 + p->B <= p->Bcap, "%s: streams [%d, %d) outside the ring's %d", who, p->b0, p->b0 + p->B,
+            p->Bcap);
+  DMG_CHECK(p->Dcap >= (long long)p->M + p->T + 1, "%s: rel-pos cache too small (Dcap %d < M + T + 1 = %lld)", who, p->Dcap,
+            (long long)p->M + p->T + 1);
+  DMG_CHECK(p->win >= 1 && (bert || (p->win == 1 && p->k == 1) || p->k == 0), "%s: window mask (%d,%d) unsupported", who, p->win, p->k);
+  SegShape s;
+  s.bf16 = p->dtype == DMG_BF16; s.use_tc = s.bf16; s.bert = bert; s.ring_tm = true;
+  s.T = p->T; s.H = p->H; s.M = p->M; s.Dcap = p->Dcap; s.mem_count = (int)(p->pos_total < p->M ? p->pos_total : p->M);
+  s.win = p->win; s.k = p->k; s.kflags = 0; s.pos_total = p->pos_total;
+  int kernel = p->kernel;
+  if (kernel == DMG_SEG_AUTO) {
+    kernel = segment_route(s);
+    DMG_CHECK(kernel != SEG_DECODE, "%s: a one-token bf16 Transformer-XL segment runs on the decode kernel: test it through dmg_attn_decode",
+              who);
+  } else {
+    const bool ok = kernel == DMG_SEG_GENERAL || (kernel == DMG_SEG_FLASH && seg_flash_ok(s)) ||
+                    (kernel == DMG_SEG_TC_RING && seg_tc_ring_ok(s)) || (kernel == DMG_SEG_BERT_TC && seg_bert_tc_ok(s));
+    DMG_CHECK(ok, "%s: kernel %d does not support this segment (arch %d, dtype %d, T %d, H %d, M %d, mem_count %d, pos_total %lld, mask "
+              "(%d,%d), Dcap %d)", who, kernel, p->arch, p->dtype, p->T, p->H, p->M, s.mem_count, (long long)p->pos_total, p->win, p->k,
+              p->Dcap);
+  }
+  p->kernel_ran = kernel;
+  SegBufs b;
+  b.qkv = p->qkv; b.kring = p->kring; b.vring = p->vring; b.rd = p->rd; b.u = p->u; b.v = p->v; b.out = p->out;
+  b.Bcap = p->Bcap; b.fp32_strip = 0; b.vp = nullptr;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int rc = s.bf16 ? segment_attention<bf16>(kernel, s, b, p->B, p->b0, p->append != 0, st)
+                        : segment_attention<float>(kernel, s, b, p->B, p->b0, p->append != 0, st);
   const cudaError_t e = cudaStreamSynchronize(st);
   if (rc) return rc;
   DMG_CUDA_OK(e);

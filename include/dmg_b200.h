@@ -116,7 +116,8 @@ int dmg_mem_count(dmg_model* m);
 
 /* model(x) (deep_music_genre.py:1617-1647 + LinearDecoder; deep_music_remix.py:1874-1881 for DMG_ARCH_BERT).
  * ids_dev/pos_dev: int64 [bs, x_len] (pos_dev may be NULL unless encode_position).  mask_win/mask_k: the
- * (win_size, k) pair of window_mask (:1577-1584); eval mode is (1, 1).  logits_dev: fp32 [bs, x_len, V]
+ * (win_size, k) pair of window_mask (:1577-1584); eval mode is (1, 1).  DMG_ARCH_TXL takes the pairs rand_window_mask draws,
+ * (1, 1) and (w >= 1, 0), and refuses any other (the kernels hide every key after the query); DMG_ARCH_BERT has no mask.  logits_dev: fp32 [bs, x_len, V]
  * (DMG_LOGITS_ALL) or [bs, V] (DMG_LOGITS_LAST) or NULL.  core_out_dev: fp32 [bs, x_len, d_model] or NULL.
  * Appends the segment to the memory exactly like _update_mems. */
 int dmg_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, int bs, int x_len, int mask_win,
@@ -430,6 +431,38 @@ int dmg_decode_layer_step(const dmg_decode_layer_args* f, void* stream);
  * a->kernel must be 0 and M supported by it) in ONE launch.  attn_clusters = 0: as many 8-CTA attention clusters as the step gives
  * it (the co-resident clusters left by the fused role, at most one per 8 items); > 0: that many, if the items fit them. */
 int dmg_decode_dual(const dmg_decode_layer_args* f, const dmg_decode_attn_args* a, int attn_clusters, void* stream);
+
+/* Unit-test entry of the attention of a segment of T tokens (dmg_forward's attention for x_len > 1, and for x_len = 1 where the decode
+ * kernel does not run): the kernel choice and the launches of dmg_forward, on caller-owned buffers laid out as the model lays them
+ * out.  Query rows [0, B*T) of qkv / out are streams [b0, b0 + B) of the rings; head size 64 (scale 1/8).
+ *   qkv [B*T, 3*H*64] (q | k | v): bf16 for the flash and tcgen05 kernels, fp32 for the general kernel (as the q|k|v GEMM writes it
+ *   for each); kring / vring [Bcap][H][M][64], rd [H][Dcap][64] (rel-pos keys by distance), out [B*T, H*64]: fp32 for dtype DMG_F32,
+ *   bf16 for DMG_BF16; u / v fp32 [H*64].  The memory is mem_count = min(pos_total, M) tokens, token j (oldest first) in ring slot
+ *   (pos_total - mem_count + j) mod M; query i sees memory token j at distance mem_count + i - j.  (win, k): the window_mask of
+ *   DMG_ARCH_TXL, (1, 1) or (w >= 1, 0); DMG_ARCH_BERT has no memory (M = 0, pos_total = 0) and no mask.  Dcap >= M + T + 1 (as the
+ *   model sizes it).  append = 1: then writes the K/V of the segment's last min(T, M) tokens into slots (pos_total + t) mod M of the
+ *   streams [b0, b0 + B), as dmg_forward does.  kernel: DMG_SEG_AUTO = dmg_forward's choice under kernel flags 0 (a one-token bf16
+ *   Transformer-XL segment that the decode kernel serves is refused: dmg_attn_decode tests that kernel), or one of the others, which
+ *   must support the shape; kernel_ran receives the kernel that ran.  Arguments are checked before anything is launched; the entry
+ *   synchronises the stream. */
+enum { DMG_SEG_AUTO = 0,
+       DMG_SEG_GENERAL = 1,   /* attn_general_kernel (attention.cu), FFMA, fp32 or bf16 rings                                   */
+       DMG_SEG_FLASH = 2,     /* attn_flash (attention_flash.cu), mma.sync, bf16, no memory: TXL with mask (1, 1), or BERT         */
+       DMG_SEG_TC_RING = 3,   /* attn_fwd_tc_ring (attention_train_tc.cu), tcgen05, bf16, T / M / mem_count / pos_total % 128 == 0 */
+       DMG_SEG_BERT_TC = 4    /* attn_bert_tc (attention_bert_tc.cu), tcgen05, bf16, BERT with T >= 128                           */ };
+typedef struct dmg_segment_attn_args {
+  const void* qkv;
+  void* kring;
+  void* vring;
+  const void* rd;
+  const float* u;
+  const float* v;
+  void* out;
+  int64_t pos_total;
+  int32_t arch, dtype, B, T, H, M, Dcap, Bcap, b0, win, k, append, kernel;
+  int32_t kernel_ran;        /* out: DMG_SEG_GENERAL .. DMG_SEG_BERT_TC */
+} dmg_segment_attn_args;
+int dmg_attn_segment(dmg_segment_attn_args* a, void* stream);
 
 /* ---- training data feed (SURVEY.md section 8 f4) ------------------------------------------------------------------------
  * dmg_preload_fill = MusicPreloader.__getitem__ / fill_row (deep_music_genre.py:1088-1125) for all `bs` rows of one batch.

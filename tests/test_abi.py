@@ -45,6 +45,9 @@ def test_struct_layouts_match_header():
     assert _lib.DecodeAttnArgs.pos_total.offset == 64 and _lib.DecodeAttnArgs.kernel.offset == 100
     assert C.sizeof(_lib.DecodeLayerArgs) == 17 * 8 + 8 + 8 * 4
     assert _lib.DecodeLayerArgs.pp_stride.offset == 136 and _lib.DecodeLayerArgs.d_inner.offset == 172
+    assert C.sizeof(_lib.SegmentAttnArgs) == 7 * 8 + 8 + 14 * 4
+    assert _lib.SegmentAttnArgs.pos_total.offset == 56 and _lib.SegmentAttnArgs.arch.offset == 64
+    assert _lib.SegmentAttnArgs.kernel.offset == 112 and _lib.SegmentAttnArgs.kernel_ran.offset == 116
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason='CPU-only check')
