@@ -74,6 +74,7 @@ SYMBOLS = {
     'dmg_reset': (c_i32, [c_vp, c_i32]),
     'dmg_select_hidden': (c_i32, [c_vp, c_vp, c_i32]),
     'dmg_mem_count': (c_i32, [c_vp]),
+    'dmg_mem_counts': (c_i32, [c_vp, c_vp, c_i32]),
     'dmg_forward': (c_i32, [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp]),
     'dmg_forward_varlen': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp]),
     'dmg_predict_mask_batch': (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, C.POINTER(VocabLayout),
@@ -136,9 +137,11 @@ SYMBOLS = {
                                    c_i32, c_i32, c_i32, c_f32, c_u32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'dmg_attn_bert_varlen': (c_i32, [c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp]),
     'dmg_attn_decode': (c_i32, [C.POINTER(DecodeAttnArgs), c_vp]),
+    'dmg_attn_decode_streams': (c_i32, [C.POINTER(DecodeAttnArgs), c_vp, c_vp]),
     'dmg_decode_layer_step': (c_i32, [C.POINTER(DecodeLayerArgs), c_vp]),
     'dmg_decode_dual': (c_i32, [C.POINTER(DecodeLayerArgs), C.POINTER(DecodeAttnArgs), c_i32, c_vp]),
     'dmg_attn_segment': (c_i32, [C.POINTER(SegmentAttnArgs), c_vp]),
+    'dmg_attn_segment_streams': (c_i32, [C.POINTER(SegmentAttnArgs), c_vp, c_vp]),
     'dmg_attn_bert_train_fwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32, c_vp]),
     'dmg_attn_bert_train_bwd': (c_i32, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_f32, c_u32,
                                         c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),

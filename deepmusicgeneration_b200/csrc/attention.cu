@@ -49,7 +49,8 @@ __global__ void __launch_bounds__(128) attn_general_kernel(AttnGeneralArgs a) {
   const int i0 = blockIdx.x * GQ, h = blockIdx.y, b = blockIdx.z;
   const int T_len = VARLEN ? a.lens[b] : a.T, H = a.H, HD = H * 64, M = a.M;
   if (VARLEN && i0 >= T_len) return;
-  const int m = a.mem_count, S = m + T_len;
+  const int* st = a.state + (size_t)a.state_stride * (a.b0 + b);   // this stream's memory: streams of a batch may hold different counts
+  const int pos_total = st[0], m = st[1], S = m + T_len;
   const T* kring = (const T*)a.kring;
   const T* vring = (const T*)a.vring;
   const T* rd = (const T*)a.rd + (size_t)h * a.Dcap * 64;
@@ -84,7 +85,7 @@ __global__ void __launch_bounds__(128) attn_general_kernel(AttnGeneralArgs a) {
       float kv[16], vv[16];
       if (j < S) {
         if (j < m) {
-          const int slot = (int)((a.pos_total - m + j) % M);
+          const int slot = (int)(((long long)pos_total - m + j) % M);
           const size_t off = (((size_t)(a.b0 + b) * H + h) * M + slot) * 64 + c16;
 #pragma unroll
           for (int e = 0; e < 16; e++) {

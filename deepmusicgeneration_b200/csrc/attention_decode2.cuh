@@ -92,6 +92,13 @@ __device__ unsigned long long* d2_prof_ptr;
 #define D2_ACC(k) do {} while (0)
 #endif
 
+// {pos_total, mem_count} of the stream of (stream, head) item `it` (head-major: stream b0 + it mod B): the streams of a batch may hold
+// memories of different lengths.  The producer fetches it one item ahead and stores it beside the item's q slot before the arrive that
+// releases the slot, so the consumers read it from shared memory.
+__device__ __forceinline__ int2 item_ring_state(const AttnDecodeArgs& a, int b0, int it) {
+  return *(const int2*)(a.state + a.state_stride * (b0 + it % a.B));
+}
+
 // The kernel body as a device function: `cta` of `ncta` persistent CTAs (the stand-alone kernel passes blockIdx.x / gridDim.x; the
 // dual-role decode kernel of decode_layer.cu gives it the CTAs that are not busy with the fused layer step of the other half of the
 // streams).  Runs on the first (4 G + 1) * 32 threads of the block; `d2_smem` is the block's dynamic shared memory.
@@ -116,6 +123,7 @@ __device__ __forceinline__ void attn_decode2_body(const CUtensorMap& tmK, const 
   uint64_t* q_empty = q_full + 2;         // [2]
   uint64_t* r_full = q_empty + 2;
   uint64_t* r_free = r_full + 1;
+  int2* qstate = (int2*)(psum + NW);      // [2] ring state of the item in q slot 0 / 1
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int nT = M / TR;                  // K tiles (= V tiles) per item
@@ -174,6 +182,7 @@ __device__ __forceinline__ void attn_decode2_body(const CUtensorMap& tmK, const 
         }
       }
       pdl_wait();
+      int2 rs = lo < hi ? item_ring_state(a, b0, lo) : make_int2(0, 0);
       for (int it = lo, n = 0; it < hi; ++it, ++n) {
         const int h = it / B, b = it - h * B;
         const int qs = n & 1;
@@ -187,6 +196,8 @@ __device__ __forceinline__ void attn_decode2_body(const CUtensorMap& tmK, const 
           for (int bx = 0; bx < L.r_boxes; bx++) tma_load_2d(Rres + bx * 8192, &tmR, 0, h * a.Dcap + bx * 64, r_full);
           cur_h = h;
         }
+        qstate[qs] = rs;                             // the item's ring state goes with its q|k|v: released by the arrive below
+        if (it + 1 < hi) rs = item_ring_state(a, b0, it + 1);
         mbar_expect_tx(&q_full[qs], 768);
         const float* qrow = a.qkv + (size_t)b * 3 * HD + h * 64;
         bulk_g2s(qbuf + qs * 192, qrow, 256, &q_full[qs]);
@@ -216,8 +227,6 @@ __device__ __forceinline__ void attn_decode2_body(const CUtensorMap& tmK, const 
   long long t_last = t_begin;
 #endif
   pdl_wait();
-  const int pos_total = a.dev_state[0], mc = a.dev_state[1];
-  const int head = pos_total % M;
   const int grp = warp >> 2, w = warp & 3;      // group: which 64 keys of a tile; w: 16-key block / 16-dim block
   const int g = lane >> 2, t4 = lane & 3;
   const float sscale = a.scale * D2_LOG2E;
@@ -240,6 +249,8 @@ __device__ __forceinline__ void attn_decode2_body(const CUtensorMap& tmK, const 
     const int qs = n & 1;
     D2_MARK(7);
     { D2_T0(); mbar_wait(&q_full[qs], (uint32_t)((n >> 1) & 1)); D2_ACC(1); }
+    const int2 rs = qstate[qs];                  // this item's stream: its memory may differ from the other streams'
+    const int mc = rs.y, head = rs.x % M;
     D2_MARK(0);
     const float* qb = qbuf + qs * 192;
     // B fragments of the query (replicated over the 8 columns): k = 16*ks + {2t, 2t+1} and {2t+8, 2t+9}

@@ -114,6 +114,7 @@ __device__ __forceinline__ void attn_decode3_body(const CUtensorMap& tmK, const 
       uint64_t *full = tb, *empty = tb + n_stages, *q_full = tb + 2 * n_stages, *q_empty = q_full + 2;
       uint8_t* ring = base + L.off_ring;
       float* qbuf = (float*)(base + L.off_team + team * L.team_bytes);
+      int2* qstate = (int2*)(base + L.off_team + team * L.team_bytes + 2 * 768 + (((M + 16) * 2 + 15) & ~15) + 40);   // = consumers' wmax + 10
       // stage s of team t lives at slot s * T + t of the ring region: the first stages of every team are outside the rel-pos alias
       int s = 0, use = 0, pre = 0;
       bool alias_ok = false;
@@ -135,10 +136,13 @@ __device__ __forceinline__ void attn_decode3_body(const CUtensorMap& tmK, const 
         if (s == n_stages) { s = 0; use = 1; }
       }
       pdl_wait();
+      int2 rs = team < n_items ? item_ring_state(a, b0, lo + team) : make_int2(0, 0);
       for (int i = team, k = 0; i < n_items; i += T, ++k) {
         const int it = lo + i, h = it / B, b = it - h * B;
         const int qs = k & 1;
         mbar_wait(&q_empty[qs], (uint32_t)(((k >> 1) & 1) ^ 1));
+        qstate[qs] = rs;                            // the item's ring state goes with its q|k|v: released by the arrive below
+        if (i + T < n_items) rs = item_ring_state(a, b0, it + T);
         mbar_expect_tx(&q_full[qs], 768);
         const float* qrow = a.qkv + (size_t)b * 3 * HD + h * 64;
         bulk_g2s(qbuf + qs * 192, qrow, 256, &q_full[qs]);
@@ -172,8 +176,6 @@ __device__ __forceinline__ void attn_decode3_body(const CUtensorMap& tmK, const 
   long long t_last = t_begin;
 #endif
   pdl_wait();
-  const int pos_total = a.dev_state[0], mc = a.dev_state[1];
-  const int head = pos_total % M;
   const int team = warp >> 2, w = warp & 3;
   const int g = lane >> 2, t4 = lane & 3;
   const int hi16 = lane >> 4;
@@ -256,6 +258,7 @@ __device__ __forceinline__ void attn_decode3_body(const CUtensorMap& tmK, const 
   float* wmax = (float*)(tmem_base + 2 * 768 + (((M + 16) * 2 + 15) & ~15));   // [4] warp maxima, [4] warp sums, [1] own score
   float* psum = wmax + 4;
   float* own_s = wmax + 8;
+  const int2* qstate = (const int2*)(wmax + 10);   // [2] ring state of the item in q slot 0 / 1 (written by the producer)
   const int bar_a = 6 + 2 * team, bar_b = 7 + 2 * team;
   // per-lane constants of the fragment addressing
   const int krowA = 32 * w + (lane & 15), krowB = krowA + 16;     // K phase: the lane's ldmatrix rows inside the 128-key tile
@@ -281,6 +284,8 @@ __device__ __forceinline__ void attn_decode3_body(const CUtensorMap& tmK, const 
     }
     const int qs = k & 1;
     mbar_wait(&q_full[qs], (uint32_t)((k >> 1) & 1));
+    const int2 rs = qstate[qs];                 // this item's stream: its memory may differ from the other streams'
+    const int mc = rs.y, head = rs.x % M;
     D2_MARK(0);
     const float* qb = qbuf + qs * 192;
     const float* tabrow = tab + i * S;

@@ -192,32 +192,39 @@ template int cast_f32<float>(const float*, float*, long long, cudaStream_t);
 template int cast_f32<bf16>(const float*, bf16*, long long, cudaStream_t);
 
 template <class T>
-__global__ void gather_rows_kernel(const T* __restrict__ src, T* __restrict__ dst, int rows, int d, int stride, int offset) {
+__global__ void gather_rows_kernel(const T* __restrict__ src, T* __restrict__ dst, int rows, int d, int stride, int offset,
+                                   const int* __restrict__ lens) {
   const int r = blockIdx.x;
   pdl_launch_dependents();
   pdl_wait();
-  const T* s = src + ((size_t)r * stride + offset) * d;
+  const T* s = src + ((size_t)r * stride + (lens ? lens[r] - 1 : offset)) * d;
   T* o = dst + (size_t)r * d;
   for (int c = threadIdx.x; c < d; c += blockDim.x) o[c] = s[c];
 }
 template <class T>
-int gather_rows(const T* src, T* dst, int rows, int d, int stride, int offset, cudaStream_t st) {
+int gather_rows(const T* src, T* dst, int rows, int d, int stride, int offset, cudaStream_t st, const int* lens) {
   if (rows <= 0) return 0;
-  return launch_k(gather_rows_kernel<T>, dim3(rows), dim3(128), 0, st, 1, src, dst, rows, d, stride, offset);
+  return launch_k(gather_rows_kernel<T>, dim3(rows), dim3(128), 0, st, 1, src, dst, rows, d, stride, offset, lens);
 }
-template int gather_rows<float>(const float*, float*, int, int, int, int, cudaStream_t);
-template int gather_rows<bf16>(const bf16*, bf16*, int, int, int, int, cudaStream_t);
+template int gather_rows<float>(const float*, float*, int, int, int, int, cudaStream_t, const int*);
+template int gather_rows<bf16>(const bf16*, bf16*, int, int, int, int, cudaStream_t, const int*);
 
 // ------------------------------------------------------------------ memory rings
-// K/V of the last min(T, M) new tokens of every stream -> ring slot (token index mod M).
+// K/V of the last min(len_b, M) new tokens of every stream -> ring slot (token index mod M).  Block x = the x-th of those tokens
+// (blocks past min(len_b, M) of a shorter stream of a padded batch do nothing: padding rows never reach the ring).
 // qkv row layout: [q (H*Dh) | k (H*Dh) | v (H*Dh)], ring layout [Bcap][H][M][Dh].
 template <class T, class TS>
 __global__ void ring_append_kv_kernel(const TS* __restrict__ qkv, T* __restrict__ kring, T* __restrict__ vring, int T_len,
-                                      int H, int Dh, int M, long long pos_total, int b0, int first) {
-  // grid: (T_len - first, B); block: H*Dh/4 threads (each 4 elements)
-  const int i = first + blockIdx.x, b = blockIdx.y;
+                                      int H, int Dh, int M, const int* __restrict__ state, int state_stride,
+                                      const int* __restrict__ lens, int b0) {
+  // grid: (min(T_len, M), B); block: H*Dh/4 threads (each 4 elements)
+  const int b = blockIdx.y;
+  const int len = lens ? lens[b] : T_len;
+  const int first = len > M ? len - M : 0;
+  const int i = first + blockIdx.x;
+  if (i >= len) return;
   const int HD = H * Dh;
-  const int slot = (int)((pos_total + i) % M);
+  const int slot = (int)(((long long)state[(size_t)state_stride * (b0 + b)] + i) % M);
   const TS* row = qkv + ((size_t)b * T_len + i) * 3 * HD;
   for (int e = threadIdx.x * 4; e < HD; e += blockDim.x * 4) {
     const int h = e / Dh, c = e % Dh;
@@ -232,67 +239,76 @@ __global__ void ring_append_kv_kernel(const TS* __restrict__ qkv, T* __restrict_
   }
 }
 template <class T, class TS>
-int ring_append_kv(const TS* qkv, T* kring, T* vring, int B, int T_len, int H, int Dh, int M, long long pos_total,
-                   int b0, int Bcap, cudaStream_t st) {
+int ring_append_kv(const TS* qkv, T* kring, T* vring, int B, int T_len, int H, int Dh, int M, const int* state, int state_stride,
+                   const int* lens, int b0, cudaStream_t st) {
   if (M <= 0 || B <= 0 || T_len <= 0) return 0;
-  (void)Bcap;
-  const int first = T_len > M ? T_len - M : 0;
   int threads = H * Dh / 4;
   if (threads > 256) threads = 256;
-  ring_append_kv_kernel<T, TS><<<dim3(T_len - first, B), threads, 0, st>>>(qkv, kring, vring, T_len, H, Dh, M, pos_total, b0, first);
+  ring_append_kv_kernel<T, TS><<<dim3(T_len < M ? T_len : M, B), threads, 0, st>>>(qkv, kring, vring, T_len, H, Dh, M, state,
+                                                                                    state_stride, lens, b0);
   g_launch_count++;
   DMG_CUDA_OK(cudaGetLastError());
   return 0;
 }
-template int ring_append_kv<float, float>(const float*, float*, float*, int, int, int, int, int, long long, int, int, cudaStream_t);
-template int ring_append_kv<bf16, float>(const float*, bf16*, bf16*, int, int, int, int, int, long long, int, int, cudaStream_t);
-template int ring_append_kv<bf16, bf16>(const bf16*, bf16*, bf16*, int, int, int, int, int, long long, int, int, cudaStream_t);
+template int ring_append_kv<float, float>(const float*, float*, float*, int, int, int, int, int, const int*, int, const int*, int,
+                                          cudaStream_t);
+template int ring_append_kv<bf16, float>(const float*, bf16*, bf16*, int, int, int, int, int, const int*, int, const int*, int,
+                                         cudaStream_t);
+template int ring_append_kv<bf16, bf16>(const bf16*, bf16*, bf16*, int, int, int, int, int, const int*, int, const int*, int,
+                                        cudaStream_t);
 
 __global__ void ring_append_hidden_kernel(const float* __restrict__ x32, float* __restrict__ hring, int T_len, int d, int M,
-                                          long long pos_total, int b0, int first) {
-  const int i = first + blockIdx.x, b = blockIdx.y;
-  const int slot = (int)((pos_total + i) % M);
+                                          const int* __restrict__ state, int state_stride, const int* __restrict__ lens, int b0) {
+  const int b = blockIdx.y;
+  const int len = lens ? lens[b] : T_len;
+  const int first = len > M ? len - M : 0;
+  const int i = first + blockIdx.x;
+  if (i >= len) return;
+  const int slot = (int)(((long long)state[(size_t)state_stride * (b0 + b)] + i) % M);
   const float4* s = (const float4*)(x32 + ((size_t)b * T_len + i) * d);
   float4* o = (float4*)(hring + ((size_t)(b0 + b) * M + slot) * d);
   for (int c = threadIdx.x; c < d / 4; c += blockDim.x) o[c] = s[c];
 }
-int ring_append_hidden(const float* x32, float* hring, int B, int T_len, int d, int M, long long pos_total, int b0,
-                       cudaStream_t st) {
+int ring_append_hidden(const float* x32, float* hring, int B, int T_len, int d, int M, const int* state, int state_stride,
+                       const int* lens, int b0, cudaStream_t st) {
   if (M <= 0 || B <= 0 || T_len <= 0) return 0;
-  const int first = T_len > M ? T_len - M : 0;
-  ring_append_hidden_kernel<<<dim3(T_len - first, B), 128, 0, st>>>(x32, hring, T_len, d, M, pos_total, b0, first);
+  ring_append_hidden_kernel<<<dim3(T_len < M ? T_len : M, B), 128, 0, st>>>(x32, hring, T_len, d, M, state, state_stride, lens, b0);
   g_launch_count++;
   DMG_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
-// out[b][j][:] = ring[b][slot(pos_total - mem_count + j)][:], j = 0..mem_count-1  (oldest first, like the reference)
-__global__ void ring_export_hidden_kernel(const float* __restrict__ hring, float* __restrict__ out, int d, int M,
-                                          long long pos_total, int mem_count) {
+// out[b][j][:] = ring[b][slot(pos_total_b - mem_count + j)][:], j = 0..mem_count-1  (oldest first, like the reference)
+__global__ void ring_export_hidden_kernel(const float* __restrict__ hring, float* __restrict__ out, int d, int M, int mem_count,
+                                          const int* __restrict__ state, int state_stride) {
   const int j = blockIdx.x, b = blockIdx.y;
-  const int slot = (int)((pos_total - mem_count + j) % M);
+  const int slot = (int)(((long long)state[(size_t)state_stride * b] - mem_count + j) % M);
   const float4* s = (const float4*)(hring + ((size_t)b * M + slot) * d);
   float4* o = (float4*)(out + ((size_t)b * mem_count + j) * d);
   for (int c = threadIdx.x; c < d / 4; c += blockDim.x) o[c] = s[c];
 }
-int ring_export_hidden(const float* hring, float* out, int B, int d, int M, long long pos_total, int mem_count,
+int ring_export_hidden(const float* hring, float* out, int B, int d, int M, int mem_count, const int* state, int state_stride,
                        cudaStream_t st) {
   if (mem_count <= 0 || B <= 0) return 0;
-  ring_export_hidden_kernel<<<dim3(mem_count, B), 128, 0, st>>>(hring, out, d, M, pos_total, mem_count);
+  ring_export_hidden_kernel<<<dim3(mem_count, B), 128, 0, st>>>(hring, out, d, M, mem_count, state, state_stride);
   g_launch_count++;
   DMG_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
-__global__ void state_advance_kernel(int* st, int T_len, int M) {
+__global__ void state_advance_kernel(int* st, int n, int T_len, const int* __restrict__ lens, int M) {
   pdl_launch_dependents();
   pdl_wait();
-  st[0] += T_len;
-  int m = st[1] + T_len;
-  st[1] = m > M ? M : m;
+  for (int b = threadIdx.x; b < n; b += blockDim.x) {
+    const int len = lens ? lens[b] : T_len;
+    st[2 * b] += len;
+    const int m = st[2 * b + 1] + len;
+    st[2 * b + 1] = m > M ? M : m;
+  }
 }
-int state_advance(int* dev_state, int T_len, int M, cudaStream_t st) {
-  return launch_k(state_advance_kernel, dim3(1), dim3(1), 0, st, 1, dev_state, T_len, M);
+int state_advance(int* state, int n, int T_len, const int* lens, int M, cudaStream_t st) {
+  if (n <= 0) return 0;
+  return launch_k(state_advance_kernel, dim3(1), dim3(n < 256 ? (n + 31) / 32 * 32 : 256), 0, st, 1, state, n, T_len, lens, M);
 }
 
 }  // namespace dmg

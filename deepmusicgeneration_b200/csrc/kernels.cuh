@@ -87,22 +87,29 @@ int rd_relayout(const float* src, T* dst, int n, int H, int Dh, cudaStream_t st)
 template <class T>
 int cast_f32(const float* src, T* dst, long long n, cudaStream_t st);
 
-// gather rows: dst[r] = src[idx(r)] with idx(r) = r*stride + offset   (last position of every stream)
+// gather rows: dst[r] = src[idx(r)] with idx(r) = r*stride + offset, or r*stride + lens[r] - 1 where lens (device [rows]) is
+// given   (last position of every stream)
 template <class T>
-int gather_rows(const T* src, T* dst, int rows, int d, int stride, int offset, cudaStream_t st);
+int gather_rows(const T* src, T* dst, int rows, int d, int stride, int offset, cudaStream_t st, const int* lens = nullptr);
 
 // ------------------------------------------------------------------ memory rings
-// Device-side ring state read by graph-captured kernels: [0] = pos_total (tokens appended since reset),
-// [1] = mem_count (valid memory positions, <= M).
+// Device-side ring state, read by graph-captured kernels: one row {pos_total, mem_count} per stream (tokens appended since reset,
+// valid memory positions <= M).  Kernels take it as (state, state_stride): stream s (absolute, as the ring index) reads
+// state + state_stride * s - the model passes its [max_batch][2] array with stride 2, stride 0 gives every stream the same row.
+// lens (device, indexed by the chunk-local stream b like the qkv rows) or NULL: stream b's segment is its first lens[b] of the T_len
+// rows (a right-padded batch); NULL = all T_len.
+// K/V of the last min(len_b, M) valid tokens of stream b into ring slots (pos_total_b + i) mod M
 template <class T, class TS>
-int ring_append_kv(const TS* qkv, T* kring, T* vring, int B, int T_len, int H, int Dh, int M, long long pos_total,
-                   int b0, int Bcap, cudaStream_t st);
+int ring_append_kv(const TS* qkv, T* kring, T* vring, int B, int T_len, int H, int Dh, int M, const int* state, int state_stride,
+                   const int* lens, int b0, cudaStream_t st);
 // hidden-state mems (model[0].hidden): ring [B][M][d] fp32
-int ring_append_hidden(const float* x32, float* hring, int B, int T_len, int d, int M, long long pos_total, int b0,
+int ring_append_hidden(const float* x32, float* hring, int B, int T_len, int d, int M, const int* state, int state_stride,
+                       const int* lens, int b0, cudaStream_t st);
+// the last mem_count tokens of streams [0, B), which all hold that many
+int ring_export_hidden(const float* hring, float* out, int B, int d, int M, int mem_count, const int* state, int state_stride,
                        cudaStream_t st);
-int ring_export_hidden(const float* hring, float* out, int B, int d, int M, long long pos_total, int mem_count,
-                       cudaStream_t st);
-int state_advance(int* dev_state, int T_len, int M, cudaStream_t st);
+// rows [0, n) of the model's state: pos_total += len_b, mem_count = min(mem_count + len_b, M); len_b = lens[b] or T_len
+int state_advance(int* state, int n, int T_len, const int* lens, int M, cudaStream_t st);
 
 // ------------------------------------------------------------------ attention
 struct AttnGeneralArgs {
@@ -114,8 +121,8 @@ struct AttnGeneralArgs {
   const float* v;
   void* out;            // T [rows, H*Dh]
   int B, T, H, M, Dcap;
-  int mem_count;        // valid memory positions
-  long long pos_total;  // tokens appended since reset (ring slot = token index mod M)
+  const int* state;     // ring state of stream b0 + b at state + state_stride * (b0 + b): {pos_total, mem_count} (ring slot = token
+  int state_stride;     // index mod M)
   int b0;               // first stream of this chunk (ring offset)
   int bert;             // 1: no mask, _line_shift wrap-around live (deep_music_remix.py:2096, r_mask=False)
   int win, k;           // window_mask (win_size, k); eval = (1, 1)
@@ -138,7 +145,8 @@ struct AttnDecodeArgs {
   const float* u;
   const float* v;
   bf16* out;            // [B, H*64]
-  const int* dev_state; // [0] pos_total, [1] mem_count
+  const int* state;     // ring state {pos_total, mem_count} of stream s (absolute: b0 + row) at state + state_stride * s
+  int state_stride;
   int B, H, M, Dcap;
   float scale;
   unsigned long long* dbg = nullptr;   // timeline probe (third kernel, CTA 0 and the last CTA): [48] start, [49] table built, [50] end, [51] last CTA's end

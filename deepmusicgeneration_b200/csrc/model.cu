@@ -100,7 +100,7 @@ struct DecodeStep {
     a.rd = (const bf16*)La.rd;
     a.u = m->u; a.v = m->v;
     a.out = (bf16*)m->attn + (size_t)r0 * HD;
-    a.dev_state = m->dev_state;
+    a.state = m->dev_state; a.state_stride = 2;
     a.B = r1 - r0; a.H = c.n_heads; a.M = M; a.Dcap = m->Dcap;
     a.scale = 1.f / sqrtf((float)c.d_head);
     a.force_v2 = (m->kflags & DMG_KF_ATTN_DECODE_V2) ? 1 : 0;
@@ -145,17 +145,19 @@ constexpr int SEG_DECODE = -1;   // a one-token bf16 step: the decode kernel (at
 struct SegShape {
   bool bf16, use_tc, bert;
   bool ring_tm;                 // the rings and Rd have the decode kernel's tensor maps
+  bool uniform;                 // every stream of the segment holds the same memory: mem_count / pos_total are theirs
   int T, H, M, Dcap, mem_count, win, k, kflags;
   long long pos_total;
 };
 
 // What each kernel supports (head size 64).  Flash: segments without memory (prefill after reset(), every BERT forward).  tcgen05
-// ring: whole 128-token tiles over a warm memory.  BERT tcgen05: sequences of at least 128 tokens.
+// ring: whole 128-token tiles over a warm memory.  BERT tcgen05: sequences of at least 128 tokens.  Both take one memory for all
+// streams; streams of unequal memories (after a varlen prefill) run on the general kernel, which reads each stream's own.
 static bool seg_flash_ok(const SegShape& s) {
-  return s.bf16 && s.T > 1 && (s.bert || (s.mem_count == 0 && s.win == 1 && s.k == 1)) && s.Dcap >= s.T;
+  return s.bf16 && s.T > 1 && (s.bert || (s.uniform && s.mem_count == 0 && s.win == 1 && s.k == 1)) && s.Dcap >= s.T;
 }
 static bool seg_tc_ring_ok(const SegShape& s) {
-  return s.bf16 && !s.bert && s.T > 1 && attn_fwd_tc_ring_supported(s.T, 64, s.M, s.mem_count, (int)s.pos_total);
+  return s.bf16 && !s.bert && s.T > 1 && s.uniform && attn_fwd_tc_ring_supported(s.T, 64, s.M, s.mem_count, (int)s.pos_total);
 }
 static bool seg_bert_tc_ok(const SegShape& s) { return s.bf16 && s.bert && attn_bert_tc_supported(s.T, s.H, s.Dcap); }
 static bool seg_decode_ok(const SegShape& s) {
@@ -184,18 +186,22 @@ struct SegBufs {
   const float *u, *v;
   void* out;                    // [B*T, H*64]
   int Bcap;
+  const int* state;          // ring state (kernels.cuh): stream s at state + state_stride * s
+  int state_stride;
   int fp32_strip;               // BERT tcgen05 kernel: DMG_KF_BERT_FP32_STRIP
-  const VarlenPlan* vp;         // BERT only: per-sequence lengths, or NULL
+  const VarlenPlan* vp;         // per-sequence lengths, or NULL.  BERT: the attention's plan; Transformer-XL: lens only (ring append)
 };
 
 // The attention of streams [b0, b0 + B) on the kernel `kernel` (not SEG_DECODE), then - over a memory and with `append` - the K/V of
-// the segment's last min(T, M) tokens into the rings.  T: element type of the rings / Rd / output of the general kernel.
+// each stream's last min(len, M) tokens into the rings.  T: element type of the rings / Rd / output of the general kernel.
 template <class T>
 static int segment_attention(int kernel, const SegShape& s, const SegBufs& p, int B, int b0, bool append, cudaStream_t st) {
   const float scale = 0.125f;   // 1 / sqrt(64)
+  const VarlenPlan* bert_vp = s.bert ? p.vp : nullptr;
+  const int* lens = !s.bert && p.vp ? p.vp->lens : nullptr;   // Transformer-XL: the causal mask keeps every row off the padding keys
   if (kernel == DMG_SEG_FLASH || kernel == DMG_SEG_BERT_TC) {
     const bf16* qkv = (const bf16*)p.qkv;
-    if (p.vp) {
+    if (bert_vp) {
       if (attn_bert_varlen_bf16(qkv, (const bf16*)p.rd, s.Dcap, p.u, p.v, (bf16*)p.out, *p.vp, B, s.T, s.H, scale, p.fp32_strip, st))
         return -1;
     } else if (kernel == DMG_SEG_BERT_TC) {
@@ -203,15 +209,16 @@ static int segment_attention(int kernel, const SegShape& s, const SegBufs& p, in
     } else if (attn_flash(qkv, (const bf16*)p.rd, s.Dcap, p.u, p.v, (bf16*)p.out, B, s.T, s.H, s.bert ? 1 : 0, scale, st)) {
       return -1;
     }
-    if (append && s.M > 0 && ring_append_kv<bf16, bf16>(qkv, (bf16*)p.kring, (bf16*)p.vring, B, s.T, s.H, 64, s.M, s.pos_total, b0,
-                                                       p.Bcap, st)) return -1;
+    if (append && s.M > 0 && ring_append_kv<bf16, bf16>(qkv, (bf16*)p.kring, (bf16*)p.vring, B, s.T, s.H, 64, s.M, p.state,
+                                                       p.state_stride, lens, b0, st)) return -1;
     return 0;
   }
   if (kernel == DMG_SEG_TC_RING) {
     const bf16* qkv = (const bf16*)p.qkv;
     if (attn_fwd_tc_ring(qkv, (const bf16*)p.kring, (const bf16*)p.vring, (const bf16*)p.rd, s.Dcap, p.u, p.v, (bf16*)p.out, B, s.T, s.H,
                          s.M, s.mem_count, s.win, s.k, (int)s.pos_total, b0, p.Bcap, scale, st)) return -1;
-    if (append && ring_append_kv<bf16, bf16>(qkv, (bf16*)p.kring, (bf16*)p.vring, B, s.T, s.H, 64, s.M, s.pos_total, b0, p.Bcap, st))
+    if (append && ring_append_kv<bf16, bf16>(qkv, (bf16*)p.kring, (bf16*)p.vring, B, s.T, s.H, 64, s.M, p.state, p.state_stride, lens,
+                                             b0, st))
       return -1;
     return 0;
   }
@@ -219,17 +226,31 @@ static int segment_attention(int kernel, const SegShape& s, const SegBufs& p, in
   AttnGeneralArgs a;
   a.qkv = (const float*)p.qkv; a.kring = p.kring; a.vring = p.vring; a.rd = p.rd; a.u = p.u; a.v = p.v; a.out = p.out;
   a.B = B; a.T = s.T; a.H = s.H; a.M = s.M; a.Dcap = s.Dcap;
-  a.mem_count = s.mem_count; a.pos_total = s.pos_total; a.b0 = b0; a.bert = s.bert ? 1 : 0; a.win = s.win; a.k = s.k;
+  a.state = p.state; a.state_stride = p.state_stride; a.b0 = b0; a.bert = s.bert ? 1 : 0; a.win = s.win; a.k = s.k;
   a.scale = scale;
-  a.lens = p.vp ? p.vp->lens : nullptr;
+  a.lens = bert_vp ? bert_vp->lens : nullptr;
   if (attn_general<T>(a, st)) return -1;
-  if (p.vp && varlen_zero_rows<T>((T*)p.out, p.vp->lens, B, s.T, s.H * 64, st)) return -1;
-  if (append && s.M > 0 && ring_append_kv<T, float>((const float*)p.qkv, (T*)p.kring, (T*)p.vring, B, s.T, s.H, 64, s.M, s.pos_total,
-                                                    b0, p.Bcap, st)) return -1;
+  if (bert_vp && varlen_zero_rows<T>((T*)p.out, bert_vp->lens, B, s.T, s.H * 64, st)) return -1;
+  if (append && s.M > 0 && ring_append_kv<T, float>((const float*)p.qkv, (T*)p.kring, (T*)p.vring, B, s.T, s.H, 64, s.M, p.state,
+                                                    p.state_stride, lens, b0, st)) return -1;
   return 0;
 }
 
-// vp (BERT only): the nb sequences have their own lengths (a padded batch, T_len = the padded length; see remix_batch.cu)
+// Rows [r0, r1) of the host mirror hold one memory: *pt / *mc receive it (those of row r0 when they differ)
+static bool uniform_state(const dmg_model* m, int r0, int r1, long long* pt, int* mc) {
+  *pt = m->pos_total[r0]; *mc = m->mem_count[r0];
+  for (int b = r0 + 1; b < r1; b++)
+    if (m->pos_total[b] != *pt || m->mem_count[b] != *mc) return false;
+  return true;
+}
+static bool mem_empty(const dmg_model* m) {
+  for (int b = 0; b < m->batch; b++)
+    if (m->mem_count[b]) return false;
+  return true;
+}
+
+// vp: the nb sequences have their own lengths (a padded batch, T_len = the padded length).  BERT: the attention plan of remix_batch.cu;
+// Transformer-XL: vp->lens only (chunk-local), the streams start from an empty memory.
 template <class T>
 static int forward_chunk(dmg_model* m, const long long* ids, const long long* pos, int b0, int nb, int T_len, int win,
                          int k, int logits_mode, float* logits, float* core_out, cudaStream_t st, const VarlenPlan* vp = nullptr) {
@@ -238,11 +259,12 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
   const bool bert = c.arch == DMG_ARCH_BERT;
   T* xa = (T*)m->xa;
   if (embed<T>(ids, c.encode_position ? pos : nullptr, m->emb.f32, m->beat, m->bar, m->x32, xa, rows, d, c.vocab, st)) return -1;
-  if (c.keep_hidden && M > 0 && ring_append_hidden(m->x32, m->hrings[0], nb, T_len, d, M, m->pos_total, b0, st)) return -1;
+  const int* lens = vp && !bert ? vp->lens : nullptr;
+  if (c.keep_hidden && M > 0 && ring_append_hidden(m->x32, m->hrings[0], nb, T_len, d, M, m->dev_state, 2, lens, b0, st)) return -1;
   SegShape sh;
   sh.bf16 = m->is_bf16; sh.use_tc = m->use_tc; sh.bert = bert; sh.ring_tm = m->layers[0].has_ring_tm;
-  sh.T = T_len; sh.H = c.n_heads; sh.M = M; sh.Dcap = m->Dcap; sh.mem_count = m->mem_count; sh.win = win; sh.k = k; sh.kflags = m->kflags;
-  sh.pos_total = m->pos_total;
+  sh.T = T_len; sh.H = c.n_heads; sh.M = M; sh.Dcap = m->Dcap; sh.win = win; sh.k = k; sh.kflags = m->kflags;
+  sh.uniform = uniform_state(m, b0, b0 + nb, &sh.pos_total, &sh.mem_count);
   const int route = segment_route(sh);
   const bool fast_decode = route == SEG_DECODE, qkv_bf16 = seg_qkv_bf16(route);
   // one-token step, product path: per layer ONE decode-attention launch + ONE fused layer launch (decode_layer.cu)
@@ -285,7 +307,7 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
       a.rd = (const bf16*)L.rd;
       a.u = m->u; a.v = m->v;
       a.out = (bf16*)m->attn;
-      a.dev_state = m->dev_state;
+      a.state = m->dev_state; a.state_stride = 2;
       a.B = nb; a.H = c.n_heads; a.M = M; a.Dcap = m->Dcap;
       a.scale = 1.f / sqrtf((float)c.d_head);
       a.force_v2 = (m->kflags & DMG_KF_ATTN_DECODE_V2) ? 1 : 0;
@@ -294,7 +316,8 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
       SegBufs p;
       p.qkv = qkv_bf16 ? (const void*)m->qkv16 : (const void*)m->qkv;
       p.kring = L.kring; p.vring = L.vring; p.rd = L.rd; p.u = m->u; p.v = m->v; p.out = m->attn;
-      p.Bcap = c.max_batch; p.fp32_strip = (m->kflags & DMG_KF_BERT_FP32_STRIP) ? 1 : 0; p.vp = vp;
+      p.Bcap = c.max_batch; p.state = m->dev_state; p.state_stride = 2;
+      p.fp32_strip = (m->kflags & DMG_KF_BERT_FP32_STRIP) ? 1 : 0; p.vp = vp;
       if (segment_attention<T>(route, sh, p, nb, b0, true, st)) return -1;
     }
     if (bert) {
@@ -306,35 +329,40 @@ static int forward_chunk(dmg_model* m, const long long* ids, const long long* po
       if (linear(m, A_H, m->hbuf, L.w2, L.b2, m->proj, d, rows, 0, 0, st)) return -1;
       if (residual_layernorm<T, float>(m->x32, m->proj, L.ln2w, L.ln2b, xa, rows, d, st)) return -1;
     }
-    if (c.keep_hidden && M > 0 && ring_append_hidden(m->x32, m->hrings[l + 1], nb, T_len, d, M, m->pos_total, b0, st)) return -1;
+    if (c.keep_hidden && M > 0 && ring_append_hidden(m->x32, m->hrings[l + 1], nb, T_len, d, M, m->dev_state, 2, lens, b0, st))
+      return -1;
   }
   if (core_out)
     DMG_CUDA_OK(cudaMemcpyAsync(core_out + (size_t)b0 * T_len * d, m->x32, (size_t)rows * d * 4, cudaMemcpyDeviceToDevice, st));
   if (logits_mode == DMG_LOGITS_ALL && logits) {
     if (linear(m, A_XA, xa, m->emb, m->head_b, logits + (size_t)b0 * T_len * c.vocab, c.vocab, rows, 0, 0, st)) return -1;
   } else if (logits_mode == DMG_LOGITS_LAST && !(T_len == 1 && nb == m->batch)) {
-    if (gather_rows<T>(xa, (T*)m->xlast + (size_t)b0 * d, nb, d, T_len, T_len - 1, st)) return -1;
+    if (gather_rows<T>(xa, (T*)m->xlast + (size_t)b0 * d, nb, d, T_len, T_len - 1, st, lens)) return -1;
   }
   return 0;
 }
 
+// lens_host (Transformer-XL, [bs], already validated and uploaded to vl_lens by dmg_forward_varlen) or NULL: stream b's segment is
+// the first lens_host[b] tokens of its row
 static int forward_impl(dmg_model* m, const long long* ids, const long long* pos, int bs, int T_len, int win, int k,
-                        int logits_mode, float* logits, float* core_out, cudaStream_t st) {
+                        int logits_mode, float* logits, float* core_out, cudaStream_t st, const int32_t* lens_host = nullptr) {
   const dmg_config& c = m->cfg;
   DMG_CHECK(m->committed, "dmg_forward: weights not committed (call dmg_commit_weights)");
   DMG_CHECK(bs >= 1 && bs <= c.max_batch, "dmg_forward: batch %d outside [1, max_batch=%d]", bs, c.max_batch);
   DMG_CHECK(T_len >= 1 && T_len <= c.max_seq, "dmg_forward: x_len %d outside [1, max_seq=%d]", T_len, c.max_seq);
   DMG_CHECK(T_len <= m->max_rows, "dmg_forward: x_len %d exceeds the activation workspace (%d rows)", T_len, m->max_rows);
   DMG_CHECK(!c.encode_position || pos != nullptr, "dmg_forward: model encodes position but pos is NULL");
-  if (c.arch == DMG_ARCH_BERT) { m->mem_count = 0; m->pos_total = 0; }
-  if (m->mem_count == 0) m->batch = bs;   // fastai: memory is (re)created by the first forward after reset()
+  if (mem_empty(m)) m->batch = bs;   // fastai: memory is (re)created by the first forward after reset()
   DMG_CHECK(bs == m->batch, "dmg_forward: batch %d does not match the %d streams held in memory", bs, m->batch);
   const int cb = m->max_rows / T_len;
   for (int b0 = 0; b0 < bs; b0 += cb) {
     const int nb = bs - b0 < cb ? bs - b0 : cb;
     const long long* p = pos ? pos + (size_t)b0 * T_len : nullptr;
-    int rc = m->is_bf16 ? forward_chunk<bf16>(m, ids + (size_t)b0 * T_len, p, b0, nb, T_len, win, k, logits_mode, logits, core_out, st)
-                        : forward_chunk<float>(m, ids + (size_t)b0 * T_len, p, b0, nb, T_len, win, k, logits_mode, logits, core_out, st);
+    VarlenPlan vp;
+    vp.lens = m->vl_lens + b0;
+    const VarlenPlan* v = lens_host ? &vp : nullptr;
+    int rc = m->is_bf16 ? forward_chunk<bf16>(m, ids + (size_t)b0 * T_len, p, b0, nb, T_len, win, k, logits_mode, logits, core_out, st, v)
+                        : forward_chunk<float>(m, ids + (size_t)b0 * T_len, p, b0, nb, T_len, win, k, logits_mode, logits, core_out, st, v);
     if (rc) return rc;
   }
   if (logits_mode == DMG_LOGITS_LAST) {
@@ -344,9 +372,12 @@ static int forward_impl(dmg_model* m, const long long* ids, const long long* pos
     m->logits_valid = true;
   }
   if (c.arch == DMG_ARCH_TXL && c.mem_len > 0) {
-    if (state_advance(m->dev_state, T_len, c.mem_len, st)) return -1;
-    m->pos_total += T_len;
-    m->mem_count = m->mem_count + T_len > c.mem_len ? c.mem_len : m->mem_count + T_len;
+    if (state_advance(m->dev_state, bs, T_len, lens_host ? m->vl_lens : nullptr, c.mem_len, st)) return -1;
+    for (int b = 0; b < bs; b++) {
+      const int len = lens_host ? lens_host[b] : T_len;
+      m->pos_total[b] += len;
+      m->mem_count[b] = m->mem_count[b] + len > c.mem_len ? c.mem_len : m->mem_count[b] + len;
+    }
   }
   return 0;
 }
@@ -373,7 +404,7 @@ static int varlen_setup(dmg_model* m, const int32_t* lens_host, int bs, int T_ma
   p->lens = m->vl_lens;
   p->tc_items = m->vl_items; p->n_tc_items = (int)items.size();
   p->fl_seqs = m->vl_seqs; p->n_fl_seqs = (int)seqs.size(); p->fl_max_len = fl_max;
-  m->mem_count = 0; m->pos_total = 0; m->batch = bs;
+  m->batch = bs;
   return 0;
 }
 
@@ -423,7 +454,7 @@ static int decode_forward(dmg_model* m, int bs, cudaStream_t st) {
                       nullptr, st);
 }
 
-// The one-token forward as a CUDA graph (all pointers are model-owned and static; the ring position is read from
+// The one-token forward as a CUDA graph (all pointers are model-owned and static; the ring positions are read from
 // dev_state on the device, so replay stays valid while the memory advances).
 static int decode_forward_graphed(dmg_model* m, int bs, cudaStream_t st) {
   const bool graph_ok = m->is_bf16 && m->cfg.arch == DMG_ARCH_TXL && !m->cfg.keep_hidden && m->cfg.max_rows >= bs &&
@@ -438,7 +469,8 @@ static int decode_forward_graphed(dmg_model* m, int bs, cudaStream_t st) {
       return decode_forward(m, bs, st);
     }
     const long long before = g_launch_count;
-    const long long pt = m->pos_total; const int mc = m->mem_count;
+    const std::vector<long long> pt = m->pos_total;
+    const std::vector<int> mc = m->mem_count;
     cudaGraph_t g = nullptr;
     DMG_CUDA_OK(cudaStreamBeginCapture(m->cap_stream, cudaStreamCaptureModeThreadLocal));
     int rc = decode_forward(m, bs, m->cap_stream);
@@ -454,8 +486,10 @@ static int decode_forward_graphed(dmg_model* m, int bs, cudaStream_t st) {
   }
   DMG_CUDA_OK(cudaGraphLaunch(m->step_graph, st));
   g_launch_count += m->graph_launches;
-  m->pos_total += 1;
-  m->mem_count = m->mem_count + 1 > m->cfg.mem_len ? m->cfg.mem_len : m->mem_count + 1;
+  for (int b = 0; b < bs; b++) {
+    m->pos_total[b] += 1;
+    m->mem_count[b] = m->mem_count[b] + 1 > m->cfg.mem_len ? m->cfg.mem_len : m->mem_count[b] + 1;
+  }
   m->logits_valid = true;
   return 0;
 }
@@ -473,7 +507,20 @@ long long dmg_launch_count_ll(void) { return g_launch_count; }
 int64_t dmg_launch_count(void) { return (int64_t)g_launch_count; }
 int64_t dmg_device_bytes(dmg_model* m) { return m ? m->bytes : 0; }
 int dmg_uses_tcgen05(dmg_model* m) { return m && m->use_tc ? 1 : 0; }
-int dmg_mem_count(dmg_model* m) { return m ? m->mem_count : -1; }
+int dmg_mem_count(dmg_model* m) {
+  DMG_CHECK(m, "dmg_mem_count: null model");
+  for (int b = 1; b < m->batch; b++)
+    DMG_CHECK(m->mem_count[b] == m->mem_count[0], "dmg_mem_count: the %d streams hold memories of different lengths (stream 0: %d, "
+              "stream %d: %d); read them with dmg_mem_counts", m->batch, m->mem_count[0], b, m->mem_count[b]);
+  return m->batch ? m->mem_count[0] : 0;
+}
+
+int dmg_mem_counts(dmg_model* m, int32_t* out_host, int n) {
+  DMG_CHECK(m && out_host, "dmg_mem_counts: null argument");
+  DMG_CHECK(n >= 0 && n <= m->cfg.max_batch, "dmg_mem_counts: %d streams outside [0, max_batch=%d]", n, m->cfg.max_batch);
+  for (int b = 0; b < n; b++) out_host[b] = m->mem_count[b];
+  return 0;
+}
 
 void dmg_destroy(dmg_model* m) {
   if (!m) return;
@@ -616,7 +663,9 @@ int dmg_create(const dmg_config* cfg, int device, dmg_model** out) {
   }
   { char* t = nullptr; TRY(dalloc(m, &t, RB * d * m->esz)); m->xlast = t; }
   TRY(dalloc(m, &m->logits_buf, (size_t)c.max_batch * V));
-  TRY(dalloc(m, &m->dev_state, 4));
+  TRY(dalloc(m, &m->dev_state, (size_t)2 * c.max_batch));
+  m->pos_total.assign(c.max_batch, 0);
+  m->mem_count.assign(c.max_batch, 0);
   TRY(dalloc(m, &m->ids_buf, (size_t)c.max_batch));
   TRY(dalloc(m, &m->pos_buf, (size_t)c.max_batch));
   TRY(dalloc(m, &m->tok_buf, (size_t)c.max_batch));
@@ -651,9 +700,9 @@ int dmg_create(const dmg_config* cfg, int device, dmg_model** out) {
       if (!rc && getenv("DMG_DECODE_TIMELINE")) TRY(dalloc(m, &m->dl_dbg, 64));
     }
   }
+  TRY(dalloc(m, &m->vl_lens, (size_t)c.max_batch));
   if (bert) {
     const size_t items = (size_t)c.max_batch * c.n_heads * ((c.max_seq + 127) / 128);
-    TRY(dalloc(m, &m->vl_lens, (size_t)c.max_batch));
     TRY(dalloc(m, &m->vl_items, items));
     TRY(dalloc(m, &m->vl_seqs, (size_t)c.max_batch));
     TRY(dalloc(m, &m->mk_pos, (size_t)c.max_batch * c.max_seq));
@@ -716,11 +765,11 @@ int dmg_reset(dmg_model* m, int batch) {
   DMG_CHECK(m, "dmg_reset: null model");
   DMG_CHECK(batch >= 0 && batch <= m->cfg.max_batch, "dmg_reset: batch %d outside [0, %d]", batch, m->cfg.max_batch);
   DMG_CUDA_OK(cudaSetDevice(m->device));
-  m->pos_total = 0;
-  m->mem_count = 0;
+  m->pos_total.assign(m->cfg.max_batch, 0);
+  m->mem_count.assign(m->cfg.max_batch, 0);
   m->batch = batch;
   m->logits_valid = false;
-  DMG_CUDA_OK(cudaMemset(m->dev_state, 0, 16));
+  DMG_CUDA_OK(cudaMemset(m->dev_state, 0, (size_t)m->cfg.max_batch * 8));
   return 0;
 }
 
@@ -728,7 +777,7 @@ int dmg_select_hidden(dmg_model* m, const int32_t* idx_host, int n) {
   DMG_CHECK(m && idx_host, "dmg_select_hidden: null argument");
   const dmg_config& c = m->cfg;
   DMG_CHECK(n >= 1 && n <= c.max_batch, "dmg_select_hidden: %d streams outside [1, %d]", n, c.max_batch);
-  if (c.mem_len == 0 || m->mem_count == 0) { m->batch = n; return 0; }
+  if (c.mem_len == 0 || mem_empty(m)) { m->batch = n; return 0; }
   for (int j = 0; j < n; j++)
     DMG_CHECK(idx_host[j] >= 0 && idx_host[j] < m->batch, "dmg_select_hidden: index %d out of range", idx_host[j]);
   DMG_CUDA_OK(cudaSetDevice(m->device));
@@ -753,6 +802,18 @@ int dmg_select_hidden(dmg_model* m, const int32_t* idx_host, int n) {
     if (!rc) rc = permute(h, per_h);
   cudaFree(tmp);
   if (rc) return rc;
+  // the ring state rows follow their rings; rows past the n streams are cleared
+  std::vector<long long> pt(c.max_batch, 0);
+  std::vector<int> mc(c.max_batch, 0), dev(2 * (size_t)c.max_batch, 0);
+  for (int j = 0; j < n; j++) {
+    pt[j] = m->pos_total[idx_host[j]];
+    mc[j] = m->mem_count[idx_host[j]];
+    dev[2 * j] = (int)pt[j];
+    dev[2 * j + 1] = mc[j];
+  }
+  DMG_CUDA_OK(cudaMemcpy(m->dev_state, dev.data(), dev.size() * 4, cudaMemcpyHostToDevice));
+  m->pos_total = pt;
+  m->mem_count = mc;
   m->batch = n;
   m->logits_valid = false;
   return 0;
@@ -773,10 +834,29 @@ int dmg_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, in
 
 int dmg_forward_varlen(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, const int32_t* lens_host, int bs, int T_max,
                        int logits_mode, float* logits_dev, float* core_out_dev, void* stream) {
-  DMG_CHECK(m && ids_dev && pos_dev && lens_host, "dmg_forward_varlen: null argument");
-  DMG_CHECK(logits_mode == DMG_LOGITS_NONE || logits_mode == DMG_LOGITS_ALL, "dmg_forward_varlen: logits_mode must be NONE or ALL");
+  DMG_CHECK(m && ids_dev && lens_host, "dmg_forward_varlen: null argument");
+  DMG_CHECK(pos_dev || (m->cfg.arch == DMG_ARCH_TXL && !m->cfg.encode_position), "dmg_forward_varlen: pos is NULL");
   DMG_CUDA_OK(cudaSetDevice(m->device));
   cudaStream_t st = (cudaStream_t)stream;
+  if (m->cfg.arch == DMG_ARCH_TXL) {
+    // every stream is one memory-less forward over its own seed (predict after reset()); the streams are independent, so the batch
+    // may go through the activation workspace in chunks of streams
+    const dmg_config& c = m->cfg;
+    DMG_CHECK(logits_mode >= DMG_LOGITS_NONE && logits_mode <= DMG_LOGITS_LAST, "dmg_forward_varlen: logits_mode %d", logits_mode);
+    DMG_CHECK(m->committed, "dmg_forward_varlen: weights not committed (call dmg_commit_weights)");
+    DMG_CHECK(bs >= 1 && bs <= c.max_batch, "dmg_forward_varlen: batch %d outside [1, max_batch=%d]", bs, c.max_batch);
+    DMG_CHECK(T_max >= 1 && T_max <= c.max_seq, "dmg_forward_varlen: T_max %d outside [1, max_seq=%d]", T_max, c.max_seq);
+    for (int b = 0; b < bs; b++)
+      DMG_CHECK(lens_host[b] >= 1 && lens_host[b] <= T_max, "dmg_forward_varlen: length %d of stream %d outside [1, T_max=%d]",
+                lens_host[b], b, T_max);
+    for (int b = 0; b < m->batch; b++)
+      DMG_CHECK(m->mem_count[b] == 0, "dmg_forward_varlen: stream %d holds %d memory tokens; the Transformer-XL form starts every "
+                "stream from an empty memory (call dmg_reset first)", b, m->mem_count[b]);
+    DMG_CUDA_OK(cudaMemcpyAsync(m->vl_lens, lens_host, (size_t)bs * 4, cudaMemcpyHostToDevice, st));
+    return forward_impl(m, (const long long*)ids_dev, (const long long*)pos_dev, bs, T_max, 1, 1, logits_mode, logits_dev, core_out_dev,
+                        st, lens_host);
+  }
+  DMG_CHECK(logits_mode == DMG_LOGITS_NONE || logits_mode == DMG_LOGITS_ALL, "dmg_forward_varlen: logits_mode must be NONE or ALL");
   VarlenPlan p;
   if (varlen_setup(m, lens_host, bs, T_max, &p, st)) return -1;
   return forward_varlen(m, (const long long*)ids_dev, (const long long*)pos_dev, p, bs, T_max, logits_mode, logits_dev, core_out_dev, st);
@@ -889,8 +969,13 @@ int dmg_get_hidden(dmg_model* m, int level, float* out_dev, void* stream) {
   DMG_CHECK(m && out_dev, "dmg_get_hidden: null argument");
   DMG_CHECK(m->cfg.keep_hidden && !m->hrings.empty(), "dmg_get_hidden: model was created without keep_hidden");
   DMG_CHECK(level >= 0 && level <= m->cfg.n_layers, "dmg_get_hidden: level %d out of range", level);
+  if (m->batch == 0) return 0;
+  for (int b = 1; b < m->batch; b++)
+    DMG_CHECK(m->mem_count[b] == m->mem_count[0], "dmg_get_hidden: the %d streams hold memories of different lengths (stream 0: %d, "
+              "stream %d: %d), which one [bs, mem_count, d_model] tensor cannot hold; read the per-stream counts with dmg_mem_counts",
+              m->batch, m->mem_count[0], b, m->mem_count[b]);
   DMG_CUDA_OK(cudaSetDevice(m->device));
-  return ring_export_hidden(m->hrings[level], out_dev, m->batch, m->cfg.d_model, m->cfg.mem_len, m->pos_total, m->mem_count,
+  return ring_export_hidden(m->hrings[level], out_dev, m->batch, m->cfg.d_model, m->cfg.mem_len, m->mem_count[0], m->dev_state, 2,
                             (cudaStream_t)stream);
 }
 
@@ -1040,7 +1125,7 @@ int dmg_attn_decode_layer(dmg_model* m, int layer, void* stream) {
   LayerW& L = m->layers[layer];
   AttnDecodeArgs a;
   a.qkv = m->qkv; a.kring = (bf16*)L.kring; a.vring = (bf16*)L.vring; a.rd = (const bf16*)L.rd;
-  a.u = m->u; a.v = m->v; a.out = (bf16*)m->attn; a.dev_state = m->dev_state;
+  a.u = m->u; a.v = m->v; a.out = (bf16*)m->attn; a.state = m->dev_state; a.state_stride = 2;
   a.B = m->batch; a.H = c.n_heads; a.M = c.mem_len; a.Dcap = m->Dcap;
   a.scale = 1.f / sqrtf((float)c.d_head);
   return attn_decode2(&L.tmK, &L.tmV, &L.tmR, a, 0, m->num_sms, (cudaStream_t)stream);
@@ -1073,8 +1158,24 @@ struct DecodeAttnPlan {
   int state[2] = {0, 0};
 };
 
-static int plan_decode_attn(const dmg_decode_attn_args* p, DecodeAttnPlan& o, const char* who) {
-  DMG_CHECK(p && p->qkv && p->kring && p->vring && p->rd && p->u && p->v && p->out && p->state, "%s: null argument", who);
+// Rows [b0, b0 + B) of a caller's per-stream ring state [Bcap][2] (device): each must be {pos_total, min(pos_total, M)} (the invariant
+// the model keeps) with pos_total + T < 2^31.  Returns them in rows (host).
+static int check_stream_state(const int32_t* state_dev, int b0, int B, int M, int T, std::vector<int>& rows, const char* who) {
+  rows.assign(2 * (size_t)B, 0);
+  DMG_CUDA_OK(cudaMemcpy(rows.data(), state_dev + 2 * (size_t)b0, rows.size() * 4, cudaMemcpyDeviceToHost));
+  for (int b = 0; b < B; b++) {
+    const int pt = rows[2 * b], mc = rows[2 * b + 1];
+    DMG_CHECK(pt >= 0 && (long long)pt + T <= 0x7fffffffLL && mc == (pt < M ? pt : M),
+              "%s: state of stream %d is {%d, %d}, not {pos_total, min(pos_total, M = %d)} with pos_total in [0, 2^31 - %d)", who, b0 + b,
+              pt, mc, M, T);
+  }
+  return 0;
+}
+
+// stream_state: NULL = the args' own state buffer, which receives the uniform pos_total (stride 0); else the per-stream state [Bcap][2]
+// of dmg_attn_decode_streams (stride 2; the args' state and pos_total are not used)
+static int plan_decode_attn(const dmg_decode_attn_args* p, DecodeAttnPlan& o, const char* who, const int32_t* stream_state = nullptr) {
+  DMG_CHECK(p && p->qkv && p->kring && p->vring && p->rd && p->u && p->v && p->out && (p->state || stream_state), "%s: null argument", who);
   DMG_CHECK(p->Dh == 64, "%s: head size %d (only 64)", who, p->Dh);
   DMG_CHECK(p->kernel == 0 || p->kernel == 1, "%s: kernel %d (0 = the step's choice, 1 = the second-generation kernel)", who, p->kernel);
   // kernel 0 falls back to the second kernel where the third does not apply, so both choices need what the second one supports
@@ -1082,7 +1183,12 @@ static int plan_decode_attn(const dmg_decode_attn_args* p, DecodeAttnPlan& o, co
   DMG_CHECK(p->Dcap >= p->M + 1, "%s: rel-pos cache too small (Dcap %d < M + 1 = %d)", who, p->Dcap, p->M + 1);
   DMG_CHECK(p->B >= 1 && p->H >= 1 && p->H <= 64 && p->b0 >= 0 && (long long)p->b0 + p->B <= p->Bcap,
             "%s: B %d, H %d, streams [%d, %d) outside the ring's %d", who, p->B, p->H, p->b0, p->b0 + p->B, p->Bcap);
-  DMG_CHECK(p->pos_total >= 0 && p->pos_total <= 0x7fffffffLL, "%s: pos_total %lld outside [0, 2^31)", who, (long long)p->pos_total);
+  if (stream_state) {
+    std::vector<int> rows;
+    if (check_stream_state(stream_state, p->b0, p->B, p->M, 1, rows, who)) return -1;
+  } else {
+    DMG_CHECK(p->pos_total >= 0 && p->pos_total <= 0x7fffffffLL, "%s: pos_total %lld outside [0, 2^31)", who, (long long)p->pos_total);
+  }
   const long long ring_rows = (long long)p->Bcap * p->H * p->M;
   if (make_tmap_bf16(&o.tmK, p->kring, 64, ring_rows, 64, 64) || make_tmap_bf16(&o.tmV, p->vring, 64, ring_rows, 64, 64) ||
       make_tmap_bf16(&o.tmR, p->rd, 64, (long long)p->H * p->Dcap, 64, 64)) return -1;
@@ -1092,7 +1198,8 @@ static int plan_decode_attn(const dmg_decode_attn_args* p, DecodeAttnPlan& o, co
   AttnDecodeArgs& a = o.a;
   const size_t chunk = (size_t)p->b0 * p->H * p->M * 64;      // the kernels take ring pointers offset by b0 streams
   a.qkv = p->qkv; a.kring = (bf16*)p->kring + chunk; a.vring = (bf16*)p->vring + chunk; a.rd = (const bf16*)p->rd;
-  a.u = p->u; a.v = p->v; a.out = (bf16*)p->out; a.dev_state = p->state;
+  a.u = p->u; a.v = p->v; a.out = (bf16*)p->out;
+  a.state = stream_state ? stream_state : p->state; a.state_stride = stream_state ? 2 : 0;
   a.B = p->B; a.H = p->H; a.M = p->M; a.Dcap = p->Dcap;
   a.scale = 0.125f;
   a.force_v2 = p->kernel;
@@ -1145,16 +1252,27 @@ static int plan_decode_layer(const dmg_decode_layer_args* p, DecodeLayerPlan& o,
 
 extern "C" {
 
-int dmg_attn_decode(const dmg_decode_attn_args* p, void* stream) {
-  DecodeAttnPlan o;
-  if (plan_decode_attn(p, o, "dmg_attn_decode")) return -1;
-  cudaStream_t st = (cudaStream_t)stream;
-  DMG_CUDA_OK(cudaMemcpyAsync(p->state, o.state, sizeof(o.state), cudaMemcpyHostToDevice, st));
+static int run_decode_attn(const DecodeAttnPlan& o, cudaStream_t st) {
   const int rc = attn_decode2(&o.tmK, &o.tmV, &o.tmR, o.a, o.b0, o.num_sms, st);
   const cudaError_t e = cudaStreamSynchronize(st);
   if (rc) return rc;
   DMG_CUDA_OK(e);
   return 0;
+}
+
+int dmg_attn_decode(const dmg_decode_attn_args* p, void* stream) {
+  DecodeAttnPlan o;
+  if (plan_decode_attn(p, o, "dmg_attn_decode")) return -1;
+  cudaStream_t st = (cudaStream_t)stream;
+  DMG_CUDA_OK(cudaMemcpyAsync(p->state, o.state, sizeof(o.state), cudaMemcpyHostToDevice, st));
+  return run_decode_attn(o, st);
+}
+
+int dmg_attn_decode_streams(const dmg_decode_attn_args* p, const int32_t* stream_state_dev, void* stream) {
+  DecodeAttnPlan o;
+  DMG_CHECK(stream_state_dev, "dmg_attn_decode_streams: null state");
+  if (plan_decode_attn(p, o, "dmg_attn_decode_streams", stream_state_dev)) return -1;
+  return run_decode_attn(o, (cudaStream_t)stream);
 }
 
 int dmg_decode_layer_step(const dmg_decode_layer_args* f, void* stream) {
@@ -1194,9 +1312,14 @@ int dmg_decode_dual(const dmg_decode_layer_args* f, const dmg_decode_attn_args* 
   return 0;
 }
 
-int dmg_attn_segment(dmg_segment_attn_args* p, void* stream) {
+}  // extern "C"
+
+namespace dmg {
+
+// dmg_attn_segment (stream_state NULL: one pos_total for every stream, passed to the kernels with stride 0) and
+// dmg_attn_segment_streams (the caller's per-stream state [Bcap][2], stride 2)
+static int attn_segment(dmg_segment_attn_args* p, const int32_t* stream_state, const char* who, cudaStream_t st) {
   static_assert(sizeof(dmg_segment_attn_args) == 120, "tests/test_abi.py mirrors this layout");
-  const char* who = "dmg_attn_segment";
   DMG_CHECK(p, "%s: null argument", who);
   DMG_CHECK(p->arch == DMG_ARCH_TXL || p->arch == DMG_ARCH_BERT, "%s: arch %d (0 = Transformer-XL, 1 = BERT)", who, p->arch);
   DMG_CHECK(p->dtype == DMG_F32 || p->dtype == DMG_BF16, "%s: dtype %d (0 = fp32, 1 = bf16)", who, p->dtype);
@@ -1205,20 +1328,27 @@ int dmg_attn_segment(dmg_segment_attn_args* p, void* stream) {
   DMG_CHECK(p->append == 0 || p->append == 1, "%s: append %d (0 or 1)", who, p->append);
   const bool bert = p->arch == DMG_ARCH_BERT;
   DMG_CHECK(p->B >= 1 && p->T >= 1 && p->H >= 1 && p->H <= 256 && p->M >= 0, "%s: B %d, T %d, H %d, M %d", who, p->B, p->T, p->H, p->M);
-  DMG_CHECK(p->pos_total >= 0 && p->pos_total + p->T <= 0x7fffffffLL, "%s: pos_total %lld outside [0, 2^31 - T)", who,
-            (long long)p->pos_total);
-  DMG_CHECK(!bert || (p->M == 0 && p->pos_total == 0), "%s: the BERT encoder has no memory (M %d, pos_total %lld)", who, p->M,
-            (long long)p->pos_total);
-  DMG_CHECK(p->qkv && p->rd && p->u && p->v && p->out && (p->M == 0 || (p->kring && p->vring)), "%s: null argument", who);
   DMG_CHECK(p->b0 >= 0 && (long long)p->b0 + p->B <= p->Bcap, "%s: streams [%d, %d) outside the ring's %d", who, p->b0, p->b0 + p->B,
             p->Bcap);
+  SegShape s;
+  std::vector<int> rows;
+  if (stream_state) {
+    if (check_stream_state(stream_state, p->b0, p->B, p->M, p->T, rows, who)) return -1;
+    s.pos_total = rows[0]; s.mem_count = rows[1]; s.uniform = true;
+    for (int b = 1; b < p->B; b++) s.uniform = s.uniform && rows[2 * b] == rows[0];
+  } else {
+    DMG_CHECK(p->pos_total >= 0 && p->pos_total + p->T <= 0x7fffffffLL, "%s: pos_total %lld outside [0, 2^31 - T)", who,
+              (long long)p->pos_total);
+    s.pos_total = p->pos_total; s.mem_count = (int)(p->pos_total < p->M ? p->pos_total : p->M); s.uniform = true;
+  }
+  DMG_CHECK(!bert || (p->M == 0 && s.uniform && s.pos_total == 0), "%s: the BERT encoder has no memory (M %d, pos_total %lld)", who,
+            p->M, (long long)s.pos_total);
+  DMG_CHECK(p->qkv && p->rd && p->u && p->v && p->out && (p->M == 0 || (p->kring && p->vring)), "%s: null argument", who);
   DMG_CHECK(p->Dcap >= (long long)p->M + p->T + 1, "%s: rel-pos cache too small (Dcap %d < M + T + 1 = %lld)", who, p->Dcap,
             (long long)p->M + p->T + 1);
   DMG_CHECK(p->win >= 1 && (bert || (p->win == 1 && p->k == 1) || p->k == 0), "%s: window mask (%d,%d) unsupported", who, p->win, p->k);
-  SegShape s;
   s.bf16 = p->dtype == DMG_BF16; s.use_tc = s.bf16; s.bert = bert; s.ring_tm = true;
-  s.T = p->T; s.H = p->H; s.M = p->M; s.Dcap = p->Dcap; s.mem_count = (int)(p->pos_total < p->M ? p->pos_total : p->M);
-  s.win = p->win; s.k = p->k; s.kflags = 0; s.pos_total = p->pos_total;
+  s.T = p->T; s.H = p->H; s.M = p->M; s.Dcap = p->Dcap; s.win = p->win; s.k = p->k; s.kflags = 0;
   int kernel = p->kernel;
   if (kernel == DMG_SEG_AUTO) {
     kernel = segment_route(s);
@@ -1227,21 +1357,47 @@ int dmg_attn_segment(dmg_segment_attn_args* p, void* stream) {
   } else {
     const bool ok = kernel == DMG_SEG_GENERAL || (kernel == DMG_SEG_FLASH && seg_flash_ok(s)) ||
                     (kernel == DMG_SEG_TC_RING && seg_tc_ring_ok(s)) || (kernel == DMG_SEG_BERT_TC && seg_bert_tc_ok(s));
-    DMG_CHECK(ok, "%s: kernel %d does not support this segment (arch %d, dtype %d, T %d, H %d, M %d, mem_count %d, pos_total %lld, mask "
-              "(%d,%d), Dcap %d)", who, kernel, p->arch, p->dtype, p->T, p->H, p->M, s.mem_count, (long long)p->pos_total, p->win, p->k,
-              p->Dcap);
+    DMG_CHECK(ok, "%s: kernel %d does not support this segment (arch %d, dtype %d, T %d, H %d, M %d, mem_count %d, pos_total %lld%s, mask "
+              "(%d,%d), Dcap %d)", who, kernel, p->arch, p->dtype, p->T, p->H, p->M, s.mem_count, (long long)s.pos_total,
+              s.uniform ? "" : " in stream b0, others differ", p->win, p->k, p->Dcap);
   }
   p->kernel_ran = kernel;
   SegBufs b;
   b.qkv = p->qkv; b.kring = p->kring; b.vring = p->vring; b.rd = p->rd; b.u = p->u; b.v = p->v; b.out = p->out;
   b.Bcap = p->Bcap; b.fp32_strip = 0; b.vp = nullptr;
-  cudaStream_t st = (cudaStream_t)stream;
+  int* own = nullptr;   // the uniform entry's one state row
+  if (stream_state) {
+    b.state = stream_state; b.state_stride = 2;
+  } else {
+    const int row[2] = {(int)s.pos_total, s.mem_count};
+    DMG_CUDA_OK(cudaMalloc(&own, sizeof(row)));
+    if (cudaMemcpyAsync(own, row, sizeof(row), cudaMemcpyHostToDevice, st) != cudaSuccess) {
+      cudaFree(own);
+      set_error("%s: state upload failed", who);
+      return -1;
+    }
+    b.state = own; b.state_stride = 0;
+  }
   const int rc = s.bf16 ? segment_attention<bf16>(kernel, s, b, p->B, p->b0, p->append != 0, st)
                         : segment_attention<float>(kernel, s, b, p->B, p->b0, p->append != 0, st);
   const cudaError_t e = cudaStreamSynchronize(st);
+  if (own) cudaFree(own);
   if (rc) return rc;
   DMG_CUDA_OK(e);
   return 0;
+}
+
+}  // namespace dmg
+
+extern "C" {
+
+int dmg_attn_segment(dmg_segment_attn_args* p, void* stream) {
+  return attn_segment(p, nullptr, "dmg_attn_segment", (cudaStream_t)stream);
+}
+
+int dmg_attn_segment_streams(dmg_segment_attn_args* p, const int32_t* stream_state_dev, void* stream) {
+  DMG_CHECK(stream_state_dev, "dmg_attn_segment_streams: null state");
+  return attn_segment(p, stream_state_dev, "dmg_attn_segment_streams", (cudaStream_t)stream);
 }
 
 int dmg_gemm_bf16(const void* a_dev, const void* w_dev, const float* bias_dev, void* c_dev, int M, int N, int K, int gelu,

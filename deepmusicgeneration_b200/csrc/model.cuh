@@ -58,9 +58,11 @@ struct dmg_model {
   std::map<std::string, RegEntry> reg;
   std::vector<void*> allocs;
   long long bytes = 0;
-  // memory state
-  long long pos_total = 0;
-  int mem_count = 0, batch = 0;
+  // memory state: per stream {pos_total (tokens appended since reset), mem_count (valid memory positions, <= mem_len)}, on the device
+  // ([max_batch][2], read by the kernels, also under graph replay) and its host mirror.  Rows >= batch are zero.
+  std::vector<long long> pos_total;
+  std::vector<int> mem_count;
+  int batch = 0;
   int* dev_state = nullptr;
   // workspaces
   float *x32 = nullptr, *qkv = nullptr, *proj = nullptr, *logits_buf = nullptr;

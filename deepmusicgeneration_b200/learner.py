@@ -181,7 +181,8 @@ class MusicLearner:
         tr.sync_for_inference()
         return tr.losses()
 
-    def _prefill(self, x, pos):
+    def _prefill(self, x, pos, lens=None):
+        "x / pos [B, T]; lens: the seed length of every row of a right-padded x (dmg_forward_varlen), or None (all T)"
         max_seq = self.model._e.cfg.max_seq
         if x.shape[1] > max_seq:
             # the reference runs the whole seed as ONE forward (memory-less attention over every seed token); splitting it into
@@ -190,7 +191,7 @@ class MusicLearner:
                              f'music_model_learner(..., max_seq=<longest seed>) or cut the seed with item.trim_to_beat(...)')
         enc = self.model[0]
         enc._bs = x.shape[0]
-        self.model._e.forward(x, pos if enc.encode_position else None, _lib.LOGITS_LAST)
+        self.model._e.forward(x, pos if enc.encode_position else None, _lib.LOGITS_LAST, lens=lens)
 
     def _run_loop(self, n_words, prev_idx, last_pos, params):
         e = self.model._e
@@ -235,18 +236,74 @@ class MusicLearner:
         return pred, full
 
     def generate_batch(self, x, pos=None, n_words=128, temperatures=(1.0, 1.0, 1.0), min_bars=4, top_k=30, top_p=0.6,
-                       seed=0, early_stop=False, mask_unused=False):
-        """`predict` over B independent streams: x LongTensor [B, T] of seeds (equal length), returns int32
-        [n_words, B] on the device (-1 = stream stopped, -2 = stream hit the reference's AssertionError case)."""
+                       seed=0, early_stop=False, mask_unused=False, lens=None):
+        """`predict` over B independent streams: x LongTensor [B, T] of seeds, returns int32 [n_words, B] on the device (-1 = stream
+        stopped, -2 = stream hit the reference's AssertionError case).  lens: the seed length of every row of a right-padded x (seeds
+        of different lengths; stream b continues from column lens[b] - 1), or None (every row is a whole seed of T tokens)."""
         self.model.reset()
         x = x.to(self.model._e.device)
         B, T = x.shape
         if pos is None:
             pos = torch.zeros_like(x)
-        self._prefill(x, pos)
+        self._prefill(x, pos, lens)
         flags = (_lib.SAMPLE_EARLY_STOP if early_stop else 0) | (_lib.SAMPLE_MASK_UNUSED if mask_unused else 0)
         params = sampler_params(self.data.vocab, n_words, temperatures, min_bars, top_k, top_p, None, flags=flags, seed=seed)
-        return self._run_loop(n_words, x[:, -1].cpu().numpy(), pos[:, -1].cpu().numpy(), params)
+        last = np.full(B, T - 1) if lens is None else np.asarray(lens, dtype=np.int64) - 1
+        rows = np.arange(B)
+        return self._run_loop(n_words, x.cpu().numpy()[rows, last], pos.cpu().numpy()[rows, last], params)
+
+    def predict_batch(self, items, n_words=128, temperatures=(1.0, 1.0, 1.0), min_bars=4, top_k=30, top_p=0.6, allowed_ins=None,
+                      seed=None):
+        """`predict` over many seeds of their own lengths at once: returns one (pred, full) per item, as predict(item) returns it.  The
+        seeds are prefilled together (each as one memory-less forward over itself, dmg_forward_varlen) and the token loop runs on the
+        device for all of them; a stream that stops (BOS, or the bar rule) only emits stop marks from then on.  Item i draws from
+        Philox stream i of `seed`, so predict_batch([item], seed=s) makes the draws of predict(item, seed=s).  The sampling parameters
+        and allowed_ins (rewritten in place once, as predict does) are shared by every item.  At most max_batch items, each of 1 to
+        max_seq tokens."""
+        e = self.model._e
+        vocab = self.data.vocab
+        cfg = e.cfg
+        items = list(items)
+        if len(items) > cfg.max_batch:
+            raise ValueError(f'{len(items)} items exceed max_batch={cfg.max_batch}: build the learner with '
+                             f'music_model_learner(..., max_batch=<items>) or call predict_batch on fewer items')
+        datas = [np.asarray(it.data, dtype=np.int64) for it in items]
+        for i, d in enumerate(datas):
+            if len(d) == 0:
+                raise ValueError(f'item {i} is empty')
+            if len(d) > cfg.max_seq:
+                raise ValueError(f'item {i} has {len(d)} tokens and exceeds max_seq={cfg.max_seq}: build the learner with '
+                                 f'music_model_learner(..., max_seq=<longest seed>) or cut the item with item.trim_to_beat(...)')
+        if not items:
+            return []
+        if allowed_ins is not None:                   # the reference rewrites the caller's list in place (:1878-1880)
+            for i, ins in enumerate(allowed_ins):
+                allowed_ins[i] = 'i' + str(ACCEP_INS[ins])
+        B, T = len(items), max(len(d) for d in datas)
+        lens = np.array([len(d) for d in datas], dtype=np.int32)
+        x = np.full((B, T), vocab.pad_idx, dtype=np.int64)
+        pos = np.zeros((B, T), dtype=np.int64)
+        for b, it in enumerate(items):
+            x[b, :lens[b]] = datas[b]
+            pos[b, :lens[b]] = np.asarray(it.position, dtype=np.int64)
+        self.model.reset()
+        self._prefill(torch.from_numpy(x).to(e.device), torch.from_numpy(pos).to(e.device), lens)
+        params = sampler_params(vocab, n_words, temperatures, min_bars, top_k, top_p, allowed_ins, seed=seed)
+        rows = np.arange(B)
+        toks = self._run_loop(n_words, x[rows, lens - 1], pos[rows, lens - 1], params).cpu().numpy()
+        out = []
+        for b, it in enumerate(items):
+            new_idx = []
+            for t in toks[:, b]:
+                if t == -2:
+                    bad = new_idx[-1] if new_idx else int(datas[b][-1])
+                    raise AssertionError(f'item {b}: Assertion error: prev_idx = {vocab.itos[bad]}')
+                if t < 0:
+                    break
+                new_idx.append(int(t))
+            pred = vocab.to_music_item(np.array(new_idx, dtype=np.int64), it.ins)
+            out.append((pred, it.append(pred)))
+        return out
 
     def beam_search(self, xb, n_words, top_k=10, beam_sz=10, temperature=1., return_beams=False):
         """Return the `n_words` that come after `xb` using beam search (signature of deep_music_genre.py:1823-1851).

@@ -124,8 +124,9 @@ class _Engine:
 
     # ---- forward
     def forward(self, ids, pos, logits_mode, want_core=False, mask=(1, 1), lens=None):
-        """One forward over ids [bs, T].  lens (BERT encoder only): the length of every row, a padded batch of sequences that are each
-        computed as if alone at their length (dmg_forward_varlen); logits_mode LOGITS_NONE or LOGITS_ALL."""
+        """One forward over ids [bs, T].  lens: the length of every row, a padded batch of sequences that are each computed as if alone
+        at their length (dmg_forward_varlen).  BERT encoder: logits_mode LOGITS_NONE or LOGITS_ALL.  Transformer-XL: the prefill of
+        bs seeds after reset() (every stream then holds its own seed as memory); LOGITS_LAST gives the logits of row lens[b] - 1."""
         assert ids.dim() == 2
         ids = ids.to(self.device, torch.int64).contiguous()
         if pos is not None:
@@ -154,7 +155,18 @@ class _Engine:
         check(self.lib.dmg_reset(self.h, batch), 'dmg_reset')
 
     def mem_count(self):
-        return self.lib.dmg_mem_count(self.h)
+        "memory positions held by every stream (ValueError when the streams hold memories of different lengths: see mem_counts)"
+        m = self.lib.dmg_mem_count(self.h)
+        if m < 0:
+            raise ValueError(self.lib.dmg_last_error().decode())
+        return m
+
+    def mem_counts(self, n=None):
+        "memory positions held by each of the first n streams (default: max_batch), a list"
+        n = self.cfg.max_batch if n is None else n
+        out = np.zeros(n, dtype=np.int32)
+        check(self.lib.dmg_mem_counts(self.h, out.ctypes.data_as(C.c_void_p), n), 'dmg_mem_counts')
+        return out.tolist()
 
     def hidden(self, level, bs):
         m = self.mem_count()
@@ -217,6 +229,10 @@ class MusicTransformerXL:
         "List of L+1 tensors [bs, <=mem_len, d] (empty 1-D tensors right after reset), fetched from the device rings."
         if not self._e.cfg.keep_hidden:
             raise RuntimeError('model was built with keep_hidden=False (generation-only engine)')
+        counts = self._e.mem_counts(self._bs)
+        if len(set(counts)) > 1:
+            raise ValueError(f'the {self._bs} streams hold memories of different lengths (per-stream counts {counts}), which one '
+                             f'[bs, mem, d] tensor per layer cannot hold; read them with the engine\'s mem_counts()')
         return [self._e.hidden(l, self._bs) for l in range(self.n_layers + 1)]
 
     def select_hidden(self, idxs):

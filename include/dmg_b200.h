@@ -105,14 +105,21 @@ int dmg_get_weight(dmg_model* m, const char* name, float* out_host, int64_t nume
  * PositionalEncoding) into the per-layer key cache, builds the TMA tensor maps. */
 int dmg_commit_weights(dmg_model* m);
 
+/* The Transformer-XL memory is kept per stream: stream b holds pos_total_b tokens appended since the reset and mem_count_b =
+ * min(pos_total_b, mem_len) memory positions.  Streams of a dmg_forward advance together; after a dmg_forward_varlen prefill every
+ * stream holds its own seed. */
+
 /* SequentialRNN.reset() -> TransformerXL.reset() (deep_music_genre.py:1857): drop all memory; `batch`
  * streams become active. */
 int dmg_reset(dmg_model* m, int batch);
 /* TransformerXL.select_hidden(idxs) (used by beam_search, deep_music_genre.py:1847): new stream j takes
- * the memory of old stream idx[j]. */
+ * the memory of old stream idx[j], with its counts. */
 int dmg_select_hidden(dmg_model* m, const int32_t* idx_host, int n);
-/* hidden[0].size(1) of the reference: number of memory positions currently held. */
+/* hidden[0].size(1) of the reference: number of memory positions currently held by every stream.  Fails when the streams hold
+ * memories of different lengths (read those with dmg_mem_counts). */
 int dmg_mem_count(dmg_model* m);
+/* mem_count of streams [0, n) into out_host[n] (host memory), n <= max_batch; streams past the active ones hold 0. */
+int dmg_mem_counts(dmg_model* m, int32_t* out_host, int n);
 
 /* model(x) (deep_music_genre.py:1617-1647 + LinearDecoder; deep_music_remix.py:1874-1881 for DMG_ARCH_BERT).
  * ids_dev/pos_dev: int64 [bs, x_len] (pos_dev may be NULL unless encode_position).  mask_win/mask_k: the
@@ -123,7 +130,18 @@ int dmg_mem_count(dmg_model* m);
 int dmg_forward(dmg_model* m, const int64_t* ids_dev, const int64_t* pos_dev, int bs, int x_len, int mask_win,
                 int mask_k, int logits_mode, float* logits_dev, float* core_out_dev, void* stream);
 
-/* The BERT encoder (DMG_ARCH_BERT) over a padded batch of bs sequences of their own lengths: ids_dev / pos_dev int64 [bs, T_max],
+/* A padded batch of bs sequences of their own lengths.
+ *
+ * DMG_ARCH_TXL: the prefill of predict for bs seeds at once.  ids_dev / pos_dev int64 [bs, T_max] (pos_dev may be NULL unless
+ * encode_position), seed b is the first lens_host[b] in [1, T_max] tokens of row b.  Needs an empty memory (dmg_reset first; refused
+ * otherwise).  Every stream is computed as one memory-less forward over its own seed (the rows < lens[b] of the segment; the padding
+ * rows compute values of no meaning and never reach the memory); afterwards stream b holds pos_total = lens[b] and mem_count =
+ * min(lens[b], mem_len).  logits_mode DMG_LOGITS_NONE, DMG_LOGITS_ALL (logits_dev fp32 [bs, T_max, V]) or DMG_LOGITS_LAST (the logits of
+ * row lens[b] - 1 of every stream, logits_dev fp32 [bs, V] or NULL; dmg_sampler_init + dmg_generate continue from them).  The batch
+ * runs through the activation workspace in chunks of max_rows / T_max streams.  A later multi-token dmg_forward over streams of
+ * unequal memories runs on the general attention kernel.
+ *
+ * DMG_ARCH_BERT: the encoder over a padded batch of bs sequences of their own lengths: ids_dev / pos_dev int64 [bs, T_max],
  * sequence b is row b of length lens_host[b] in [1, T_max] (host memory); what its padding positions hold does not matter.  Every
  * sequence is computed as if it were alone at its length (dmg_forward with x_len = lens[b]): the same attention kernel - except a
  * one-token sequence in a batch with T_max > 1, which runs on the flash kernel in bf16 where alone it runs on the FFMA kernel - and
@@ -148,7 +166,7 @@ int dmg_predict_mask_batch(dmg_model* m, int64_t* ids_dev, const int64_t* pos_de
                            const dmg_vocab_layout* vocab, const dmg_sampler_params* params, void* stream);
 
 /* raw_outputs[level] of the reference forward (= model[0].hidden[level]): fp32 [bs, mem_count, d_model].
- * Needs cfg.keep_hidden. */
+ * Needs cfg.keep_hidden, and fails when the streams hold memories of different lengths (see dmg_mem_counts). */
 int dmg_get_hidden(dmg_model* m, int level, float* out_dev, void* stream);
 
 /* MusicLearner.predict state (deep_music_genre.py:1856-1881): per stream the previous token (item.data[-1]),
@@ -405,6 +423,10 @@ typedef struct dmg_decode_attn_args {
   int32_t B, H, Dh, M, Dcap, Bcap, b0, kernel;
 } dmg_decode_attn_args;
 int dmg_attn_decode(const dmg_decode_attn_args* a, void* stream);
+/* The same over streams of their own memories: stream_state_dev is a per-stream ring state int32 [Bcap][2] on the device, row s =
+ * {pos_total_s, min(pos_total_s, M)} (checked), and rows b0 .. b0 + B - 1 take the place of pos_total; the state and pos_total fields
+ * of the args are not used.  The kernels read it as the model's one-token step reads its state (stride 2). */
+int dmg_attn_decode_streams(const dmg_decode_attn_args* a, const int32_t* stream_state_dev, void* stream);
 
 /* dmg_decode_layer_args: the fused one-token layer step over rows [row_base, B) (d_model 512, d_inner 2048, 8 heads of 64: the
  * geometry the kernel supports).  mode bit 0 = layer body: x32 = LN2(x1 + W2 gelu_tanh(W1 x1 + b1) + b2) with
@@ -463,6 +485,10 @@ typedef struct dmg_segment_attn_args {
   int32_t kernel_ran;        /* out: DMG_SEG_GENERAL .. DMG_SEG_BERT_TC */
 } dmg_segment_attn_args;
 int dmg_attn_segment(dmg_segment_attn_args* a, void* stream);
+/* The same over streams of their own memories: stream_state_dev as for dmg_attn_decode_streams (rows b0 .. b0 + B - 1 take the place
+ * of pos_total, the field is not used).  Kernel choice as dmg_forward's: the flash and tcgen05 ring kernels need one memory for all B
+ * streams; over unequal memories the general kernel runs. */
+int dmg_attn_segment_streams(dmg_segment_attn_args* a, const int32_t* stream_state_dev, void* stream);
 
 /* ---- training data feed (SURVEY.md section 8 f4) ------------------------------------------------------------------------
  * dmg_preload_fill = MusicPreloader.__getitem__ / fill_row (deep_music_genre.py:1088-1125) for all `bs` rows of one batch.
